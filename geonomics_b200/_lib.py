@@ -192,7 +192,6 @@ SIGNATURES = {
     'gnx_set_draws': (C.c_int, [_ctx, C.POINTER(Draws)]),
     'gnx_set_burn': (C.c_int, [_ctx, C.c_int32]),
     'gnx_set_debug': (C.c_int, [_ctx, C.c_int32]),
-    'gnx_set_gamete_tma': (C.c_int, [_ctx, C.c_int32]),
     'gnx_upload_population': (C.c_int, [_ctx, C.POINTER(Population)]),
     'gnx_download_population': (C.c_int, [_ctx, C.POINTER(Population)]),
     'gnx_population_size': (C.c_int, [_ctx, c_int64_p]),

@@ -45,7 +45,6 @@ struct ProfSpan {
 struct gnx_ctx {
   gnx_config_t cfg;
   bool profiling = false;
-  bool no_tma = true;               // TMA-staged gamete kernel is opt-in: measured 2.3x slower (profiles/r01_notes.md)
   std::vector<ProfSpan> spans;
   cudaStream_t stream = nullptr;
   cudaStream_t stream2 = nullptr;          // density chain of the fused step (one_step)
@@ -371,12 +370,6 @@ static int create_impl(const gnx_config_t* cfg, gnx_ctx* ctx) {
   DM(ctx, &W.N_rast, plane);
   DM(ctx, &W.NP_rast, plane);
   DM(ctx, &W.d_rast, plane);
-  W.envd_stride = 1 + cfg->n_traits;
-#if GNX_ENVD_PLANAR
-  W.envd = nullptr;
-#else
-  DM(ctx, &W.envd, plane * (size_t)W.envd_stride);
-#endif
   DM(ctx, &W.e_out, (size_t)cap * cfg->n_layers);
   DM(ctx, &W.fix_list, plane);
   DM(ctx, &W.fix_count, 1);
@@ -472,17 +465,6 @@ extern "C" int gnx_destroy(gnx_ctx* ctx) {
   return GNX_OK;
 }
 
-static int pack_env(gnx_ctx* ctx) {
-#if GNX_ENVD_PLANAR
-  return GNX_OK;               // the death kernel reads the layers themselves
-#endif
-  if (!ctx->have_traits || ctx->cfg.n_traits == 0 || !ctx->have_rasters) return GNX_OK;
-  PROF(ctx, "k_pack_env");
-  k_pack_env<<<grid_for(ctx, 4), 256, 0, ctx->stream>>>(ctx->land, ctx->traits, ctx->work, ctx->cfg.n_traits);
-  LAUNCHED(ctx);
-  return GNX_OK;
-}
-
 // refresh the float32 conductance copies after `layer` (or every layer, -1) changed
 static int refresh_surf_f32(gnx_ctx* ctx, int layer) {
   const size_t plane = (size_t)ctx->cfg.dim_x * ctx->cfg.dim_y;
@@ -513,9 +495,8 @@ extern "C" int gnx_set_rasters(gnx_ctx* ctx, const double* host_rasters) {
   CK(cudaMemcpyAsync(ctx->d_rasters, host_rasters, plane * ctx->cfg.n_layers * sizeof(double),
                      cudaMemcpyHostToDevice, ctx->stream));
   ctx->have_rasters = true;
-  int r = pack_env(ctx);
+  int r = refresh_surf_f32(ctx, -1);
   if (r != GNX_OK) return r;
-  if ((r = refresh_surf_f32(ctx, -1)) != GNX_OK) return r;
   return set_K(ctx);
 }
 
@@ -525,9 +506,8 @@ extern "C" int gnx_set_raster(gnx_ctx* ctx, int32_t layer, const double* host_ra
   const size_t plane = (size_t)ctx->cfg.dim_x * ctx->cfg.dim_y;
   CK(cudaMemcpyAsync(ctx->d_rasters + plane * layer, host_raster, plane * sizeof(double), cudaMemcpyHostToDevice,
                      ctx->stream));
-  int r = pack_env(ctx);
+  int r = refresh_surf_f32(ctx, layer);
   if (r != GNX_OK) return r;
-  if ((r = refresh_surf_f32(ctx, layer)) != GNX_OK) return r;
   if (layer == ctx->cfg.K_layer) return set_K(ctx);      // model.py:651-652 (Species._set_K)
   return GNX_OK;
 }
@@ -662,7 +642,7 @@ extern "C" int gnx_set_traits(gnx_ctx* ctx, int32_t n_traits, const gnx_trait_t*
   for (int t = 0; t < n_traits; ++t) if (traits[t].n_loci <= 1) ctx->pair_phenotype = false;
   ctx->have_traits = true;
   ctx->traits_as_set = T;
-  return pack_env(ctx);
+  return GNX_OK;
 }
 
 extern "C" int gnx_set_recomb_paths(gnx_ctx* ctx, const uint32_t* host_packed_paths) {
@@ -1365,31 +1345,8 @@ static int offspring_gametes(gnx_ctx* ctx) {
                                                                        fnb, stage);                       \
   } while (0)
     const int fnb = ctx->cfg.n_births_fixed ? (int)ctx->cfg.n_births_lambda : 0;
-    if (Wq >= 4 && Wq <= 32 && !ctx->no_tma) {
-      // rows >= 128 B: TMA-staged pipeline (k_gametes_tma)
-      const size_t Wb = 16 * (size_t)Wq, RB = 2 * Wb;
-      const size_t smem = GT_STAGES * (GT_NB * (2 * RB + 2 * Wb) + GT_NB * RB);
-      const int per_sm = smem <= 100 * 1024 ? 2 : 1;
-#define MT(GW)                                                                                              \
-  do {                                                                                                      \
-    auto kern = ctx->cfg.n_traits <= 2 ? k_gametes_tma<GW, 2> : k_gametes_tma<GW, GNX_MAX_TRAITS>;           \
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                 \
-    kern<<<grid_for(ctx, per_sm), GT_THREADS, smem, s>>>(ctx->pop, ctx->prm, ctx->traits, ctx->draws,      \
-                                                         ctx->work, ctx->d_c, fnb);                         \
-  } while (0)
-      PROF(ctx, "k_gametes");
-      if (Wq <= 4) MT(4);
-      else if (Wq <= 8) MT(8);
-      else if (Wq <= 16) MT(16);
-      else MT(32);
-#undef MT
-      LAUNCHED(ctx);
-    } else {
     PROF(ctx, "k_gametes");
-#ifndef GNX_GAM_W1
-#define GNX_GAM_W1 1
-#endif
-    if (Wq <= 1) MO(GNX_GAM_W1);
+    if (Wq <= 1) MO(1);
     else if (Wq <= 2) MO(2);
     else if (Wq <= 4) MO(4);
     else if (Wq <= 8) MO(8);
@@ -1397,7 +1354,6 @@ static int offspring_gametes(gnx_ctx* ctx) {
     else MO(32);
 #undef MO
     LAUNCHED(ctx);
-    }
   }
   return GNX_OK;
 }
@@ -1928,7 +1884,7 @@ static void step_key(const gnx_ctx* ctx, std::vector<unsigned char>* key) {
   put(&ctx->dens, sizeof ctx->dens);
   put(&ctx->tsk, sizeof ctx->tsk);
   put(&ctx->mut, sizeof ctx->mut);
-  const int flags[4] = {ctx->burn, ctx->no_tma ? 1 : 0, ctx->have_density ? 1 : 0, ctx->mut_delet ? 1 : 0};
+  const int flags[3] = {ctx->burn, ctx->have_density ? 1 : 0, ctx->mut_delet ? 1 : 0};
   put(flags, sizeof flags);
 }
 
@@ -2430,9 +2386,6 @@ extern "C" int gnx_device_ptr(gnx_ctx* ctx, int32_t field, void** dev_ptr, int64
     case GNX_F_K_RAST: p = ctx->d_K; b = plane * 8; break;
     case GNX_F_DISP_TRIES: p = W.disp_tries; b = (size_t)h.B * 4; break;
     case GNX_F_COUNTERS: p = ctx->d_c; b = sizeof(Counters); break;
-#ifdef GNX_GS_TIMING
-    case 31: p = D.coef + (size_t)2 * D.ntri * CT_STRIDE; b = 64 * 8; break;   /* clock64 phase timings (tools/gs_time.py) */
-#endif
     default: g_last_error = "unknown field"; return GNX_ERR_ARG;
   }
   CK(cudaGetLastError());
@@ -2505,15 +2458,6 @@ extern "C" int gnx_set_debug(gnx_ctx* ctx, int32_t on) {
   ARG(ctx, "null ctx");
   USE_DEVICE(ctx);
   ctx->prm.store_debug = on ? 1 : 0;
-  return GNX_OK;
-}
-
-
-/* A/B switch for the gamete kernel: 1 = TMA-staged pipeline when rows >= 128 B (default), 0 = register streaming */
-extern "C" int gnx_set_gamete_tma(gnx_ctx* ctx, int32_t on) {
-  ARG(ctx, "null ctx");
-  USE_DEVICE(ctx);
-  ctx->no_tma = !on;
   return GNX_OK;
 }
 

@@ -179,8 +179,6 @@ struct Work {
   double* N_rast;
   double* NP_rast;
   double* d_rast;
-  double* envd;            // [Y*X][1 + T]: d raster slot + each trait's environment value
-  int32_t envd_stride;
   double* e_out;
   int32_t* fix_list;       // landscape cells whose N needs the exact-order re-evaluation
   int32_t* fix_count;
@@ -561,19 +559,4 @@ __device__ __forceinline__ void mbar_wait(unsigned long long* bar, uint32_t pari
       "WAIT_DONE:\n"
       "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
 }
-
-__device__ __forceinline__ void mbar_arrive(unsigned long long* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void bulk_s2g(void* gmem_dst, const void* smem_src, uint32_t bytes) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
-               ::"l"(gmem_dst), "r"(smem_u32(smem_src)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-template <int NTHREADS>
-__device__ __forceinline__ void named_bar_sync_1() { asm volatile("bar.sync 1, %0;" ::"n"(NTHREADS) : "memory"); }
 

@@ -11,9 +11,6 @@
 #include "gnx_common.cuh"
 #include "gnx_scan.cuh"
 
-#ifndef GNX_ENVD_PLANAR
-#define GNX_ENVD_PLANAR 1      // 0: the round-1 packed [cell][d | e...] raster (A/B)
-#endif
 #define GTID (blockIdx.x * blockDim.x + threadIdx.x)
 #define GSTRIDE (gridDim.x * blockDim.x)
 
@@ -1358,164 +1355,6 @@ __global__ void __launch_bounds__(256, GNX_GAM_MINB) k_gametes(Pop pop, Params p
   }
 }
 
-// ----- k_gametes_tma: genotype streaming staged through shared memory by the TMA ----------
-// For rows of >= 128 B (L > 256 loci).  One producer warp per CTA resolves a batch of
-// GT_NB offspring (one per lane: parents' slots, recombination keys, start homologues) and
-// issues four bulk copies per offspring (cp.async.bulk, SASS UBLKCP): both parents' whole
-// rows and the two cached recombination paths, GT_STAGES batches deep.  Four consumer
-// warps wait on the stage's mbarrier, form the gametes with 128-bit shared-memory loads,
-// accumulate the phenotype, write the child rows to a staging buffer and hand them back
-// to the TMA as bulk stores.  No parental byte passes through a register before it is used,
-// and ~3 x 24 KB per CTA are in flight whatever the occupancy.
-#define GT_NB 32
-#define GT_STAGES 3
-#define GT_CONSUMERS 128
-#define GT_THREADS (GT_CONSUMERS + 32)
-
-struct GtMeta {            // per stage, per offspring of the batch
-  int cslot[GT_NB];
-  uint32_t f0[GT_NB];      // start homologue of parent 0 as an all-ones / all-zeros mask
-  uint32_t f1[GT_NB];
-  int nvalid;
-  int pad[3];
-};
-
-template <int GW, int NT>
-__global__ void __launch_bounds__(GT_THREADS) k_gametes_tma(Pop pop, Params prm, Traits tr, DevDraws dr, Work w,
-                                                             const Counters* c, int fixed_nb) {
-  extern __shared__ __align__(128) unsigned char gt_smem[];
-  const int n = c->n, B = c->B, cur = c->cur, n_free = c->n_free, n_slots = c->n_slots;
-  const int64_t t = c->t, max_idx = c->max_idx;
-  const int Wq = pop.Wq, T = pop.T;
-  const uint32_t Wb = 16u * Wq, RB = 2u * Wb;                 // bytes per homologue, per row
-  const uint32_t stage_in = GT_NB * (2 * RB + 2 * Wb);        // P0 | P1 | M0 | M1
-  const uint32_t stage_bytes = stage_in + GT_NB * RB;         // + child staging
-  __shared__ __align__(8) unsigned long long full_bar[GT_STAGES], empty_bar[GT_STAGES];
-  __shared__ GtMeta meta[GT_STAGES];
-  const int warp = threadIdx.x >> 5, lane32 = threadIdx.x & 31;
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < GT_STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
-  }
-  __syncthreads();
-  const int nbatch = (B + GT_NB - 1) / GT_NB;
-  if (warp == GT_CONSUMERS / 32) {
-    // ================================ producer warp =====================================
-    int it = 0;
-    for (int b = blockIdx.x; b < nbatch; b += gridDim.x, ++it) {
-      const int s = it % GT_STAGES;
-      const uint32_t ph = (it / GT_STAGES) & 1;
-      mbar_wait(&empty_bar[s], ph ^ 1);                       // stage free (first pass: immediate)
-      unsigned char* base = gt_smem + (size_t)s * stage_bytes;
-      const int o = b * GT_NB + lane32;
-      const int nvalid = min(GT_NB, B - b * GT_NB);
-      int s0 = 0, s1 = 0, k0 = 0, k1 = 0;
-      if (lane32 < nvalid) {
-        const int p = fixed_nb > 0 ? o / fixed_nb : w.off_pair[o];
-        const int2 sl = reinterpret_cast<const int2*>(w.pair_slots)[p];
-        s0 = sl.x;
-        s1 = sl.y;
-        const int cslot = o < n_free ? pop.free_slots[n_free - 1 - o] : n_slots + (o - n_free);
-        int h0, h1;
-        RngStream gg(prm.seed_lo, prm.seed_hi, max_idx + 1 + o, SITE_GAMETE, t);
-        if (dr.recomb_keys) {
-          const int j = o - w.off_start[p];
-          const int e = 2 * (w.off_start[p] + w.nb[p]);
-          k0 = dr.recomb_keys[e - 1 - 2 * j];                 // mating.py:176-181
-          k1 = dr.recomb_keys[e - 2 - 2 * j];
-        } else {
-          k0 = (int)choose_k(gg.u32(), prm.n_paths);          // species.py:625-627
-          k1 = (int)choose_k(gg.u32(), prm.n_paths);
-        }
-        if (dr.start_homs) {
-          h0 = dr.start_homs[2 * o];
-          h1 = dr.start_homs[2 * o + 1];
-        } else {
-          const uint32_t bits = gg.u32();                     // mating.py:133
-          h0 = bits & 1;
-          h1 = (bits >> 1) & 1;
-        }
-        meta[s].cslot[lane32] = cslot;
-        meta[s].f0[lane32] = h0 ? 0xffffffffu : 0u;
-        meta[s].f1[lane32] = h1 ? 0xffffffffu : 0u;
-        pop.gslot[cur][n + o] = cslot;
-      }
-      if (lane32 == 0) meta[s].nvalid = nvalid;
-      __syncwarp();
-      if (lane32 == 0) mbar_expect_tx(&full_bar[s], (uint32_t)nvalid * (2 * RB + 2 * Wb));
-      __syncwarp();
-      if (lane32 < nvalid) {
-        bulk_g2s(base + (size_t)lane32 * RB, pop.G + (size_t)s0 * 2 * Wq, RB, &full_bar[s]);
-        bulk_g2s(base + (size_t)GT_NB * RB + (size_t)lane32 * RB, pop.G + (size_t)s1 * 2 * Wq, RB, &full_bar[s]);
-        bulk_g2s(base + (size_t)2 * GT_NB * RB + (size_t)lane32 * Wb, prm.paths + (size_t)k0 * Wq, Wb, &full_bar[s]);
-        bulk_g2s(base + (size_t)2 * GT_NB * RB + (size_t)GT_NB * Wb + (size_t)lane32 * Wb,
-                 prm.paths + (size_t)k1 * Wq, Wb, &full_bar[s]);
-      }
-    }
-  } else {
-    // ================================ consumer warps ====================================
-    const int lane = threadIdx.x & (GW - 1);
-    const int lane0 = lane32 & ~(GW - 1);
-    const unsigned gmask = GW == 32 ? 0xffffffffu : (((1u << GW) - 1u) << lane0);
-    const int grp = threadIdx.x / GW;                          // offspring slot handled in a pass
-    const int ngrp = GT_CONSUMERS / GW;
-    int it = 0;
-    for (int b = blockIdx.x; b < nbatch; b += gridDim.x, ++it) {
-      const int s = it % GT_STAGES;
-      const uint32_t ph = (it / GT_STAGES) & 1;
-      unsigned char* base = gt_smem + (size_t)s * stage_bytes;
-      unsigned char* outb = base + stage_in;
-      // the child staging buffer of this stage was handed to the TMA GT_STAGES batches ago
-      if (warp == 0) bulk_wait_read<GT_STAGES - 1>();
-      mbar_wait(&full_bar[s], ph);
-      named_bar_sync_1<GT_CONSUMERS>();
-      const int nvalid = meta[s].nvalid;
-      for (int k = grp; k < nvalid; k += ngrp) {
-        const uint4* P0 = reinterpret_cast<const uint4*>(base + (size_t)k * RB);
-        const uint4* P1 = reinterpret_cast<const uint4*>(base + (size_t)GT_NB * RB + (size_t)k * RB);
-        const uint4* M0 = reinterpret_cast<const uint4*>(base + (size_t)2 * GT_NB * RB + (size_t)k * Wb);
-        const uint4* M1 = reinterpret_cast<const uint4*>(base + (size_t)2 * GT_NB * RB + (size_t)GT_NB * Wb + (size_t)k * Wb);
-        uint4* C = reinterpret_cast<uint4*>(outb + (size_t)k * RB);
-        const uint32_t f0 = meta[s].f0[k], f1 = meta[s].f1[k];
-        double zacc[NT];
-#pragma unroll
-        for (int tt = 0; tt < NT; ++tt) zacc[tt] = 0.0;
-        for (int q = lane; q < Wq; q += GW) {
-          const uint4 a0 = P0[q], a1 = P0[Wq + q], b0 = P1[q], b1 = P1[Wq + q];
-          uint4 m0 = M0[q], m1 = M1[q];
-          m0 = make_uint4(m0.x ^ f0, m0.y ^ f0, m0.z ^ f0, m0.w ^ f0);
-          m1 = make_uint4(m1.x ^ f1, m1.y ^ f1, m1.z ^ f1, m1.w ^ f1);
-          const uint4 g0 = bitsel(a0, a1, m0), g1 = bitsel(b0, b1, m1);     // mating.py:161-168
-          C[q] = g0;
-          C[Wq + q] = g1;
-#pragma unroll
-          for (int tt = 0; tt < NT; ++tt)
-            if (tt < T) zacc[tt] += trait_partial(tr, tt, q, Wq, g0, g1);
-        }
-        const int o = b * GT_NB + k;
-#pragma unroll
-        for (int tt = 0; tt < NT; ++tt) {
-          if (tt < T) {
-            double v = zacc[tt];
-#pragma unroll
-            for (int d = GW / 2; d >= 1; d >>= 1) v += __shfl_xor_sync(gmask, v, d);
-            if (lane == 0) pop.z[cur][(size_t)tt * pop.cap + n + o] = (trait_n_loci(tr, tt) > 1) ? 0.5 + v : v;
-          }
-        }
-      }
-      fence_async_smem();                    // generic-proxy writes of the child rows -> async proxy
-      named_bar_sync_1<GT_CONSUMERS>();                       // all rows written, all inputs consumed
-      if (warp == 0) {
-        if (lane32 < nvalid)
-          bulk_s2g(pop.G + (size_t)meta[s].cslot[lane32] * 2 * Wq, outb + (size_t)lane32 * RB, RB);
-        bulk_commit();
-        __syncwarp();
-        if (lane32 == 0) mbar_arrive(&empty_bar[s]);           // hand the stage back to the producer
-      }
-    }
-    if (warp == 0) bulk_wait_all();
-  }
-}
-
 // ----- k_newborns: natal dispersal, sex, newborn record (one thread per offspring) -------
 #ifndef GNX_NB_MINB
 #define GNX_NB_MINB 4     // 64 registers instead of 77: 83 -> 68 us at c4
@@ -2382,12 +2221,7 @@ __device__ __forceinline__ void raster_d_cell(const Land& land, const Params& pr
   double dv = N_d / N;                              // demography.py:159-160
   if (isnan(dv)) dv = 0.0;
   dv = dv < prm.c.d_min ? prm.c.d_min : (dv > prm.c.d_max ? prm.c.d_max : dv);
-#if GNX_ENVD_PLANAR
   w.d_rast[id] = dv;                                // its own plane: a full-sector streaming write
-#else
-  w.envd[(size_t)id * w.envd_stride] = dv;          // packed [cell][d | e_trait0 | e_trait1 ...]
-  if (prm.store_debug) w.d_rast[id] = dv;
-#endif
 }
 
 __global__ void __launch_bounds__(256) k_raster_d(Dens d, Land land, Params prm, Work w, const Counters* c, int row_lo,
@@ -2418,7 +2252,7 @@ __global__ void __launch_bounds__(256) k_raster_d_fix(Dens d, Land land, Params 
 // a3 + a15 + a16 (draw): environment gather (species.py:913-922), fitness
 // (selection.py:51-112), death probability (selection.py:119-125, demography.py:306-321),
 // Bernoulli mortality draw (demography.py:175-176).  The first n entries are in mating-grid
-// order, so the packed (d, e...) raster records of a warp's 32 individuals sit in a few
+// order, so the d and environment raster reads of a warp's 32 individuals share a few
 // neighbouring sectors.  With end_step = 1 (fused step) the last block to finish also closes
 // the time step (Species._set_Nt species.py:554, the bookkeeping of demography.py:324-329):
 // the dead are only FLAGGED here -- the next step's re-grid drops them.
@@ -2446,25 +2280,16 @@ __global__ void __launch_bounds__(256, GNX_DEATH_MINB) k_death(Pop pop, Land lan
     const double x = xy.x, y = xy.y;
     const int cx = (int)x, cy = (int)y;
     const size_t cell = (size_t)cy * land.X + cx;
-#if GNX_ENVD_PLANAR
     // d and the environment layers are read as planes: with the state in mating-grid order a warp's
     // 32 individuals sit in a few neighbouring landscape cells, so the plane reads share sectors,
     // and the d raster is written by k_raster_d as whole sectors (interleaved with the environment
     // values it was a read-modify-write of 8 bytes in every 24: 2.6x its algorithmic traffic)
     const size_t plane_sz = (size_t)land.X * land.Y;
     double p = w.d_rast[cell];                                     // demography.py:306
-#else
-    const double* __restrict__ ed = w.envd + cell * w.envd_stride;   // one sector: d and the traits' e
-    double p = ed[0];                                              // demography.py:306
-#endif
     if (prm.selection) {
       double wfit = 1.0;
       for (int tt = 0; tt < T; ++tt) {
-#if GNX_ENVD_PLANAR
         const double e = tr.univ_adv[tt] ? 1.0 : __ldg(&land.rasters[(size_t)tr.layer[tt] * plane_sz + cell]);
-#else
-        const double e = tr.univ_adv[tt] ? 1.0 : ed[1 + tt];     // species.py:913-922 gather
-#endif
         const double z = pop.z[cur][(size_t)tt * pop.cap + i];
         const double phi = tr.phi_rast[tt] ? __ldg(&tr.phi_rast[tt][cell]) : tr.phi[tt];
         const double diff = fabs(e - z);
@@ -2832,16 +2657,8 @@ __global__ void __launch_bounds__(256) k_gather_genomes(Pop pop, const int32_t* 
   }
 }
 
-// environment values of each trait's layer packed next to the d slot (setup / env change)
 __global__ void __launch_bounds__(256) k_raster_to_f32(const double* src, float* dst, size_t n) {
   for (size_t id = GTID; id < n; id += GSTRIDE) dst[id] = (float)src[id];
-}
-
-__global__ void __launch_bounds__(256) k_pack_env(Land land, Traits tr, Work w, int T) {
-  const size_t plane = (size_t)land.X * land.Y;
-  for (size_t id = GTID; id < plane; id += GSTRIDE)
-    for (int tt = 0; tt < T; ++tt)
-      w.envd[id * w.envd_stride + 1 + tt] = land.rasters[(size_t)tr.layer[tt] * plane + id];
 }
 
 // upload epilogue: identity genome slots, default ids, z [n][T] -> [T][cap], counters reset

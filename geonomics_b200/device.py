@@ -167,9 +167,6 @@ class DeviceSpecies:
         """Keep n_nbrs / death_p / disp_tries / n_pairs raster readable (parity tests)."""
         _lib.check(self._L.gnx_set_debug(self._ctx, int(bool(on))), 'gnx_set_debug')
 
-    def set_gamete_tma(self, on=True):
-        _lib.check(self._L.gnx_set_gamete_tma(self._ctx, int(bool(on))), 'gnx_set_gamete_tma')
-
     @staticmethod
     def _fill_life_history(cfg, prm):
         """The scalar parameters the step reads off the Species (species.py:405-425)."""

@@ -6,14 +6,14 @@ contiguous range of the (mating cell, id) order and the rank-major order of pair
 offspring ids is the order of the undecomposed run).  The data path is in the library:
 individuals are written by the sender straight into the receiver's buffer (NVLink peer memory
 mapped through CUDA IPC) and the device reads every size from device memory, so a time step
-is enqueued without a host round trip.  This module supplies what the library leaves to the
-caller: the plan (which rows, which individuals go where at upload), the barrier between
-phases and the three small collectives (births all-gather, density-count sum, max(N)).
+is enqueued without a host round trip.  This module supplies the plan (which rows, which
+individuals go where at upload) and, where the host sequences the phases, the barrier between
+them and the three small collectives (births all-gather, density-count sum, max(N)).
 
 Two transports:
-  * `NcclStrips`   one process per GPU (`torch.distributed`, backend nccl): the barrier is a
-                   one-element all-reduce enqueued on the context's stream, the collectives act
-                   on the context's own device buffers.
+  * `NcclStrips`   one process per GPU (`torch.distributed`, backend nccl, which only exchanges
+                   the CUDA IPC handles): the barrier and the collectives are one-CTA kernels
+                   over peer memory (gnx_strip_barrier) inside each step's CUDA graph.
   * `LocalStrips`  all ranks as contexts of ONE process on one GPU (tests; a box with fewer GPUs
                    than ranks): the same kernels write into the other contexts' buffers, the
                    host runs each phase on every context before the next and does the
@@ -273,17 +273,12 @@ class NcclStrips:
     """This process's strip of a landscape decomposed over the ranks of `torch.distributed`
     (backend nccl, one GPU each, one node: the receive buffers are shared through CUDA IPC)."""
 
-    def __init__(self, land_dim, rasters, prm, gen_arch, capacity, seed=0, bounds=None, group=None,
-                 device_barrier=None, **kw):
-        import os
+    def __init__(self, land_dim, rasters, prm, gen_arch, capacity, seed=0, bounds=None, group=None, **kw):
         import torch
         import torch.distributed as dist
-        self.torch, self.dist, self.group = torch, dist, group
         # the barriers and the three small collectives of a step run as one-CTA kernels over peer memory
-        # (gnx_strip_barrier); GNX_STRIP_NCCL=1 (or device_barrier=False) keeps them on NCCL for comparison
-        if device_barrier is None:
-            device_barrier = os.environ.get('GNX_STRIP_NCCL', '0') in ('', '0')
-        self.device_barrier = bool(device_barrier)
+        # (gnx_strip_barrier), never on the host
+        self.device_barrier = True
         self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
         self.cs, self.ncx, self.ncy = mating_grid(land_dim, prm['mating_radius'])
         K = np.asarray(rasters)[int(prm.get('K_layer', 0))] * float(prm.get('K_factor', 1.0))
@@ -298,9 +293,6 @@ class NcclStrips:
             if r != self.rank:
                 self.me.connect(r, _lib.StripEndpoints.from_buffer_copy(raw), same_process=False)
         self.stream = torch.cuda.ExternalStream(self.me.dev.stream_ptr)
-        self.births, self.counts, self.nmax = self.me.tensors()
-        self._token = torch.zeros(1, device='cuda', dtype=torch.int32)
-        self._mine = torch.zeros(1, device='cuda', dtype=torch.int64)
         dist.barrier(group=group)
 
     @property
@@ -320,23 +312,7 @@ class NcclStrips:
                            max_ind_idx=int(idx.max()) if max_ind_idx is None else max_ind_idx)
 
     def step(self, n=1):
-        torch, dist = self.torch, self.dist
-        if self.device_barrier:
-            self.me.dev.step(n)                            # gnx_step: eight phases + gnx_strip_barrier, one graph per step
-            return
-        with torch.cuda.stream(self.stream):               # collectives are ordered on the context's stream
-            for _ in range(n):
-                for k in range(N_PHASES):
-                    self.me.phase(k)
-                    if k in (0, 1, 2, 4):
-                        dist.all_reduce(self._token, group=self.group)            # stream-ordered barrier
-                    elif k == 3:
-                        self._mine.copy_(self.births[self.rank:self.rank + 1])
-                        dist.all_gather_into_tensor(self.births[:self.world], self._mine, group=self.group)
-                    elif k == 5:
-                        dist.all_reduce(self.counts, op=dist.ReduceOp.SUM, group=self.group)
-                    elif k == 6:
-                        dist.all_reduce(self.nmax, op=dist.ReduceOp.MAX, group=self.group)
+        self.me.dev.step(n)            # gnx_step: eight phases + gnx_strip_barrier, one graph per step
 
     def sync(self):
         self.me.check()

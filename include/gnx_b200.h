@@ -196,10 +196,6 @@ int gnx_set_burn(gnx_ctx* ctx, int32_t burn);   /* burn-in: no genomes, no selec
 /* keep per-individual intermediates (n_nbrs, death_p, disp_tries, n_pairs raster) readable
  * through gnx_read_field; off by default (they cost extra HBM writes) */
 int gnx_set_debug(gnx_ctx* ctx, int32_t on);
-/* gamete kernel variant: 0 (default) = register-streaming kernel (128-bit gathers) for every
- * row size; 1 = TMA-staged shared-memory pipeline for rows >= 128 B (kept for A/B
- * measurements: bulk copies of 128-256 B rows are issue-rate bound, profiles/r01_notes.md) */
-int gnx_set_gamete_tma(gnx_ctx* ctx, int32_t on);
 int gnx_upload_population(gnx_ctx* ctx, const gnx_population_t* pop);
 int gnx_download_population(gnx_ctx* ctx, gnx_population_t* pop /* buffers sized >= gnx_population_size */);
 int gnx_population_size(gnx_ctx* ctx, int64_t* n);          /* synchronises */

@@ -126,7 +126,7 @@ def test_production_step_matches_oracle(name):
 @pytest.mark.parametrize('L,n_traits,lpt', [(100, 5, 7), (300, 8, 9), (1000, 3, 40)])
 def test_many_traits(L, n_traits, lpt):
     """More than two traits (the reference allows any number, genome.py:826-867): the 8-accumulator
-    instantiations of the gamete / phenotype kernels, the wider packed (d, e...) raster record and
+    instantiations of the gamete / phenotype kernels, the per-trait environment reads of k_death and
     the z planes of the compaction, against the oracle -- staged and as the production step."""
     from oracle import step_oracle as so
     from parity_util import synthetic_case

@@ -1,8 +1,8 @@
 """Multi-process check of the strip decomposition (run under torchrun, one rank per GPU):
 the ranks jointly advance one landscape through NcclStrips (records written into the peers'
-buffers over NVLink through CUDA IPC, NCCL collectives as barriers); rank 0 also runs the same
-population undecomposed and compares -- ids, positions, ages, genomes, phenotypes, fitness and
-the step records must be identical.
+buffers over NVLink through CUDA IPC, barriers and collectives by gnx_strip_barrier over peer
+memory); rank 0 also runs the same population undecomposed and compares -- ids, positions,
+ages, genomes, phenotypes, fitness and the step records must be identical.
 
   python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 \
       --master-port 29511 tools/strips_nccl_check.py [steps]
@@ -48,8 +48,9 @@ def main():
             ok = ok and np.array_equal(ref[k], got[k])
         ok = ok and all((a['Nt'], a['n_births'], a['n_deaths'], a['n_pairs']) ==
                         (b['Nt'], b['n_births'], b['n_deaths'], b['n_pairs']) for a, b in zip(ref_recs, got_recs))
-        print('strips over %d GPUs (CUDA IPC peer writes; barriers and collectives by %s), %d steps: %s; N %d -> %d; per-rank shares %s'
-              % (world, 'gnx_strip_barrier over peer memory' if st.device_barrier else 'NCCL', steps, 'IDENTICAL to the undecomposed run' if ok else 'MISMATCH', len(pop['x']),
+        print('strips over %d GPUs (CUDA IPC peer writes; barriers and collectives by gnx_strip_barrier over '
+              'peer memory), %d steps: %s; N %d -> %d; per-rank shares %s'
+              % (world, steps, 'IDENTICAL to the undecomposed run' if ok else 'MISMATCH', len(pop['x']),
                  len(got['idx']), [len(s[0]['idx']) for s in shares]), flush=True)
     st.close()
     dist.destroy_process_group()
