@@ -212,7 +212,9 @@ SIGNATURES = {
     'gnx_strip_connect': (C.c_int, [_ctx, C.c_int32, C.POINTER(StripEndpoints), C.c_int32]),
     'gnx_strip_collective_ptrs': (C.c_int, [_ctx, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
                                             C.POINTER(C.c_int64), C.POINTER(C.c_void_p)]),
+    'gnx_strip_pairs_ptr': (C.c_int, [_ctx, C.POINTER(C.c_void_p)]),
     'gnx_strip_phase': (C.c_int, [_ctx, C.c_int32]),
+    'gnx_strip_phase_order': (C.c_int, [C.c_int32, c_int32_p, c_int32_p, c_int32_p]),
     'gnx_strip_barrier': (C.c_int, [_ctx, C.c_int32]),
     'gnx_strip_check': (C.c_int, [_ctx]),
     'gnx_set_K': (C.c_int, [_ctx, c_double_p]),

@@ -893,6 +893,7 @@ extern "C" int gnx_set_density(gnx_ctx* ctx, const gnx_density_t* dn) {
 extern "C" int gnx_set_draws(gnx_ctx* ctx, const gnx_draws_t* dr) {
   ARG(ctx, "null ctx");
   USE_DEVICE(ctx);
+  ARG(!(dr && ctx->d_strip), "injected draws are not supported under strip decomposition");
   CK(cudaStreamSynchronize(ctx->stream));
   const int R = ctx->draws.disp_R;
   memset(&ctx->draws, 0, sizeof ctx->draws);
@@ -1291,24 +1292,32 @@ static int find_mates(gnx_ctx* ctx) {
   return GNX_OK;
 }
 
-extern "C" int gnx_dedup_pairs(gnx_ctx* ctx) {
-  ARG(ctx, "null ctx");
-  USE_DEVICE(ctx);
+// the pair list (and, with n_births_fixed, the births)
+static int scan_pairs(gnx_ctx* ctx) {
   const bool fixed = ctx->cfg.n_births_fixed != 0;
   PairScan ps{ctx->pop, ctx->work, ctx->d_c, ctx->cfg.sex, fixed ? (int32_t)ctx->cfg.n_births_lambda : 0,
               ctx->cfg.mating_radius <= 0 ? 1 : 0, ctx->prm.ordered};
   if (fixed) ARG(ps.fixed_nb >= 1, "n_births_fixed needs n_births_distr_lambda >= 1");
-  int r = run_scan(ctx, ps, "scan_pairs");
+  return run_scan(ctx, ps, "scan_pairs");
+}
+
+// Poisson births of the pairs (under strips keyed by the pairs' species-wide positions: the pair
+// counts of the lower ranks must have been all-gathered)
+static int draw_births(gnx_ctx* ctx) {
+  PROF(ctx, "k_draw_births");
+  k_draw_births<<<grid_for(ctx, 4), 256, 0, ctx->stream>>>(ctx->pop, ctx->prm, ctx->draws, ctx->work, ctx->d_c,
+                                                           ctx->d_strip);
+  LAUNCHED(ctx);
+  BirthScan bs{ctx->work, ctx->pop.cap};
+  return run_scan(ctx, bs, "scan_births");
+}
+
+extern "C" int gnx_dedup_pairs(gnx_ctx* ctx) {
+  ARG(ctx, "null ctx");
+  USE_DEVICE(ctx);
+  int r = scan_pairs(ctx);
   if (r != GNX_OK) return r;
-  if (!fixed) {
-    PROF(ctx, "k_draw_births");
-    k_draw_births<<<grid_for(ctx, 4), 256, 0, ctx->stream>>>(ctx->pop, ctx->prm, ctx->draws, ctx->work, ctx->d_c);
-    LAUNCHED(ctx);
-    BirthScan bs{ctx->work, ctx->pop.cap};
-    r = run_scan(ctx, bs, "scan_births");
-    if (r != GNX_OK) return r;
-  }
-  return GNX_OK;
+  return ctx->cfg.n_births_fixed ? GNX_OK : draw_births(ctx);
 }
 
 extern "C" int gnx_mutate(gnx_ctx* ctx);
@@ -1398,6 +1407,13 @@ extern "C" int gnx_make_offspring(gnx_ctx* ctx) {
 extern "C" int gnx_set_mutation(gnx_ctx* ctx, const gnx_mutation_t* m) {
   ARG(ctx, "null ctx");
   USE_DEVICE(ctx);
+  if (ctx->d_strip && m) {
+    // every rank replays the species-wide draws on by-locus rows; the tskit layout would also need the path
+    // patches and node ids of offspring held by other ranks
+    ARG(!m->tskit_layout, "the tskit genotype layout is not supported under strip decomposition");
+    for (int t = 0; m->host_trait_mu && t < ctx->cfg.n_traits; ++t)
+      ARG(!(m->host_trait_mu[t] > 0), "trait mutation is not supported under strip decomposition");
+  }
   CK(cudaStreamSynchronize(ctx->stream));
   if (ctx->mut.enabled && ctx->mut.own_tables) {
     ctx->traits = ctx->traits_as_set;                  // back to the tables gnx_set_traits built
@@ -1590,8 +1606,11 @@ extern "C" int gnx_mutate(gnx_ctx* ctx) {
   if (!ctx->mut.enabled || ctx->burn) return GNX_OK;
   if (ctx->mut.mu_tot <= 0) return GNX_OK;             // tskit layout without mutation: nothing to draw
   PROF(ctx, "k_mutate");
-  k_mutate<<<1, 256, 0, ctx->stream>>>(ctx->pop, ctx->prm, ctx->traits, ctx->draws, ctx->mut, ctx->d_c,
-                                       ctx->tsk.enabled ? 1 : 0);
+  if (ctx->d_strip)
+    k_mutate<true><<<1, 256, 0, ctx->stream>>>(ctx->pop, ctx->prm, ctx->traits, ctx->draws, ctx->mut, ctx->d_c, 0);
+  else
+    k_mutate<false><<<1, 256, 0, ctx->stream>>>(ctx->pop, ctx->prm, ctx->traits, ctx->draws, ctx->mut, ctx->d_c,
+                                                ctx->tsk.enabled ? 1 : 0);
   LAUNCHED(ctx);
   return GNX_OK;
 }
@@ -1975,8 +1994,10 @@ extern "C" int gnx_strip_enable(gnx_ctx* ctx, const gnx_strip_config_t* sc) {
   ARG(!ctx->d_strip, "strip decomposition is already enabled for this context");
   ARG(sc->world >= 1 && sc->world <= GNX_STRIP_MAX_WORLD && sc->rank >= 0 && sc->rank < sc->world, "rank / world");
   ARG(ctx->cfg.mating_radius > 0, "strip decomposition needs a mating radius (panmixia has no locality)");
-  ARG(ctx->cfg.n_births_fixed, "strip decomposition supports n_births_fixed only");
-  ARG(!ctx->tsk.enabled && !ctx->mut.enabled, "strip decomposition does not carry tskit rows or mutation");
+  ARG(!ctx->tsk.enabled, "strip decomposition does not carry tskit rows");
+  ARG(!ctx->mut.enabled || !ctx->mut.own_tables,
+      "strip decomposition does not carry the tskit genotype layout or trait mutation");
+  ARG(!ctx->prm.ordered, "injected draws are not supported under strip decomposition");
   Strip& S = ctx->strip_h;
   memset(&S, 0, sizeof S);
   S.enabled = 1;
@@ -2025,6 +2046,7 @@ extern "C" int gnx_strip_enable(gnx_ctx* ctx, const gnx_strip_config_t* sc) {
   S.err = S.list_n + 1;
   DM(ctx, &S.sent, (size_t)ctx->pop.cap, &ctx->strip_allocs);
   DM(ctx, &S.births, GNX_STRIP_MAX_WORLD, &ctx->strip_allocs);
+  DM(ctx, &S.pairs, GNX_STRIP_MAX_WORLD, &ctx->strip_allocs);
   DM(ctx, &S.epoch, 4, &ctx->strip_allocs);
   CK(cudaMemsetAsync(S.epoch, 0, 16, ctx->stream));
   DM(ctx, &ctx->d_strip, 1, &ctx->strip_allocs);
@@ -2076,14 +2098,15 @@ extern "C" int gnx_strip_connect(gnx_ctx* ctx, int32_t peer_rank, const gnx_stri
   return strip_upload(ctx);
 }
 
-// Barrier (kind 0) or one of the three small collectives of a time step (1: births all-gather after phase
-// 3, 2: density-count sum after phase 5, 3: max(N) after phase 6) over peer memory, enqueued on the rank's
-// stream: see k_strip_barrier.  Every rank must make the same sequence of calls.
+// Barrier (kind 0) or one of the small collectives of a time step (1: births all-gather after phase 3, or
+// after phase 8 with Poisson births; 2: density-count sum after phase 5; 3: max(N) after phase 6; 4: pairs
+// all-gather after phase 3 with Poisson births) over peer memory, enqueued on the rank's stream: see
+// k_strip_barrier.  Every rank must make the same sequence of calls.
 static int strip_barrier_launch(gnx_ctx* ctx, int kind);
 extern "C" int gnx_strip_barrier(gnx_ctx* ctx, int32_t kind) {
   ARG(ctx && ctx->d_strip, "strip decomposition is not enabled");
   USE_DEVICE(ctx);
-  ARG(kind >= 0 && kind <= 3, "kind");
+  ARG(kind >= 0 && kind <= 4, "kind");
   if (ctx->strip_connected != ctx->strip_h.world - 1) { g_last_error = "gnx_strip_barrier: not every peer is connected"; return GNX_ERR_STATE; }
   if (kind == 2 && (!ctx->have_density || ctx->strip_h.counts_cap < 2 * ctx->dens.npts)) {
     g_last_error = "gnx_strip_barrier: the density lattice was set after gnx_strip_enable";
@@ -2098,6 +2121,12 @@ extern "C" int gnx_strip_collective_ptrs(gnx_ctx* ctx, void** births, void** cou
   if (counts) *counts = ctx->dens.counts;
   if (n_counts) *n_counts = 2 * (int64_t)ctx->dens.npts;
   if (nmax) *nmax = &ctx->d_c->nmax_bits;
+  return GNX_OK;
+}
+
+extern "C" int gnx_strip_pairs_ptr(gnx_ctx* ctx, void** pairs) {
+  ARG(ctx && pairs && ctx->d_strip, "strip decomposition is not enabled");
+  *pairs = ctx->strip_h.pairs;
   return GNX_OK;
 }
 
@@ -2126,10 +2155,15 @@ static int strip_recv(gnx_ctx* ctx, int which, int mode) {
 //   1 receive migrants; list and send the halo                 | barrier
 //   2 receive ghosts; re-grid; mate search; send edge choices  | barrier
 //   3 receive choices; pair list; publish the births           | all-gather of `births`
-//   4 id base; offspring; route and send dispersed newborns    | barrier
+//   4 id base; offspring, mutation; route and send dispersed newborns | barrier
 //   5 receive newborns; density counts                         | all-reduce (sum) of `counts`
 //   6 N raster over the strip's rows                           | all-reduce (max) of `nmax`
 //   7 d raster; death probabilities and mortality draw; end of step
+// With Poisson births (n_births_fixed = 0) the births of a rank depend on the pairs of the lower ranks, so
+// phase 3 ends after the pair list and publishes the pairs, and a ninth phase follows the pairs all-gather:
+//   3 receive choices; pair list; publish the pairs            | all-gather of `pairs`
+//   8 Poisson births keyed by the species-wide pair positions; publish the births | all-gather of `births`
+// and then phases 4 to 7 as above.
 static int strip_phase_launch(gnx_ctx* ctx, int phase) {
   cudaStream_t s = ctx->stream;
   int r;
@@ -2157,7 +2191,18 @@ static int strip_phase_launch(gnx_ctx* ctx, int phase) {
       LAUNCHED(ctx);
       k_strip_choice_finish<<<1, 1, 0, s>>>(ctx->d_strip);
       LAUNCHED(ctx);
-      if ((r = gnx_dedup_pairs(ctx))) return r;
+      if ((r = scan_pairs(ctx))) return r;
+      if (!ctx->cfg.n_births_fixed) {
+        k_strip_publish_pairs<<<1, 1, 0, s>>>(ctx->d_c, ctx->d_strip);
+        LAUNCHED(ctx);
+        return GNX_OK;
+      }
+      k_strip_publish_births<<<1, 1, 0, s>>>(ctx->d_c, ctx->d_strip);
+      LAUNCHED(ctx);
+      return GNX_OK;
+    case 8:
+      ARG(!ctx->cfg.n_births_fixed, "phase 8 (Poisson births) with n_births_fixed");
+      if ((r = draw_births(ctx))) return r;
       k_strip_publish_births<<<1, 1, 0, s>>>(ctx->d_c, ctx->d_strip);
       LAUNCHED(ctx);
       return GNX_OK;
@@ -2181,7 +2226,7 @@ static int strip_phase_launch(gnx_ctx* ctx, int phase) {
       LAUNCHED(ctx);
       return GNX_OK;
     default:
-      ARG(false, "phase must be 0..7");
+      ARG(false, "phase must be 0..8");
   }
   return GNX_OK;
 }
@@ -2194,12 +2239,35 @@ static int strip_barrier_launch(gnx_ctx* ctx, int kind) {
   return GNX_OK;
 }
 
+// The phases of one strip time step in order and the gnx_strip_barrier kind after each (-1: the step ends);
+// gnx_strip_phase_order hands the same table to callers that sequence the phases themselves.
+static void strip_step_plan(bool fixed, const int** phase, const int** sync_after, int* n) {
+  static const int fixed_phase[8] = {0, 1, 2, 3, 4, 5, 6, 7}, fixed_sync[8] = {0, 0, 0, 1, 0, 2, 3, -1};
+  static const int poisson_phase[9] = {0, 1, 2, 3, 8, 4, 5, 6, 7}, poisson_sync[9] = {0, 0, 0, 4, 1, 0, 2, 3, -1};
+  *phase = fixed ? fixed_phase : poisson_phase;
+  *sync_after = fixed ? fixed_sync : poisson_sync;
+  *n = fixed ? 8 : 9;
+}
+
+extern "C" int gnx_strip_phase_order(int32_t n_births_fixed, int32_t* phases, int32_t* sync_after, int32_t* n) {
+  ARG(phases && sync_after && n, "null");
+  const int *ph, *sy;
+  int k;
+  strip_step_plan(n_births_fixed != 0, &ph, &sy, &k);
+  for (int i = 0; i < k; ++i) { phases[i] = ph[i]; sync_after[i] = sy[i]; }
+  *n = k;
+  return GNX_OK;
+}
+
 // the whole time step of one strip: phase, then the barrier / collective that follows it (gnx_step captures
-// this into one CUDA graph; the spin barriers inside it order the ranks' graphs against each other)
+// this into one CUDA graph; the spin barriers inside it order the ranks' graphs against each other).  The
+// sequence is fixed when the step is captured: a change of n_births_fixed changes prm, hence the step key.
 static int strip_whole_step(gnx_ctx* ctx) {
-  static const int sync_after[8] = {0, 0, 0, 1, 0, 2, 3, -1};
-  for (int k = 0; k < 8; ++k) {
-    int r = strip_phase_launch(ctx, k);
+  const int *phase, *sync_after;
+  int n;
+  strip_step_plan(ctx->cfg.n_births_fixed != 0, &phase, &sync_after, &n);
+  for (int k = 0; k < n; ++k) {
+    int r = strip_phase_launch(ctx, phase[k]);
     if (r != GNX_OK) return r;
     if (sync_after[k] >= 0 && (r = strip_barrier_launch(ctx, sync_after[k])) != GNX_OK) return r;
   }
@@ -2586,6 +2654,7 @@ static int tskit_renumber(gnx_ctx* ctx, int reset_t0) {
 extern "C" int gnx_tskit_enable(gnx_ctx* ctx, int64_t edge_capacity, int64_t birth_capacity) {
   ARG(ctx && edge_capacity > 0 && birth_capacity > 0, "capacities");
   USE_DEVICE(ctx);
+  ARG(!ctx->d_strip, "tskit recording is not supported under strip decomposition");
   ARG(edge_capacity < (1ll << 31) && birth_capacity < (1ll << 31), "capacities");
   if (!ctx->have_paths) { g_last_error = "recombination paths not set"; return GNX_ERR_STATE; }
   CK(cudaStreamSynchronize(ctx->stream));

@@ -53,6 +53,10 @@ struct Counters {
   int32_t tail_sent;    // newborns of this step shipped to the strip they dispersed into
   int32_t pad3;
   int64_t max_idx_global;   // species-wide max_ind_idx while Counters.max_idx carries this rank's id base
+  // set by k_strip_id_base for the rest of the step (k_mutate replays the species-wide mutation draws)
+  int64_t max_idx_base;     // species-wide max_ind_idx at the start of the step
+  int32_t births_lo;        // births of the lower ranks: offspring number of this rank's first newborn
+  int32_t births_all;       // births of the species
 };
 #define GNX_ERRBIT_CAPACITY 1
 #define GNX_ERRBIT_DRAWS 2
@@ -222,7 +226,8 @@ struct StripPeer {
 #define STRIP_SYNC_FLAGS 0           // uint32[MAX_WORLD]: barrier epoch each rank has reached
 #define STRIP_SYNC_BIRTHS 128        // int64[MAX_WORLD]: births of each rank this step
 #define STRIP_SYNC_NMAX 256          // uint64[MAX_WORLD]: bits of each rank's max(N)
-#define STRIP_SYNC_COUNTS 384        // int32[MAX_WORLD][counts_cap]: each rank's coarse density counts
+#define STRIP_SYNC_PAIRS 384         // int64[MAX_WORLD]: pairs of each rank this step (Poisson births)
+#define STRIP_SYNC_COUNTS 512        // int32[MAX_WORLD][counts_cap]: each rank's coarse density counts
 struct Strip {
   int32_t enabled;
   int32_t rank, world;
@@ -234,6 +239,7 @@ struct Strip {
   StripPeer peer[GNX_STRIP_MAX_WORLD];       // peer[rank] = this rank's own buffers
   uint8_t* sent;                     // [cap] tail entries shipped away this step
   int64_t* births;                   // [world] births of every rank this step (all-gathered)
+  int64_t* pairs;                    // [world] pairs of every rank this step (all-gathered; Poisson births only)
   // individuals to ship, listed by the kernel that finds them (k_move_key: leavers; k_strip_halo_list:
   // the strip's edge rows; k_strip_newborn_route: newborns that dispersed out), sent by k_strip_send
   int32_t* list_entry;

@@ -1002,16 +1002,21 @@ struct PairScan {
   }
 };
 
-// Poisson births: second scan over the P pairs
-__global__ void __launch_bounds__(256) k_draw_births(Pop pop, Params prm, DevDraws dr, Work w, const Counters* c) {
-  const int P = c->P, cur = c->cur;
+// Poisson births: second scan over the P pairs.  `st` (strip decomposition, else NULL): this rank's
+// pairs are the slice of the species-wide pair list that follows the pairs of the lower ranks.
+__global__ void __launch_bounds__(256) k_draw_births(Pop pop, Params prm, DevDraws dr, Work w, const Counters* c,
+                                                     const Strip* st) {
+  const int P = c->P;
+  long long pair_base = 0;
+  if (st)
+    for (int r = 0; r < st->rank; ++r) pair_base += st->pairs[r];
   for (int p = GTID; p < P; p += GSTRIDE) {
     int nbv;
     if (dr.poisson) nbv = dr.poisson[p];
     else {
       // keyed by the pair's position in the canonical pair list (an individual can belong to
       // several pairs under panmixia)
-      RngStream g(prm.seed_lo, prm.seed_hi, (int64_t)p, SITE_BIRTHS, c->t);
+      RngStream g(prm.seed_lo, prm.seed_hi, (int64_t)(pair_base + p), SITE_BIRTHS, c->t);
       nbv = sample_poisson(g, prm.c.n_births_lambda);
     }
     w.nb[p] = max(nbv, 1);                   // mating.py:125
@@ -1634,14 +1639,20 @@ __global__ void k_mut_rebuild(Mut mu, Counters* c) {
   if (threadIdx.x == 0 && blockIdx.x == 0) mut_rebuild_tables(mu, c);
 }
 
+// STRIP: one strip of a decomposed landscape (by-locus layout only: no tskit layout, trait mutation or
+// tskit rows).  Every rank replays the species-wide sequence -- the births of all ranks, keyed by the
+// species-wide max_ind_idx (k_strip_id_base left both in Counters) -- and so keeps identical tables and
+// logs; only the rank that holds offspring o (offspring are rank-major) edits its row and z.
+template <bool STRIP>
 __global__ void __launch_bounds__(256) k_mutate(Pop pop, Params prm, Traits tr, DevDraws dr, Mut mu, Counters* c, int tsk_on) {
   __shared__ int new_loci[GNX_MUT_MAX_NEW];
   __shared__ int n_new;
   if (blockIdx.x != 0) return;
   if (threadIdx.x == 0) {
     n_new = 0;
-    const int B = c->B, n = c->n, cur = c->cur, Wq = pop.Wq;
-    RngStream g(prm.seed_lo, prm.seed_hi, c->max_idx + 1, SITE_MUTATE, c->t);
+    // B: births of the species; under strips this rank's newborns are offspring [births_lo, births_lo + c->B)
+    const int B = STRIP ? c->births_all : c->B, n = c->n, cur = c->cur, Wq = pop.Wq;
+    RngStream g(prm.seed_lo, prm.seed_hi, (STRIP ? c->max_idx_base : c->max_idx) + 1, SITE_MUTATE, c->t);
     const long long n_muts = B == 0 ? 0 : (dr.mut_n ? (long long)dr.mut_n[0]
                                       : sample_binomial_wait(g, (long long)B * mu.L, mu.mu_tot));   // mutation.py:172-173
     for (long long m = 0; m < n_muts; ++m) {
@@ -1658,7 +1669,7 @@ __global__ void __launch_bounds__(256) k_mutate(Pop pop, Params prm, Traits tr, 
       const uint32_t R = dr.mut_ind_R ? dr.mut_ind_R[m] : g.u32();
       // r.choice(offspring): the list holds the new ids in DESCENDING order (species.py:615-622)
       const int o = B - 1 - (int)choose_k(R, (uint32_t)B);
-      const int i = n + o;
+      const int i = STRIP ? n + (o - c->births_lo) : n + o;
       int row = -1;
       double alpha = 0.0;
       if (type >= 1) {
@@ -1712,27 +1723,29 @@ __global__ void __launch_bounds__(256) k_mutate(Pop pop, Params prm, Traits tr, 
         // mutation.py:117: spp[individ].g[idx, homol] = 1
         row = lower_bound_i32(mu.nonneut, mu.counts[1], locus);
         const int bit = mu.tskit_layout ? locus : row;
-        uint32_t* hw = reinterpret_cast<uint32_t*>(pop.G + ((size_t)pop.gslot[cur][i] * 2 + homol) * Wq);
-        hw[bit >> 5] |= 1u << (bit & 31);
-        // species.py:929 _set_z_individ
-        const uint4* Gi = pop.G + (size_t)pop.gslot[cur][i] * 2 * Wq;
-        for (int tt = 0; tt < pop.T; ++tt) {
-          double acc = 0.0;
-          const int nl = mu.own_tables ? mu.counts[4 + tt] : tr.n_loci[tt];
-          for (int q = 0; q < Wq; ++q) {
-            const int* ptr = tr.chunk_ptr + tt * (4 * Wq + 1) + 4 * q;
-            if (ptr[0] == ptr[4]) continue;
-            const uint4 h0 = Gi[q], h1 = Gi[Wq + q];
-            const uint32_t w0[4] = {h0.x, h0.y, h0.z, h0.w}, w1[4] = {h1.x, h1.y, h1.z, h1.w};
-            for (int ww = 0; ww < 4; ++ww)
-              for (int k = ptr[ww]; k < ptr[ww + 1]; ++k) {                 // plain loads: the tables were just rewritten
-                const int sh = tr.te_locus[k] & 31;
-                double geno = 0.5 * (double)((int)((w0[ww] >> sh) & 1u) + (int)((w1[ww] >> sh) & 1u));
-                if (tr.te_dom) geno = fmin(geno * tr.te_dom[k], 1.0);
-                acc += nl > 1 ? geno * tr.te_alpha[k] : geno;
-              }
+        if (!STRIP || (unsigned)(o - c->births_lo) < (unsigned)c->B) {      // this rank holds offspring o
+          uint32_t* hw = reinterpret_cast<uint32_t*>(pop.G + ((size_t)pop.gslot[cur][i] * 2 + homol) * Wq);
+          hw[bit >> 5] |= 1u << (bit & 31);
+          // species.py:929 _set_z_individ
+          const uint4* Gi = pop.G + (size_t)pop.gslot[cur][i] * 2 * Wq;
+          for (int tt = 0; tt < pop.T; ++tt) {
+            double acc = 0.0;
+            const int nl = mu.own_tables ? mu.counts[4 + tt] : tr.n_loci[tt];
+            for (int q = 0; q < Wq; ++q) {
+              const int* ptr = tr.chunk_ptr + tt * (4 * Wq + 1) + 4 * q;
+              if (ptr[0] == ptr[4]) continue;
+              const uint4 h0 = Gi[q], h1 = Gi[Wq + q];
+              const uint32_t w0[4] = {h0.x, h0.y, h0.z, h0.w}, w1[4] = {h1.x, h1.y, h1.z, h1.w};
+              for (int ww = 0; ww < 4; ++ww)
+                for (int k = ptr[ww]; k < ptr[ww + 1]; ++k) {                 // plain loads: the tables were just rewritten
+                  const int sh = tr.te_locus[k] & 31;
+                  double geno = 0.5 * (double)((int)((w0[ww] >> sh) & 1u) + (int)((w1[ww] >> sh) & 1u));
+                  if (tr.te_dom) geno = fmin(geno * tr.te_dom[k], 1.0);
+                  acc += nl > 1 ? geno * tr.te_alpha[k] : geno;
+                }
+            }
+            pop.z[cur][(size_t)tt * pop.cap + i] = nl > 1 ? 0.5 + acc : acc;
           }
-          pop.z[cur][(size_t)tt * pop.cap + i] = nl > 1 ? 0.5 + acc : acc;
         }
         if (mu.tskit_layout) new_loci[n_new++] = locus;
       }
@@ -1740,7 +1753,7 @@ __global__ void __launch_bounds__(256) k_mutate(Pop pop, Params prm, Traits tr, 
       if (nl < mu.log_cap) {
         gnx_mutation_row_t r;
         r.t = c->t;
-        r.individual = c->max_idx + 1 + o;
+        r.individual = (STRIP ? c->max_idx_base : c->max_idx) + 1 + o;
         r.locus = locus;
         r.row = row;
         r.homologue = homol;

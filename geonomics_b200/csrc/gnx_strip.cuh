@@ -19,7 +19,10 @@
 //   newborns  -- offspring that dispersed out of the strip (movement.py:98-141), before the
 //                density counts and the mortality of the same step
 // plus three collectives on small arrays: births per rank (id bases, species.py:614-619), the
-// 2 x 4 coarse density-count grids (sum, spatial.py:73-97) and max(N) (demography.py:104-119).
+// 2 x 4 coarse density-count grids (sum, spatial.py:73-97) and max(N) (demography.py:104-119); with
+// Poisson births a fourth, pairs per rank, comes first: the birth draws are keyed by the pair's
+// species-wide position (mating.py:120-126).  Mutation needs no exchange: every rank replays the
+// step's draws and keeps the tables, and the owner of a mutated offspring edits its genome row.
 #pragma once
 #include "gnx_common.cuh"
 
@@ -240,6 +243,9 @@ __global__ void k_strip_id_base(Counters* c, const Strip* st) {
     if (r < st->rank) off += st->births[r];
     tot += st->births[r];
   }
+  c->max_idx_base = c->max_idx;
+  c->births_lo = (int32_t)off;
+  c->births_all = (int32_t)tot;
   c->max_idx_global = c->max_idx + tot;      // species-wide max_ind_idx once this step's births exist
   c->max_idx += off;
 }
@@ -250,6 +256,8 @@ __global__ void k_strip_end_step(Counters* c) {
 }
 // this rank's births, where the all-gather picks them up
 __global__ void k_strip_publish_births(const Counters* c, const Strip* st) { st->births[st->rank] = (long long)c->B; }
+// this rank's pairs (Poisson births: the lower ranks' pairs key this rank's draws, k_draw_births)
+__global__ void k_strip_publish_pairs(const Counters* c, const Strip* st) { st->pairs[st->rank] = (long long)c->P; }
 
 // ========================================================================================
 // Barrier and the three small collectives of a strip time step, over peer memory.
@@ -257,7 +265,9 @@ __global__ void k_strip_publish_births(const Counters* c, const Strip* st) { st-
 // CUDA IPC / NVLink like the record buffers); rank w writes only slot w of every page, so nothing
 // is ever contended: the payload first (kind 1: this rank's births -> all-gather; kind 2: its
 // coarse density counts -> sum over the ranks in rank order, so the integers are the same on every
-// rank; kind 3: the bits of its max(N) -> maximum), a system-scope fence, then the rank's barrier
+// rank; kind 3: the bits of its max(N) -> maximum; kind 4: its pairs -> all-gather, in a slot of its own
+// because the births all-gather of the same step follows it only one phase later), a system-scope
+// fence, then the rank's barrier
 // epoch with release semantics into every peer's flag word; the lanes then spin (acquire loads) on
 // the flags of this rank's own page until every peer has reached the same epoch.  Kernels of a rank
 // are stream-ordered, so a peer that reads a slot has finished with it before the writer can get to
@@ -292,6 +302,8 @@ __global__ void __launch_bounds__(256) k_strip_barrier(const Strip* stp, int kin
     }
   } else if (kind == 3) {
     if (tid < W) reinterpret_cast<unsigned long long*>(st.peer[tid].sync + STRIP_SYNC_NMAX)[me] = *nmax;
+  } else if (kind == 4) {
+    if (tid < W) reinterpret_cast<int64_t*>(st.peer[tid].sync + STRIP_SYNC_PAIRS)[me] = st.pairs[me];
   }
   __threadfence_system();
   __syncthreads();
@@ -323,5 +335,7 @@ __global__ void __launch_bounds__(256) k_strip_barrier(const Strip* stp, int kin
       for (int r = 0; r < W; ++r) m = in[r] > m ? in[r] : m;
       *nmax = m;
     }
+  } else if (kind == 4) {
+    if (tid < W) st.pairs[tid] = reinterpret_cast<const volatile int64_t*>(mine + STRIP_SYNC_PAIRS)[tid];
   }
 }

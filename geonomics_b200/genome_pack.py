@@ -34,7 +34,7 @@ def unpack_genomes(packed, L):
     """u32[N, 2, W] -> int8[N, L, 2]."""
     packed = np.ascontiguousarray(packed, dtype=np.uint32)
     n = packed.shape[0]
-    bits = np.unpackbits(packed.view(np.uint8).reshape(n, 2, -1), axis=-1, bitorder='little')
+    bits = np.unpackbits(packed.view(np.uint8).reshape(n, 2, 4 * packed.shape[2]), axis=-1, bitorder='little')
     return np.ascontiguousarray(np.transpose(bits[:, :, :L], (0, 2, 1))).astype(np.int8)
 
 

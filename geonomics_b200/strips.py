@@ -8,7 +8,8 @@ individuals are written by the sender straight into the receiver's buffer (NVLin
 mapped through CUDA IPC) and the device reads every size from device memory, so a time step
 is enqueued without a host round trip.  This module supplies the plan (which rows, which
 individuals go where at upload) and, where the host sequences the phases, the barrier between
-them and the three small collectives (births all-gather, density-count sum, max(N)).
+them and the small collectives (births all-gather, density-count sum, max(N), and with Poisson
+births the pairs all-gather).
 
 Two transports:
   * `NcclStrips`   one process per GPU (`torch.distributed`, backend nccl, which only exchanges
@@ -25,8 +26,6 @@ import numpy as np
 
 from . import _lib
 from .device import DeviceSpecies
-
-N_PHASES = 8
 
 
 # ---------------------------------------------------------------------------------------------
@@ -73,6 +72,18 @@ def owner_of(y, bounds, cell_size, ncy):
     """Rank that owns an individual at ordinate y (its mating-grid row, clamped like the kernel)."""
     row = np.minimum(np.floor(np.asarray(y) / cell_size).astype(np.int64), ncy - 1)
     return np.searchsorted(np.asarray(bounds)[1:-1], row, side='right')
+
+
+def phase_sequence(n_births_fixed):
+    """The phases of one time step in order, each with the gnx_strip_barrier kind that follows it
+    (0 barrier, 1 births all-gather, 2 density-count sum, 3 max(N), 4 pairs all-gather; None: the
+    step ends), as the library's gnx_step runs them.  Poisson births are keyed by the species-wide
+    position of each pair, so phase 3 publishes the pairs and phase 8 draws the births once the
+    pairs of every rank are known."""
+    phases, syncs, n = (C.c_int32 * 16)(), (C.c_int32 * 16)(), C.c_int32()
+    _lib.check(_lib.lib().gnx_strip_phase_order(int(bool(n_births_fixed)), phases, syncs, C.byref(n)),
+               'gnx_strip_phase_order')
+    return [(phases[k], None if syncs[k] < 0 else syncs[k]) for k in range(n.value)]
 
 
 def merge_records(per_rank):
@@ -129,6 +140,9 @@ class StripRank:
         _lib.check(L.gnx_strip_collective_ptrs(self.dev._ctx, C.byref(b), C.byref(c), C.byref(n), C.byref(m)),
                    'gnx_strip_collective_ptrs')
         self.births_ptr, self.counts_ptr, self.n_counts, self.nmax_ptr = b.value, c.value, int(n.value), m.value
+        p = C.c_void_p()
+        _lib.check(L.gnx_strip_pairs_ptr(self.dev._ctx, C.byref(p)), 'gnx_strip_pairs_ptr')
+        self.pairs_ptr = p.value
 
     def connect(self, peer_rank, endpoints, same_process):
         _lib.check(self.dev._L.gnx_strip_connect(self.dev._ctx, int(peer_rank), C.byref(endpoints),
@@ -138,7 +152,8 @@ class StripRank:
         _lib.check(self.dev._L.gnx_strip_phase(self.dev._ctx, int(k)), 'gnx_strip_phase')
 
     def barrier(self, kind=0):
-        """gnx_strip_barrier: the barrier (0) or a collective (1 births, 2 counts, 3 max(N)) over peer memory."""
+        """gnx_strip_barrier: the barrier (0) or a collective (1 births, 2 counts, 3 max(N), 4 pairs) over peer
+        memory."""
         _lib.check(self.dev._L.gnx_strip_barrier(self.dev._ctx, int(kind)), 'gnx_strip_barrier')
 
     def check(self):
@@ -149,11 +164,8 @@ class StripRank:
         births = torch.as_tensor(_DevArray(self.births_ptr, self.world, '<i8'), device='cuda')
         counts = torch.as_tensor(_DevArray(self.counts_ptr, self.n_counts, '<i4'), device='cuda')
         nmax = torch.as_tensor(_DevArray(self.nmax_ptr, 1, '<i8'), device='cuda')      # bits of a double >= 0
-        return births, counts, nmax
-
-
-# what follows each phase: the barrier / collective kind of gnx_strip_barrier (phase 7 ends the step)
-PHASE_SYNC = {0: 0, 1: 0, 2: 0, 3: 1, 4: 0, 5: 2, 6: 3}
+        pairs = torch.as_tensor(_DevArray(self.pairs_ptr, self.world, '<i8'), device='cuda')
+        return births, counts, nmax, pairs
 
 
 def _subset(pop, mask):
@@ -191,6 +203,26 @@ class LocalStrips:
     def set_burn(self, burn):
         for r in self.ranks:
             r.dev.set_burn(burn)
+
+    def set_mutation(self, *args, **kw):
+        """Mutation of each step's offspring (DeviceSpecies.set_mutation, by-locus layout): every rank gets
+        the same tables and replays the same species-wide draws."""
+        for r in self.ranks:
+            r.dev.set_mutation(*args, **kw)
+
+    def read_mutations(self, max_rows=4096):
+        """Drain every rank's mutation log; each must equal the undecomposed run's, so they must agree.
+        Returns rank 0's (rows, state) as DeviceSpecies.read_mutations does."""
+        for r in self.ranks:
+            r.check()
+        out = [r.dev.read_mutations(max_rows) for r in self.ranks]
+        rows0, st0 = out[0]
+        for rank, (rows, st) in enumerate(out[1:], 1):
+            same = rows == rows0 and st['n_mutables'] == st0['n_mutables'] and \
+                all(np.array_equal(st[k], st0[k]) for k in ('nonneut_loci', 'delet_loci', 'delet_s'))
+            if not same:
+                raise RuntimeError('strip rank %d: mutation log or tables differ from rank 0' % rank)
+        return rows0, st0
 
     def upload(self, x, y, age=None, sex=None, idx=None, g=None, genomes_packed=None, max_ind_idx=None):
         n = len(x)
@@ -231,23 +263,24 @@ class LocalStrips:
                 self.device_barrier = True
             return self.step(n - 1) if n > 1 else None
         for _ in range(n):
-            for k in range(N_PHASES):
+            for k, sync in phase_sequence(self.ranks[0].dev._cfg.n_births_fixed):
                 for r in self.ranks:
                     r.phase(k)
                 self._sync()                               # the barrier: every context finished phase k
-                if k == 3:                                 # births of every rank, everywhere
-                    b = torch.stack([t[0][r] for r, t in enumerate(self._t)])
+                if sync in (1, 4):                         # births (pairs) of every rank, everywhere
+                    j = 0 if sync == 1 else 3
+                    b = torch.stack([t[j][r] for r, t in enumerate(self._t)])
                     for t in self._t:
-                        t[0][:self.world] = b
-                elif k == 5:                               # density counts summed over the strips
+                        t[j][:self.world] = b
+                elif sync == 2:                            # density counts summed over the strips
                     tot = sum(t[1] for t in self._t)
                     for t in self._t:
                         t[1].copy_(tot)
-                elif k == 6:                               # max(N): non-negative doubles order like their bits
+                elif sync == 3:                            # max(N): non-negative doubles order like their bits
                     mx = torch.stack([t[2] for t in self._t]).max()
                     for t in self._t:
                         t[2].fill_(mx)
-                if k in (3, 5, 6):
+                if sync:
                     torch.cuda.synchronize()
 
     def step_records(self):
@@ -302,6 +335,14 @@ class NcclStrips:
     def set_burn(self, burn):
         self.me.dev.set_burn(burn)
 
+    def set_mutation(self, *args, **kw):
+        """DeviceSpecies.set_mutation on this rank; every rank must make the same call."""
+        self.me.dev.set_mutation(*args, **kw)
+
+    def read_mutations(self, max_rows=4096):
+        """This rank's mutation log and tables, which equal every other rank's."""
+        return self.me.dev.read_mutations(max_rows)
+
     def upload_owned(self, x, y, age=None, sex=None, idx=None, g=None, genomes_packed=None, max_ind_idx=None):
         """Upload this rank's share of a population every rank holds on the host."""
         idx = np.arange(len(x), dtype=np.int64) if idx is None else np.asarray(idx)
@@ -312,7 +353,7 @@ class NcclStrips:
                            max_ind_idx=int(idx.max()) if max_ind_idx is None else max_ind_idx)
 
     def step(self, n=1):
-        self.me.dev.step(n)            # gnx_step: eight phases + gnx_strip_barrier, one graph per step
+        self.me.dev.step(n)            # gnx_step: the phases + gnx_strip_barrier, one graph per step
 
     def sync(self):
         self.me.check()

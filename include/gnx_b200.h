@@ -255,7 +255,8 @@ int gnx_step(gnx_ctx* ctx, int32_t n_steps);
  * offspring ids species.py:614-619 (based at the births of the lower ranks).  Records travel by
  * direct writes into the receiver's buffer (NVLink peer memory through CUDA IPC, or plain device
  * pointers when the ranks are contexts of one process); the caller supplies the barrier between
- * phases (a stream-ordered collective) and the three small collectives named at gnx_strip_phase. */
+ * phases (a stream-ordered collective) and the small collectives named at gnx_strip_collective_ptrs
+ * and gnx_strip_pairs_ptr, or gnx_strip_barrier does both over peer memory. */
 typedef struct {
   int32_t rank, world;
   const int32_t* first_rows;     /* [world + 1] first mating-grid row of every rank, first_rows[world] = rows of the grid */
@@ -278,18 +279,30 @@ int gnx_strip_connect(gnx_ctx* ctx, int32_t peer_rank, const gnx_strip_endpoints
  * counts int32[n_counts] (all-reduce sum after phase 5), nmax uint64[1] holding the bits of a
  * non-negative double (all-reduce max after phase 6) */
 int gnx_strip_collective_ptrs(gnx_ctx* ctx, void** births, void** counts, int64_t* n_counts, void** nmax);
-/* one phase (0..7) of a time step on this rank's stream; every rank must have finished phase k
- * before any rank starts phase k + 1 */
+/* device buffer of the pairs int64[world] (all-gather after phase 3 with Poisson births) */
+int gnx_strip_pairs_ptr(gnx_ctx* ctx, void** pairs);
+/* one phase of a time step on this rank's stream; every rank must have finished a phase before any
+ * rank starts the next.  With n_births_fixed the step is phases 0..7 (births all-gather after phase 3).
+ * With Poisson births the births of a rank are keyed by the species-wide positions of its pairs, so
+ * phase 3 ends after the pair list and publishes the pairs; the step is then phases 0, 1, 2, 3, 8, 4, 5,
+ * 6, 7 with the pairs all-gather after phase 3 and the births all-gather after phase 8 (the Poisson
+ * draws).  Phase 8 with n_births_fixed is an error.  Mutation (by-locus layout) runs inside phase 4:
+ * every rank replays the species-wide draws, so their tables and mutation logs stay identical. */
 int gnx_strip_phase(gnx_ctx* ctx, int32_t phase);
-/* The barrier between two phases (kind 0) and the three collectives (1 births all-gather, 2 density-count sum,
- * 3 max(N)) done by ONE one-CTA kernel over peer memory on the rank's stream: every rank writes its slot of
+/* That order, as gnx_step runs it: phases[k] then the gnx_strip_barrier kind sync_after[k] (-1: the step
+ * ends), for k < *n (at most 9). */
+int gnx_strip_phase_order(int32_t n_births_fixed, int32_t* phases, int32_t* sync_after, int32_t* n);
+/* The barrier between two phases (kind 0) and the four collectives (1 births all-gather, 2 density-count sum,
+ * 3 max(N), 4 pairs all-gather) done by ONE one-CTA kernel over peer memory on the rank's stream: every rank writes its slot of
  * every peer's synchronisation page (NVLink stores), publishes its barrier epoch with release semantics and
  * spins on its own page until every peer has arrived.  Replaces the caller-supplied NCCL collectives; all
  * ranks must make the same sequence of calls; a peer that never arrives sets an error after ~5 s. */
 int gnx_strip_barrier(gnx_ctx* ctx, int32_t kind);
 /* gnx_step on a context that holds a strip runs WHOLE time steps this way -- the eight phases with
- * gnx_strip_barrier after each of the first seven, captured as one CUDA graph per step like the undecomposed
- * run; the spin barriers inside order the ranks' graphs against each other.  Every rank makes the same call. */
+ * gnx_strip_barrier after each of the first seven (nine and eight with Poisson births), captured as one CUDA
+ * graph per step like the undecomposed run; the spin barriers inside order the ranks' graphs against each
+ * other.  Every rank makes the same call.  Not supported on a strip context, and refused by the call that
+ * would set them up: tskit recording, the tskit genotype layout, trait mutation and injected draws. */
 int gnx_strip_check(gnx_ctx* ctx);      /* synchronises; exchange overflow -> GNX_ERR_CAPACITY */
 
 int gnx_sync(gnx_ctx* ctx);
