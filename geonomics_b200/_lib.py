@@ -170,6 +170,16 @@ class TskitRows(C.Structure):
     ]
 
 
+class GenomeInit(C.Structure):
+    _fields_ = [
+        ('seed', C.c_uint64),
+        ('n_loci', C.c_int32),
+        ('host_n_carriers', c_int64_p),
+        ('host_write_mask', C.POINTER(C.c_uint8)),
+        ('tskit_rows', C.c_int32),
+    ]
+
+
 FIELDS = dict(
     X=1, Y=2, AGE=3, SEX=4, IDX=5, Z=6, FIT=7, GSLOT=8, N_NBRS=9, MATE=10, PAIRS=11, NB=12,
     PERM=13, CELL_START=14, COUNTS_N=15, COUNTS_P=16, VALS_N=17, VALS_P=18, GRAD_N=19, GRAD_P=20,
@@ -234,6 +244,10 @@ SIGNATURES = {
     'gnx_read_mutations': (C.c_int, [_ctx, C.POINTER(MutationRow), C.c_int32, c_int32_p, c_int32_p, c_int32_p,
                                      c_int32_p, c_int32_p, c_double_p, c_int32_p]),
     'gnx_read_mutation_tables': (C.c_int, [_ctx, C.c_int32, c_int32_p, c_int32_p, c_double_p, c_int32_p, c_int32_p]),
+    'gnx_genome_init_begin': (C.c_int, [_ctx, C.POINTER(GenomeInit), C.POINTER(C.c_void_p), c_int64_p]),
+    'gnx_genome_init_pass': (C.c_int, [_ctx, c_int32_p]),
+    'gnx_genome_init_end': (C.c_int, [_ctx]),
+    'gnx_genome_init_rows': (C.c_int, [_ctx, c_int32_p, c_int64_p, c_int8_p, C.c_int64, c_int64_p]),
     'gnx_stats_genotypes': (C.c_int, [_ctx, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), c_double_p, c_int64_p]),
     'gnx_stats_genotypes_region': (C.c_int, [_ctx, C.c_double, C.c_double, C.c_double, C.c_double,
                                              C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), c_double_p, c_int64_p]),

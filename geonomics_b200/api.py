@@ -25,6 +25,7 @@ from collections import OrderedDict
 
 import numpy as np
 
+from . import genome_pack as gp
 from .device import DeviceSpecies
 
 
@@ -1024,24 +1025,23 @@ class Species:
         return self._dev.stats()['mean_fit'] if self.gen_arch.traits is not None else np.nan
 
     # ---- post burn-in genome assignment (species.py:956-1094, genome.py:1108-1157) ----
-    def _set_genomes_and_tables(self, burn_T=None, T=None):
+    def _set_genomes_and_tables(self, burn_T=None, T=None, genome_init='host'):
         s = self._dev.download(genomes=False)
         n = len(s['x'])
         ga = self.gen_arch
         L = ga.L
         tsk = ga.use_tskit
+        if genome_init == 'device':
+            self._set_genomes_on_device(s, burn_T, T)
+            return
         g = np.zeros((n, L, 2), dtype=np.int8)
         flat = g.reshape(n, L, 2)
         p = ga.p
         nonneut = set(int(v) for v in ga.nonneut_loci)
         mut_site, mut_node = [], []
+        n_muts = gp.carrier_counts(n, p[:L])
         for site in range(L):
-            freq = p[site]
-            n_mut = int(round(2 * n * freq, 0))
-            if n_mut == n * 2 and freq < 1:
-                n_mut -= 1
-            if n_mut == 0 and freq > 0:
-                n_mut = 1
+            n_mut = int(n_muts[site])
             if n_mut > 0:
                 hom = np.random.permutation(2 * n)[:n_mut]
                 if not tsk or site in nonneut:            # genome.py:1137-1142: only non-neutral rows are carried
@@ -1051,6 +1051,32 @@ class Species:
                     mut_node.append(hom.astype(np.int32))  # is 2k + h (see below)
         self._dev.set_burn(False)
         self._dev.upload(s['x'], s['y'], s['age'], s['sex'], s['idx'], g=g, max_ind_idx=s['max_ind_idx'])
+        self._finish_genome_assignment(s, burn_T, T, mut_site, mut_node)
+
+    def _set_genomes_on_device(self, s, burn_T, T):
+        """The same assignment drawn on the device (DeviceSpecies.init_genomes): the same per-locus 1-allele
+        counts, no genotype download and no host array.  The device seed comes from numpy's stream, so a
+        seeded model stays reproducible and every rand_genarch iteration gets new genomes."""
+        ga = self.gen_arch
+        seed = int(np.random.randint(0, 2 ** 63 - 1, dtype=np.int64))
+        mask = None
+        if ga.use_tskit:                                  # genome.py:1137-1142: only non-neutral rows are carried
+            mask = np.zeros(ga.L, np.uint8)
+            mask[np.asarray(ga.nonneut_loci, dtype=np.int64)] = 1
+        rows = self._dev.init_genomes(np.asarray(ga.p, dtype=np.float64)[:ga.L], seed, write_mask=mask,
+                                      tskit_rows=ga.use_tskit)
+        self._dev.set_burn(False)
+        mut_site, mut_node = [], []
+        if rows is not None and len(rows['site']):
+            # node of (individual k in species order, homologue h) is 2k + h; rows come sorted by (site, node)
+            mut_site = [rows['site']]
+            mut_node = [(2 * np.searchsorted(s['idx'], rows['idx']) + rows['homologue']).astype(np.int32)]
+        self._finish_genome_assignment(s, burn_T, T, mut_site, mut_node)
+
+    def _finish_genome_assignment(self, s, burn_T, T, mut_site, mut_node):
+        ga = self.gen_arch
+        n = len(s['x'])
+        tsk = ga.use_tskit
         # everyone up to this id was alive at the assignment (the FASTA writer tells them apart, writers.py)
         self._genome_assignment_max_idx = int(s['max_ind_idx'])
         self._tc = None
@@ -1247,10 +1273,22 @@ def _make_species(land, name, idx, spp_params, seed=0):
 # ---------------------------------------------------------------------------------------------
 # model (sim/model.py)
 # ---------------------------------------------------------------------------------------------
-class Model:
-    """sim/model.py:47.  `walk` / `run` keep their reference signatures."""
+def _check_genome_init(genome_init):
+    if genome_init not in ('host', 'device'):
+        raise ValueError("genome_init must be 'host' or 'device', not %r" % (genome_init,))
 
-    def __init__(self, name, params, verbose=False):
+
+class Model:
+    """sim/model.py:47.  `walk` / `run` keep their reference signatures.
+
+    genome_init selects how the starting genomes are assigned after the burn-in: 'host' (the
+    default) draws them with numpy's stream exactly as the reference does; 'device' draws them on the
+    GPU with the same exact per-locus allele counts (DeviceSpecies.init_genomes) and never builds the
+    N x L x 2 host array, which is what makes populations of millions of individuals startable."""
+
+    def __init__(self, name, params, verbose=False, genome_init='host'):
+        _check_genome_init(genome_init)
+        self.genome_init = genome_init
         self.params = copy.deepcopy(params)
         m = self.params.model
         self.name = name or 'unnamed_model'
@@ -1300,7 +1338,7 @@ class Model:
                 if self.reassign_genomes:
                     for spp in self.comm.values():
                         if spp.gen_arch is not None:
-                            spp._set_genomes_and_tables(self.burn_T, self.T)
+                            spp._set_genomes_and_tables(self.burn_T, self.T, self.genome_init)
                     self.reassign_genomes = False
                 self.comm.burned = True
         elif mode == 'main':
@@ -1460,7 +1498,7 @@ class Model:
                 ga = _make_genomic_architecture(self.params.comm.species[spp.name], self.land)
             spp._restore(self.orig_comm[n], self.land, gen_arch=ga)
             if ga is not None and not self.repeat_burn and spp.burned:
-                spp._set_genomes_and_tables(self.burn_T, self.T)
+                spp._set_genomes_and_tables(self.burn_T, self.T, self.genome_init)
         self.comm.burned = all(spp.burned for spp in self.comm.values())
         self.comm.t = -1
 
@@ -1569,8 +1607,10 @@ class Model:
         return writers.write_geodata(filepath, self._spp(spp), n=n)
 
 
-def make_model(parameters=None, verbose=False, name=None):
-    """main.py:442: a Model from a parameters-file path, a dict or a ParametersDict."""
+def make_model(parameters=None, verbose=False, name=None, genome_init='host'):
+    """main.py:442: a Model from a parameters-file path, a dict or a ParametersDict.  genome_init: how the
+    starting genomes are assigned after the burn-in (Model)."""
+    _check_genome_init(genome_init)
     if isinstance(parameters, str):
         params = read_parameters_file(parameters)
     elif isinstance(parameters, ParametersDict):
@@ -1579,4 +1619,5 @@ def make_model(parameters=None, verbose=False, name=None):
         params = make_params_dict(parameters, name or 'unnamed_model')
     else:
         raise ValueError('parameters must be a filepath, a dict or a ParametersDict')
-    return Model(name or params.get('model', {}).get('name', 'unnamed_model'), params, verbose=verbose)
+    return Model(name or params.get('model', {}).get('name', 'unnamed_model'), params, verbose=verbose,
+                 genome_init=genome_init)

@@ -9,6 +9,7 @@
 #include <vector>
 #include <algorithm>
 #include "gnx_kernels.cuh"
+#include "gnx_genome_init.cuh"
 
 static thread_local std::string g_last_error;
 
@@ -115,6 +116,17 @@ struct gnx_ctx {
   int64_t strip_buf_off[STRIP_N_BUF] = {0, 0, 0, 0};
   std::vector<void*> strip_allocs;
   std::vector<void*> strip_ipc_opened;
+  // staged device genome assignment (gnx_genome_init_*): 0 idle, 1 selecting, 3 selected, 2 genomes written
+  int gi_stage = 0;
+  bool gi_tskit = false;
+  std::vector<long long> gi_carriers;   // n_carriers as given to gnx_genome_init_begin
+  GiLocus* d_gi_state = nullptr;
+  uint32_t* d_gi_lkey = nullptr;
+  uint8_t* d_gi_write = nullptr;        // [L] loci whose bits are written
+  int32_t* d_gi_hist = nullptr;         // [L][GI_BINS]
+  int32_t* d_gi_active = nullptr;       // [2]: loci still active, loci with more carriers than keys
+  int64_t gi_t = 0;                     // Counters.t when the genomes were written (the rows describe that population)
+  std::vector<void*> gi_allocs;
 };
 
 template <class T>
@@ -450,6 +462,7 @@ extern "C" int gnx_destroy(gnx_ctx* ctx) {
   free_bucket(ctx->tsk_allocs);
   free_bucket(ctx->mut_allocs);
   free_bucket(ctx->strip_allocs);
+  free_bucket(ctx->gi_allocs);
   for (void* m : ctx->strip_ipc_opened) cudaIpcCloseMemHandle(m);
   ctx->strip_ipc_opened.clear();
   if (ctx->strip_block) cudaFree(ctx->strip_block);
@@ -2769,4 +2782,176 @@ extern "C" int gnx_tskit_drain(gnx_ctx* ctx, gnx_tskit_rows_t* rows) {
   rows->n_edges = h.n_edges;
   rows->n_births = h.n_born;
   return GNX_OK;
+}
+
+// ---- device assignment of the starting genomes (gnx_genome_init.cuh) ---------------------------
+// One histogram pass over the keys of every still-active locus; synchronises (the caller may sum the
+// histograms of several strips before the next gnx_genome_init_pass).
+static int gi_hist_pass(gnx_ctx* ctx) {
+  const int L = ctx->cfg.L;
+  cudaStream_t s = ctx->stream;
+  CK(cudaMemsetAsync(ctx->d_gi_hist, 0, (size_t)L * GI_BINS * sizeof(int32_t), s));
+  const int tiles = (L + GI_TILE - 1) / GI_TILE;
+  const long long n = std::max<long long>(ctx->n_hint, 1);
+  const int gx = (int)std::max<long long>(1, std::min<long long>((n + 2047) / 2048, (8ll * ctx->num_sms + tiles - 1) / tiles));
+  PROF(ctx, "k_gi_hist");
+  k_gi_hist<<<dim3(gx, tiles), 256, 0, s>>>(ctx->pop, ctx->d_c, ctx->d_gi_state, ctx->d_gi_lkey, ctx->d_gi_hist, L);
+  LAUNCHED(ctx);
+  CK(cudaStreamSynchronize(s));
+  return GNX_OK;
+}
+
+extern "C" int gnx_genome_init_begin(gnx_ctx* ctx, const gnx_genome_init_t* gi, void** dev_hist, int64_t* hist_len) {
+  ARG(ctx && gi && dev_hist && hist_len, "null");
+  const int L = ctx->cfg.L;
+  ARG(L > 0, "the context carries no genomes (L = 0)");
+  ARG(gi->n_loci == L, "n_loci differs from the L of the context");
+  ARG(gi->host_n_carriers, "host_n_carriers is required");
+  ARG(!(gi->tskit_rows && ctx->d_strip), "tskit rows are not supported under strip decomposition");
+  ARG((L + GI_TILE - 1) / GI_TILE <= 65535, "L too large for the device genome assignment");
+  USE_DEVICE(ctx);
+  int r = materialise(ctx);
+  if (r != GNX_OK) return r;
+  Counters h;
+  if ((r = read_counters(ctx, &h)) != GNX_OK) return r;
+  if ((r = check_device_err(h)) != GNX_OK) return r;
+  // a strip holds part of the species: its k_gi_select checks the counts against the summed histogram
+  for (int l = 0; l < L; ++l)
+    ARG(gi->host_n_carriers[l] >= 0 && (ctx->d_strip || gi->host_n_carriers[l] <= 2ll * h.n),
+        "n_carriers must lie in [0, 2n]");
+  ctx->gi_stage = 0;
+  free_bucket(ctx->gi_allocs);
+  ctx->d_gi_hist = nullptr;
+  long long* d_nc = nullptr;
+  uint8_t* d_sel = nullptr;
+  DM(ctx, &ctx->d_gi_state, (size_t)L, &ctx->gi_allocs);
+  DM(ctx, &ctx->d_gi_lkey, (size_t)L, &ctx->gi_allocs);
+  DM(ctx, &ctx->d_gi_write, (size_t)L, &ctx->gi_allocs);
+  DM(ctx, &ctx->d_gi_hist, (size_t)L * GI_BINS, &ctx->gi_allocs);
+  DM(ctx, &ctx->d_gi_active, (size_t)2, &ctx->gi_allocs);
+  DM(ctx, &d_nc, (size_t)L, &ctx->gi_allocs);
+  DM(ctx, &d_sel, (size_t)L, &ctx->gi_allocs);
+  ctx->gi_carriers.assign(gi->host_n_carriers, gi->host_n_carriers + L);
+  ctx->gi_tskit = gi->tskit_rows != 0;
+  // select: loci whose carriers are needed -- the written ones, and every locus for the tskit listing
+  std::vector<uint8_t> wr(L), sel(L);
+  for (int l = 0; l < L; ++l) {
+    wr[l] = gi->host_write_mask ? (gi->host_write_mask[l] ? 1 : 0) : 1;
+    sel[l] = ctx->gi_tskit ? 1 : wr[l];
+  }
+  cudaStream_t s = ctx->stream;
+  CK(cudaMemcpyAsync(d_nc, ctx->gi_carriers.data(), (size_t)L * 8, cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(d_sel, sel.data(), (size_t)L, cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(ctx->d_gi_write, wr.data(), (size_t)L, cudaMemcpyHostToDevice, s));
+  PROF(ctx, "k_gi_slots");
+  k_gi_slots<<<grid_for(ctx, 4), 256, 0, s>>>(ctx->pop, ctx->d_c);
+  LAUNCHED(ctx);
+  PROF(ctx, "k_gi_setup");
+  k_gi_setup<<<std::max(1, std::min((L + 255) / 256, grid_for(ctx, 4))), 256, 0, s>>>(
+      ctx->d_gi_state, ctx->d_gi_lkey, d_nc, d_sel, L, (uint32_t)gi->seed, (uint32_t)(gi->seed >> 32));
+  LAUNCHED(ctx);
+  if ((r = gi_hist_pass(ctx)) != GNX_OK) return r;
+  ctx->gi_stage = 1;
+  *dev_hist = ctx->d_gi_hist;
+  *hist_len = (int64_t)L * GI_BINS;
+  return GNX_OK;
+}
+
+extern "C" int gnx_genome_init_pass(gnx_ctx* ctx, int32_t* all_done) {
+  ARG(ctx && all_done, "null");
+  if (ctx->gi_stage != 1) { g_last_error = "gnx_genome_init_pass outside gnx_genome_init_begin / _end"; return GNX_ERR_STATE; }
+  USE_DEVICE(ctx);
+  cudaStream_t s = ctx->stream;
+  CK(cudaMemsetAsync(ctx->d_gi_active, 0, 2 * sizeof(int32_t), s));
+  PROF(ctx, "k_gi_select");
+  k_gi_select<<<ctx->cfg.L, 256, 0, s>>>(ctx->d_gi_state, ctx->d_gi_hist, ctx->d_gi_active);
+  LAUNCHED(ctx);
+  int32_t act[2];
+  CK(cudaMemcpyAsync(act, ctx->d_gi_active, sizeof act, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  if (act[1]) {
+    ctx->gi_stage = 0;
+    g_last_error = "invalid argument: n_carriers exceeds the 2n homologues of the population at some locus (or ids repeat)";
+    return GNX_ERR_ARG;
+  }
+  *all_done = act[0] == 0;
+  if (act[0]) return gi_hist_pass(ctx);
+  ctx->gi_stage = 3;                               // selected, not yet written
+  return GNX_OK;
+}
+
+extern "C" int gnx_genome_init_end(gnx_ctx* ctx) {
+  ARG(ctx, "null ctx");
+  if (ctx->gi_stage != 3) {
+    g_last_error = "gnx_genome_init_end before gnx_genome_init_pass reported every locus selected";
+    return GNX_ERR_STATE;
+  }
+  USE_DEVICE(ctx);
+  cudaStream_t s = ctx->stream;
+  PROF(ctx, "k_gi_write");
+  k_gi_write<<<grid_for(ctx, 8), 256, 0, s>>>(ctx->pop, ctx->d_c, ctx->d_gi_state, ctx->d_gi_lkey, ctx->d_gi_write,
+                                              ctx->cfg.L);
+  LAUNCHED(ctx);
+  if (ctx->cfg.n_traits > 0 && ctx->have_traits) {
+    int r = gnx_phenotype(ctx);
+    if (r != GNX_OK) return r;
+  }
+  Counters h;
+  int r = read_counters(ctx, &h);
+  if (r != GNX_OK) return r;
+  // the histograms are not needed any more (L x 8 KB)
+  auto it = std::find(ctx->gi_allocs.begin(), ctx->gi_allocs.end(), (void*)ctx->d_gi_hist);
+  if (it != ctx->gi_allocs.end()) ctx->gi_allocs.erase(it);
+  CK(cudaFree(ctx->d_gi_hist));
+  ctx->d_gi_hist = nullptr;
+  ctx->gi_stage = 2;
+  ctx->gi_t = h.t;
+  return check_device_err(h);
+}
+
+extern "C" int gnx_genome_init_rows(gnx_ctx* ctx, int32_t* host_site, int64_t* host_id, int8_t* host_homologue,
+                                    int64_t capacity, int64_t* n_rows) {
+  ARG(ctx && n_rows, "null");
+  USE_DEVICE(ctx);
+  Counters h;
+  int r = read_counters(ctx, &h);
+  if (r != GNX_OK) return r;
+  if (ctx->gi_stage != 2 || !ctx->gi_tskit || ctx->pending || h.t != ctx->gi_t) {
+    g_last_error = "gnx_genome_init_rows needs a finished assignment begun with tskit_rows, before any step";
+    return GNX_ERR_STATE;
+  }
+  const int L = ctx->cfg.L;
+  std::vector<long long> off(L + 1, 0);
+  for (int l = 0; l < L; ++l) off[l + 1] = off[l] + ctx->gi_carriers[l];
+  const long long total = off[L];
+  *n_rows = total;
+  if (!host_site && !host_id && !host_homologue) return GNX_OK;
+  ARG(host_site && host_id && host_homologue && capacity >= total, "host buffers missing or too small");
+  std::vector<void*> tmp;
+  long long* d_off = nullptr;
+  unsigned long long* d_cur = nullptr;
+  int32_t* d_site = nullptr;
+  long long* d_id = nullptr;
+  int8_t* d_h = nullptr;
+  auto run = [&]() -> int {
+    DM(ctx, &d_off, (size_t)L, &tmp);
+    DM(ctx, &d_cur, (size_t)L, &tmp);
+    DM(ctx, &d_site, (size_t)total, &tmp);
+    DM(ctx, &d_id, (size_t)total, &tmp);
+    DM(ctx, &d_h, (size_t)total, &tmp);
+    cudaStream_t s = ctx->stream;
+    CK(cudaMemcpyAsync(d_off, off.data(), (size_t)L * 8, cudaMemcpyHostToDevice, s));
+    PROF(ctx, "k_gi_rows");
+    k_gi_rows<<<grid_for(ctx, 8), 256, 0, s>>>(ctx->pop, ctx->d_c, ctx->d_gi_state, ctx->d_gi_lkey, d_off, d_cur,
+                                               d_site, d_id, d_h, L);
+    LAUNCHED(ctx);
+    CK(cudaMemcpyAsync(host_site, d_site, (size_t)total * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(host_id, d_id, (size_t)total * 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(host_homologue, d_h, (size_t)total, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return GNX_OK;
+  };
+  r = run();
+  free_bucket(tmp);
+  return r;
 }

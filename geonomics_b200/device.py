@@ -30,6 +30,14 @@ def _ptr(a, typ):
     return None if a is None else a.ctypes.data_as(typ)
 
 
+class _DevArray:
+    """A ctx-owned device array as a __cuda_array_interface__ object (zero-copy torch view)."""
+
+    def __init__(self, ptr, n, typestr):
+        self.__cuda_array_interface__ = {'shape': (int(n),), 'typestr': typestr, 'data': (int(ptr), False),
+                                         'version': 2, 'strides': None}
+
+
 class DeviceSpecies:
     """One Species resident on the GPU.
 
@@ -485,6 +493,71 @@ class DeviceSpecies:
         bufs['n'] = int(p.n)
         bufs['max_ind_idx'] = int(p.max_ind_idx)
         return bufs
+
+    # ---- device assignment of the starting genomes (gnx_genome_init_*) ----------------------
+    def genome_init_begin(self, n_carriers, seed, write_mask=None, tskit_rows=False):
+        """Start the staged assignment: exactly n_carriers[l] 1-alleles at locus l.  Returns the
+        int32[L * 2048] digit histogram of this context as a torch view (summed over the strips of a
+        decomposed landscape before every genome_init_pass)."""
+        import torch
+        nc = np.ascontiguousarray(n_carriers, dtype=np.int64)
+        gi = _lib.GenomeInit()
+        gi.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+        gi.n_loci = len(nc)
+        gi.host_n_carriers = _ptr(nc, _lib.c_int64_p)
+        wm = None
+        if write_mask is not None:
+            wm = np.ascontiguousarray(write_mask, dtype=np.uint8)
+            assert wm.shape == nc.shape, 'write_mask must hold one flag per locus'
+            gi.host_write_mask = wm.ctypes.data_as(C.POINTER(C.c_uint8))
+        gi.tskit_rows = int(bool(tskit_rows))
+        ptr, n = C.c_void_p(), C.c_int64()
+        _lib.check(self._L.gnx_genome_init_begin(self._ctx, C.byref(gi), C.byref(ptr), C.byref(n)),
+                   'gnx_genome_init_begin')
+        return torch.as_tensor(_DevArray(ptr.value, n.value, '<i4'), device='cuda')
+
+    def genome_init_pass(self):
+        """Select from the (summed) histogram; True when every locus is resolved."""
+        done = C.c_int32()
+        _lib.check(self._L.gnx_genome_init_pass(self._ctx, C.byref(done)), 'gnx_genome_init_pass')
+        return bool(done.value)
+
+    def genome_init_end(self):
+        _lib.check(self._L.gnx_genome_init_end(self._ctx), 'gnx_genome_init_end')
+
+    def genome_init_rows(self):
+        """(site, idx, homologue) of every starting carrier at every locus, sorted by (site, idx, homologue)."""
+        n = C.c_int64()
+        _lib.check(self._L.gnx_genome_init_rows(self._ctx, None, None, None, 0, C.byref(n)), 'gnx_genome_init_rows')
+        site, idx, hom = np.empty(n.value, np.int32), np.empty(n.value, np.int64), np.empty(n.value, np.int8)
+        _lib.check(self._L.gnx_genome_init_rows(self._ctx, _ptr(site, _lib.c_int32_p), _ptr(idx, _lib.c_int64_p),
+                                                _ptr(hom, _lib.c_int8_p), n.value, C.byref(n)), 'gnx_genome_init_rows')
+        o = np.lexsort((hom, idx, site))
+        return dict(site=site[o], idx=idx[o], homologue=hom[o])
+
+    def init_genomes(self, p, seed, write_mask=None, tskit_rows=False, allreduce=None):
+        """Assign the starting genomes on the device (the post-burn-in assignment of species.py:956-1094
+        without a host genotype array): locus l gets exactly genome_pack.carrier_counts(n, p)[l] 1-alleles,
+        on the homologues with the smallest Philox keys (include/gnx_b200.h).  write_mask [L]: loci whose
+        bits are set (the non-neutral loci of the tskit layout), None: all.  tskit_rows: return the
+        starting carriers of every locus (genome_init_rows).  allreduce: an in-place sum over the ranks of
+        a strip-decomposed landscape (e.g. torch.distributed.all_reduce) applied to the population size and
+        to the histograms, so every rank makes the same selection."""
+        import torch
+        n = self.population_size()
+        if allreduce is not None:
+            t = torch.tensor([n], dtype=torch.int64, device='cuda')
+            allreduce(t)
+            n = int(t.item())
+        hist = self.genome_init_begin(gp.carrier_counts(n, p), seed, write_mask, tskit_rows)
+        while True:
+            if allreduce is not None:
+                allreduce(hist)
+                torch.cuda.synchronize()
+            if self.genome_init_pass():
+                break
+        self.genome_init_end()
+        return self.genome_init_rows() if tskit_rows else None
 
     # ---- stepping ------------------------------------------------------------------------
     def step(self, n_steps=1, sync=False):

@@ -48,6 +48,17 @@ def pack_paths(paths):
     return pack_bits(bits).reshape(n, W)
 
 
+def carrier_counts(n, p):
+    """1-alleles per locus of a starting population of n individuals with allele frequencies p
+    (genome.py:1108-1157): round(2n p) (numpy's half-to-even), one fewer where that makes a locus fixed
+    although p < 1, one where it makes a locus lost although p > 0."""
+    p = np.asarray(p, dtype=np.float64)
+    c = np.round((2 * int(n)) * p, 0).astype(np.int64)
+    c[(c == 2 * int(n)) & (p < 1)] -= 1
+    c[(c == 0) & (p > 0)] = 1
+    return c
+
+
 def rows_to_loci(g_rows, nonneut_loci, L):
     """gen_arch.use_tskit = True (species.py:891-905): the reference's genotype arrays hold one ROW per
     non-neutral locus, int8[N, n_nonneut, 2].  The device keeps one bit per LOCUS: row r becomes locus

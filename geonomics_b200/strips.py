@@ -25,7 +25,8 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from .device import DeviceSpecies
+from . import genome_pack as gp
+from .device import DeviceSpecies, _DevArray
 
 
 # ---------------------------------------------------------------------------------------------
@@ -111,14 +112,6 @@ def merge_states(states):
 # ---------------------------------------------------------------------------------------------
 # one rank
 # ---------------------------------------------------------------------------------------------
-class _DevArray:
-    """A ctx-owned device array as a __cuda_array_interface__ object (zero-copy torch view)."""
-
-    def __init__(self, ptr, n, typestr):
-        self.__cuda_array_interface__ = {'shape': (int(n),), 'typestr': typestr, 'data': (int(ptr), False),
-                                         'version': 2, 'strides': None}
-
-
 class StripRank:
     """One rank's DeviceSpecies with strip decomposition enabled."""
 
@@ -224,6 +217,27 @@ class LocalStrips:
                 raise RuntimeError('strip rank %d: mutation log or tables differ from rank 0' % rank)
         return rows0, st0
 
+    def init_genomes(self, p, seed, write_mask=None):
+        """DeviceSpecies.init_genomes over the strips: the counts follow the species-wide size, the ranks'
+        histograms are summed between the passes and every rank makes the same selection, so the genomes
+        equal those of the undecomposed population."""
+        torch = self.torch
+        n = sum(self.population_sizes())
+        counts = gp.carrier_counts(n, p)
+        hists = [r.dev.genome_init_begin(counts, seed, write_mask) for r in self.ranks]
+        while True:
+            torch.cuda.synchronize()
+            tot = torch.stack(hists).sum(dim=0, dtype=torch.int32)
+            for h in hists:
+                h.copy_(tot)
+            torch.cuda.synchronize()
+            done = [r.dev.genome_init_pass() for r in self.ranks]
+            assert len(set(done)) == 1, 'strip ranks disagree on the genome selection'
+            if done[0]:
+                break
+        for r in self.ranks:
+            r.dev.genome_init_end()
+
     def upload(self, x, y, age=None, sex=None, idx=None, g=None, genomes_packed=None, max_ind_idx=None):
         n = len(x)
         idx = np.arange(n, dtype=np.int64) if idx is None else np.asarray(idx)
@@ -313,6 +327,7 @@ class NcclStrips:
         # (gnx_strip_barrier), never on the host
         self.device_barrier = True
         self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
+        self.group = group
         self.cs, self.ncx, self.ncy = mating_grid(land_dim, prm['mating_radius'])
         K = np.asarray(rasters)[int(prm.get('K_layer', 0))] * float(prm.get('K_factor', 1.0))
         self.bounds = plan_rows(self.ncy, self.world, row_weights_from_K(K, self.cs, self.ncy)) if bounds is None \
@@ -342,6 +357,12 @@ class NcclStrips:
     def read_mutations(self, max_rows=4096):
         """This rank's mutation log and tables, which equal every other rank's."""
         return self.me.dev.read_mutations(max_rows)
+
+    def init_genomes(self, p, seed, write_mask=None):
+        """DeviceSpecies.init_genomes on this rank with the size and the histograms summed over the ranks
+        (every rank makes the same call)."""
+        import torch.distributed as dist
+        self.me.dev.init_genomes(p, seed, write_mask, allreduce=lambda t: dist.all_reduce(t, group=self.group))
 
     def upload_owned(self, x, y, age=None, sex=None, idx=None, g=None, genomes_packed=None, max_ind_idx=None):
         """Upload this rank's share of a population every rank holds on the host."""

@@ -426,6 +426,40 @@ int gnx_read_mutations(gnx_ctx* ctx, gnx_mutation_row_t* rows, int32_t max_rows,
 int gnx_read_mutation_tables(gnx_ctx* ctx, int32_t trait, int32_t* n_loci, int32_t* host_loci, double* host_alpha,
                              int32_t* host_loci_idxs, int32_t* host_delet_loci_idxs);
 
+/* ---- device assignment of the starting genomes (species.py:956-1094, genome.py:1108-1157) -----------
+ * An alternative to uploading host-built genotypes after the burn-in.  Locus l gets exactly
+ * host_n_carriers[l] 1-alleles (the caller applies the reference's rounding rule to the species-wide
+ * live count n and the starting frequencies): homologue h of the individual with id i has the key
+ * K_l(i, h) = Philox2x32-10(counter 2i + h, key k_l), k_l derived from (seed, l), and the carriers of
+ * locus l are the n_l homologues with the smallest keys (keys never tie).  The genomes therefore depend
+ * only on the seed, the set of live ids and the counts -- not on the entry order or on a strip cut.
+ * The n_l-th smallest key is found by an MSB-first radix select (11 bits per pass) over keys that are
+ * regenerated in every pass; the passes are separate calls so that the ranks of a strip-decomposed
+ * landscape can sum their histograms (int32[L][2048]) between them:
+ *   gnx_genome_init_begin  applies pending deaths, gives every live individual its own genome row
+ *                          (burn-in newborns have none), counts the first digit; returns the histogram
+ *   gnx_genome_init_pass   selects from the (summed) histogram; counts the next digit unless *all_done
+ *   gnx_genome_init_end    after *all_done: writes every row (both homologues, padding zero, loci outside
+ *                          host_write_mask zero) and recomputes the phenotypes, as an upload does
+ *   gnx_genome_init_rows   tskit_rows only, before any step: (site, id, homologue) of every carrier at
+ *                          every locus with carriers, sum(n_carriers) rows grouped by site (order within
+ *                          a site unspecified); NULL arrays: *n_rows only
+ * Each call synchronises.  Every rank of a strip makes the same calls with the same arguments.  Refused
+ * (GNX_ERR_ARG): L = 0, n_loci != L, n_l outside [0, 2n], tskit_rows under strip decomposition. */
+typedef struct {
+  uint64_t seed;
+  int32_t n_loci;                     /* = L */
+  const int64_t* host_n_carriers;     /* [L] 1-alleles per locus */
+  const uint8_t* host_write_mask;     /* [L] loci whose bits are set (the non-neutral loci of the tskit
+                                         layout), or NULL: every locus */
+  int32_t tskit_rows;                 /* 1: keep the selection of every locus for gnx_genome_init_rows */
+} gnx_genome_init_t;
+int gnx_genome_init_begin(gnx_ctx* ctx, const gnx_genome_init_t* gi, void** dev_hist, int64_t* hist_len);
+int gnx_genome_init_pass(gnx_ctx* ctx, int32_t* all_done);
+int gnx_genome_init_end(gnx_ctx* ctx);
+int gnx_genome_init_rows(gnx_ctx* ctx, int32_t* host_site, int64_t* host_id, int8_t* host_homologue,
+                         int64_t capacity, int64_t* n_rows);
+
 /* ---- on-device statistics (sim/stats.py:399-435 _calc_het / _calc_maf / _calc_mean_fitness;
  *      SURVEY.md section 8f rank 2): per-locus 1-allele counts and heterozygote counts by
  *      vertical popcount over the packed genotypes, and the sum of fitness.  Synchronises. */

@@ -5,10 +5,12 @@ memory); rank 0 also runs the same population undecomposed and compares -- ids, 
 ages, genomes, phenotypes, fitness and the step records must be identical.
 
   python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 \
-      --master-port 29511 tools/strips_nccl_check.py [steps] [--mutation] [--poisson]
+      --master-port 29511 tools/strips_nccl_check.py [steps] [--mutation] [--poisson] [--genome-init]
 
 --mutation adds neutral + deleterious mutation (the mutation logs must be identical as well);
---poisson draws the births per pair from Poisson(2.5) instead of one per pair.
+--poisson draws the births per pair from Poisson(2.5) instead of one per pair;
+--genome-init assigns the starting genomes on the device (NcclStrips.init_genomes, histograms summed by
+all_reduce) instead of uploading them; they must equal the undecomposed assignment before the first step too.
 """
 import os
 import sys
@@ -20,6 +22,28 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, 'tests'))
 
 
+def _run_single_device_genomes(wl, steps, seed, mut, p, genome_seed):
+    """_run_single with the starting genomes assigned on the device instead of uploaded."""
+    from geonomics_b200.device import DeviceSpecies
+    dim, rasters, prm, ga, pop, _ = wl
+    dev = DeviceSpecies(dim, rasters, prm, ga, capacity=4 * len(pop['x']), seed=seed)
+    try:
+        dev.upload(pop['x'], pop['y'], pop['age'], pop['sex'], pop['idx'])
+        dev.init_genomes(p, genome_seed)
+        start = dev.download()
+        if mut:
+            dev.set_mutation(**mut)
+        out, logs = [], []
+        for _ in range(steps):
+            dev.step(1)
+            dev.sync()
+            out.append(dev.download())
+            logs.append(dev.read_mutations() if mut else None)
+        return dict(start=start, states=out, records=dev.step_records(), logs=logs)
+    finally:
+        dev.close()
+
+
 def main():
     import torch
     import torch.distributed as dist
@@ -29,6 +53,7 @@ def main():
     pos = [a for a in sys.argv[1:] if not a.startswith('--')]
     steps = int(pos[0]) if pos else 8
     mutation, poisson = '--mutation' in sys.argv, '--poisson' in sys.argv
+    genome_init = '--genome-init' in sys.argv
     rank, local = int(os.environ['RANK']), int(os.environ['LOCAL_RANK'])
     torch.cuda.set_device(local)
     dist.init_process_group('nccl', device_id=torch.device('cuda', local))
@@ -40,7 +65,14 @@ def main():
         wl = (dim, rasters, prm, ga, pop, g)
     mut = _mutation(wl, seed=5, mu=1e-5) if mutation else None
     st = strips.NcclStrips(dim, rasters, prm, ga, capacity=4 * len(pop['x']) // world + 4096, seed=77)
-    st.upload_owned(pop['x'], pop['y'], pop['age'], pop['sex'], pop['idx'], g=g)
+    p = np.random.default_rng(3).random(ga['L'])
+    start = None
+    if genome_init:
+        st.upload_owned(pop['x'], pop['y'], pop['age'], pop['sex'], pop['idx'])
+        st.init_genomes(p, 1234)
+        start = st.dev.download()
+    else:
+        st.upload_owned(pop['x'], pop['y'], pop['age'], pop['sex'], pop['idx'], g=g)
     if mut:
         st.set_mutation(**mut)
     st.step(steps)
@@ -49,14 +81,21 @@ def main():
     recs = st.step_records_local()
     log = st.read_mutations() if mut else None
     shares = [None] * world
-    dist.all_gather_object(shares, (mine, recs, log))
+    dist.all_gather_object(shares, (mine, recs, log, start))
     ok = True
     if rank == 0:
         got = strips.merge_states([s[0] for s in shares])
         got_recs = strips.merge_records([s[1] for s in shares])
-        single = _run_single(wl, steps, seed=77, mut=mut)
+        if genome_init:
+            single = _run_single_device_genomes(wl, steps, 77, mut, p, 1234)
+            got0 = strips.merge_states([s[3] for s in shares])
+            ok = all(np.array_equal(single['start'][k], got0[k]) for k in ('idx', 'g', 'z'))
+            print('starting genomes assigned on the device over %d GPUs: %s' % (
+                world, 'IDENTICAL to the undecomposed assignment' if ok else 'MISMATCH'), flush=True)
+        else:
+            single = _run_single(wl, steps, seed=77, mut=mut)
         ref, ref_recs = single['states'][-1], single['records']
-        ok = np.array_equal(ref['idx'], got['idx'])
+        ok = ok and np.array_equal(ref['idx'], got['idx'])
         for k in ('x', 'y', 'age', 'sex', 'g', 'z', 'fit'):
             ok = ok and np.array_equal(ref[k], got[k])
         ok = ok and all((a['Nt'], a['n_births'], a['n_deaths'], a['n_pairs']) ==
@@ -64,7 +103,7 @@ def main():
         if mut:
             ref_rows = [r for rows, _ in single['logs'] for r in rows]
             ref_state = single['logs'][-1][1]
-            for _, _, (rows, state) in shares:
+            for _, _, (rows, state), _ in shares:
                 ok = ok and rows == ref_rows and state['n_mutables'] == ref_state['n_mutables']
                 ok = ok and all(np.array_equal(state[k], ref_state[k]) for k in ('nonneut_loci', 'delet_loci', 'delet_s'))
         print('strips over %d GPUs (CUDA IPC peer writes; barriers and collectives by gnx_strip_barrier over '
