@@ -384,7 +384,7 @@ static int create_impl(const gnx_config_t* cfg, gnx_ctx* ctx) {
   DM(ctx, &W.d_rast, plane);
   DM(ctx, &W.e_out, (size_t)cap * cfg->n_layers);
   DM(ctx, &W.fix_list, plane);
-  DM(ctx, &W.fix_count, 1);
+  DM(ctx, &W.fix_count, 3);
   W.max_records = 1 << 16;
   DM(ctx, &W.records, (size_t)W.max_records);
   DM(ctx, &ctx->d_c, 1);
@@ -1727,9 +1727,9 @@ extern "C" int gnx_density_counts(gnx_ctx* ctx) {
   return GNX_OK;
 }
 
-// gnx_density_eval in two parts: the N raster (and its maximum), then the d raster that needs the
-// maximum -- under strip decomposition each rank evaluates its own landscape rows and the maximum
-// is reduced over the ranks in between
+// gnx_density_eval in two parts: both rasters in one pass and the exact-order N of the fix list, then the d
+// of the cells that need max(N) -- under strip decomposition each rank evaluates its own landscape rows and
+// the maximum is reduced over the ranks in between
 static void raster_grid(const gnx_ctx* ctx, int* row_lo, int* row_hi, int* rgrid) {
   *row_lo = ctx->d_strip ? ctx->strip_h.ly0 : 0;
   *row_hi = ctx->d_strip ? ctx->strip_h.ly1 : ctx->cfg.dim_y;
@@ -1740,7 +1740,7 @@ static void raster_grid(const gnx_ctx* ctx, int* row_lo, int* row_hi, int* rgrid
   *rgrid = (rows + rows_per_cta - 1) / rows_per_cta;
 }
 
-static int density_eval_N(gnx_ctx* ctx) {
+static int density_eval_rasters(gnx_ctx* ctx) {
   if (!ctx->have_density) { g_last_error = "density grids not set"; return GNX_ERR_STATE; }
   cudaStream_t s = ctx->stream;
   // scipy defaults reached through griddata: CloughTocher2DInterpolator(tol=1e-6, maxiter=400)
@@ -1757,29 +1757,22 @@ static int density_eval_N(gnx_ctx* ctx) {
   }
   LAUNCHED(ctx);
   PROF(ctx, "k_ct_coefficients");
-  k_ct_coefficients<<<std::max(1, (6 * ctx->dens.ntri + 127) / 128), 128, 0, s>>>(ctx->dens);
+  k_ct_coefficients<<<(2 * ctx->dens.ntri + CT_ITEMS - 1) / CT_ITEMS, CT_COEF_THREADS, 0, s>>>(ctx->dens);
   LAUNCHED(ctx);
-  CK(cudaMemsetAsync(ctx->work.fix_count, 0, sizeof(int32_t), s));
   int row_lo, row_hi, rgrid;
   raster_grid(ctx, &row_lo, &row_hi, &rgrid);
-  PROF(ctx, "k_raster_N");
-  k_raster_N<<<rgrid, 256, 0, s>>>(ctx->dens, ctx->land, ctx->work, ctx->d_c, row_lo, row_hi);
+  PROF(ctx, "k_raster_Nd");
+  k_raster_Nd<<<rgrid, 256, 0, s>>>(ctx->dens, ctx->land, ctx->prm, ctx->work, ctx->d_c, row_lo, row_hi);
   LAUNCHED(ctx);
-  PROF(ctx, "k_raster_N_fix");
-  k_raster_N_fix<<<grid_for(ctx, 2), 256, 0, s>>>(ctx->dens, ctx->land, ctx->work, ctx->d_c);
+  PROF(ctx, "k_raster_fix_N");
+  k_raster_fix_N<<<grid_for(ctx, 2), 256, 0, s>>>(ctx->dens, ctx->land, ctx->work, ctx->d_c);
   LAUNCHED(ctx);
   return GNX_OK;
 }
 
-static int density_eval_d(gnx_ctx* ctx) {
-  cudaStream_t s = ctx->stream;
-  int row_lo, row_hi, rgrid;
-  raster_grid(ctx, &row_lo, &row_hi, &rgrid);
-  PROF(ctx, "k_raster_d");
-  k_raster_d<<<rgrid, 256, 0, s>>>(ctx->dens, ctx->land, ctx->prm, ctx->work, ctx->d_c, row_lo, row_hi);
-  LAUNCHED(ctx);
-  PROF(ctx, "k_raster_d_fix");
-  k_raster_d_fix<<<grid_for(ctx, 2), 256, 0, s>>>(ctx->dens, ctx->land, ctx->prm, ctx->work, ctx->d_c);
+static int density_eval_deferred(gnx_ctx* ctx) {
+  PROF(ctx, "k_raster_fix_d");
+  k_raster_fix_d<<<grid_for(ctx, 2), 256, 0, ctx->stream>>>(ctx->dens, ctx->land, ctx->prm, ctx->work, ctx->d_c);
   LAUNCHED(ctx);
   return GNX_OK;
 }
@@ -1787,9 +1780,9 @@ static int density_eval_d(gnx_ctx* ctx) {
 extern "C" int gnx_density_eval(gnx_ctx* ctx) {
   ARG(ctx, "null ctx");
   USE_DEVICE(ctx);
-  int r = density_eval_N(ctx);
+  int r = density_eval_rasters(ctx);
   if (r != GNX_OK) return r;
-  return density_eval_d(ctx);
+  return density_eval_deferred(ctx);
 }
 
 static int death_prob(gnx_ctx* ctx, int end_step) {
@@ -1864,7 +1857,7 @@ static int one_step(gnx_ctx* ctx) {
   if (ctx->stream2 && !ctx->profiling && !(ctx->tsk.enabled && !ctx->burn)) {
     // Newborn records first (positions do not depend on genotypes), then two branches:
     //   stream  : gametes -> mutation -> birth bookkeeping
-    //   stream2 : density counts -> gradients -> Clough-Tocher coefficients -> N, d rasters
+    //   stream2 : gradients -> Clough-Tocher coefficients -> N and d rasters -> fix-list N -> fix and deferred d
     // The density chain is a string of small latency-bound kernels; it hides under the
     // genotype streaming.  They join before the death probabilities.
     if ((r = offspring_check(ctx))) return r;
@@ -2170,8 +2163,8 @@ static int strip_recv(gnx_ctx* ctx, int which, int mode) {
 //   3 receive choices; pair list; publish the births           | all-gather of `births`
 //   4 id base; offspring, mutation; route and send dispersed newborns | barrier
 //   5 receive newborns; density counts                         | all-reduce (sum) of `counts`
-//   6 N raster over the strip's rows                           | all-reduce (max) of `nmax`
-//   7 d raster; death probabilities and mortality draw; end of step
+//   6 N and d rasters over the strip's rows (d of the cells that need max(N) deferred) | all-reduce (max) of `nmax`
+//   7 deferred d cells; death probabilities and mortality draw; end of step
 // With Poisson births (n_births_fixed = 0) the births of a rank depend on the pairs of the lower ranks, so
 // phase 3 ends after the pair list and publishes the pairs, and a ninth phase follows the pairs all-gather:
 //   3 receive choices; pair list; publish the pairs            | all-gather of `pairs`
@@ -2231,9 +2224,9 @@ static int strip_phase_launch(gnx_ctx* ctx, int phase) {
       if ((r = strip_recv(ctx, STRIP_BUF_NEWBORNS, 1))) return r;
       return gnx_density_counts(ctx);
     case 6:
-      return density_eval_N(ctx);
+      return density_eval_rasters(ctx);
     case 7:
-      if ((r = density_eval_d(ctx))) return r;
+      if ((r = density_eval_deferred(ctx))) return r;
       if ((r = death_prob(ctx, 1))) return r;
       k_strip_end_step<<<1, 1, 0, s>>>(ctx->d_c);
       LAUNCHED(ctx);

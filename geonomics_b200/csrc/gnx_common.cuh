@@ -57,6 +57,7 @@ struct Counters {
   int64_t max_idx_base;     // species-wide max_ind_idx at the start of the step
   int32_t births_lo;        // births of the lower ranks: offspring number of this rank's first newborn
   int32_t births_all;       // births of the species
+  int32_t dens_lists[2];    // fix-list and deferred-list lengths of the last density evaluation (k_raster_fix_d)
 };
 #define GNX_ERRBIT_CAPACITY 1
 #define GNX_ERRBIT_DRAWS 2
@@ -184,8 +185,9 @@ struct Work {
   double* NP_rast;
   double* d_rast;
   double* e_out;
-  int32_t* fix_list;       // landscape cells whose N needs the exact-order re-evaluation
-  int32_t* fix_count;
+  int32_t* fix_list;       // [Y*X]: from the front the cells whose N needs the exact-order re-evaluation,
+                           // from the back the cells whose d waits for max(N) (k_raster_Nd)
+  int32_t* fix_count;      // [3]: both list lengths and k_raster_fix_d's last-block ticket; reset by that block
   gnx_step_record_t* records;
   int32_t max_records;
   void* scratch;           // species-order staging of one per-individual field (gnx_read_field)

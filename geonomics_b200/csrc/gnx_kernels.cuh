@@ -2039,12 +2039,20 @@ __global__ void __launch_bounds__(128) k_ct_setup_g(Dens d, double* tri_g) {
   }
 }
 
-// Bezier ordinates of every triangle (`_clough_tocher_2d_single`, point-independent part)
-__global__ void __launch_bounds__(128) k_ct_coefficients(Dens d) {
-  // 3 threads per (density, triangle): each converts the ordinates to one micro-triangle's monomials
-  const int total = 6 * d.ntri;
-  for (int id3 = GTID; id3 < total; id3 += GSTRIDE) {
-    const int id = id3 / 3, kpart = id3 - 3 * id;
+// Bezier ordinates of every triangle (`_clough_tocher_2d_single`, point-independent part) and the
+// monomial coefficients of its micro-triangles.  A CTA takes CT_ITEMS (density, triangle) items: one
+// thread per item computes the 19 ordinates once and stages them in shared memory, then every thread
+// runs ONE of the 30 coefficients' 19-term FMA chains for one item (the chain's order is fixed, so the
+// bits are).  Warp w owns coefficient w for all CT_ITEMS items, so its CT_MONO reads are warp-uniform
+// (constant-cache broadcasts) and its shared-memory reads are stride-1.
+#define CT_ITEMS 32
+#define CT_COEF_THREADS (30 * CT_ITEMS)
+__global__ void __launch_bounds__(CT_COEF_THREADS) k_ct_coefficients(Dens d) {
+  __shared__ double so[19][CT_ITEMS];
+  const int total = 2 * d.ntri;
+  const int base = blockIdx.x * CT_ITEMS;
+  if (threadIdx.x < CT_ITEMS && base + (int)threadIdx.x < total) {
+    const int id = base + threadIdx.x;
     const int which = id / d.ntri, t = id - which * d.ntri;
     const double* f = d.vals + (size_t)which * d.npts;
     const double* gr = d.grad + (size_t)which * d.npts * 2;
@@ -2083,21 +2091,22 @@ __global__ void __launch_bounds__(128) k_ct_coefficients(Dens d) {
     const double c0003 = (c1002 + c0102 + c0012) / 3;
     const double o[19] = {c3000, c0300, c0030, c0003, c2100, c2010, c2001, c0210, c0201, c0021,
                           c1200, c1020, c1002, c0120, c0102, c0012, c1101, c1011, c0111};
-    // Bezier ordinates -> monomial coefficients in (b0, b1) for each micro-triangle
-    double* mo = d.coef + ((size_t)which * d.ntri + t) * CT_STRIDE;
-    if (kpart == 0) {
+    double* mo = d.coef + (size_t)id * CT_STRIDE;
 #pragma unroll
-      for (int cidx = 0; cidx < 19; ++cidx) mo[30 + cidx] = o[cidx];
+    for (int cidx = 0; cidx < 19; ++cidx) {
+      mo[30 + cidx] = o[cidx];
+      so[cidx][threadIdx.x] = o[cidx];
     }
-    {
-      const int k = kpart;
-      for (int r = 0; r < 10; ++r) {
-        double acc = 0.0;
+  }
+  __syncthreads();
+  // Bezier ordinates -> monomial coefficients in (b0, b1): coefficient r of micro-triangle k is row
+  // k * 10 + r of CT_MONO
+  const int item = threadIdx.x % CT_ITEMS, row = threadIdx.x / CT_ITEMS;
+  if (base + item < total) {
+    double acc = 0.0;
 #pragma unroll
-        for (int cidx = 0; cidx < 19; ++cidx) acc = fma(CT_MONO[(k * 10 + r) * 19 + cidx], o[cidx], acc);
-        mo[k * 10 + r] = acc;
-      }
-    }
+    for (int cidx = 0; cidx < 19; ++cidx) acc = fma(CT_MONO[row * 19 + cidx], so[cidx][item], acc);
+    d.coef[(size_t)(base + item) * CT_STRIDE + row] = acc;
   }
 }
 
@@ -2153,7 +2162,13 @@ __device__ __forceinline__ int lattice_index(double q, double hww, double inv_hw
   return min(max(s, 0), smax);
 }
 
-__device__ __forceinline__ double ct_eval_point(const Dens& d, int which, double qi, double qj, int si, double inv_hww) {
+// the cell's place in the triangulation, shared by both densities: triangle t, micro-triangle k and
+// the barycentric coordinates (b0, b1)
+struct CtLoc {
+  int t, k;
+  double b0, b1;
+};
+__device__ __forceinline__ CtLoc ct_locate(const Dens& d, double qi, double qj, int si, double inv_hww) {
   const int sj = lattice_index(qj, d.hww, inv_hww, d.lat_nj - 2);
   const int2 st = __ldg(reinterpret_cast<const int2*>(d.square_tri) + (si * (d.lat_nj - 1) + sj));
   int t = st.x;
@@ -2169,7 +2184,12 @@ __device__ __forceinline__ double ct_eval_point(const Dens& d, int which, double
     b2 = 1.0 - b0 - b1;
   }
   const int k = (b0 <= b1 && b0 <= b2) ? 0 : ((b1 <= b2) ? 1 : 2);
-  const double* m = d.coef + ((size_t)which * d.ntri + t) * CT_STRIDE + k * 10;
+  return CtLoc{t, k, b0, b1};
+}
+
+__device__ __forceinline__ double ct_eval_at(const Dens& d, int which, const CtLoc& l) {
+  const double* m = d.coef + ((size_t)which * d.ntri + l.t) * CT_STRIDE + l.k * 10;
+  const double b0 = l.b0, b1 = l.b1;
   // order: 1, b1, b1^2, b1^3, b0, b0 b1, b0 b1^2, b0^2, b0^2 b1, b0^3
   const double r0 = fma(b1, fma(b1, fma(b1, m[3], m[2]), m[1]), m[0]);
   const double r1 = fma(b1, fma(b1, m[6], m[5]), m[4]);
@@ -2177,24 +2197,79 @@ __device__ __forceinline__ double ct_eval_point(const Dens& d, int which, double
   return fma(b0, fma(b0, fma(b0, m[9], r2), r1), r0);
 }
 
-// N raster (Species._calc_density species.py:845-882, clip >= 0) + its maximum
-// (rows are dealt to CTAs, columns to threads: no integer division per cell, the lattice row
-// index is computed once per row)
-__global__ void __launch_bounds__(256) k_raster_N(Dens d, Land land, Work w, Counters* c, int row_lo, int row_hi) {
+__device__ __forceinline__ double ct_eval_point(const Dens& d, int which, double qi, double qj, int si, double inv_hww) {
+  return ct_eval_at(d, which, ct_locate(d, qi, qj, si, inv_hww));
+}
+
+// a7 + a14: n_pairs raster (demography.py:60-91) and the logistic d raster
+// (demography.py:104-172), never materialising dNdt / N_b / N_d.
+__device__ __forceinline__ double raster_np(const Params& prm, const Work& w, int id, double np) {
+  np = np < 0.0 ? 0.0 : np;
+  if (isnan(np)) np = 0.0;
+  if (prm.store_debug) w.NP_rast[id] = np;
+  return np;
+}
+
+__device__ __forceinline__ void raster_d_store(const Params& prm, const Work& w, int id, double np, double N,
+                                               double dNdt) {
+  const double N_b = prm.c.b * prm.c.n_births_lambda * np;     // demography.py:142
+  const double N_d = N_b - dNdt;                    // demography.py:149
+  double dv = N_d / N;                              // demography.py:159-160
+  if (isnan(dv)) dv = 0.0;
+  dv = dv < prm.c.d_min ? prm.c.d_min : (dv > prm.c.d_max ? prm.c.d_max : dv);
+  w.d_rast[id] = dv;                                // its own plane: a full-sector streaming write
+}
+
+__device__ __forceinline__ void raster_d_cell(const Land& land, const Params& prm, const Work& w, int id,
+                                              double np, double Nmax) {
+  np = raster_np(prm, w, id, np);
+  const double N = w.N_rast[id], K = land.K[id];
+  double dNdt = prm.c.R * (1 - (N / K)) * N;        // demography.py:95-97
+  if (dNdt < -Nmax) dNdt = -Nmax;                   // np.clip(a_min=-N.max())
+  if (isnan(dNdt) || isinf(dNdt)) dNdt = -Nmax;
+  raster_d_store(prm, w, id, np, N, dNdt);
+}
+
+// The d of a cell needs max(N) only through the clip of dNdt at -Nmax.  Nmax >= N (N is one of the
+// values it is the maximum of, and under strips it is also reduced over the ranks), so when dNdt is
+// finite and >= -N neither clip can fire and d is final without Nmax.  Returns false for the other
+// cells (K = 0, N > K (1 + 1/R), NaN): they are deferred to k_raster_fix_d.
+__device__ __forceinline__ bool raster_d_cell_no_clip(const Land& land, const Params& prm, const Work& w, int id,
+                                                      double np, double N) {
+  const double K = land.K[id];
+  const double dNdt = prm.c.R * (1 - (N / K)) * N;
+  if (!(isfinite(dNdt) && dNdt >= -N)) return false;
+  raster_d_store(prm, w, id, raster_np(prm, w, id, np), N, dNdt);
+  return true;
+}
+
+// Both rasters in one pass over the landscape (Species._calc_density species.py:845-882 for N, clip
+// >= 0, and the d raster), plus max(N).  Each cell is located once and both interpolants are
+// evaluated there.  Two lists share Work.fix_list: from the front the cells whose N is at
+// rounding-noise level, from the back the cells whose d waits for max(N) (raster_d_cell_no_clip).
+// Rows are dealt to CTAs, columns to threads: no integer division per cell, the lattice row index is
+// computed once per row.
+__global__ void __launch_bounds__(256) k_raster_Nd(Dens d, Land land, Params prm, Work w, Counters* c, int row_lo,
+                                                    int row_hi) {
   double mx = 0.0;
   const double inv_hww = 1.0 / d.hww;
+  const int last = land.X * land.Y - 1;
   for (int i = row_lo + blockIdx.x; i < row_hi; i += gridDim.x) {
    const int si = lattice_index(i + 0.5, d.hww, inv_hww, d.lat_ni - 2);
    for (int j = threadIdx.x; j < land.X; j += blockDim.x) {
     const int id = i * land.X + j;
-    double v = ct_eval_point(d, 0, i + 0.5, j + 0.5, si, inv_hww);
+    const CtLoc loc = ct_locate(d, i + 0.5, j + 0.5, si, inv_hww);
+    double v = ct_eval_at(d, 0, loc);
+    const double np = ct_eval_at(d, 1, loc);
     // where the interpolant is at rounding-noise level its sign / exact zero-ness is what
     // d = N_d / N amplifies: those cells are re-evaluated in scipy's exact operation order
-    // by k_raster_N_fix (none in a populated landscape)
-    if (fabs(v) < 1e-7) w.fix_list[atomicAdd(w.fix_count, 1)] = id;
+    // by k_raster_fix_N and k_raster_fix_d (none in a populated landscape)
+    const bool fix = fabs(v) < 1e-7;
+    if (fix) w.fix_list[atomicAdd(&w.fix_count[0], 1)] = id;
     v = v < 0.0 ? 0.0 : v;                    // np.clip(dens, a_min=0)
     w.N_rast[id] = v;
     mx = fmax(mx, v);
+    if (!fix && !raster_d_cell_no_clip(land, prm, w, id, np, v)) w.fix_list[last - atomicAdd(&w.fix_count[1], 1)] = id;
    }
   }
 #pragma unroll
@@ -2202,8 +2277,9 @@ __global__ void __launch_bounds__(256) k_raster_N(Dens d, Land land, Work w, Cou
   if ((threadIdx.x & 31) == 0 && mx > 0.0) atomicMax(&c->nmax_bits, (unsigned long long)__double_as_longlong(mx));
 }
 
-__global__ void __launch_bounds__(256) k_raster_N_fix(Dens d, Land land, Work w, Counters* c) {
-  const int nfix = *w.fix_count;
+// exact-order N of the fix list, and their part of max(N)
+__global__ void __launch_bounds__(256) k_raster_fix_N(Dens d, Land land, Work w, Counters* c) {
+  const int nfix = w.fix_count[0];
   double mx = 0.0;
   for (int k = GTID; k < nfix; k += GSTRIDE) {
     const int id = w.fix_list[k];
@@ -2218,46 +2294,36 @@ __global__ void __launch_bounds__(256) k_raster_N_fix(Dens d, Land land, Work w,
   if ((threadIdx.x & 31) == 0 && mx > 0.0) atomicMax(&c->nmax_bits, (unsigned long long)__double_as_longlong(mx));
 }
 
-// a7 + a14: n_pairs raster (demography.py:60-91) and the logistic d raster
-// (demography.py:104-172), never materialising dNdt / N_b / N_d.
-__device__ __forceinline__ void raster_d_cell(const Land& land, const Params& prm, const Work& w, int id,
-                                              double np, double Nmax) {
-  np = np < 0.0 ? 0.0 : np;
-  if (isnan(np)) np = 0.0;
-  if (prm.store_debug) w.NP_rast[id] = np;
-  const double N = w.N_rast[id], K = land.K[id];
-  double dNdt = prm.c.R * (1 - (N / K)) * N;        // demography.py:95-97
-  if (dNdt < -Nmax) dNdt = -Nmax;                   // np.clip(a_min=-N.max())
-  if (isnan(dNdt) || isinf(dNdt)) dNdt = -Nmax;
-  const double N_b = prm.c.b * prm.c.n_births_lambda * np;     // demography.py:142
-  const double N_d = N_b - dNdt;                    // demography.py:149
-  double dv = N_d / N;                              // demography.py:159-160
-  if (isnan(dv)) dv = 0.0;
-  dv = dv < prm.c.d_min ? prm.c.d_min : (dv > prm.c.d_max ? prm.c.d_max : dv);
-  w.d_rast[id] = dv;                                // its own plane: a full-sector streaming write
-}
-
-__global__ void __launch_bounds__(256) k_raster_d(Dens d, Land land, Params prm, Work w, const Counters* c, int row_lo,
-                                                   int row_hi) {
+// d of both lists with the final max(N).  On the fix list d = N_d / N turns the noise of the
+// pair-density interpolant into 0 or 1, so it too is evaluated in scipy's exact operation order;
+// the deferred cells evaluate it as k_raster_Nd did.  The last CTA to finish keeps the list lengths
+// in Counters.dens_lists and resets the list cursors for the next evaluation.
+__global__ void __launch_bounds__(256) k_raster_fix_d(Dens d, Land land, Params prm, Work w, Counters* c) {
+  const int nfix = w.fix_count[0], ndef = w.fix_count[1];
+  const int last = land.X * land.Y - 1;
   const double Nmax = __longlong_as_double((long long)c->nmax_bits);
   const double inv_hww = 1.0 / d.hww;
-  for (int i = row_lo + blockIdx.x; i < row_hi; i += gridDim.x) {
-    const int si = lattice_index(i + 0.5, d.hww, inv_hww, d.lat_ni - 2);
-    for (int j = threadIdx.x; j < land.X; j += blockDim.x)
-      raster_d_cell(land, prm, w, i * land.X + j, ct_eval_point(d, 1, i + 0.5, j + 0.5, si, inv_hww), Nmax);
-  }
-}
-
-// cells whose density is at rounding-noise level (fix_list, built by k_raster_N): there
-// d = N_d / N turns the noise of the pair-density interpolant into 0 or 1, so it too is
-// evaluated in scipy's exact operation order
-__global__ void __launch_bounds__(256) k_raster_d_fix(Dens d, Land land, Params prm, Work w, const Counters* c) {
-  const int nfix = *w.fix_count;
-  const double Nmax = __longlong_as_double((long long)c->nmax_bits);
   for (int k = GTID; k < nfix; k += GSTRIDE) {
     const int id = w.fix_list[k];
     const int i = id / land.X, j = id - i * land.X;
     raster_d_cell(land, prm, w, id, ct_eval_exact(d, 1, i + 0.5, j + 0.5), Nmax);
+  }
+  for (int k = GTID; k < ndef; k += GSTRIDE) {
+    const int id = w.fix_list[last - k];
+    const int i = id / land.X, j = id - i * land.X;
+    const int si = lattice_index(i + 0.5, d.hww, inv_hww, d.lat_ni - 2);
+    raster_d_cell(land, prm, w, id, ct_eval_point(d, 1, i + 0.5, j + 0.5, si, inv_hww), Nmax);
+  }
+  __shared__ bool is_last;
+  __syncthreads();
+  if (threadIdx.x == 0) is_last = atomicAdd(reinterpret_cast<unsigned int*>(&w.fix_count[2]), 1u) == gridDim.x - 1;
+  __syncthreads();
+  if (is_last && threadIdx.x == 0) {
+    c->dens_lists[0] = nfix;
+    c->dens_lists[1] = ndef;
+    w.fix_count[0] = 0;
+    w.fix_count[1] = 0;
+    w.fix_count[2] = 0;
   }
 }
 
@@ -2295,7 +2361,7 @@ __global__ void __launch_bounds__(256, GNX_DEATH_MINB) k_death(Pop pop, Land lan
     const size_t cell = (size_t)cy * land.X + cx;
     // d and the environment layers are read as planes: with the state in mating-grid order a warp's
     // 32 individuals sit in a few neighbouring landscape cells, so the plane reads share sectors,
-    // and the d raster is written by k_raster_d as whole sectors (interleaved with the environment
+    // and the d raster is written by k_raster_Nd as whole sectors (interleaved with the environment
     // values it was a read-modify-write of 8 bytes in every 24: 2.6x its algorithmic traffic)
     const size_t plane_sz = (size_t)land.X * land.Y;
     double p = w.d_rast[cell];                                     // demography.py:306

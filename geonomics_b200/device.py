@@ -681,7 +681,7 @@ class DeviceSpecies:
         return out
 
     def counters(self):
-        c = self.read('COUNTERS', 24)
+        c = self.read('COUNTERS', 48)
         names = ['n', 'n_pre', 'P', 'B', 'deaths', 'n_free', 'n_slots', 'cur']
         out = {k: int(c[i]) for i, k in enumerate(names)}
         out['max_idx'] = int(c[8:10].view(np.int64)[0])
@@ -689,6 +689,9 @@ class DeviceSpecies:
         out['err'] = int(c[12])
         out['n_rec'] = int(c[13])
         out['gs_iters'] = (int(c[14]), int(c[15]))
+        # lengths of the fix list (exact-order cells) and the deferred list (d waits for max(N)) of the last
+        # density evaluation
+        out['density_lists'] = (int(c[46]), int(c[47]))
         return out
 
     def read(self, field, count):
