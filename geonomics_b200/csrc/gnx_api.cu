@@ -96,7 +96,6 @@ struct gnx_ctx {
   bool have_density = false, have_paths = false, have_traits = false, have_rasters = false;
   int64_t launches = 0;
   int burn = 0;
-  int host_n_hint = 0;
   bool gs_attr_set = false;
   bool capturing = false;               // inside cudaStreamBeginCapture/EndCapture of the whole-step graph
   bool pending = false;                 // host mirror of Counters.pending (set by the fused step, cleared by materialise / upload)
@@ -157,25 +156,12 @@ static inline int grid_cap(const gnx_ctx* ctx, int per_sm, int threads, double s
   if (ctx->n_hint <= 0) return (int)hi;
   return (int)std::max<long long>(ctx->num_sms, std::min(hi, want));
 }
-// experiment knobs: CTAs per SM of the grid-stride kernels whose per-item cost varies
-#ifndef GNX_G_AGE
-#define GNX_G_AGE 8
-#endif
-#ifndef GNX_G_NEWB
-#define GNX_G_NEWB 8
-#endif
-#ifndef GNX_G_DEATH
-#define GNX_G_DEATH 32
-#endif
-#ifndef GNX_G_SORT
-#define GNX_G_SORT 8
-#endif
-#ifndef GNX_G_GATHER
-#define GNX_G_GATHER 8
-#endif
-#ifndef GNX_G_SCAN
-#define GNX_G_SCAN 8
-#endif
+// CTAs per SM of grid-stride kernels whose per-item cost varies
+constexpr int MOVE_KEY_GRID = 8;     // k_move_key
+constexpr int NEWBORNS_GRID = 8;     // k_newborns
+constexpr int DEATH_GRID = 32;       // k_death
+constexpr int REGRID_GRID = 8;       // k_bucket, k_regrid
+constexpr int SCAN_GRID = 8;         // scan_reduce_kernel, scan_apply_kernel
 
 // ---- optional per-kernel timing (bench.py roofline): CUDA events on the ctx stream around
 // every launch, accumulated by kernel name.
@@ -359,7 +345,7 @@ static int create_impl(const gnx_config_t* cfg, gnx_ctx* ctx) {
     W.scratch = sc;
   }
   DM(ctx, &W.mate, cap);
-  // a cell is crowded when focals x candidates of its 3x3 block reaches GNX_FM_HEAVY_WORK; it
+  // a cell is crowded when focals x candidates of its 3x3 block reaches FM_HEAVY_WORK; it
   // contributes one work item per 32 focals, so n / 32 items plus one per crowded cell (few
   // hundred candidates are shared by the at most 9 cells around them): below n / 4 in all
   W.heavy_cap = (int32_t)(cap / 4 + 1024);
@@ -1090,7 +1076,6 @@ static int upload_population(gnx_ctx* ctx, const gnx_population_t* pop, bool wai
     if (r != GNX_OK) return r;
   }
   if (wait) CK(cudaStreamSynchronize(s));
-  ctx->host_n_hint = (int)n;
   return GNX_OK;
 }
 
@@ -1173,12 +1158,12 @@ static int run_scan(gnx_ctx* ctx, F f, const char* name) {
   char nm[64];
   snprintf(nm, sizeof nm, "%s.reduce", name);
   PROF(ctx, nm);
-  scan_reduce_kernel<F><<<grid_for(ctx, GNX_G_SCAN), SCAN_BLOCK, 0, s>>>(f, ctx->d_c, ctx->work.tile_sums,
-                                                                ctx->work.scan_ticket);
+  scan_reduce_kernel<F><<<grid_for(ctx, SCAN_GRID), SCAN_BLOCK, 0, s>>>(f, ctx->d_c, ctx->work.tile_sums,
+                                                                       ctx->work.scan_ticket);
   LAUNCHED(ctx);
   snprintf(nm, sizeof nm, "%s.apply", name);
   PROF(ctx, nm);
-  scan_apply_kernel<F><<<grid_for(ctx, GNX_G_SCAN), SCAN_BLOCK, 0, s>>>(f, ctx->d_c, ctx->work.tile_sums);
+  scan_apply_kernel<F><<<grid_for(ctx, SCAN_GRID), SCAN_BLOCK, 0, s>>>(f, ctx->d_c, ctx->work.tile_sums);
   LAUNCHED(ctx);
   return GNX_OK;
 }
@@ -1200,8 +1185,9 @@ static int move_key(gnx_ctx* ctx, int do_age, int do_move, int do_key) {
     return GNX_ERR_STATE;
   }
   PROF(ctx, "k_move_key");
-  k_move_key<<<grid_for(ctx, GNX_G_AGE), 256, 0, ctx->stream>>>(ctx->pop, ctx->land, ctx->prm, ctx->draws, ctx->work,
-                                                       ctx->d_c, do_age, do_move, do_key, ctx->d_strip);
+  k_move_key<<<grid_for(ctx, MOVE_KEY_GRID), 256, 0, ctx->stream>>>(ctx->pop, ctx->land, ctx->prm, ctx->draws,
+                                                                    ctx->work, ctx->d_c, do_age, do_move, do_key,
+                                                                    ctx->d_strip);
   LAUNCHED(ctx);
   return GNX_OK;
 }
@@ -1230,10 +1216,10 @@ static int finish_regrid(gnx_ctx* ctx, int age_inc) {
   if (r != GNX_OK) return r;
   cudaStream_t s = ctx->stream;
   PROF(ctx, "k_bucket");
-  k_bucket<<<grid_for(ctx, GNX_G_GATHER), 256, 0, s>>>(ctx->pop, ctx->land, ctx->work, ctx->d_c);
+  k_bucket<<<grid_for(ctx, REGRID_GRID), 256, 0, s>>>(ctx->pop, ctx->land, ctx->work, ctx->d_c);
   LAUNCHED(ctx);
   PROF(ctx, "k_regrid");
-  k_regrid<<<grid_for(ctx, GNX_G_GATHER), 256, 0, s>>>(ctx->pop, ctx->land, ctx->work, ctx->d_c, age_inc,
+  k_regrid<<<grid_for(ctx, REGRID_GRID), 256, 0, s>>>(ctx->pop, ctx->land, ctx->work, ctx->d_c, age_inc,
                                                       ctx->prm.ordered, ctx->d_strip);
   LAUNCHED(ctx);
   return GNX_OK;
@@ -1260,6 +1246,18 @@ extern "C" int gnx_find_mates(gnx_ctx* ctx) {
   return find_mates(ctx);
 }
 
+// Bernoulli(b) first: list the focals that may mate (and announce the crowded cells' work items),
+// then search the listed focals' neighbours on a grid of g CTAs
+template <int MODE>
+static int launch_mate_search(gnx_ctx* ctx, int g) {
+  k_mate_select<MODE><<<grid_for(ctx, 8), 256, 0, ctx->stream>>>(ctx->pop, ctx->land, ctx->prm, ctx->draws, ctx->work,
+                                                                  ctx->d_c);
+  LAUNCHED(ctx);
+  k_find_mates<MODE><<<g, FM_BLOCK, 0, ctx->stream>>>(ctx->pop, ctx->land, ctx->prm, ctx->draws, ctx->work, ctx->d_c);
+  LAUNCHED(ctx);
+  return GNX_OK;
+}
+
 static int find_mates(gnx_ctx* ctx) {
   if (ctx->cfg.mating_radius <= 0) {          // mating_radius = None: Wright-Fisher style panmixia
     PROF(ctx, "k_panmixia");
@@ -1267,39 +1265,26 @@ static int find_mates(gnx_ctx* ctx) {
     LAUNCHED(ctx);
     return GNX_OK;
   }
+  constexpr int FM_GRID = 128, FMD_GRID = 6;   // CTAs per SM of k_find_mates (at most) and k_find_mates_dense
   PROF(ctx, "k_find_mates");
-#ifndef GNX_FM_GRID
-#define GNX_FM_GRID 128
-#endif
-#ifndef GNX_FM_BLOCK
-#define GNX_FM_BLOCK 128
-#endif
-#ifndef GNX_FMD_GRID
-#define GNX_FMD_GRID 6
-#endif
   // the thread-per-focal search walks the list of focals that may mate: a fraction b of the population
-  const int g = grid_cap(ctx, GNX_FM_GRID, GNX_FM_BLOCK, ctx->prm.store_debug ? 1.0 : std::min(1.0, ctx->cfg.b + 0.05));
-  const bool uniform_choice = !ctx->cfg.choose_nearest && !ctx->cfg.inverse_dist;
-  if (uniform_choice)     // n_heavy, heavy_next: the crowded-cell list starts empty
+  const int g = grid_cap(ctx, FM_GRID, FM_BLOCK, ctx->prm.store_debug ? 1.0 : std::min(1.0, ctx->cfg.b + 0.05));
+  // MODE of the search kernels: 0 uniform random neighbour, 1 nearest, 2 inverse-distance weighting
+  const int mode = ctx->cfg.choose_nearest ? 1 : ctx->cfg.inverse_dist ? 2 : 0;
+  if (mode == 0)     // n_heavy, heavy_next: the crowded-cell list starts empty
     CK(cudaMemsetAsync(&ctx->d_c->n_heavy, 0, 2 * sizeof(int32_t), ctx->stream));
   CK(cudaMemsetAsync(ctx->work.fm_count, 0, sizeof(int32_t), ctx->stream));
-  // Bernoulli(b) first: list the focals that may mate (and announce the crowded cells' work items)
-#define FS(MODE) k_mate_select<MODE><<<grid_for(ctx, 8), 256, 0, ctx->stream>>>(ctx->pop, ctx->land, ctx->prm, ctx->draws, ctx->work, ctx->d_c)
-  if (ctx->cfg.choose_nearest) FS(1);
-  else if (ctx->cfg.inverse_dist) FS(2);
-  else FS(0);
-#undef FS
-  LAUNCHED(ctx);
-#define FM(MODE) k_find_mates<MODE><<<g, GNX_FM_BLOCK, 0, ctx->stream>>>(ctx->pop, ctx->land, ctx->prm, ctx->draws, ctx->work, ctx->d_c)
-  if (ctx->cfg.choose_nearest) FM(1);
-  else if (ctx->cfg.inverse_dist) FM(2);
-  else FM(0);
-#undef FM
-  LAUNCHED(ctx);
-  if (uniform_choice) {
+  int r;
+  switch (mode) {
+    case 1: r = launch_mate_search<1>(ctx, g); break;
+    case 2: r = launch_mate_search<2>(ctx, g); break;
+    default: r = launch_mate_search<0>(ctx, g); break;
+  }
+  if (r != GNX_OK) return r;
+  if (mode == 0) {
     PROF(ctx, "k_find_mates_dense");
-    k_find_mates_dense<<<grid_for(ctx, GNX_FMD_GRID), 32 * FMD_WARPS, 0, ctx->stream>>>(ctx->pop, ctx->land, ctx->prm,
-                                                                                   ctx->draws, ctx->work, ctx->d_c);
+    k_find_mates_dense<<<grid_for(ctx, FMD_GRID), 32 * FMD_WARPS, 0, ctx->stream>>>(ctx->pop, ctx->land, ctx->prm,
+                                                                               ctx->draws, ctx->work, ctx->d_c);
     LAUNCHED(ctx);
   }
   return GNX_OK;
@@ -1345,36 +1330,36 @@ static int offspring_check(gnx_ctx* ctx) {
   return GNX_OK;
 }
 
-static int offspring_gametes(gnx_ctx* ctx) {
-  cudaStream_t s = ctx->stream;
-  const int Wq = ctx->Wq;
+// k_gametes with GW lanes per offspring (fnb: births per pair when fixed, else 0)
+template <int GW>
+static void launch_gametes(gnx_ctx* ctx, int fnb) {
   const int g = grid_for(ctx, 8);
+  // child rows staged in shared memory for the phenotype when they fit (32 KB per block)
+  const size_t rows_b = (size_t)(256 / GW) * 2 * ctx->Wq * 16;
+  int stage = (GW > 1 && ctx->cfg.n_traits > 0 && rows_b <= 32 * 1024) ? 1 : 0;
+  // 2 = two staged rows per group and one trait-table walk for both: every trait polygenic, no dominance
+  constexpr int NB = (GAM_NB < GW) ? GAM_NB : GW;
+  if (stage && NB >= 2 && NB * rows_b <= 44 * 1024 && ctx->pair_phenotype) stage = NB;
+  const size_t smem = stage ? stage * rows_b : 0;
+  if (ctx->cfg.n_traits <= 2)
+    k_gametes<GW, 2><<<g, 256, smem, ctx->stream>>>(ctx->pop, ctx->prm, ctx->traits, ctx->draws, ctx->work, ctx->d_c,
+                                                    fnb, stage);
+  else
+    k_gametes<GW, GNX_MAX_TRAITS><<<g, 256, smem, ctx->stream>>>(ctx->pop, ctx->prm, ctx->traits, ctx->draws,
+                                                                 ctx->work, ctx->d_c, fnb, stage);
+}
+
+static int offspring_gametes(gnx_ctx* ctx) {
   if (!ctx->burn) {
-#define MO(GW)                                                                                            \
-  do {                                                                                                    \
-    /* child rows staged in shared memory for the phenotype when they fit (32 KB per block) */           \
-    const size_t rows_b = (size_t)(256 / GW) * 2 * Wq * 16;                                               \
-    /* 2 = two staged rows per group and one trait-table walk for both: every trait polygenic, no dominance */  \
-    int stage = (GW > 1 && ctx->cfg.n_traits > 0 && rows_b <= 32 * 1024) ? 1 : 0;                         \
-    { constexpr int NB = (GNX_GAM_NB < GW) ? GNX_GAM_NB : GW;                                              \
-      if (stage && NB >= 2 && NB * rows_b <= 44 * 1024 && ctx->pair_phenotype) stage = NB; }              \
-    if (ctx->cfg.n_traits <= 2)                                                                           \
-      k_gametes<GW, 2><<<g, 256, stage ? stage * rows_b : 0, s>>>(ctx->pop, ctx->prm, ctx->traits, ctx->draws,   \
-                                                          ctx->work, ctx->d_c, fnb, stage);               \
-    else                                                                                                  \
-      k_gametes<GW, GNX_MAX_TRAITS><<<g, 256, stage ? stage * rows_b : 0, s>>>(ctx->pop, ctx->prm, ctx->traits,  \
-                                                                       ctx->draws, ctx->work, ctx->d_c,   \
-                                                                       fnb, stage);                       \
-  } while (0)
+    const int Wq = ctx->Wq;
     const int fnb = ctx->cfg.n_births_fixed ? (int)ctx->cfg.n_births_lambda : 0;
     PROF(ctx, "k_gametes");
-    if (Wq <= 1) MO(1);
-    else if (Wq <= 2) MO(2);
-    else if (Wq <= 4) MO(4);
-    else if (Wq <= 8) MO(8);
-    else if (Wq <= 16) MO(16);
-    else MO(32);
-#undef MO
+    if (Wq <= 1) launch_gametes<1>(ctx, fnb);
+    else if (Wq <= 2) launch_gametes<2>(ctx, fnb);
+    else if (Wq <= 4) launch_gametes<4>(ctx, fnb);
+    else if (Wq <= 8) launch_gametes<8>(ctx, fnb);
+    else if (Wq <= 16) launch_gametes<16>(ctx, fnb);
+    else launch_gametes<32>(ctx, fnb);
     LAUNCHED(ctx);
   }
   return GNX_OK;
@@ -1382,8 +1367,8 @@ static int offspring_gametes(gnx_ctx* ctx) {
 
 static int offspring_newborns(gnx_ctx* ctx) {
   PROF(ctx, "k_newborns");
-  k_newborns<<<grid_for(ctx, GNX_G_NEWB), 256, 0, ctx->stream>>>(ctx->pop, ctx->land, ctx->prm, ctx->draws, ctx->work,
-                                                        ctx->d_c, ctx->tsk);
+  k_newborns<<<grid_for(ctx, NEWBORNS_GRID), 256, 0, ctx->stream>>>(ctx->pop, ctx->land, ctx->prm, ctx->draws,
+                                                                    ctx->work, ctx->d_c, ctx->tsk);
   LAUNCHED(ctx);
   return GNX_OK;
 }
@@ -1787,7 +1772,7 @@ extern "C" int gnx_density_eval(gnx_ctx* ctx) {
 
 static int death_prob(gnx_ctx* ctx, int end_step) {
   PROF(ctx, "k_death");
-  k_death<<<grid_cap(ctx, GNX_G_DEATH, 256, 1.0 + ctx->cfg.b * ctx->cfg.n_births_lambda), 256, 0, ctx->stream>>>(
+  k_death<<<grid_cap(ctx, DEATH_GRID, 256, 1.0 + ctx->cfg.b * ctx->cfg.n_births_lambda), 256, 0, ctx->stream>>>(
       ctx->pop, ctx->land, ctx->prm, ctx->traits, ctx->draws, ctx->work, ctx->d_c, ctx->mut, end_step, ctx->d_strip);
   LAUNCHED(ctx);
   return GNX_OK;

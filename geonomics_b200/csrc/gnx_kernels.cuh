@@ -410,7 +410,7 @@ __global__ void __launch_bounds__(256) k_regrid(Pop pop, Land land, Work w, Coun
 //   reference's cKDTree does).
 //   MODE 0: uniform random neighbour (spatial.py:232-242); valid candidates are kept as bit
 //           masks and the k-th is picked, k = (R * count) >> 32.  Cells whose 3x3 block is
-//           crowded (a row range longer than 64 entries, or focals x candidates >= GNX_FM_HEAVY_WORK)
+//           crowded (a row range longer than 64 entries, or focals x candidates >= FM_HEAVY_WORK)
 //           are not searched here: k_mate_select appends one work item per 32 focals of such a cell
 //           to Work.heavy and k_find_mates_dense takes them, one warp per item with the lanes across
 //           candidates.  All three kernels search only the focals whose Bernoulli(b) draw lets them
@@ -418,9 +418,7 @@ __global__ void __launch_bounds__(256) k_regrid(Pop pop, Land land, Work w, Coun
 //   MODE 1: nearest neighbour (spatial.py:194-203)
 //   MODE 2: inverse-distance weighting, p ~ (radius - dist) (spatial.py:209-229)
 // ========================================================================================
-#ifndef GNX_FM_HEAVY_WORK
-#define GNX_FM_HEAVY_WORK 4096   // measured flat from 3072 to 16384 at c4 (t = 300); 256-768 are 10-35 % slower
-#endif
+constexpr int FM_HEAVY_WORK = 4096;   // measured flat from 3072 to 16384 at c4 (t = 300); 256-768 are 10-35 % slower
 // position of the (k+1)-th set bit of m: popcount bisection (branch-free; __fns is a software loop)
 __device__ __forceinline__ int kth_set_bit(uint32_t m, int k) {
   int bit = 0;
@@ -434,7 +432,9 @@ __device__ __forceinline__ int kth_set_bit(uint32_t m, int k) {
 
 // the crowded-cell test of MODE 0 (see k_find_mates): l0..l2 = lengths of the three candidate row ranges,
 // nf = focals of the cell
-#define GNX_FM_IS_HEAVY(l0, l1, l2, nf) (max(l0, max(l1, l2)) > 64 || (nf) * ((l0) + (l1) + (l2)) >= GNX_FM_HEAVY_WORK)
+__device__ __forceinline__ bool fm_is_heavy(int l0, int l1, int l2, int nf) {
+  return max(l0, max(l1, l2)) > 64 || nf * (l0 + l1 + l2) >= FM_HEAVY_WORK;
+}
 
 // Bernoulli(b) FIRST.  The reference lists every focal's neighbours, lets each focal pick one and only then
 // keeps the pair with probability b (species.py:2212-2214) -- the draw is independent of the search, so a
@@ -482,7 +482,7 @@ __global__ void __launch_bounds__(256) k_mate_select(Pop pop, Land land, Params 
                      : (int)w.cell_start[row * land.ncx + x1 + 1] - (int)w.cell_start[row * land.ncx + x0];
             }
             const int nf = (int)w.cell_start[cy * land.ncx + cx + 1] - fs;
-            heavy = GNX_FM_IS_HEAVY(len[0], len[1], len[2], nf);
+            heavy = fm_is_heavy(len[0], len[1], len[2], nf);
             hkey = key;
           }
         }
@@ -522,24 +522,16 @@ __global__ void __launch_bounds__(256) k_mate_select(Pop pop, Land land, Params 
   }
 }
 
+constexpr int FM_BLOCK = 128;   // threads per CTA of k_find_mates (its launch bound and its launch)
 template <int MODE>
-#ifndef GNX_FM_BLOCK
-#define GNX_FM_BLOCK 128
-#endif
-#ifdef GNX_FM_MINB
-#define GNX_FM_BOUNDS __launch_bounds__(GNX_FM_BLOCK, GNX_FM_MINB)
-#else
-#define GNX_FM_BOUNDS __launch_bounds__(GNX_FM_BLOCK)
-#endif
-__global__ void GNX_FM_BOUNDS k_find_mates(Pop pop, Land land, Params prm, DevDraws dr, Work w,
-                                                     Counters* c) {
-  const int n = c->n, cur = c->cur;
+__global__ void __launch_bounds__(FM_BLOCK) k_find_mates(Pop pop, Land land, Params prm, DevDraws dr, Work w,
+                                                         Counters* c) {
+  const int cur = c->cur;
   const int64_t t = c->t;
   const double r2 = prm.r2, radius = prm.c.mating_radius;
   const double2* __restrict__ sxy = pop.xy[cur];
   const int32_t* __restrict__ ord = prm.ordered ? pop.ord[cur] : nullptr;
   const int n_list = *w.fm_count;                  // the focals k_mate_select let through
-  (void)n;
   for (int li = GTID; li < n_list; li += GSTRIDE) {
     const int p = w.fm_list[li];
     const double2 f = sxy[p];
@@ -564,7 +556,7 @@ __global__ void GNX_FM_BOUNDS k_find_mates(Pop pop, Land land, Params prm, DevDr
       // kernel loses lanes to padding (candidates in chunks of 32, focals in batches of 32), this
       // one to trip-count divergence: a cell moves over when its focals x candidates product is
       // large enough for the padding not to matter (or a row range exceeds the masks here)
-      if (GNX_FM_IS_HEAVY(l0, l1, l2, nf)) continue;      // (its work items were announced by k_mate_select)
+      if (fm_is_heavy(l0, l1, l2, nf)) continue;      // (its work items were announced by k_mate_select)
     }
     // MODE 0 keeps the valid candidates of each row range as two 32-bit masks in registers
     // (candidates 0-31 and 32-63 of the range)
@@ -1114,14 +1106,10 @@ struct BirthPlan {
   int s0, s1, cslot, kk0, kk1;     // parents' slots, child slot, key | start << 30
 };
 
-#ifndef GNX_GAM_NB
-#define GNX_GAM_NB 2           // offspring per trait-table walk in the staged path
-#endif
-#ifndef GNX_GAM_MINB
-#define GNX_GAM_MINB 4          // 64 registers: 4 CTAs per SM measured fastest (3, 5, 6 are slower)
-#endif
+constexpr int GAM_NB = 2;     // offspring per trait-table walk in the staged path
+constexpr int GAM_MINB = 4;   // 64 registers: 4 CTAs per SM measured fastest (3, 5, 6 are slower)
 template <int GW, int NT>
-__global__ void __launch_bounds__(256, GNX_GAM_MINB) k_gametes(Pop pop, Params prm, Traits tr, DevDraws dr, Work w,
+__global__ void __launch_bounds__(256, GAM_MINB) k_gametes(Pop pop, Params prm, Traits tr, DevDraws dr, Work w,
                                                   const Counters* c, int fixed_nb, int stage_rows) {
   // stage_rows: the child's row is also kept in shared memory (2*Wq uint4 per group) and the
   // phenotype is accumulated over the trait table with the entries dealt round-robin to the
@@ -1188,7 +1176,7 @@ __global__ void __launch_bounds__(256, GNX_GAM_MINB) k_gametes(Pop pop, Params p
     // NB offspring per group and pass: their rows are streamed and staged (one buffer each), then
     // ONE walk over the trait table serves all of them -- entry load, address arithmetic and
     // loop control are paid once per NB offspring.
-    constexpr int NB = (GNX_GAM_NB < GW) ? GNX_GAM_NB : GW;
+    constexpr int NB = (GAM_NB < GW) ? GAM_NB : GW;
     const int buf_stride = 8 * Wq * (blockDim.x / GW);       // uint32 words between the staging buffers
 #pragma unroll 1
     for (int j = 0; j < GW; j += NB) {
@@ -1361,10 +1349,8 @@ __global__ void __launch_bounds__(256, GNX_GAM_MINB) k_gametes(Pop pop, Params p
 }
 
 // ----- k_newborns: natal dispersal, sex, newborn record (one thread per offspring) -------
-#ifndef GNX_NB_MINB
-#define GNX_NB_MINB 4     // 64 registers instead of 77: 83 -> 68 us at c4
-#endif
-__global__ void __launch_bounds__(256, GNX_NB_MINB) k_newborns(Pop pop, Land land, Params prm, DevDraws dr, Work w,
+constexpr int NB_MINB = 4;   // 64 registers instead of 77: 83 -> 68 us at c4
+__global__ void __launch_bounds__(256, NB_MINB) k_newborns(Pop pop, Land land, Params prm, DevDraws dr, Work w,
                                                    Counters* c, Tsk tsk) {
   const int n = c->n, B = c->B, cur = c->cur;
   const int n_nodes = c->n_nodes, n_born = c->n_born;
@@ -2338,10 +2324,8 @@ __global__ void __launch_bounds__(256) k_raster_fix_d(Dens d, Land land, Params 
 // ========================================================================================
 // 8 resident CTAs (<= 32 registers): the kernel waits on its per-individual raster and genome gathers,
 // so residency beats registers (measured at c4: 262 us without the bound, 245 at 6, 233 at 8)
-#ifndef GNX_DEATH_MINB
-#define GNX_DEATH_MINB 8
-#endif
-__global__ void __launch_bounds__(256, GNX_DEATH_MINB) k_death(Pop pop, Land land, Params prm, Traits tr, DevDraws dr, Work w,
+constexpr int DEATH_MINB = 8;
+__global__ void __launch_bounds__(256, DEATH_MINB) k_death(Pop pop, Land land, Params prm, Traits tr, DevDraws dr, Work w,
                                                 Counters* c, Mut mu, int end_step, const Strip* st) {
   const int n0 = c->n, n = c->n + c->B, cur = c->cur, T = pop.T;
   const int64_t t = c->t;

@@ -108,11 +108,9 @@ __global__ void __launch_bounds__(SCAN_BLOCK) scan_reduce_kernel(F f, Counters* 
   }
 }
 
-#ifndef GNX_SCAN_MINB
-#define GNX_SCAN_MINB 3      // 80 registers: measured best of 1, 3, 4, 5 CTAs per SM
-#endif
+constexpr int SCAN_MINB = 3;   // 80 registers: measured best of 1, 3, 4, 5 CTAs per SM
 template <class F>
-__global__ void __launch_bounds__(SCAN_BLOCK, GNX_SCAN_MINB) scan_apply_kernel(F f, const Counters* c, const u64* tile_sums) {
+__global__ void __launch_bounds__(SCAN_BLOCK, SCAN_MINB) scan_apply_kernel(F f, const Counters* c, const u64* tile_sums) {
   const int n = f.size(c);
   const int ntiles = (n + SCAN_TILE - 1) / SCAN_TILE;
   for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
