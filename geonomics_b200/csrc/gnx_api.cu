@@ -96,7 +96,6 @@ struct gnx_ctx {
   bool have_density = false, have_paths = false, have_traits = false, have_rasters = false;
   int64_t launches = 0;
   int burn = 0;
-  bool gs_attr_set = false;
   bool capturing = false;               // inside cudaStreamBeginCapture/EndCapture of the whole-step graph
   bool pending = false;                 // host mirror of Counters.pending (set by the fused step, cleared by materialise / upload)
   bool order_valid = false;             // pop.ord / work.inv describe the current entries
@@ -836,17 +835,6 @@ extern "C" int gnx_set_density(gnx_ctx* ctx, const gnx_density_t* dn) {
     for (int i = 0; i < D.npts; ++i)
       for (int cc = 0; cc < 3; ++cc) vinv_t[(size_t)cc * D.npts + i] = vinv[3 * i + cc];
     if ((r = up(vinv_t.data(), sizeof(double) * vinv_t.size(), (const void**)&D.v_inv_t))) return r;
-    {
-      // one blob in the kernel's shared-memory layout: [8][4][npts] f64 | [3][npts] f64 | [8][npts] i32
-      const size_t nb = ((size_t)D.npts * GS_TABLE_BYTES_PER_PT + 15) / 16 * 16;
-      std::vector<unsigned char> blob(nb, 0);
-      memcpy(blob.data(), pe.data(), pe.size() * 8);
-      memcpy(blob.data() + pe.size() * 8, vinv_t.data(), vinv_t.size() * 8);
-      memcpy(blob.data() + pe.size() * 8 + vinv_t.size() * 8, pj.data(), pj.size() * 4);
-      if ((r = up(blob.data(), nb, (const void**)&D.gs_table))) return r;
-      D.gs_table_bytes = (int32_t)nb;
-      CK(cudaStreamSynchronize(ctx->stream));
-    }
     if ((r = up(pj.data(), sizeof(int32_t) * pj.size(), (const void**)&D.p_j))) return r;
     if ((r = up(pe.data(), sizeof(double) * pe.size(), (const void**)&D.p_e))) return r;
     CK(cudaStreamSynchronize(ctx->stream));     // the host vectors go out of scope below
@@ -1730,13 +1718,8 @@ static int density_eval_rasters(gnx_ctx* ctx) {
   cudaStream_t s = ctx->stream;
   // scipy defaults reached through griddata: CloughTocher2DInterpolator(tol=1e-6, maxiter=400)
   PROF(ctx, "k_ct_gradients");
-  const size_t gs_bytes = (size_t)ctx->dens.gs_table_bytes + (size_t)ctx->dens.npts * 24 + 16;
-  if (ctx->dens.colourable && ctx->dens.padded && gs_bytes <= 220 * 1024) {
-    if (!ctx->gs_attr_set) {              // per device, so per ctx (a process may drive several GPUs)
-      CK(cudaFuncSetAttribute(k_ct_gradients_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-      ctx->gs_attr_set = true;
-    }
-    k_ct_gradients_smem<<<2, GS_BLOCK, gs_bytes, s>>>(ctx->dens, ctx->d_c, 400, 1e-6);
+  if (ctx->dens.colourable && ctx->dens.padded && ctx->dens.npts <= GS_REG_PTS) {
+    k_ct_gradients_reg<<<2, (ctx->dens.npts + 31) / 32 * 32, 0, s>>>(ctx->dens, ctx->d_c, 400, 1e-6);
   } else {
     k_ct_gradients<<<2, GS_BLOCK, 0, s>>>(ctx->dens, ctx->d_c, 400, 1e-6);
   }
@@ -1848,8 +1831,8 @@ static int one_step(gnx_ctx* ctx) {
     if ((r = offspring_check(ctx))) return r;
     if ((r = offspring_newborns(ctx))) return r;
     // The counts stay on the main stream, IN FRONT of the gamete kernel: the gradient solve that follows them
-    // is two CTAs that each need a whole SM's shared memory, and once the gamete kernel's CTAs hold the SMs it
-    // cannot start before they are all gone.  Forking after the counts makes the gradient solve and the gamete
+    // is two CTAs that each need a whole SM's register file (one thread per lattice vertex, its tables in
+    // registers), and once the gamete kernel's CTAs hold the SMs it cannot start before they are all gone.  Forking after the counts makes the gradient solve and the gamete
     // kernel eligible at the same moment, the solve's two CTAs are placed first, and the chain's latency-bound
     // head runs UNDER the genotype streaming instead of behind it.
     if ((r = gnx_density_counts(ctx))) return r;

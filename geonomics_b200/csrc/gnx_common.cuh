@@ -138,8 +138,6 @@ struct Dens {
   const int32_t* p_j;      // [8][npts] neighbours padded with self (transposed)
   const double* p_e;       // [8][4][npts] (ex, ey, ex/L^3, ey/L^3), padded with zeros (transposed)
   const double* v_inv_t;   // [3][npts]
-  const void* gs_table;    // contiguous blob [p_e | v_inv_t | p_j | pad16] staged into shared memory by TMA
-  int32_t gs_table_bytes;
   int32_t padded;          // every vertex has <= 8 neighbours
   int32_t lat_ni, lat_nj;
   const int32_t* square_tri;
@@ -542,29 +540,3 @@ __device__ __forceinline__ void sincos_half(__half h, double* s, double* c) {
   *c = (double)__half2float(__float2half_rn(cf));
   *s = (double)__half2float(__float2half_rn(sf));
 }
-
-// ---- TMA bulk copy (cp.async.bulk, SASS UBLKCP) + mbarrier helpers ------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gmem_src, uint32_t bytes, unsigned long long* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(smem_u32(smem_dst)), "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "WAIT_LOOP:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra WAIT_DONE;\n"
-      "bra WAIT_LOOP;\n"
-      "WAIT_DONE:\n"
-      "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-

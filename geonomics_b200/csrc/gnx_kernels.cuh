@@ -1840,37 +1840,8 @@ __global__ void __launch_bounds__(512) k_density_counts(Pop pop, Work w, const C
 // Per-vertex update with the data-independent parts hoisted to setup (gnx_set_density):
 // the 2x2 matrix Q of `_estimate_gradients_2d_global` depends only on the triangulation,
 // so its inverse (v_inv) and the per-edge weights ex/L^3, ey/L^3 are precomputed; a sweep
-// then costs 6 flops per edge and no sqrt.  Edges are stored padded to GS_DEG slots per
-// vertex (pad: neighbour = self, weights = 0), so the loop is fully unrolled and all loads
-// of a vertex are independent.
+// then costs 6 flops per edge and no sqrt.
 #define GS_DEG 8
-// Edge table layout is transposed: slot k, component c of vertex v is at [(4*k + c)*npts + v],
-// neighbour ids at [k*npts + v], inverse-matrix entries at [c*npts + v]; the threads of a
-// colour phase own consecutive vertices, so every shared-memory access is stride-1 across the
-// warp (the [vertex][slot] layout costs a 32-way bank conflict on every load).
-__device__ __forceinline__ double gs_vertex_padded(const int* __restrict__ pj, const double* __restrict__ pe,
-                                                   const double* __restrict__ vinv, const double* f, double* yv,
-                                                   int i, int npts) {
-  double s0 = 0, s1 = 0;
-  const double f1 = f[i];
-#pragma unroll
-  for (int k = 0; k < GS_DEG; ++k) {
-    const int j = pj[k * npts + i];
-    const double ex = pe[(4 * k + 0) * npts + i], ey = pe[(4 * k + 1) * npts + i];
-    // (6*(f1 - f2) - 2*df2) with df2 = -ex*y_j0 - ey*y_j1
-    const double tt = 6 * (f1 - f[j]) + 2 * (ex * yv[j] + ey * yv[npts + j]);
-    s0 += tt * pe[(4 * k + 2) * npts + i];
-    s1 += tt * pe[(4 * k + 3) * npts + i];
-  }
-  const double i00 = vinv[i], i01 = vinv[npts + i], i11 = vinv[2 * npts + i];
-  const double r0 = i00 * s0 + i01 * s1;
-  const double r1 = i01 * s0 + i11 * s1;
-  double change = fmax(fabs(yv[i] + r0), fabs(yv[npts + i] + r1));
-  yv[i] = -r0;
-  yv[npts + i] = -r1;
-  change /= fmax(1.0, fmax(fabs(r0), fabs(r1)));
-  return change;
-}
 
 // general form (any degree, CSR), used when a vertex has more than GS_DEG neighbours or the
 // triangulation is not 4-colourable by grid
@@ -1894,68 +1865,98 @@ __device__ __forceinline__ double gs_vertex_csr(const Dens& d, const double* f, 
 }
 
 #define GS_BLOCK 256
-#define GS_SMEM_PTS 1536
-// bytes of dynamic shared memory per lattice point when the whole solve lives in shared
-// memory: edge table (8 slots x 4 doubles), inverse matrices (3), neighbour ids (8 ints),
-// gradients (2), values (1)
-#define GS_TABLE_BYTES_PER_PT (GS_DEG * 32 + 24 + GS_DEG * 4)
-extern __shared__ __align__(128) unsigned char gs_dyn_smem[];
+// Largest lattice of the register-resident solve: one thread per vertex in one CTA.  Its
+// edge tables take 64 registers a thread; an SM's four schedulers hold 16384 registers each,
+// so up to 20 warps (5 a scheduler) may use 96.  The default window width gives lattices of
+// about 23 x 23 = 529 points.
+#define GS_REG_PTS 640
 
-// Fast path: the whole solve in shared memory (default lattices have <= 529 points = 178 KB).
-// The constant tables (one contiguous blob, already in the transposed shared-memory layout)
-// are staged by the TMA with one bulk copy per 32 KB chunk while the threads compute the
-// lattice values; everything after that touches shared memory only.
-__global__ void __launch_bounds__(GS_BLOCK) k_ct_gradients_smem(Dens d, Counters* c, int maxiter, double tol) {
+// Fast path (lattices of <= GS_REG_PTS points, every vertex of degree <= GS_DEG, 4-colourable
+// by grid): thread v owns vertex v for the whole solve.  The vertices are numbered grid by
+// grid, so each colour phase is a contiguous range of threads.  The edge vectors and weights
+// of the vertex's GS_DEG slots (pad: neighbour = self, weights = 0) do not change during the
+// solve and stay in registers; shared memory holds the values and gradients, the 2x2 inverses
+// and the neighbour ids, so an update gathers its 8 neighbours' values and gradients, one
+// address each.  (Keeping the value differences or the unpacked ids in registers as well
+// exceeds the 96 and spills.)  The arithmetic is spelled out with _rn intrinsics: it is the
+// contraction nvcc chose for the shared-memory kernel this replaced, and no rounding of the
+// solve may change (density feeds the death draws).
+__global__ void __launch_bounds__(GS_REG_PTS, 1) k_ct_gradients_reg(Dens d, Counters* c, int maxiter, double tol) {
   const int which = blockIdx.x;          // 0 = species density N, 1 = pair-midpoint density
   const int npts = d.npts;
-  const int* counts = d.counts + (size_t)which * npts;
-  double* gf = d.vals + (size_t)which * npts;
-  double* gy = d.grad + (size_t)which * npts * 2;
-  __shared__ __align__(8) unsigned long long bar;
-  const uint32_t table_bytes = (uint32_t)d.gs_table_bytes;                // multiple of 16
-  double* spe = reinterpret_cast<double*>(gs_dyn_smem);                   // [8][4][npts]
-  double* svinv = spe + (size_t)npts * GS_DEG * 4;                        // [3][npts]
-  int* spj = reinterpret_cast<int*>(svinv + 3 * npts);                    // [8][npts]
-  double* sy = reinterpret_cast<double*>(gs_dyn_smem + table_bytes);      // [2][npts]
-  double* sf = sy + 2 * npts;                                             // [npts]
-  if (threadIdx.x == 0) mbar_init(&bar, 1);
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    mbar_expect_tx(&bar, table_bytes);
-    const unsigned char* src = reinterpret_cast<const unsigned char*>(d.gs_table);
-    for (uint32_t off = 0; off < table_bytes; off += 32768) {
-      const uint32_t nb = min(32768u, table_bytes - off);
-      bulk_g2s(gs_dyn_smem + off, src + off, nb, &bar);
+  const int v = threadIdx.x;
+  const bool own = v < npts;
+  struct __align__(16) Vert { double2 y; double f; };   // gradient and value: one address per neighbour
+  __shared__ Vert sv[GS_REG_PTS];
+  __shared__ double sinv[3][GS_REG_PTS];
+  __shared__ uint4 snb[GS_REG_PTS];      // neighbour ids of slots 2q, 2q+1 in the low, high half of word q
+  double ex[GS_DEG], ey[GS_DEG], wx[GS_DEG], wy[GS_DEG];
+  int colour = -1;
+  if (own) {
+    // table layout is transposed ([(4*k + c)*npts + v], [k*npts + v], [c*npts + v]): coalesced loads
+#pragma unroll
+    for (int k = 0; k < GS_DEG; ++k) {
+      ex[k] = d.p_e[(4 * k + 0) * npts + v];
+      ey[k] = d.p_e[(4 * k + 1) * npts + v];
+      wx[k] = d.p_e[(4 * k + 2) * npts + v];
+      wy[k] = d.p_e[(4 * k + 3) * npts + v];
     }
+    uint32_t w[GS_DEG / 2];
+#pragma unroll
+    for (int q = 0; q < GS_DEG / 2; ++q)
+      w[q] = (uint32_t)d.p_j[2 * q * npts + v] | ((uint32_t)d.p_j[(2 * q + 1) * npts + v] << 16);
+    snb[v] = make_uint4(w[0], w[1], w[2], w[3]);
+#pragma unroll
+    for (int cc = 0; cc < 3; ++cc) sinv[cc][v] = d.v_inv_t[cc * npts + v];
+#pragma unroll
+    for (int g = 0; g < 4; ++g)
+      if (v >= d.g_off[g] && v < d.g_off[g] + d.g_ni[g] * d.g_nj[g]) colour = g;
+    const double f = (double)d.counts[(size_t)which * npts + v] / d.areas[v];   // spatial.py:95
+    sv[v].f = f;
+    d.vals[(size_t)which * npts + v] = f;
+    sv[v].y = make_double2(0.0, 0.0);
   }
-  for (int k = threadIdx.x; k < npts; k += blockDim.x) {
-    const double v = (double)counts[k] / d.areas[k];       // spatial.py:95
-    sf[k] = v;
-    gf[k] = v;
-    sy[k] = 0.0;
-    sy[npts + k] = 0.0;
-  }
-  mbar_wait(&bar, 0);
   __syncthreads();
-  int iters = 0;
-  for (int it = 0; it < maxiter; ++it) {
+  int it = 0;
+  for (; it < maxiter; ++it) {
     double err = 0.0;
 #pragma unroll
     for (int g = 0; g < 4; ++g) {
-      const int s = d.g_off[g], e = s + d.g_ni[g] * d.g_nj[g];
-      for (int v = s + threadIdx.x; v < e; v += GS_BLOCK)
-        err = fmax(err, gs_vertex_padded(spj, spe, svinv, sf, sy, v, npts));
+      if (colour == g) {
+        const double f1 = sv[v].f;
+        const uint4 nbw = snb[v];
+        const uint32_t nbp[GS_DEG / 2] = {nbw.x, nbw.y, nbw.z, nbw.w};
+        double s0 = 0.0, s1 = 0.0;
+#pragma unroll
+        for (int k = 0; k < GS_DEG; ++k) {
+          // (6*(f1 - f2) - 2*df2) with df2 = -ex*y_j0 - ey*y_j1
+          const Vert& nv = sv[(nbp[k >> 1] >> (16 * (k & 1))) & 0xffff];
+          const double2 yj = nv.y;
+          const double q = __fma_rn(ex[k], yj.x, __dmul_rn(ey[k], yj.y));
+          const double tt = __fma_rn(__dsub_rn(f1, nv.f), 6.0, __dadd_rn(q, q));
+          s0 = __fma_rn(tt, wx[k], s0);
+          s1 = __fma_rn(tt, wy[k], s1);
+        }
+        const double i00 = sinv[0][v], i01 = sinv[1][v], i11 = sinv[2][v];
+        const double r0 = __fma_rn(i00, s0, __dmul_rn(i01, s1));
+        const double r1 = __fma_rn(i01, s0, __dmul_rn(i11, s1));
+        const double2 yi = sv[v].y;
+        const double change = fmax(fabs(__dadd_rn(yi.x, r0)), fabs(__dadd_rn(yi.y, r1)));
+        sv[v].y = make_double2(-r0, -r1);
+        err = fmax(err, __ddiv_rn(change, fmax(1.0, fmax(fabs(r0), fabs(r1)))));
+      }
       // the barrier that ends the last colour phase also carries the convergence vote:
-      // max over vertices of `change` < tol  <=>  every thread's local maximum < tol
+      // max over vertices of `change` < tol  <=>  every thread's `change` < tol
       if (g < 3) __syncthreads();
     }
-    if (__syncthreads_and(err < tol)) { iters = it + 1; break; }
+    if (__syncthreads_and(err < tol)) break;
   }
-  for (int k = threadIdx.x; k < npts; k += blockDim.x) {
-    gy[2 * k] = sy[k];
-    gy[2 * k + 1] = sy[npts + k];
+  if (own) {
+    double* gy = d.grad + (size_t)which * npts * 2;
+    gy[2 * v] = sv[v].y.x;
+    gy[2 * v + 1] = sv[v].y.y;
   }
-  if (threadIdx.x == 0) c->gs_iters[which] = iters;     // 0: maxiter reached (scipy only warns)
+  if (threadIdx.x == 0) c->gs_iters[which] = it < maxiter ? it + 1 : 0;     // 0: maxiter reached (scipy only warns)
 }
 
 // General path: larger lattices, vertices of degree > 8, or triangulations that are not

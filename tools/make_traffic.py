@@ -24,7 +24,7 @@ def bench_name(ncu_name):
     if m:
         return '%s.%s' % (SCAN.get(m.group(2), m.group(2)), m.group(1))
     n = re.sub(r'<.*>', '', n)
-    return {'k_ct_gradients_smem': 'k_ct_gradients'}.get(n, n)
+    return {'k_ct_gradients_reg': 'k_ct_gradients'}.get(n, n)
 
 
 def to_bytes(v, unit):

@@ -9,7 +9,10 @@ torch.profiler (CUDA activities) and writes, for every kernel of those steps, it
   * gametes_us:      fork -> end of the last other kernel before k_death (k_gametes ... k_after_births);
   * exposed_us:      density_us - gametes_us (> 0: k_death waits for the density branch);
   * death_us:        k_death;
-  * step_us:         first kernel start -> next step's first kernel start.
+  * step_us:         first kernel start -> next step's first kernel start;
+  * gaps:            idle stretches of a stream between two of its kernels longer than GAP_US, each with the
+                     memset and memcpy nodes of the step that run inside it (the graph's non-kernel work).
+`gap_median_us` gives the median of every such gap over the traced steps, keyed 'kernel -> kernel'.
 The raster kernels have no row in bench.py's algorithmic-bytes table, so their bytes per launch (landscape
 cells x bytes per cell) are reported here.  The library is the in-tree build, or GNX_B200_LIB.
 
@@ -26,7 +29,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
 
-DENSITY = ('k_ct_gradients', 'k_ct_gradients_smem', 'k_ct_coefficients')
+GAP_US = 2.0
 # algorithmic bytes per landscape cell of the raster passes
 RASTER_BYTES_PER_CELL = {'k_raster_N': 8, 'k_raster_d': 24, 'k_raster_Nd': 24}
 
@@ -38,7 +41,7 @@ def short_name(name):
 
 
 def is_density(name):
-    return name in DENSITY or name.startswith('k_raster_')
+    return name.startswith(('k_ct_', 'k_raster_'))
 
 
 def split_steps(kernels):
@@ -51,6 +54,22 @@ def split_steps(kernels):
         if cur is not None:
             cur.append(k)
     return steps
+
+
+def step_gaps(ks, others):
+    """Idle stretches of each stream between consecutive kernels, and the memset / memcpy nodes inside them."""
+    out = []
+    streams = sorted({k['stream'] for k in ks}, key=str)
+    for st in streams:
+        sk = [k for k in ks if k['stream'] == st]
+        for a, b in zip(sk, sk[1:]):
+            if b['start'] - a['end'] <= GAP_US:
+                continue
+            inside = [{'name': o['name'], 'kind': o['kind'], 'stream': o['stream'], 'us': o['end'] - o['start']}
+                      for o in others if o['end'] > a['end'] and o['start'] < b['start']]
+            out.append({'after': a['name'], 'before': b['name'], 'stream': st, 'us': b['start'] - a['end'],
+                        'activity': inside})
+    return out
 
 
 def step_summary(ks, next_start):
@@ -72,6 +91,16 @@ def step_summary(ks, next_start):
     if next_start is not None:
         out['step_us'] = next_start - t0
     return out
+
+
+def power_limit_w():
+    try:
+        import pynvml
+        pynvml.nvmlInit()
+        h = pynvml.nvmlDeviceGetHandleByIndex(0)
+        return pynvml.nvmlDeviceGetEnforcedPowerLimit(h) / 1000.0
+    except Exception:
+        return None
 
 
 def main():
@@ -110,17 +139,27 @@ def main():
     prof.export_chrome_trace(trace)
     with open(trace) as f:
         events = json.load(f)['traceEvents']
-    kernels = sorted(({'name': short_name(e['name']), 'stream': e.get('args', {}).get('stream', e.get('tid')),
-                       'start': float(e['ts']), 'end': float(e['ts']) + float(e['dur'])}
-                      for e in events if e.get('cat') == 'kernel'), key=lambda k: k['start'])
+    acts = sorted(({'name': short_name(e['name']), 'kind': e['cat'],
+                    'stream': e.get('args', {}).get('stream', e.get('tid')),
+                    'start': float(e['ts']), 'end': float(e['ts']) + float(e['dur'])}
+                   for e in events if e.get('cat') in ('kernel', 'gpu_memset', 'gpu_memcpy')), key=lambda k: k['start'])
+    kernels = [a for a in acts if a['kind'] == 'kernel']
     steps = split_steps(kernels)
     rows = []
+    gap_us = {}
     for s, ks in enumerate(steps):
         nxt = steps[s + 1][0]['start'] if s + 1 < len(steps) else None
         r = step_summary(ks, nxt)
         if r is not None and nxt is not None:
+            others = [a for a in acts if a['kind'] != 'kernel' and ks[0]['start'] <= a['start'] < nxt]
+            r['gaps'] = step_gaps(ks, others)
+            for g in r['gaps']:
+                gap_us.setdefault(g['after'] + ' -> ' + g['before'], []).append(g['us'])
             r['kernels'] = [{'name': k['name'], 'stream': k['stream'], 'start_us': k['start'] - ks[0]['start'],
                              'end_us': k['end'] - ks[0]['start']} for k in ks]
+            r['non_kernel'] = [{'name': o['name'], 'kind': o['kind'], 'stream': o['stream'],
+                                'start_us': o['start'] - ks[0]['start'], 'end_us': o['end'] - ks[0]['start']}
+                               for o in others]
             rows.append(r)
     cells = w['land_dim'][0] * w['land_dim'][1]
     durs = {}
@@ -135,11 +174,13 @@ def main():
            'library': os.path.relpath(_lib.LIB_PATH, os.path.dirname(HERE)),
            'presteps': args.presteps, 'steps_traced': len(rows),
            'gpu': torch.cuda.get_device_name(0),
+           'power_limit_w': power_limit_w(),
            'kernels_listed': len(kernels) > 0,
            'median': {k: float(np.median([r[k] for r in rows])) for k in keys} if rows else None,
            'min': {k: float(np.min([r[k] for r in rows])) for k in keys} if rows else None,
            'max': {k: float(np.max([r[k] for r in rows])) for k in keys} if rows else None,
            'kernel_median_us': {n: float(np.median(v)) for n, v in sorted(durs.items())},
+           'gap_median_us': {n: float(np.median(v)) for n, v in sorted(gap_us.items())},
            'raster_bytes': raster,
            # (fix list, deferred list); libraries without k_raster_Nd keep no such lengths
            'density_lists_last_step': counters.get('density_lists') if 'k_raster_Nd' in durs else None,
@@ -148,7 +189,8 @@ def main():
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, 'w') as f:
         json.dump(out, f, indent=1)
-    print(json.dumps({k: out[k] for k in ('workload', 'library', 'steps_traced', 'median', 'density_lists_last_step')}))
+    print(json.dumps({k: out[k] for k in ('workload', 'library', 'gpu', 'power_limit_w', 'steps_traced', 'median',
+                                          'gap_median_us', 'density_lists_last_step')}))
 
 
 if __name__ == '__main__':
