@@ -190,6 +190,45 @@ def compare_step(out, new_o, im_o, rtol=1e-6, exact_xy_tol=1e-9):
     assert rec['n_deaths'] == im_o['n_deaths']
 
 
+# Genome sizes and trait kinds that reach every k_gametes<GW, NT> instantiation and phenotype mode
+# (gnx_api.cu launch_gametes): GW = 1, 2, 4, 8, 16, 32 lanes per offspring; at GW 32 two staged rows
+# (L 3000), one staged row (L 12000: two 94-unit rows exceed 44 KB) and no staging (L 17000: one row
+# exceeds 32 KB).  Kinds: polygenic; polygenic with dominance; a monogenic trait beside a polygenic
+# one; five traits with dominance (the GNX_MAX_TRAITS accumulators).
+GAMETE_MATRIX_L = (100, 200, 400, 1000, 1500, 3000, 12000, 17000)
+TRAIT_KINDS = ('poly', 'dom', 'mono', 'dom5')
+
+
+def trait_set(L, kind, seed=0, lyr_nums=(1, 2), phi=0.1):
+    """(traits, dom) of one trait kind, with trait loci on the word and unit edges 0, 31, 32, 127,
+    128 and L - 1 (those below L) dealt round-robin to the traits; traits hold disjoint loci."""
+    rng = np.random.default_rng(seed)
+    n_traits = 5 if kind == 'dom5' else 2
+    edges = [l for l in (0, 31, 32, 127, 128, L - 1) if l < L]
+    edges = list(dict.fromkeys(edges))
+    per = max(2, min(9, (L - len(edges)) // (2 * n_traits)))
+    rest = rng.permutation(np.setdiff1d(np.arange(L), edges))[:per * n_traits]
+    loci = [[] for _ in range(n_traits)]
+    for k, l in enumerate(edges):
+        loci[k % n_traits].append(l)
+    for k, l in enumerate(rest):
+        loci[k % n_traits].append(int(l))
+    if kind == 'mono':                       # trait 0 keeps one locus (31 where the genome has it)
+        one = 31 if 31 in loci[0] else loci[0][0]
+        loci[1] += [l for l in loci[0] if l != one]
+        loci[0] = [one]
+    traits = []
+    for t in range(n_traits):
+        lc = np.array(sorted(loci[t]), dtype=np.int64)
+        traits.append(dict(loci=lc, alpha=rng.normal(0, 0.1, len(lc)), phi=phi, gamma=1.0,
+                           lyr_num=lyr_nums[t % len(lyr_nums)], univ_adv=False))
+    dom = np.zeros(L, np.int8)
+    if kind in ('dom', 'dom5'):
+        for tr in traits:
+            dom[tr['loci'][::2]] = 1         # every other trait locus, the first (an edge locus) included
+    return traits, dom
+
+
 def synthetic_case(L=1000, n=1500, n_traits=2, loci_per_trait=20, dim=(40, 40), seed=0, max_tries=8, cap=None):
     """A synthetic population in the golden-case format (arch, prm, state, draws), for parity
     of the CUDA path against the (golden-pinned) oracle at genome sizes the reference-recorded
