@@ -253,6 +253,8 @@ SIGNATURES = {
                                              C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), c_double_p, c_int64_p]),
     'gnx_stats_ld': (C.c_int, [_ctx, C.POINTER(C.c_uint64), c_int64_p]),
     'gnx_burnin_cell_stats': (C.c_int, [_ctx, c_int64_p, c_int64_p]),
+    'gnx_strip_burnin_count': (C.c_int, [_ctx, c_int32_p, c_int32_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)]),
+    'gnx_strip_burnin_diff': (C.c_int, [_ctx, C.c_int32, c_int64_p, c_int64_p]),
     'gnx_read_field': (C.c_int, [_ctx, C.c_int32, C.c_void_p, C.c_int64]),
     'gnx_device_ptr': (C.c_int, [_ctx, C.c_int32, C.POINTER(C.c_void_p), c_int64_p]),
     'gnx_stream': (C.c_void_p, [_ctx]),

@@ -602,7 +602,7 @@ class Species:
     DeviceSpecies.  Parameter attributes (`spp.b`, `spp.mating_radius`, ...) resolve through
     `_pv` like the reference (species.py:71-74, 405-425)."""
 
-    def __init__(self, name, idx, land, spp_params, genomic_architecture=None, N=0, seed=0):
+    def __init__(self, name, idx, land, spp_params, genomic_architecture=None, N=0, seed=0, strips=None):
         self.idx = idx
         self.name = str(name)
         self._land = land
@@ -648,6 +648,7 @@ class Species:
                 self.mut_log = '%s_mutations.log' % name
         self.mutations = []                    # drained device mutation log (dict rows)
         self._seed = seed
+        self._strips = strips                  # None, a strip count or a process group (strips.StripSpecies)
         self._tc = None                        # tskit tables as numpy columns (tables.TableColumns), use_tskit only
         self._dev = None
         self._cache = None                     # host copy of the device state (lazy)
@@ -691,12 +692,17 @@ class Species:
                                    univ_adv=t.univ_adv))
             ga = dict(L=self.gen_arch.L, paths=self.gen_arch.recombinations._paths, traits=traits,
                       dom=np.asarray(self.gen_arch.dom, dtype=np.int8))
-        if capacity is None:
-            capacity = int(max(4096, 3.0 * float(np.sum(self.K)), 2 * self.start_N))
-        self._dev = DeviceSpecies(land.dim, rasters, self._device_params(), ga, capacity=capacity,
-                                  seed=self._seed, res_ratio=self._land_res_ratio)
-        land._listeners.append(self)
         p = self._init_pop
+        if self._strips is not None:
+            from .strips import StripSpecies
+            self._dev = StripSpecies(land.dim, rasters, self._device_params(), ga, self.K, p['y'], self._strips,
+                                     seed=self._seed, res_ratio=self._land_res_ratio, capacity=capacity)
+        else:
+            if capacity is None:
+                capacity = int(max(4096, 3.0 * float(np.sum(self.K)), 2 * self.start_N))
+            self._dev = DeviceSpecies(land.dim, rasters, self._device_params(), ga, capacity=capacity,
+                                      seed=self._seed, res_ratio=self._land_res_ratio)
+        land._listeners.append(self)
         self._dev.set_burn(not self.burned)
         self._dev.upload(p['x'], p['y'], p['age'], p['sex'], p['idx'], max_ind_idx=self.max_ind_idx,
                          genomes_packed=p.get('genomes'))
@@ -1234,12 +1240,12 @@ class Community(dict):
         self.burned = False
 
 
-def _make_species(land, name, idx, spp_params, seed=0):
+def _make_species(land, name, idx, spp_params, seed=0, strips=None):
     """species.py:3276-3397."""
     init = dict(spp_params.init)
     ga = _make_genomic_architecture(spp_params, land) if 'gen_arch' in spp_params else None
     N = int(init.pop('N'))
-    spp = Species(name, idx, land, spp_params, ga, N=N, seed=seed)
+    spp = Species(name, idx, land, spp_params, ga, N=N, seed=seed, strips=strips)
     # individual.py:188-229: uniform positions, Bernoulli(0.5) sex (with the re-draw quirk of
     # Individual.__init__, individual.py:110-115: a drawn 0 is re-drawn)
     xy = np.random.rand(N, 2) * np.array(land.dim)
@@ -1278,17 +1284,61 @@ def _check_genome_init(genome_init):
         raise ValueError("genome_init must be 'host' or 'device', not %r" % (genome_init,))
 
 
+def _strip_world(strips):
+    """The number of strips of `strips` (None, an int >= 2 or an initialised nccl process group)."""
+    if strips is None:
+        return None
+    if isinstance(strips, (int, np.integer)) and not isinstance(strips, bool):
+        if strips < 2:
+            raise ValueError('strips must be at least 2 (or None, or a process group), not %d' % strips)
+        return int(strips)
+    import torch.distributed as dist
+    if not isinstance(strips, dist.ProcessGroup) or not dist.is_initialized():
+        raise ValueError('strips must be None, an int >= 2 or an initialised torch.distributed process group')
+    if dist.get_backend(strips) != 'nccl':
+        raise ValueError('a strip process group needs the nccl backend, not %s' % dist.get_backend(strips))
+    return dist.get_world_size(strips)
+
+
+def _check_strip_species(spp, world):
+    """What strip decomposition does not carry, refused before any device work."""
+    from .strips import mating_grid
+    ga = spp.gen_arch
+    if ga is not None and ga.use_tskit:
+        raise ValueError("species '%s': use_tskit=True is not supported under strip decomposition" % spp.name)
+    if ga is not None and any((t.mu or 0) > 0 for t in (ga.traits or {}).values()):
+        raise ValueError("species '%s': trait mutation (Trait.mu > 0) is not supported under strip decomposition"
+                         % spp.name)
+    if getattr(spp, 'mating_radius', None) is None:
+        raise ValueError("species '%s': a panmictic species (no mating radius) cannot be cut into strips" % spp.name)
+    ncy = mating_grid(spp._land_dim, spp.mating_radius)[2]
+    if ncy < 2 * world:
+        raise ValueError("species '%s': %d strips need %d mating-grid rows, the landscape has %d"
+                         % (spp.name, world, 2 * world, ncy))
+
+
 class Model:
     """sim/model.py:47.  `walk` / `run` keep their reference signatures.
 
     genome_init selects how the starting genomes are assigned after the burn-in: 'host' (the
     default) draws them with numpy's stream exactly as the reference does; 'device' draws them on the
     GPU with the same exact per-locus allele counts (DeviceSpecies.init_genomes) and never builds the
-    N x L x 2 host array, which is what makes populations of millions of individuals startable."""
+    N x L x 2 host array, which is what makes populations of millions of individuals startable.
 
-    def __init__(self, name, params, verbose=False, genome_init='host'):
+    strips cuts every species into horizontal strips of its mating grid (geonomics_b200/strips.py) and
+    reproduces the undecomposed model with the same seed: None (the default) keeps each species on one
+    context; an int k >= 2 holds k strips as contexts of this process on the current GPU (a check, no
+    speed-up); an initialised torch.distributed process group (nccl, one rank per GPU of one node) gives
+    every rank its own strip.  Under a group every rank runs the same script and makes the same calls in
+    the same order, and builds the same host state from numpy's global stream: without a seed in the
+    parameters rank 0 draws one and every rank seeds numpy with it.  Strips refuse use_tskit, trait
+    mutation, panmixia, fewer than two mating-grid rows per strip and Model.run(dist=...)."""
+
+    def __init__(self, name, params, verbose=False, genome_init='host', strips=None):
         _check_genome_init(genome_init)
+        world = _strip_world(strips)
         self.genome_init = genome_init
+        self.strips = strips
         self.params = copy.deepcopy(params)
         m = self.params.model
         self.name = name or 'unnamed_model'
@@ -1296,8 +1346,13 @@ class Model:
         self.seed = None
         if 'seed' in m and m.seed is not None:
             self.seed = m.seed.num if isinstance(m.seed, dict) else m.seed
-            if self.seed is not None:
-                np.random.seed(self.seed)                   # model.py:362-366
+        if world is not None and not isinstance(strips, (int, np.integer)) and self.seed is None:
+            import torch.distributed as dist
+            box = [int(np.random.SeedSequence().generate_state(1)[0]) if dist.get_rank(strips) == 0 else None]
+            dist.broadcast_object_list(box, group=strips, group_src=0)
+            self.seed = box[0]
+        if self.seed is not None:
+            np.random.seed(self.seed)                       # model.py:362-366
         self.burn_T = m.burn_T
         self.burn_t = -1
         self.T = m.T
@@ -1315,7 +1370,9 @@ class Model:
         self.land = _make_landscape(self.params)
         spps = {}
         for n, (sname, sp) in enumerate(self.params.comm.species.items()):
-            spps[n] = _make_species(self.land, sname, n, sp, seed=(self.seed or 0) * 1000003 + n)
+            spps[n] = _make_species(self.land, sname, n, sp, seed=(self.seed or 0) * 1000003 + n, strips=strips)
+            if world is not None:
+                _check_strip_species(spps[n], world)
         self.comm = Community(self.land, spps)
         for spp in self.comm.values():
             spp._attach()
@@ -1487,7 +1544,8 @@ class Model:
                 spp._detach()
             spps = {}
             for n, (sname, sp) in enumerate(self.params.comm.species.items()):
-                spps[n] = _make_species(self.land, sname, n, sp, seed=(self.seed or 0) * 1000003 + n + 7919 * (self.it + 1))
+                spps[n] = _make_species(self.land, sname, n, sp, seed=(self.seed or 0) * 1000003 + n + 7919 * (self.it + 1),
+                                        strips=self.strips)
             self.comm = Community(self.land, spps)
             for spp in self.comm.values():
                 spp._attach()
@@ -1544,6 +1602,9 @@ class Model:
         rand_genarch / repeat_burn.  With an initialised `torch.distributed` handle in `dist` the
         iterations are sharded round-robin over the ranks (they never exchange data,
         geonomics_b200/parallel.py) and rank 0 returns every iteration's trajectories."""
+        if dist is not None and self.strips is not None:
+            raise ValueError('Model.run(dist=...) shards iterations over the ranks; a strip model already spreads '
+                             'each species over them')
         self._verbose = verbose
         mine = None
         if dist is not None and dist.is_initialized() and dist.get_world_size() > 1:
@@ -1607,10 +1668,11 @@ class Model:
         return writers.write_geodata(filepath, self._spp(spp), n=n)
 
 
-def make_model(parameters=None, verbose=False, name=None, genome_init='host'):
+def make_model(parameters=None, verbose=False, name=None, genome_init='host', strips=None):
     """main.py:442: a Model from a parameters-file path, a dict or a ParametersDict.  genome_init: how the
-    starting genomes are assigned after the burn-in (Model)."""
+    starting genomes are assigned after the burn-in; strips: None, a strip count or a process group (Model)."""
     _check_genome_init(genome_init)
+    _strip_world(strips)
     if isinstance(parameters, str):
         params = read_parameters_file(parameters)
     elif isinstance(parameters, ParametersDict):
@@ -1620,4 +1682,4 @@ def make_model(parameters=None, verbose=False, name=None, genome_init='host'):
     else:
         raise ValueError('parameters must be a filepath, a dict or a ParametersDict')
     return Model(name or params.get('model', {}).get('name', 'unnamed_model'), params, verbose=verbose,
-                 genome_init=genome_init)
+                 genome_init=genome_init, strips=strips)

@@ -50,6 +50,7 @@ struct gnx_ctx {
   cudaStream_t stream = nullptr;
   cudaStream_t stream2 = nullptr;          // density chain of the fused step (one_step)
   int32_t* burnin_counts = nullptr;        // gnx_burnin_cell_stats: [2][Y][X] counts (now, previous call) + two sums
+  int32_t* strip_burnin = nullptr;         // gnx_strip_burnin_*: [2][ly1 - ly0][X] band counts + two sums + outside
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   // one fused step captured as a CUDA graph (every kernel reads its sizes from the device
   // counters, so the same graph serves every step); re-captured when any kernel argument changes
@@ -453,6 +454,7 @@ extern "C" int gnx_destroy(gnx_ctx* ctx) {
   if (ctx->strip_block) cudaFree(ctx->strip_block);
   if (ctx->d_paths) cudaFree(ctx->d_paths);
   if (ctx->burnin_counts) cudaFree(ctx->burnin_counts);
+  if (ctx->strip_burnin) cudaFree(ctx->strip_burnin);
   for (int k = 0; k < 2; ++k) if (ctx->d_surf_tab[k]) cudaFree(ctx->d_surf_tab[k]);
   if (ctx->stream) cudaStreamDestroy(ctx->stream);
   if (ctx->stream2) cudaStreamDestroy(ctx->stream2);
@@ -2597,6 +2599,71 @@ extern "C" int gnx_burnin_cell_stats(gnx_ctx* ctx, int64_t* sum_diff, int64_t* s
   PROF(ctx, "k_burnin_count");
   k_burnin_count<<<grid_for(ctx, 8), 256, 0, s>>>(ctx->pop, ctx->land, ctx->d_c, cur);
   LAUNCHED(ctx);
+  PROF(ctx, "k_burnin_diff");
+  k_burnin_diff<<<grid_for(ctx, 8), 256, 0, s>>>(cur, prev, ncell, sums);
+  LAUNCHED(ctx);
+  long long h[2] = {0, 0};
+  CK(cudaMemcpyAsync(h, sums, 16, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  *sum_diff = h[0];
+  *sum_sq_diff = h[1];
+  return GNX_OK;
+}
+
+// The statistic under strip decomposition: the rank's individuals counted into its band of landscape rows
+// [ly0, ly1) only (the host folds the row shared with the lower neighbour in between the two calls).
+// Layout of ctx->strip_burnin: cur [rows][X] | prev [rows][X] | two int64 sums | the out-of-band count.
+extern "C" int gnx_strip_burnin_count(gnx_ctx* ctx, int32_t* ly0, int32_t* ly1, void** first_row, void** last_row) {
+  ARG(ctx && ly0 && ly1 && first_row && last_row, "null");
+  USE_DEVICE(ctx);
+  if (!ctx->d_strip) { g_last_error = "gnx_strip_burnin_count: strip decomposition is not enabled"; return GNX_ERR_STATE; }
+  int r = materialise(ctx);
+  if (r != GNX_OK) return r;
+  const Strip& S = ctx->strip_h;
+  const int X = ctx->cfg.dim_x;
+  const size_t nband = (size_t)(S.ly1 - S.ly0) * X;
+  cudaStream_t s = ctx->stream;
+  if (!ctx->strip_burnin) {
+    CK(cudaMalloc((void**)&ctx->strip_burnin, (2 * nband + 6) * sizeof(int32_t)));
+    CK(cudaMemsetAsync(ctx->strip_burnin, 0, (2 * nband + 6) * sizeof(int32_t), s));
+  }
+  int32_t* cur = ctx->strip_burnin;
+  int32_t* outside = cur + 2 * nband + 4;
+  CK(cudaMemsetAsync(cur, 0, nband * sizeof(int32_t), s));
+  CK(cudaMemsetAsync(outside, 0, sizeof(int32_t), s));
+  PROF(ctx, "k_strip_burnin_count");
+  k_strip_burnin_count<<<grid_for(ctx, 8), 256, 0, s>>>(ctx->pop, ctx->land, ctx->d_c, S.ly0, S.ly1, cur, outside);
+  LAUNCHED(ctx);
+  int32_t h_out = 0;
+  CK(cudaMemcpyAsync(&h_out, outside, sizeof h_out, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  if (h_out) {
+    g_last_error = "gnx_strip_burnin_count: an individual lies outside the strip's landscape rows";
+    return GNX_ERR_STATE;
+  }
+  *ly0 = S.ly0;
+  *ly1 = S.ly1;
+  *first_row = cur;
+  *last_row = cur + (size_t)(S.ly1 - S.ly0 - 1) * X;
+  return GNX_OK;
+}
+
+extern "C" int gnx_strip_burnin_diff(gnx_ctx* ctx, int32_t skip_last_row, int64_t* sum_diff, int64_t* sum_sq_diff) {
+  ARG(ctx && sum_diff && sum_sq_diff, "null");
+  USE_DEVICE(ctx);
+  if (!ctx->d_strip || !ctx->strip_burnin) {
+    g_last_error = "gnx_strip_burnin_diff: no band counts (gnx_strip_burnin_count first)";
+    return GNX_ERR_STATE;
+  }
+  const Strip& S = ctx->strip_h;
+  const int X = ctx->cfg.dim_x;
+  const size_t nband = (size_t)(S.ly1 - S.ly0) * X;
+  const size_t ncell = nband - (skip_last_row ? (size_t)X : 0);
+  int32_t* cur = ctx->strip_burnin;
+  int32_t* prev = cur + nband;
+  long long* sums = reinterpret_cast<long long*>(prev + nband);
+  cudaStream_t s = ctx->stream;
+  CK(cudaMemsetAsync(sums, 0, 16, s));
   PROF(ctx, "k_burnin_diff");
   k_burnin_diff<<<grid_for(ctx, 8), 256, 0, s>>>(cur, prev, ncell, sums);
   LAUNCHED(ctx);

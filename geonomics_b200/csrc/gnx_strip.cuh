@@ -339,3 +339,20 @@ __global__ void __launch_bounds__(256) k_strip_barrier(const Strip* stp, int kin
     if (tid < W) st.pairs[tid] = reinterpret_cast<const volatile int64_t*>(mine + STRIP_SYNC_PAIRS)[tid];
   }
 }
+
+// Burn-in spatial statistic under strips (gnx_strip_burnin_count): this rank's individuals counted into its
+// band of landscape rows [ly0, ly1), row iy - ly0, with k_burnin_count's transposed tally; an individual
+// outside the band is counted in *outside (the caller reports it).
+__global__ void __launch_bounds__(256) k_strip_burnin_count(Pop pop, Land land, const Counters* c, int ly0, int ly1,
+                                                             int32_t* counts, int32_t* outside) {
+  const int n = c->n, cur = c->cur;
+  for (int p = GTID; p < n; p += GSTRIDE) {
+    const double2 xy = pop.xy[cur][p];
+    const int ix = (int)xy.x, iy = (int)xy.y;
+    if (iy < ly0 || iy >= ly1) {
+      atomicAdd(outside, 1);
+      continue;
+    }
+    if (ix < land.Y && iy < land.X) atomicAdd(&counts[(size_t)(iy - ly0) * land.X + ix], 1);
+  }
+}

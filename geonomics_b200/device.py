@@ -38,6 +38,36 @@ class _DevArray:
                                          'version': 2, 'strides': None}
 
 
+def stats_from_counts(c1, het, fit_sum, N):
+    """DeviceSpecies.stats from the device's counts (summed over the strips of a decomposed species)."""
+    Lg = len(c1)
+    freq = c1 / float(2 * N) if N else np.zeros(Lg)
+    return dict(N=N, freq=freq, het=het / float(N) if N else np.zeros(Lg),
+                maf=np.minimum(freq, 1 - freq), mean_fit=float(fit_sum) / N if N else float('nan'))
+
+
+def ld_from_counts(n11, n):
+    """DeviceSpecies.ld from the chromosome counts n11 [L, L] of n individuals."""
+    L = n11.shape[0]
+    N = 2 * int(n)                                        # chromosomes
+    n11 = n11.astype(np.float64)
+    n11 = np.triu(n11) + np.triu(n11, 1).T                # only one word-triangle is filled
+    f1 = np.diagonal(n11) / N
+    with np.errstate(divide='ignore', invalid='ignore'):
+        D = n11 / N - f1[:, None] * f1[None, :]
+        r2 = (D ** 2) / (((f1 * (1 - f1))[:, None] * f1[None, :]) * (1 - f1)[None, :])
+    # the reference fills (i, j) and (j, i) from the i < j evaluation
+    r2 = np.triu(r2, 1) + np.triu(r2, 1).T
+    r2[np.arange(L), np.arange(L)] = np.nan
+    return r2
+
+
+def cell_stats_from_sums(sum_diff, sum_sq_diff, ncell):
+    """(mean, std) of the per-cell count changes over ncell landscape cells from their sum and sum of squares."""
+    mean = sum_diff / float(ncell)
+    return mean, float(np.sqrt(max(sum_sq_diff / float(ncell) - mean * mean, 0.0)))
+
+
 class DeviceSpecies:
     """One Species resident on the GPU.
 
@@ -617,10 +647,8 @@ class DeviceSpecies:
         out['node_individual'] = np.repeat(out['first_individual_row'] + np.arange(nb), 2)
         return out
 
-    def stats(self, region=None):
-        """Per-locus statistics computed on the device from the packed genotypes
-        (sim/stats.py:399-435): dict(N, freq, het, maf, mean_fit).  region = (x_min, x_max,
-        y_min, y_max) restricts them to the individuals in that half-open rectangle."""
+    def stat_counts(self, region=None):
+        """The integer counts behind `stats` and the fitness sum: (c1 u64[L], het u64[L], fit_sum, n)."""
         c1 = np.zeros(max(1, self.Lg), dtype=np.uint64)
         het = np.zeros(max(1, self.Lg), dtype=np.uint64)
         fs = C.c_double()
@@ -629,41 +657,36 @@ class DeviceSpecies:
         _lib.check(self._L.gnx_stats_genotypes_region(
             self._ctx, float(x0), float(x1), float(y0), float(y1), c1.ctypes.data_as(C.POINTER(C.c_uint64)),
             het.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(fs), C.byref(n)), 'gnx_stats_genotypes_region')
-        N = int(n.value)
-        freq = c1[:self.Lg] / float(2 * N) if N else np.zeros(self.Lg)
-        return dict(N=N, freq=freq, het=het[:self.Lg] / float(N) if N else np.zeros(self.Lg),
-                    maf=np.minimum(freq, 1 - freq), mean_fit=float(fs.value) / N if N else float('nan'))
+        return c1[:self.Lg], het[:self.Lg], float(fs.value), int(n.value)
 
-    def ld(self):
-        """r^2 between every pair of loci (sim/stats.py:359-392 _calc_ld): the L x L matrix the
-        reference returns (NaN on the diagonal), formed with the reference's own expression from
-        the chromosome counts n11[i][j] that the device accumulates (gnx_stats_ld)."""
+    def stats(self, region=None):
+        """Per-locus statistics computed on the device from the packed genotypes
+        (sim/stats.py:399-435): dict(N, freq, het, maf, mean_fit).  region = (x_min, x_max,
+        y_min, y_max) restricts them to the individuals in that half-open rectangle."""
+        return stats_from_counts(*self.stat_counts(region))
+
+    def ld_counts(self):
+        """(n11 u64[L, L], n): the chromosome counts behind `ld` (gnx_stats_ld)."""
         L = self.Lg
         Lp = 32 * ((L + 31) // 32)
         n11 = np.zeros((Lp, Lp), dtype=np.uint64)
         n = C.c_int64()
         _lib.check(self._L.gnx_stats_ld(self._ctx, n11.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(n)),
                    'gnx_stats_ld')
-        N = 2 * int(n.value)                                  # chromosomes
-        n11 = n11[:L, :L].astype(np.float64)
-        n11 = np.triu(n11) + np.triu(n11, 1).T                # only one word-triangle is filled
-        f1 = np.diagonal(n11) / N
-        with np.errstate(divide='ignore', invalid='ignore'):
-            D = n11 / N - f1[:, None] * f1[None, :]
-            r2 = (D ** 2) / (((f1 * (1 - f1))[:, None] * f1[None, :]) * (1 - f1)[None, :])
-        # the reference fills (i, j) and (j, i) from the i < j evaluation
-        r2 = np.triu(r2, 1) + np.triu(r2, 1).T
-        r2[np.arange(L), np.arange(L)] = np.nan
-        return r2
+        return n11[:L, :L], int(n.value)
+
+    def ld(self):
+        """r^2 between every pair of loci (sim/stats.py:359-392 _calc_ld): the L x L matrix the
+        reference returns (NaN on the diagonal), formed with the reference's own expression from
+        the chromosome counts n11[i][j] that the device accumulates (gnx_stats_ld)."""
+        return ld_from_counts(*self.ld_counts())
 
     def burnin_cell_stats(self):
         """(mean, std) of the change of the per-cell individual counts since the previous call
         (sim/burnin.py:41-58 SpatialTester.update: np.mean(diff), np.std(diff))."""
         s1, s2 = C.c_int64(), C.c_int64()
         _lib.check(self._L.gnx_burnin_cell_stats(self._ctx, C.byref(s1), C.byref(s2)), 'gnx_burnin_cell_stats')
-        ncell = float(self.land_dim[0] * self.land_dim[1])
-        mean = s1.value / ncell
-        return mean, float(np.sqrt(max(s2.value / ncell - mean * mean, 0.0)))
+        return cell_stats_from_sums(s1.value, s2.value, self.land_dim[0] * self.land_dim[1])
 
     def fst(self, region_a, region_b, est_Hs=False):
         """Per-locus pairwise Fst = (Ht - Hs) / Ht between two rectangular sub-populations, as in the

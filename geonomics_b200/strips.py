@@ -26,7 +26,7 @@ import numpy as np
 
 from . import _lib
 from . import genome_pack as gp
-from .device import DeviceSpecies, _DevArray
+from .device import DeviceSpecies, _DevArray, cell_stats_from_sums, ld_from_counts, stats_from_counts
 
 
 # ---------------------------------------------------------------------------------------------
@@ -73,6 +73,29 @@ def owner_of(y, bounds, cell_size, ncy):
     """Rank that owns an individual at ordinate y (its mating-grid row, clamped like the kernel)."""
     row = np.minimum(np.floor(np.asarray(y) / cell_size).astype(np.int64), ncy - 1)
     return np.searchsorted(np.asarray(bounds)[1:-1], row, side='right')
+
+
+def band_rows(bounds, cell_size, dim_y):
+    """Landscape rows [ly0, ly1) that hold each rank's individuals, as gnx_strip_enable sets them: the rows
+    of y in [row0, row1) * cell_size.  A band ends on the row its upper neighbour's band starts on."""
+    b = np.asarray(bounds)
+    world = len(b) - 1
+    out = []
+    for r in range(world):
+        ly0 = max(0, int(np.floor(int(b[r]) * float(cell_size))))
+        ly1 = int(dim_y) if r == world - 1 else min(int(dim_y), int(np.floor(int(b[r + 1]) * float(cell_size))) + 1)
+        out.append((ly0, ly1))
+    return out
+
+
+def shared_band_rows(bands):
+    """The burn-in bookkeeping of rows that adjacent bands share: per rank, the lower ranks whose last band row
+    is this rank's first (their counts there are added into this rank's before the diff), and whether this
+    rank's last row is an upper rank's first (the row, and its previous counts, belong to the upper rank)."""
+    world = len(bands)
+    adds = [[q for q in range(r) if bands[q][1] - 1 == bands[r][0]] for r in range(world)]
+    skip_last = [any(bands[q][0] == bands[r][1] - 1 for q in range(r + 1, world)) for r in range(world)]
+    return adds, skip_last
 
 
 def phase_sequence(n_births_fixed):
@@ -151,6 +174,22 @@ class StripRank:
 
     def check(self):
         _lib.check(self.dev._L.gnx_strip_check(self.dev._ctx), 'gnx_strip_check')
+
+    def burnin_count(self):
+        """gnx_strip_burnin_count: (ly0, ly1, first band row, last band row), the rows as int32 torch views."""
+        import torch
+        a, b, f, l = C.c_int32(), C.c_int32(), C.c_void_p(), C.c_void_p()
+        _lib.check(self.dev._L.gnx_strip_burnin_count(self.dev._ctx, C.byref(a), C.byref(b), C.byref(f), C.byref(l)),
+                   'gnx_strip_burnin_count')
+        X = self.dev.land_dim[0]
+        return (a.value, b.value, torch.as_tensor(_DevArray(f.value, X, '<i4'), device='cuda'),
+                torch.as_tensor(_DevArray(l.value, X, '<i4'), device='cuda'))
+
+    def burnin_diff(self, skip_last_row):
+        s1, s2 = C.c_int64(), C.c_int64()
+        _lib.check(self.dev._L.gnx_strip_burnin_diff(self.dev._ctx, int(bool(skip_last_row)), C.byref(s1), C.byref(s2)),
+                   'gnx_strip_burnin_diff')
+        return int(s1.value), int(s2.value)
 
     def tensors(self):
         import torch
@@ -384,3 +423,189 @@ class NcclStrips:
 
     def close(self):
         self.me.dev.close()
+
+
+# ---------------------------------------------------------------------------------------------
+# one species over strips, behind the DeviceSpecies surface of api.Species
+# ---------------------------------------------------------------------------------------------
+def band_capacities(K, start_y, bounds, cell_size, ncy):
+    """Per-rank capacity: what DeviceSpecies gives a whole species (3 x the carrying capacity, twice the
+    starting size, at least 4096), taken over the rank's own band of mating-grid rows."""
+    b = np.asarray(bounds, dtype=np.int64)
+    kb = np.add.reduceat(row_weights_from_K(np.asarray(K, dtype=np.float64), cell_size, ncy), b[:-1])
+    nb = np.bincount(owner_of(start_y, b, cell_size, ncy), minlength=len(b) - 1) if len(start_y) else 0 * kb
+    return np.maximum(4096, np.maximum(3.0 * kb, 2.0 * nb)).astype(np.int64)
+
+
+class StripSpecies:
+    """One species cut into strips, with the members of DeviceSpecies that api.Species uses and species-wide
+    results.  `strips` is a strip count (LocalStrips: every strip a context of this process on the current
+    GPU, the host the barrier between the phases) or an initialised torch.distributed process group
+    (NcclStrips: this process's strip, device barriers, one graph per step).  Under a group every rank
+    makes the same calls in the same order and sees the whole species."""
+
+    def __init__(self, land_dim, rasters, prm, gen_arch, K, start_y, strips, seed=0, res_ratio=(1.0, 1.0),
+                 capacity=None):
+        self.land_dim = (int(land_dim[0]), int(land_dim[1]))
+        self.group = None if isinstance(strips, (int, np.integer)) else strips
+        if self.group is None:
+            self.world, self.rank = int(strips), None
+        else:
+            import torch.distributed as dist
+            self.world, self.rank = dist.get_world_size(self.group), dist.get_rank(self.group)
+        cs, ncx, ncy = mating_grid(self.land_dim, prm['mating_radius'])
+        bounds = plan_rows(ncy, self.world, row_weights_from_K(np.asarray(K, dtype=np.float64), cs, ncy))
+        self.bands = band_rows(bounds, cs, self.land_dim[1])
+        self._adds, self._skip_last = shared_band_rows(self.bands)
+        if capacity is None:
+            caps = band_capacities(K, np.asarray(start_y), bounds, cs, ncy)
+            capacity = int(caps.max() if self.group is None else caps[self.rank])
+        self.capacity = int(capacity)
+        kw = dict(seed=seed, bounds=bounds, res_ratio=res_ratio)
+        if self.group is None:
+            self._st = LocalStrips(self.world, self.land_dim, rasters, prm, gen_arch, self.capacity, **kw)
+            self._ranks = self._st.ranks
+        else:
+            self._st = NcclStrips(self.land_dim, rasters, prm, gen_arch, self.capacity, group=self.group, **kw)
+            self._ranks = [self._st.me]
+        self.Lg = self._ranks[0].dev.Lg
+
+    def _per_rank(self, fn):
+        """[fn(rank 0), ..., fn(rank world - 1)] on every rank (all-gathered under a group)."""
+        mine = [fn(r) for r in self._ranks]
+        if self.group is None:
+            return mine
+        import torch.distributed as dist
+        out = [None] * self.world
+        dist.all_gather_object(out, mine[0], group=self.group)
+        return out
+
+    def _each(self, name, *args, **kw):
+        for r in self._ranks:
+            getattr(r.dev, name)(*args, **kw)
+
+    @property
+    def _surf_tabs(self):
+        return self._ranks[0].dev._surf_tabs
+
+    # ---- setup: the same call on every strip
+    def set_burn(self, burn):
+        self._each('set_burn', burn)
+
+    def set_raster(self, layer, rast):
+        self._each('set_raster', layer, rast)
+
+    def set_K(self, K):
+        self._each('set_K', K)
+
+    def set_life_history(self, **changes):
+        self._each('set_life_history', **changes)
+
+    def set_surface_tables(self, move_tab=None, disp_tab=None):
+        self._each('set_surface_tables', move_tab, disp_tab)
+
+    def set_mutation(self, *args, **kw):
+        self._st.set_mutation(*args, **kw)
+
+    def read_mutations(self, max_rows=4096):
+        return self._st.read_mutations(max_rows)
+
+    def read_mutation_tables(self):
+        return self._ranks[0].dev.read_mutation_tables()
+
+    def init_genomes(self, p, seed, write_mask=None, tskit_rows=False):
+        if tskit_rows:
+            raise ValueError('strip decomposition does not carry tskit rows')
+        self._st.init_genomes(p, seed, write_mask)
+
+    # ---- population in / out
+    def upload(self, x, y, age=None, sex=None, idx=None, g=None, max_ind_idx=None, genomes_packed=None):
+        up = self._st.upload if self.group is None else self._st.upload_owned
+        up(x, y, age, sex, idx, g=g, genomes_packed=genomes_packed, max_ind_idx=max_ind_idx)
+
+    def _check(self):
+        """gnx_strip_check on every strip: a dropped migrant or a barrier timeout raises (on every rank)."""
+        if self.group is None:
+            for r in self._ranks:
+                r.check()
+            return
+        import torch
+        import torch.distributed as dist
+        err = None
+        try:
+            self._st.me.check()
+        except _lib.GnxError as e:
+            err = e
+        flag = torch.tensor([0 if err is None else 1], dtype=torch.int32, device='cuda')
+        dist.all_reduce(flag, op=dist.ReduceOp.MAX, group=self.group)
+        if err is not None:
+            raise err
+        if int(flag.item()):
+            raise RuntimeError('a strip rank of this species failed (see that rank\'s error)')
+
+    def step(self, n_steps=1):
+        self._st.step(n_steps)
+        self._check()
+
+    def step_records(self):
+        return merge_records(self._per_rank(lambda r: r.dev.step_records()))
+
+    def population_size(self):
+        return sum(self._per_rank(lambda r: r.dev.population_size()))
+
+    def download(self, genomes=True, unpack=True, e=False):
+        self._check()
+        out = merge_states(self._per_rank(lambda r: r.dev.download(genomes=genomes, unpack=False, e=e)))
+        if 'genomes' in out and unpack:
+            out['g'] = gp.unpack_genomes(out['genomes'], self.Lg)
+        return out
+
+    # ---- statistics: the integer counts add up over the strips, the fitness sum in rank order
+    def stats(self, region=None):
+        per = self._per_rank(lambda r: r.dev.stat_counts(region))
+        c1 = sum(p[0] for p in per)
+        het = sum(p[1] for p in per)
+        fs = 0.0
+        for p in per:
+            fs += p[2]
+        return stats_from_counts(c1, het, fs, sum(p[3] for p in per))
+
+    def ld(self):
+        per = self._per_rank(lambda r: r.dev.ld_counts())
+        return ld_from_counts(sum(p[0] for p in per), sum(p[1] for p in per))
+
+    def raster(self, field):
+        """A landscape raster of the last step, each band's rows from the rank that computes them (a row two
+        bands share from the upper one)."""
+        per = self._per_rank(lambda r: r.dev.raster(field)[slice(*self.bands[r.rank])])
+        out = None
+        for (ly0, ly1), rows in zip(self.bands, per):
+            if out is None:
+                out = np.zeros((self.land_dim[1],) + rows.shape[1:], dtype=rows.dtype)
+            out[ly0:ly1] = rows
+        return out
+
+    def burnin_cell_stats(self):
+        """DeviceSpecies.burnin_cell_stats of the whole species: every rank counts into its band, the rows two
+        bands share are added into the upper band, and each rank sums the change over the rows it accounts for."""
+        import torch
+        got = {r.rank: r.burnin_count() for r in self._ranks}
+        for k, (ly0, ly1, _, _) in got.items():
+            assert (ly0, ly1) == self.bands[k], 'strip band rows differ from the host plan'
+        if self.group is None:
+            lasts = [got[k][3].clone() for k in range(self.world)]
+        else:
+            import torch.distributed as dist
+            X = self.land_dim[0]
+            allrows = torch.empty(self.world * X, dtype=torch.int32, device='cuda')
+            dist.all_gather_into_tensor(allrows, got[self.rank][3].clone(), group=self.group)
+            lasts = list(allrows.view(self.world, X))
+        for k, (_, _, first, _) in got.items():
+            for q in self._adds[k]:
+                first += lasts[q]
+        torch.cuda.synchronize()
+        per = self._per_rank(lambda r: r.burnin_diff(self._skip_last[r.rank]))
+        return cell_stats_from_sums(sum(p[0] for p in per), sum(p[1] for p in per), self.land_dim[0] * self.land_dim[1])
+
+    def close(self):
+        self._st.close()

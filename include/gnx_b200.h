@@ -481,6 +481,20 @@ int gnx_stats_ld(gnx_ctx* ctx, uint64_t* host_n11, int64_t* n);
  * compares with all-zero counts, as SpatialTester.__init__ does).  mean(diff) and std(diff) over the
  * dim_x * dim_y cells follow from the two integers.  Synchronises. */
 int gnx_burnin_cell_stats(gnx_ctx* ctx, int64_t* sum_diff, int64_t* sum_sq_diff);
+/* The same statistic for a species cut into strips, in two calls per rank and burn-in step.  A rank's
+ * individuals lie in its landscape rows [ly0, ly1) (gnx_strip_enable), and the band of a rank ends on the
+ * row its upper neighbour's band starts on whenever a mating-grid row boundary falls inside a landscape row.
+ * gnx_strip_burnin_count counts this rank's individuals into a band raster of (ly1 - ly0) x dim_x int32
+ * with the transposed tally of gnx_burnin_cell_stats (cell (ix, iy) counted at row iy - ly0, column ix, only
+ * for ix < dim_y and iy < dim_x), and returns the band and the device addresses of its first and last rows
+ * (dim_x int32 each).  Before gnx_strip_burnin_diff the caller adds the lower neighbour's last row into this
+ * rank's first row when they are the same landscape row.  gnx_strip_burnin_diff then returns the sum and the
+ * sum of squares of the change of the band's counts since the previous call, over every band row except the
+ * last one when skip_last_row (a shared row belongs to the upper rank).  The species-wide sums are the sums
+ * over the ranks, equal to gnx_burnin_cell_stats of the undecomposed population.  Both synchronise; an
+ * individual outside [ly0, ly1) -> GNX_ERR_STATE; GNX_ERR_STATE without strip decomposition. */
+int gnx_strip_burnin_count(gnx_ctx* ctx, int32_t* ly0, int32_t* ly1, void** first_row, void** last_row);
+int gnx_strip_burnin_diff(gnx_ctx* ctx, int32_t skip_last_row, int64_t* sum_diff, int64_t* sum_sq_diff);
 
 /* ---- introspection (parity tests, lazy API views) -------------------------------------- */
 enum {
