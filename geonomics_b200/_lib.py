@@ -184,7 +184,7 @@ FIELDS = dict(
     X=1, Y=2, AGE=3, SEX=4, IDX=5, Z=6, FIT=7, GSLOT=8, N_NBRS=9, MATE=10, PAIRS=11, NB=12,
     PERM=13, CELL_START=14, COUNTS_N=15, COUNTS_P=16, VALS_N=17, VALS_P=18, GRAD_N=19, GRAD_P=20,
     N_RAST=21, NPAIRS_RAST=22, D_RAST=23, K_RAST=24, DEATH_P=25, ALIVE=26, DISP_TRIES=27, E=28,
-    COUNTERS=29, GENOMES=30, NODE0=31, NODE1=32)
+    COUNTERS=29, GENOMES=30, NODE0=31, NODE1=32, VM_TAB_MOVE=33, VM_TAB_DISP=34)
 
 # every exported entry point: name -> (restype, argtypes)
 _ctx = C.c_void_p

@@ -2430,6 +2430,12 @@ extern "C" int gnx_device_ptr(gnx_ctx* ctx, int32_t field, void** dev_ptr, int64
     case GNX_F_K_RAST: p = ctx->d_K; b = plane * 8; break;
     case GNX_F_DISP_TRIES: p = W.disp_tries; b = (size_t)h.B * 4; break;
     case GNX_F_COUNTERS: p = ctx->d_c; b = sizeof(Counters); break;
+    case GNX_F_VM_TAB_MOVE:
+    case GNX_F_VM_TAB_DISP: {
+      const int k = field == GNX_F_VM_TAB_DISP ? 1 : 0;
+      if (!ctx->prm.vm_tab[k]) { g_last_error = "that site's conductance surface is not on the fly"; return GNX_ERR_STATE; }
+      p = const_cast<float*>(ctx->prm.vm_tab[k]); b = (size_t)VM_TAB_LEN * 4; break;
+    }
     default: g_last_error = "unknown field"; return GNX_ERR_ARG;
   }
   CK(cudaGetLastError());

@@ -23,6 +23,7 @@ _DT = {
     'N_RAST': np.float64, 'NPAIRS_RAST': np.float64, 'D_RAST': np.float64, 'K_RAST': np.float64,
     'DEATH_P': np.float64, 'ALIVE': np.uint8, 'DISP_TRIES': np.int32, 'E': np.float64, 'Z': np.float64,
     'COUNTERS': np.int32, 'GENOMES': np.uint32, 'NODE0': np.int32, 'NODE1': np.int32,
+    'VM_TAB_MOVE': np.float32, 'VM_TAB_DISP': np.float32,
 }
 
 

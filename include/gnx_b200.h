@@ -503,7 +503,9 @@ enum {
   GNX_F_COUNTS_N, GNX_F_COUNTS_P, GNX_F_VALS_N, GNX_F_VALS_P, GNX_F_GRAD_N, GNX_F_GRAD_P,
   GNX_F_N_RAST, GNX_F_NPAIRS_RAST, GNX_F_D_RAST, GNX_F_K_RAST, GNX_F_DEATH_P, GNX_F_ALIVE,
   GNX_F_DISP_TRIES, GNX_F_E, GNX_F_COUNTERS, GNX_F_GENOMES,
-  GNX_F_NODE0, GNX_F_NODE1     /* tskit node id of homologue 0 / 1 (int32, Individual._nodes_tab_ids) */
+  GNX_F_NODE0, GNX_F_NODE1,    /* tskit node id of homologue 0 / 1 (int32, Individual._nodes_tab_ids) */
+  GNX_F_VM_TAB_MOVE, GNX_F_VM_TAB_DISP  /* von Mises inverse-CDF table of an on-the-fly surface (float32
+                                           [4096 + 1 + 256 + 1]); GNX_ERR_STATE when that site is not on the fly */
 };
 /* Copies a device field into a host buffer (synchronises).  For per-individual fields the
  * first `count` elements in species order are returned. */

@@ -107,3 +107,140 @@ def lognormal_f32(w1, w2, p1, p2):
     d = np.exp(arg)
     rel = abs(p2) * e_z + np.abs(arg) * 2 * _F32 + _EXPF
     return d, rel
+
+
+def wald_f32(w1, w2, w3, mean, scale):
+    """sample_distance_f32 for the Wald (numpy legacy): with Y = mean z^2 (z = normal_f32(w1, w2)),
+    X = mean + mean / (2 scale) (Y - sqrtf(4 scale Y + Y^2)), U = uniform_f32(w3), the distance is X when
+    U <= mean / (mean + X) and mean^2 / X otherwise.  Returns (distance in float64, relative bound,
+    ambiguous): `ambiguous` flags the draws whose U lies within the bound of the threshold, where the
+    device may take the other branch.  The subtraction Y - sqrt(...) cancels for large Y; the bound
+    carries the float32 roundings of Y and of the square root through it."""
+    assert float(np.float32(mean)) == mean and float(np.float32(scale)) == scale, 'use float32-exact parameters'
+    mu_2l = float(np.float32(mean) / (np.float32(2.0) * np.float32(scale)))     # the device's float32 value
+    z, e_z = normal_f32(w1, w2)
+    Y = mean * z * z
+    e_Y = mean * (2 * np.abs(z) * e_z + e_z * e_z) + Y * 2 * _F32
+    S = 4 * scale * Y + Y * Y
+    e_S = (4 * scale + 2 * Y + e_Y) * e_Y + S * 3 * _F32
+    R = np.sqrt(S)
+    e_R = np.minimum(np.sqrt(e_S), e_S / np.maximum(2 * R, 1e-300)) + R * _F32
+    D = Y - R
+    e_D = e_Y + e_R + np.abs(D) * _F32
+    X = mean + mu_2l * D
+    e_X = mu_2l * e_D + (np.abs(mu_2l * D) + np.abs(X)) * _F32
+    U = uniform_f32(w3).astype(np.float64)
+    T = mean / (mean + X)
+    e_T = T * (e_X / np.abs(mean + X) + 2 * _F32)
+    first = U <= T
+    with np.errstate(divide='ignore', invalid='ignore'):
+        d = np.where(first, X, mean * mean / X)
+        rel = np.where(first, e_X / X, e_X / X + 2 * _F32)
+    ambiguous = (np.abs(U - T) <= e_T) | ~(rel < 0.01)        # near the threshold, or X not resolved
+    return d, rel, ambiguous
+
+
+# ---- the on-the-fly conductance-surface direction (gnx_kernels.cuh vonmises_tab, surface_direction_from_neigh) ----
+VM_TAB_CELLS, VM_TAB_FINE = 4096, 256
+VM_TAB_LEN = VM_TAB_CELLS + 1 + VM_TAB_FINE + 1
+PI_F = np.float32(3.14159265358979)
+# the directions of the 8 queen neighbours in row-major order, as the device's float32 constants
+SURF_DIRS = np.array([np.float32(-3) * PI_F / np.float32(4), -PI_F / np.float32(2), -PI_F / np.float32(4), PI_F,
+                      np.float32(0), np.float32(3) * PI_F / np.float32(4), PI_F / np.float32(2), PI_F / np.float32(4)],
+                     dtype=np.float32)
+
+
+def _round_f32(q):
+    """A Fraction rounded to the nearest float32, ties to even."""
+    from fractions import Fraction
+    x = np.float32(float(q))
+    best = None
+    for c in (np.nextafter(x, np.float32(-np.inf)), x, np.nextafter(x, np.float32(np.inf))):
+        d = abs(Fraction(float(c)) - q)
+        if best is None or d < best[0] or (d == best[0] and (int(np.float32(c).view(np.uint32)) & 1) == 0):
+            best = (d, c)
+    return np.float32(best[1])
+
+
+def fma_f32(a, b, c):
+    """fmaf(a, b, c) on float32 arrays: a b is exact in float64; when the float64 sum s = a b + c is exact
+    too (TwoSum error term zero) it is rounded to float32 once.  Otherwise s differs from the exact sum x,
+    and rounding s to float32 can only go wrong when s sits exactly on a float32 midpoint (midpoints are
+    float64 numbers and rounding to float64 is monotone, so x and s lie strictly on the same side of every
+    other midpoint); those sums are rounded from a Fraction of the exact value."""
+    from fractions import Fraction
+    a, b, c = np.broadcast_arrays(*(np.atleast_1d(np.asarray(v, dtype=np.float32)) for v in (a, b, c)))
+    p = a.astype(np.float64) * b.astype(np.float64)
+    cc = np.broadcast_to(c.astype(np.float64), p.shape)
+    s = p + cc
+    bp = s - p
+    err = (p - (s - bp)) + (cc - bp)
+    out = np.asarray(s.astype(np.float32))
+    s32 = out.astype(np.float64)
+    nb = np.nextafter(out, np.where(s > s32, np.float32(np.inf), np.float32(-np.inf)).astype(np.float32))
+    mid = (s != s32) & (s == (s32 + nb.astype(np.float64)) / 2)
+    for i in zip(*np.nonzero((err != 0) & mid)):
+        out[i] = _round_f32(Fraction(float(p[i])) + Fraction(float(cc[i])))
+    return out
+
+
+def vonmises_tab(r, tab):
+    """vonmises_tab for kappa >= 1e-8 from the word r: float32 |theta| interpolated in the quantile table,
+    negated when bit 31 is set."""
+    r = np.asarray(r, dtype=np.uint32)
+    tab = np.asarray(tab, dtype=np.float32)
+    v = (r << np.uint32(1)).astype(np.uint32)
+    k = (v >> np.uint32(20)).astype(np.int64)
+    coarse = k < VM_TAB_CELLS - 1
+    k2 = ((v >> np.uint32(12)) & np.uint32(0xff)).astype(np.int64)
+    f = np.where(coarse, ((v >> np.uint32(1)) & np.uint32(0x7ffff)).astype(np.float32) * np.float32(1.0 / 524288.0),
+                 ((v >> np.uint32(1)) & np.uint32(0x7ff)).astype(np.float32) * np.float32(1.0 / 2048.0))
+    ia = np.where(coarse, k, VM_TAB_CELLS + 1 + k2)
+    a, b = tab[ia], tab[ia + 1]
+    res = fma_f32(f, b - a, a)
+    return np.where((r >> np.uint32(31)) != 0, -res, res)
+
+
+def surface_direction(words, k, nv, mixture, kappa, tab):
+    """surface_direction_from_neigh in float32 for each row: the neighbourhood nv (float32[n, 8], row-major
+    queen neighbours of the zero-embedded raster), the stream's words from column k (int or int[n]).
+    Returns (float16 direction, number of words used): the mixture draw (one uniform_f32 word) when
+    `mixture`, then one von Mises word (the table word, or a uniform_f32 word when kappa < 1e-8)."""
+    words = np.asarray(words, dtype=np.uint32)
+    nv = np.asarray(nv, dtype=np.float32)
+    n = nv.shape[0]
+    rows = np.arange(n)
+    k = np.broadcast_to(np.asarray(k, dtype=np.int64), (n,))
+    s = np.zeros(n, np.float32)
+    for j in range(8):
+        s = s + nv[:, j]
+    if mixture:
+        pos = s > 0
+        target = uniform_f32(words[rows, k]) * np.where(pos, s, np.float32(8))
+        acc = np.zeros(n, np.float32)
+        loc = np.full(n, SURF_DIRS[7], np.float32)
+        found = np.zeros(n, bool)
+        for j in range(8):
+            acc = acc + np.where(pos, nv[:, j], np.float32(1))
+            hit = ~found & (target < acc)
+            loc[hit] = SURF_DIRS[j]
+            found |= hit
+        kv = k + 1
+    else:
+        mx = nv.max(axis=1)
+        sacc = np.zeros(n, np.float32)
+        cnt = np.zeros(n, np.float32)
+        for j in range(8):
+            m = nv[:, j] == mx
+            sacc = np.where(m, sacc + SURF_DIRS[j], sacc)
+            cnt = cnt + m.astype(np.float32)
+        loc = sacc / cnt
+        kv = k
+    wv = words[rows, kv]
+    if np.float32(kappa) < np.float32(1e-8):
+        vm = PI_F * (np.float32(2) * uniform_f32(wv) - np.float32(1))
+    else:
+        vm = vonmises_tab(wv, tab)
+    v = (loc + vm).astype(np.float32)
+    v = np.where(v >= PI_F, v - np.float32(2) * PI_F, np.where(v < -PI_F, v + np.float32(2) * PI_F, v))
+    return v.astype(np.float32).astype(np.float16), (kv - k + 1)
