@@ -648,7 +648,7 @@ class Species:
                 self.mut_log = '%s_mutations.log' % name
         self.mutations = []                    # drained device mutation log (dict rows)
         self._seed = seed
-        self._strips = strips                  # None, a strip count or a process group (strips.StripSpecies)
+        self._strips = strips                  # None, a strip count or a process group (strips.LocalStrips, NcclStrips)
         self._tc = None                        # tskit tables as numpy columns (tables.TableColumns), use_tskit only
         self._dev = None
         self._cache = None                     # host copy of the device state (lazy)
@@ -694,9 +694,12 @@ class Species:
                       dom=np.asarray(self.gen_arch.dom, dtype=np.int8))
         p = self._init_pop
         if self._strips is not None:
-            from .strips import StripSpecies
-            self._dev = StripSpecies(land.dim, rasters, self._device_params(), ga, self.K, p['y'], self._strips,
-                                     seed=self._seed, res_ratio=self._land_res_ratio, capacity=capacity)
+            from .strips import LocalStrips, NcclStrips
+            kw = dict(seed=self._seed, res_ratio=self._land_res_ratio, K=self.K, start_y=p['y'])
+            if isinstance(self._strips, (int, np.integer)):
+                self._dev = LocalStrips(self._strips, land.dim, rasters, self._device_params(), ga, capacity, **kw)
+            else:
+                self._dev = NcclStrips(land.dim, rasters, self._device_params(), ga, capacity, group=self._strips, **kw)
         else:
             if capacity is None:
                 capacity = int(max(4096, 3.0 * float(np.sum(self.K)), 2 * self.start_N))

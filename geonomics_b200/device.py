@@ -566,27 +566,15 @@ class DeviceSpecies:
         o = np.lexsort((hom, idx, site))
         return dict(site=site[o], idx=idx[o], homologue=hom[o])
 
-    def init_genomes(self, p, seed, write_mask=None, tskit_rows=False, allreduce=None):
+    def init_genomes(self, p, seed, write_mask=None, tskit_rows=False):
         """Assign the starting genomes on the device (the post-burn-in assignment of species.py:956-1094
         without a host genotype array): locus l gets exactly genome_pack.carrier_counts(n, p)[l] 1-alleles,
         on the homologues with the smallest Philox keys (include/gnx_b200.h).  write_mask [L]: loci whose
         bits are set (the non-neutral loci of the tskit layout), None: all.  tskit_rows: return the
-        starting carriers of every locus (genome_init_rows).  allreduce: an in-place sum over the ranks of
-        a strip-decomposed landscape (e.g. torch.distributed.all_reduce) applied to the population size and
-        to the histograms, so every rank makes the same selection."""
-        import torch
-        n = self.population_size()
-        if allreduce is not None:
-            t = torch.tensor([n], dtype=torch.int64, device='cuda')
-            allreduce(t)
-            n = int(t.item())
-        hist = self.genome_init_begin(gp.carrier_counts(n, p), seed, write_mask, tskit_rows)
-        while True:
-            if allreduce is not None:
-                allreduce(hist)
-                torch.cuda.synchronize()
-            if self.genome_init_pass():
-                break
+        starting carriers of every locus (genome_init_rows)."""
+        self.genome_init_begin(gp.carrier_counts(self.population_size(), p), seed, write_mask, tskit_rows)
+        while not self.genome_init_pass():
+            pass
         self.genome_init_end()
         return self.genome_init_rows() if tskit_rows else None
 

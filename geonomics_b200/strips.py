@@ -11,10 +11,13 @@ individuals go where at upload) and, where the host sequences the phases, the ba
 them and the small collectives (births all-gather, density-count sum, max(N), and with Poisson
 births the pairs all-gather).
 
-Two transports:
+One species over strips is one object: `_Strips` holds the plan and every species-wide operation
+(setters, upload, download, step records, statistics, the burn-in statistic, genome assignment),
+written once over the ranks that live in this process; two subclasses supply the transport:
   * `NcclStrips`   one process per GPU (`torch.distributed`, backend nccl, which only exchanges
                    the CUDA IPC handles): the barrier and the collectives are one-CTA kernels
-                   over peer memory (gnx_strip_barrier) inside each step's CUDA graph.
+                   over peer memory (gnx_strip_barrier) inside each step's CUDA graph; species-wide
+                   results are gathered over the group.
   * `LocalStrips`  all ranks as contexts of ONE process on one GPU (tests; a box with fewer GPUs
                    than ranks): the same kernels write into the other contexts' buffers, the
                    host runs each phase on every context before the next and does the
@@ -200,41 +203,77 @@ class StripRank:
         return births, counts, nmax, pairs
 
 
-def _subset(pop, mask):
-    return {k: (v[mask] if isinstance(v, np.ndarray) and v.ndim >= 1 and len(v) == len(mask) else v)
-            for k, v in pop.items()}
-
-
 # ---------------------------------------------------------------------------------------------
-# all ranks in one process (tests / fewer GPUs than ranks)
+# one species over strips: the plan and every species-wide operation
 # ---------------------------------------------------------------------------------------------
-class LocalStrips:
-    """`world` strips as contexts of this process on the current GPU."""
+def band_capacities(K, start_y, bounds, cell_size, ncy):
+    """Per-rank capacity: what DeviceSpecies gives a whole species (3 x the carrying capacity, twice the
+    starting size, at least 4096), taken over the rank's own band of mating-grid rows."""
+    b = np.asarray(bounds, dtype=np.int64)
+    kb = np.add.reduceat(row_weights_from_K(np.asarray(K, dtype=np.float64), cell_size, ncy), b[:-1])
+    nb = np.bincount(owner_of(start_y, b, cell_size, ncy), minlength=len(b) - 1) if len(start_y) else 0 * kb
+    return np.maximum(4096, np.maximum(3.0 * kb, 2.0 * nb)).astype(np.int64)
 
-    def __init__(self, world, land_dim, rasters, prm, gen_arch, capacity, seed=0, bounds=None, device_barrier=False,
-                 **kw):
-        import torch
-        self.torch = torch
+
+class _Strips:
+    """One species cut into `world` strips, of which `self.ranks` live in this process, with the members of
+    DeviceSpecies that api.Species uses and species-wide results.  The subclasses supply the transport: how
+    the ranks are connected, how a step is sequenced, and the primitives that combine the ranks' values:
+      _gather(fn)        [fn(rank 0), ..., fn(rank world - 1)]
+      _sum(tensors)      one tensor per rank of this process, each replaced by the sum over all ranks
+                         (on the device when the call returns)
+      _gather_rows(rows) one row per rank of this process in, every rank's row out ([world, len(row)])
+      _check()           gnx_strip_check on every strip; a failure on any rank raises on every rank
+    Where the ranks live in several processes, every process makes the same calls in the same order and sees
+    the whole species.
+
+    The plan: the mating grid, the first mating-grid row of every rank (`bounds`: given, or cut by the
+    carrying capacity `K`, which defaults to the K layer of `rasters`), the landscape rows of each rank's
+    band and the rows that adjacent bands share.  capacity None: each rank's band_capacities from `K` and the
+    starting ordinates `start_y`; the ranks of one process share the largest."""
+
+    def __init__(self, world, mine, land_dim, rasters, prm, gen_arch, capacity, seed, bounds=None, K=None,
+                 start_y=(), **kw):
         self.world = int(world)
-        # device_barrier: the ranks synchronise through gnx_strip_barrier (no host round trip inside a step);
-        # otherwise the host is the barrier and does the three collectives on the ranks' tensors
-        self.device_barrier = bool(device_barrier)
-        self._warm = False
+        self.land_dim = (int(land_dim[0]), int(land_dim[1]))
         self.cs, self.ncx, self.ncy = mating_grid(land_dim, prm['mating_radius'])
-        K = np.asarray(rasters)[int(prm.get('K_layer', 0))] * float(prm.get('K_factor', 1.0))
-        self.bounds = plan_rows(self.ncy, world, row_weights_from_K(K, self.cs, self.ncy)) if bounds is None \
+        K = np.asarray(rasters)[int(prm.get('K_layer', 0))] * float(prm.get('K_factor', 1.0)) if K is None \
+            else np.asarray(K, dtype=np.float64)
+        self.bounds = plan_rows(self.ncy, self.world, row_weights_from_K(K, self.cs, self.ncy)) if bounds is None \
             else np.asarray(bounds, dtype=np.int32)
-        self.ranks = [StripRank(r, world, self.bounds, land_dim, rasters, prm, gen_arch, capacity, seed, **kw)
-                      for r in range(world)]
-        for a in self.ranks:
-            for b in self.ranks:
-                if a is not b:
-                    a.connect(b.rank, b.endpoints, same_process=True)
-        self._t = [r.tensors() for r in self.ranks]
+        self.bands = band_rows(self.bounds, self.cs, self.land_dim[1])
+        self._adds, self._skip_last = shared_band_rows(self.bands)
+        if capacity is None:
+            capacity = band_capacities(K, np.asarray(start_y), self.bounds, self.cs, self.ncy)[list(mine)].max()
+        self.capacity = int(capacity)
+        self.ranks = [StripRank(r, self.world, self.bounds, land_dim, rasters, prm, gen_arch, self.capacity, seed,
+                                **kw) for r in mine]
+        self.Lg = self.ranks[0].dev.Lg
 
+    @property
+    def _surf_tabs(self):
+        return self.ranks[0].dev._surf_tabs
+
+    # ---- setup: the same call on every strip
     def set_burn(self, burn):
         for r in self.ranks:
             r.dev.set_burn(burn)
+
+    def set_raster(self, layer, rast):
+        for r in self.ranks:
+            r.dev.set_raster(layer, rast)
+
+    def set_K(self, K):
+        for r in self.ranks:
+            r.dev.set_K(K)
+
+    def set_life_history(self, **changes):
+        for r in self.ranks:
+            r.dev.set_life_history(**changes)
+
+    def set_surface_tables(self, move_tab=None, disp_tab=None):
+        for r in self.ranks:
+            r.dev.set_surface_tables(move_tab, disp_tab)
 
     def set_mutation(self, *args, **kw):
         """Mutation of each step's offspring (DeviceSpecies.set_mutation, by-locus layout): every rank gets
@@ -243,33 +282,32 @@ class LocalStrips:
             r.dev.set_mutation(*args, **kw)
 
     def read_mutations(self, max_rows=4096):
-        """Drain every rank's mutation log; each must equal the undecomposed run's, so they must agree.
-        Returns rank 0's (rows, state) as DeviceSpecies.read_mutations does."""
-        for r in self.ranks:
-            r.check()
+        """Drain the mutation logs; each rank's must equal the undecomposed run's, so the ranks of this
+        process must agree.  Returns (rows, state) as DeviceSpecies.read_mutations does."""
+        self._check()
         out = [r.dev.read_mutations(max_rows) for r in self.ranks]
         rows0, st0 = out[0]
-        for rank, (rows, st) in enumerate(out[1:], 1):
+        for r, (rows, st) in zip(self.ranks[1:], out[1:]):
             same = rows == rows0 and st['n_mutables'] == st0['n_mutables'] and \
                 all(np.array_equal(st[k], st0[k]) for k in ('nonneut_loci', 'delet_loci', 'delet_s'))
             if not same:
-                raise RuntimeError('strip rank %d: mutation log or tables differ from rank 0' % rank)
+                raise RuntimeError('strip rank %d: mutation log or tables differ from rank %d'
+                                   % (r.rank, self.ranks[0].rank))
         return rows0, st0
 
-    def init_genomes(self, p, seed, write_mask=None):
+    def read_mutation_tables(self):
+        return self.ranks[0].dev.read_mutation_tables()
+
+    def init_genomes(self, p, seed, write_mask=None, tskit_rows=False):
         """DeviceSpecies.init_genomes over the strips: the counts follow the species-wide size, the ranks'
         histograms are summed between the passes and every rank makes the same selection, so the genomes
         equal those of the undecomposed population."""
-        torch = self.torch
-        n = sum(self.population_sizes())
-        counts = gp.carrier_counts(n, p)
+        if tskit_rows:
+            raise ValueError('strip decomposition does not carry tskit rows')
+        counts = gp.carrier_counts(self.population_size(), p)
         hists = [r.dev.genome_init_begin(counts, seed, write_mask) for r in self.ranks]
         while True:
-            torch.cuda.synchronize()
-            tot = torch.stack(hists).sum(dim=0, dtype=torch.int32)
-            for h in hists:
-                h.copy_(tot)
-            torch.cuda.synchronize()
+            self._sum(hists)
             done = [r.dev.genome_init_pass() for r in self.ranks]
             assert len(set(done)) == 1, 'strip ranks disagree on the genome selection'
             if done[0]:
@@ -277,24 +315,123 @@ class LocalStrips:
         for r in self.ranks:
             r.dev.genome_init_end()
 
-    def upload(self, x, y, age=None, sex=None, idx=None, g=None, genomes_packed=None, max_ind_idx=None):
-        n = len(x)
-        idx = np.arange(n, dtype=np.int64) if idx is None else np.asarray(idx)
-        max_ind_idx = int(idx.max()) if (max_ind_idx is None and n) else max_ind_idx
+    # ---- population in / out
+    def upload(self, x, y, age=None, sex=None, idx=None, g=None, max_ind_idx=None, genomes_packed=None):
+        """Upload each rank's share of a population every process holds on the host."""
+        idx = np.arange(len(x), dtype=np.int64) if idx is None else np.asarray(idx)
+        if max_ind_idx is None and len(idx):
+            max_ind_idx = int(idx.max())
+        cols = dict(x=x, y=y, age=age, sex=sex, idx=idx, g=g, genomes_packed=genomes_packed)
         own = owner_of(y, self.bounds, self.cs, self.ncy)
         for r in self.ranks:
             m = own == r.rank
-            r.dev.upload(x[m], y[m], None if age is None else age[m], None if sex is None else sex[m], idx[m],
-                         g=None if g is None else g[m],
-                         genomes_packed=None if genomes_packed is None else genomes_packed[m],
-                         max_ind_idx=max_ind_idx)
+            r.dev.upload(**{k: None if v is None else v[m] for k, v in cols.items()}, max_ind_idx=max_ind_idx)
+
+    def step_records(self):
+        """Species-wide records of the steps since the last call, after the strips are checked: a dropped
+        migrant or a barrier timeout raises here (on every rank)."""
+        self._check()
+        return merge_records(self._gather(lambda r: r.dev.step_records()))
+
+    def population_size(self):
+        return sum(self._gather(lambda r: r.dev.population_size()))
+
+    def download(self, genomes=True, unpack=True, e=False):
+        self._check()
+        out = merge_states(self._gather(lambda r: r.dev.download(genomes=genomes, unpack=False, e=e)))
+        if 'genomes' in out and unpack:
+            out['g'] = gp.unpack_genomes(out['genomes'], self.Lg)
+        return out
+
+    # ---- statistics: the integer counts add up over the strips, the fitness sum in rank order
+    def stats(self, region=None):
+        per = self._gather(lambda r: r.dev.stat_counts(region))
+        c1 = sum(p[0] for p in per)
+        het = sum(p[1] for p in per)
+        fs = 0.0
+        for p in per:
+            fs += p[2]
+        return stats_from_counts(c1, het, fs, sum(p[3] for p in per))
+
+    def ld(self):
+        per = self._gather(lambda r: r.dev.ld_counts())
+        return ld_from_counts(sum(p[0] for p in per), sum(p[1] for p in per))
+
+    def raster(self, field):
+        """A landscape raster of the last step, each band's rows from the rank that computes them (a row two
+        bands share from the upper one)."""
+        per = self._gather(lambda r: r.dev.raster(field)[slice(*self.bands[r.rank])])
+        out = None
+        for (ly0, ly1), rows in zip(self.bands, per):
+            if out is None:
+                out = np.zeros((self.land_dim[1],) + rows.shape[1:], dtype=rows.dtype)
+            out[ly0:ly1] = rows
+        return out
+
+    def burnin_cell_stats(self):
+        """DeviceSpecies.burnin_cell_stats of the whole species: every rank counts into its band, the rows two
+        bands share are added into the upper band, and each rank sums the change over the rows it accounts for."""
+        import torch
+        got = [r.burnin_count() for r in self.ranks]
+        for r, (ly0, ly1, _, _) in zip(self.ranks, got):
+            assert (ly0, ly1) == self.bands[r.rank], 'strip band rows differ from the host plan'
+        lasts = self._gather_rows([last for _, _, _, last in got])
+        for r, (_, _, first, _) in zip(self.ranks, got):
+            for q in self._adds[r.rank]:
+                first += lasts[q]
+        torch.cuda.synchronize()
+        per = self._gather(lambda r: r.burnin_diff(self._skip_last[r.rank]))
+        return cell_stats_from_sums(sum(p[0] for p in per), sum(p[1] for p in per), self.land_dim[0] * self.land_dim[1])
+
+    def close(self):
+        for r in self.ranks:
+            r.dev.close()
+
+
+# ---------------------------------------------------------------------------------------------
+# all ranks in one process (tests / fewer GPUs than ranks)
+# ---------------------------------------------------------------------------------------------
+class LocalStrips(_Strips):
+    """`world` strips as contexts of this process on the current GPU."""
+
+    def __init__(self, world, land_dim, rasters, prm, gen_arch, capacity, seed=0, bounds=None, device_barrier=False,
+                 **kw):
+        super().__init__(world, range(int(world)), land_dim, rasters, prm, gen_arch, capacity, seed, bounds, **kw)
+        # device_barrier: the ranks synchronise through gnx_strip_barrier (no host round trip inside a step);
+        # otherwise the host is the barrier and does the three collectives on the ranks' tensors
+        self.device_barrier = bool(device_barrier)
+        self._warm = False
+        for a in self.ranks:
+            for b in self.ranks:
+                if a is not b:
+                    a.connect(b.rank, b.endpoints, same_process=True)
+        self._t = [r.tensors() for r in self.ranks]
+
+    def _gather(self, fn):
+        return [fn(r) for r in self.ranks]
+
+    def _sum(self, tensors):
+        import torch
+        torch.cuda.synchronize()
+        tot = torch.stack(tensors).sum(dim=0, dtype=tensors[0].dtype)
+        for t in tensors:
+            t.copy_(tot)
+        torch.cuda.synchronize()
+
+    def _gather_rows(self, rows):
+        import torch
+        return torch.stack(rows)
+
+    def _check(self):
+        for r in self.ranks:
+            r.check()
 
     def _sync(self):
         for r in self.ranks:
             r.dev.sync()
 
     def step(self, n=1):
-        torch = self.torch
+        import torch
         if self.device_barrier and self._warm:
             # whole steps through gnx_step (one CUDA graph per rank and step, spin barriers inside); one step of
             # every rank is enqueued before the next, so no rank's queue fills up while a peer has nothing queued
@@ -336,204 +473,64 @@ class LocalStrips:
                 if sync:
                     torch.cuda.synchronize()
 
-    def step_records(self):
-        return merge_records([r.dev.step_records() for r in self.ranks])
-
-    def download(self, **kw):
-        for r in self.ranks:
-            r.check()
-        return merge_states([r.dev.download(**kw) for r in self.ranks])
-
-    def population_sizes(self):
-        return [r.dev.population_size() for r in self.ranks]
-
-    def close(self):
-        for r in self.ranks:
-            r.dev.close()
-
 
 # ---------------------------------------------------------------------------------------------
 # one process per GPU
 # ---------------------------------------------------------------------------------------------
-class NcclStrips:
+class NcclStrips(_Strips):
     """This process's strip of a landscape decomposed over the ranks of `torch.distributed`
     (backend nccl, one GPU each, one node: the receive buffers are shared through CUDA IPC)."""
 
     def __init__(self, land_dim, rasters, prm, gen_arch, capacity, seed=0, bounds=None, group=None, **kw):
         import torch
         import torch.distributed as dist
+        self.group = group
+        self.rank = dist.get_rank(group)
+        super().__init__(dist.get_world_size(group), [self.rank], land_dim, rasters, prm, gen_arch, capacity, seed,
+                         bounds, **kw)
         # the barriers and the three small collectives of a step run as one-CTA kernels over peer memory
         # (gnx_strip_barrier), never on the host
         self.device_barrier = True
-        self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
-        self.group = group
-        self.cs, self.ncx, self.ncy = mating_grid(land_dim, prm['mating_radius'])
-        K = np.asarray(rasters)[int(prm.get('K_layer', 0))] * float(prm.get('K_factor', 1.0))
-        self.bounds = plan_rows(self.ncy, self.world, row_weights_from_K(K, self.cs, self.ncy)) if bounds is None \
-            else np.asarray(bounds, dtype=np.int32)
-        self.me = StripRank(self.rank, self.world, self.bounds, land_dim, rasters, prm, gen_arch, capacity, seed, **kw)
         # exchange the endpoints (raw bytes of the struct: offsets + the CUDA IPC handle)
-        mine = bytes(self.me.endpoints)
         everyone = [None] * self.world
-        dist.all_gather_object(everyone, mine, group=group)
+        dist.all_gather_object(everyone, bytes(self.ranks[0].endpoints), group=group)
         for r, raw in enumerate(everyone):
             if r != self.rank:
-                self.me.connect(r, _lib.StripEndpoints.from_buffer_copy(raw), same_process=False)
-        self.stream = torch.cuda.ExternalStream(self.me.dev.stream_ptr)
+                self.ranks[0].connect(r, _lib.StripEndpoints.from_buffer_copy(raw), same_process=False)
+        self.stream = torch.cuda.ExternalStream(self.dev.stream_ptr)
         dist.barrier(group=group)
 
     @property
     def dev(self):
-        return self.me.dev
+        return self.ranks[0].dev
 
-    def set_burn(self, burn):
-        self.me.dev.set_burn(burn)
-
-    def set_mutation(self, *args, **kw):
-        """DeviceSpecies.set_mutation on this rank; every rank must make the same call."""
-        self.me.dev.set_mutation(*args, **kw)
-
-    def read_mutations(self, max_rows=4096):
-        """This rank's mutation log and tables, which equal every other rank's."""
-        return self.me.dev.read_mutations(max_rows)
-
-    def init_genomes(self, p, seed, write_mask=None):
-        """DeviceSpecies.init_genomes on this rank with the size and the histograms summed over the ranks
-        (every rank makes the same call)."""
-        import torch.distributed as dist
-        self.me.dev.init_genomes(p, seed, write_mask, allreduce=lambda t: dist.all_reduce(t, group=self.group))
-
-    def upload_owned(self, x, y, age=None, sex=None, idx=None, g=None, genomes_packed=None, max_ind_idx=None):
-        """Upload this rank's share of a population every rank holds on the host."""
-        idx = np.arange(len(x), dtype=np.int64) if idx is None else np.asarray(idx)
-        m = owner_of(y, self.bounds, self.cs, self.ncy) == self.rank
-        self.me.dev.upload(x[m], y[m], None if age is None else age[m], None if sex is None else sex[m], idx[m],
-                           g=None if g is None else g[m],
-                           genomes_packed=None if genomes_packed is None else genomes_packed[m],
-                           max_ind_idx=int(idx.max()) if max_ind_idx is None else max_ind_idx)
-
-    def step(self, n=1):
-        self.me.dev.step(n)            # gnx_step: the phases + gnx_strip_barrier, one graph per step
-
-    def sync(self):
-        self.me.check()
-
-    def step_records_local(self):
-        return self.me.dev.step_records()
-
-    def close(self):
-        self.me.dev.close()
-
-
-# ---------------------------------------------------------------------------------------------
-# one species over strips, behind the DeviceSpecies surface of api.Species
-# ---------------------------------------------------------------------------------------------
-def band_capacities(K, start_y, bounds, cell_size, ncy):
-    """Per-rank capacity: what DeviceSpecies gives a whole species (3 x the carrying capacity, twice the
-    starting size, at least 4096), taken over the rank's own band of mating-grid rows."""
-    b = np.asarray(bounds, dtype=np.int64)
-    kb = np.add.reduceat(row_weights_from_K(np.asarray(K, dtype=np.float64), cell_size, ncy), b[:-1])
-    nb = np.bincount(owner_of(start_y, b, cell_size, ncy), minlength=len(b) - 1) if len(start_y) else 0 * kb
-    return np.maximum(4096, np.maximum(3.0 * kb, 2.0 * nb)).astype(np.int64)
-
-
-class StripSpecies:
-    """One species cut into strips, with the members of DeviceSpecies that api.Species uses and species-wide
-    results.  `strips` is a strip count (LocalStrips: every strip a context of this process on the current
-    GPU, the host the barrier between the phases) or an initialised torch.distributed process group
-    (NcclStrips: this process's strip, device barriers, one graph per step).  Under a group every rank
-    makes the same calls in the same order and sees the whole species."""
-
-    def __init__(self, land_dim, rasters, prm, gen_arch, K, start_y, strips, seed=0, res_ratio=(1.0, 1.0),
-                 capacity=None):
-        self.land_dim = (int(land_dim[0]), int(land_dim[1]))
-        self.group = None if isinstance(strips, (int, np.integer)) else strips
-        if self.group is None:
-            self.world, self.rank = int(strips), None
-        else:
-            import torch.distributed as dist
-            self.world, self.rank = dist.get_world_size(self.group), dist.get_rank(self.group)
-        cs, ncx, ncy = mating_grid(self.land_dim, prm['mating_radius'])
-        bounds = plan_rows(ncy, self.world, row_weights_from_K(np.asarray(K, dtype=np.float64), cs, ncy))
-        self.bands = band_rows(bounds, cs, self.land_dim[1])
-        self._adds, self._skip_last = shared_band_rows(self.bands)
-        if capacity is None:
-            caps = band_capacities(K, np.asarray(start_y), bounds, cs, ncy)
-            capacity = int(caps.max() if self.group is None else caps[self.rank])
-        self.capacity = int(capacity)
-        kw = dict(seed=seed, bounds=bounds, res_ratio=res_ratio)
-        if self.group is None:
-            self._st = LocalStrips(self.world, self.land_dim, rasters, prm, gen_arch, self.capacity, **kw)
-            self._ranks = self._st.ranks
-        else:
-            self._st = NcclStrips(self.land_dim, rasters, prm, gen_arch, self.capacity, group=self.group, **kw)
-            self._ranks = [self._st.me]
-        self.Lg = self._ranks[0].dev.Lg
-
-    def _per_rank(self, fn):
-        """[fn(rank 0), ..., fn(rank world - 1)] on every rank (all-gathered under a group)."""
-        mine = [fn(r) for r in self._ranks]
-        if self.group is None:
-            return mine
+    def _gather(self, fn):
         import torch.distributed as dist
         out = [None] * self.world
-        dist.all_gather_object(out, mine[0], group=self.group)
+        dist.all_gather_object(out, fn(self.ranks[0]), group=self.group)
         return out
 
-    def _each(self, name, *args, **kw):
-        for r in self._ranks:
-            getattr(r.dev, name)(*args, **kw)
+    def _sum(self, tensors):
+        import torch
+        import torch.distributed as dist
+        for t in tensors:
+            dist.all_reduce(t, group=self.group)
+        torch.cuda.synchronize()
 
-    @property
-    def _surf_tabs(self):
-        return self._ranks[0].dev._surf_tabs
-
-    # ---- setup: the same call on every strip
-    def set_burn(self, burn):
-        self._each('set_burn', burn)
-
-    def set_raster(self, layer, rast):
-        self._each('set_raster', layer, rast)
-
-    def set_K(self, K):
-        self._each('set_K', K)
-
-    def set_life_history(self, **changes):
-        self._each('set_life_history', **changes)
-
-    def set_surface_tables(self, move_tab=None, disp_tab=None):
-        self._each('set_surface_tables', move_tab, disp_tab)
-
-    def set_mutation(self, *args, **kw):
-        self._st.set_mutation(*args, **kw)
-
-    def read_mutations(self, max_rows=4096):
-        return self._st.read_mutations(max_rows)
-
-    def read_mutation_tables(self):
-        return self._ranks[0].dev.read_mutation_tables()
-
-    def init_genomes(self, p, seed, write_mask=None, tskit_rows=False):
-        if tskit_rows:
-            raise ValueError('strip decomposition does not carry tskit rows')
-        self._st.init_genomes(p, seed, write_mask)
-
-    # ---- population in / out
-    def upload(self, x, y, age=None, sex=None, idx=None, g=None, max_ind_idx=None, genomes_packed=None):
-        up = self._st.upload if self.group is None else self._st.upload_owned
-        up(x, y, age, sex, idx, g=g, genomes_packed=genomes_packed, max_ind_idx=max_ind_idx)
+    def _gather_rows(self, rows):
+        import torch
+        import torch.distributed as dist
+        out = torch.empty(self.world * len(rows[0]), dtype=rows[0].dtype, device='cuda')
+        dist.all_gather_into_tensor(out, rows[0].clone(), group=self.group)
+        return out.view(self.world, -1)
 
     def _check(self):
-        """gnx_strip_check on every strip: a dropped migrant or a barrier timeout raises (on every rank)."""
-        if self.group is None:
-            for r in self._ranks:
-                r.check()
-            return
+        """Each rank checks its strip, then the error flags are all-reduced, so every rank raises."""
         import torch
         import torch.distributed as dist
         err = None
         try:
-            self._st.me.check()
+            self.ranks[0].check()
         except _lib.GnxError as e:
             err = e
         flag = torch.tensor([0 if err is None else 1], dtype=torch.int32, device='cuda')
@@ -543,69 +540,12 @@ class StripSpecies:
         if int(flag.item()):
             raise RuntimeError('a strip rank of this species failed (see that rank\'s error)')
 
-    def step(self, n_steps=1):
-        self._st.step(n_steps)
-        self._check()
+    def step(self, n=1):
+        self.dev.step(n)               # gnx_step: the phases + gnx_strip_barrier, one graph per step
 
-    def step_records(self):
-        return merge_records(self._per_rank(lambda r: r.dev.step_records()))
+    def sync(self):
+        self.ranks[0].check()
 
-    def population_size(self):
-        return sum(self._per_rank(lambda r: r.dev.population_size()))
-
-    def download(self, genomes=True, unpack=True, e=False):
-        self._check()
-        out = merge_states(self._per_rank(lambda r: r.dev.download(genomes=genomes, unpack=False, e=e)))
-        if 'genomes' in out and unpack:
-            out['g'] = gp.unpack_genomes(out['genomes'], self.Lg)
-        return out
-
-    # ---- statistics: the integer counts add up over the strips, the fitness sum in rank order
-    def stats(self, region=None):
-        per = self._per_rank(lambda r: r.dev.stat_counts(region))
-        c1 = sum(p[0] for p in per)
-        het = sum(p[1] for p in per)
-        fs = 0.0
-        for p in per:
-            fs += p[2]
-        return stats_from_counts(c1, het, fs, sum(p[3] for p in per))
-
-    def ld(self):
-        per = self._per_rank(lambda r: r.dev.ld_counts())
-        return ld_from_counts(sum(p[0] for p in per), sum(p[1] for p in per))
-
-    def raster(self, field):
-        """A landscape raster of the last step, each band's rows from the rank that computes them (a row two
-        bands share from the upper one)."""
-        per = self._per_rank(lambda r: r.dev.raster(field)[slice(*self.bands[r.rank])])
-        out = None
-        for (ly0, ly1), rows in zip(self.bands, per):
-            if out is None:
-                out = np.zeros((self.land_dim[1],) + rows.shape[1:], dtype=rows.dtype)
-            out[ly0:ly1] = rows
-        return out
-
-    def burnin_cell_stats(self):
-        """DeviceSpecies.burnin_cell_stats of the whole species: every rank counts into its band, the rows two
-        bands share are added into the upper band, and each rank sums the change over the rows it accounts for."""
-        import torch
-        got = {r.rank: r.burnin_count() for r in self._ranks}
-        for k, (ly0, ly1, _, _) in got.items():
-            assert (ly0, ly1) == self.bands[k], 'strip band rows differ from the host plan'
-        if self.group is None:
-            lasts = [got[k][3].clone() for k in range(self.world)]
-        else:
-            import torch.distributed as dist
-            X = self.land_dim[0]
-            allrows = torch.empty(self.world * X, dtype=torch.int32, device='cuda')
-            dist.all_gather_into_tensor(allrows, got[self.rank][3].clone(), group=self.group)
-            lasts = list(allrows.view(self.world, X))
-        for k, (_, _, first, _) in got.items():
-            for q in self._adds[k]:
-                first += lasts[q]
-        torch.cuda.synchronize()
-        per = self._per_rank(lambda r: r.burnin_diff(self._skip_last[r.rank]))
-        return cell_stats_from_sums(sum(p[0] for p in per), sum(p[1] for p in per), self.land_dim[0] * self.land_dim[1])
-
-    def close(self):
-        self._st.close()
+    def step_records_local(self):
+        """This rank's own records, without a check or a gather."""
+        return self.dev.step_records()

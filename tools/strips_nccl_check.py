@@ -68,11 +68,11 @@ def main():
     p = np.random.default_rng(3).random(ga['L'])
     start = None
     if genome_init:
-        st.upload_owned(pop['x'], pop['y'], pop['age'], pop['sex'], pop['idx'])
+        st.upload(pop['x'], pop['y'], pop['age'], pop['sex'], pop['idx'])
         st.init_genomes(p, 1234)
         start = st.dev.download()
     else:
-        st.upload_owned(pop['x'], pop['y'], pop['age'], pop['sex'], pop['idx'], g=g)
+        st.upload(pop['x'], pop['y'], pop['age'], pop['sex'], pop['idx'], g=g)
     if mut:
         st.set_mutation(**mut)
     st.step(steps)
