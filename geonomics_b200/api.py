@@ -681,7 +681,9 @@ class Species:
                 prm[nm] = dict(table=surf.surf, layer=surf.lyr_num, mixture=surf.mix, kappa=surf.kappa)
         return prm
 
-    def _attach(self, capacity=None):
+    def _attach(self, capacity=None, cols=None):
+        """cols: (col_locus, col_capacity) of the column layout to continue from (a snapshot's); a use_tskit
+        species otherwise starts its columns at the ascending non-neutral loci."""
         land = self._land
         rasters = np.stack([land[l].rast for l in range(len(land))])
         ga = None
@@ -692,6 +694,11 @@ class Species:
                                    univ_adv=t.univ_adv))
             ga = dict(L=self.gen_arch.L, paths=self.gen_arch.recombinations._paths, traits=traits,
                       dom=np.asarray(self.gen_arch.dom, dtype=np.int8))
+            if self.gen_arch.use_tskit:
+                # species.py:891-905: genotype rows carry the non-neutral loci only; so do the device's (gnx_create_cols)
+                if cols is None:
+                    cols = (np.sort(np.asarray(self.gen_arch.nonneut_loci, dtype=np.int64)), None)
+                ga['cols'], ga['col_capacity'] = cols
         p = self._init_pop
         if self._strips is not None:
             from .strips import LocalStrips, NcclStrips
@@ -742,6 +749,8 @@ class Species:
                     inst={k: copy.deepcopy(v) for k, v in self.__dict__.items()
                           if hasattr(self._pv, k) and not k.startswith('_')},        # life-history overrides
                     capacity=self._dev.capacity)
+        if getattr(self._dev, 'cols', False):
+            snap['cols'] = (self._dev.read_cols(), self._dev.col_capacity)
         return snap
 
     def _restore(self, snap, land, gen_arch=None):
@@ -765,13 +774,13 @@ class Species:
         self._init_pop = dict(x=st['x'], y=st['y'], age=st['age'], sex=st['sex'], idx=st['idx'])
         if gen_arch is None and st.get('genomes') is not None:
             self._init_pop['genomes'] = st['genomes']
-        self._attach(capacity=snap['capacity'])
+        self._attach(capacity=snap['capacity'], cols=snap.get('cols') if gen_arch is None else None)
         if self.burned and gen_arch is None and self.mutate:
             ga = self.gen_arch
             self._dev.set_mutation(ga.mu_neut or 0, ga.mu_delet or 0, ga._mutables,
                                    np.sort(np.asarray(ga.nonneut_loci, dtype=np.int64)), ga.delet_loci, ga.delet_loci_s,
                                    ga.delet_alpha_distr_shape, ga.delet_alpha_distr_scale,
-                                   log_capacity=max(ga.L, 16))
+                                   log_capacity=max(ga.L, 16), **self._tskit_mutation_kw())
 
     def _on_raster_change(self, lyr_num, rast):
         if self._dev is not None:
@@ -889,14 +898,8 @@ class Species:
                                    z=np.zeros((len(p['x']), 0)), fit=np.full(len(p['x']), np.nan),
                                    e=None, g=None)
             else:
+                # a use_tskit species' rows are the Individuals' own: one per non-neutral locus (species.py:891-905)
                 self._cache = self._dev.download(genomes=self.burned and self.gen_arch is not None, e=True)
-                if self._cache.get('g') is not None and self.gen_arch.use_tskit:
-                    # species.py:891-905: Individuals carry one genotype ROW per non-neutral locus
-                    # (the by-locus array the device holds is kept for _get_genotypes, which the reference
-                    # answers from the tree sequence for all L loci, species.py:1395-1425)
-                    from . import genome_pack as gp
-                    self._cache['g_loci'] = self._cache['g']
-                    self._cache['g'] = gp.loci_to_rows(self._cache['g'], self.gen_arch.nonneut_loci)
         return self._cache
 
     def _individuals(self):
@@ -984,7 +987,9 @@ class Species:
         per non-neutral locus, species.py:891-905); `all_loci=True` gives all L loci, which the
         reference reads off the tree sequence (:1395-1425) and the device holds by locus."""
         s = self._state()
-        g = self._sel(s.get('g_loci', s['g']) if all_loci else s['g'], individs)
+        g = self._sel(s['g'], individs)
+        if all_loci and s.get('col_locus') is not None:      # rows of the chosen individuals scattered to their loci
+            g = gp.rows_to_loci(g, np.sort(s['col_locus']), self.gen_arch.L)
         if loci is not None:
             g = g[:, loci, :]
         if not biallelic:
@@ -1043,18 +1048,19 @@ class Species:
         if genome_init == 'device':
             self._set_genomes_on_device(s, burn_T, T)
             return
-        g = np.zeros((n, L, 2), dtype=np.int8)
-        flat = g.reshape(n, L, 2)
         p = ga.p
-        nonneut = set(int(v) for v in ga.nonneut_loci)
+        # genome.py:1137-1142: a use_tskit species carries the non-neutral rows only, in ascending locus order
+        row_of = {int(l): r for r, l in enumerate(np.sort(np.asarray(ga.nonneut_loci, dtype=np.int64)))} if tsk \
+            else {l: l for l in range(L)}
+        g = np.zeros((n, len(row_of), 2), dtype=np.int8)
         mut_site, mut_node = [], []
         n_muts = gp.carrier_counts(n, p[:L])
         for site in range(L):
             n_mut = int(n_muts[site])
             if n_mut > 0:
                 hom = np.random.permutation(2 * n)[:n_mut]
-                if not tsk or site in nonneut:            # genome.py:1137-1142: only non-neutral rows are carried
-                    flat[hom // 2, site, hom % 2] = 1
+                if site in row_of:
+                    g[hom // 2, row_of[site], hom % 2] = 1
                 if tsk:                                   # genome.py:1143-1147: node of (individual k, homologue h)
                     mut_site.append(np.full(n_mut, site, np.int32))
                     mut_node.append(hom.astype(np.int32))  # is 2k + h (see below)
@@ -1159,14 +1165,7 @@ class Species:
         """species.py:960-967 + genome.py:1060-1104: check the rates against the infinite-sites
         budget, shuffle the mutable loci, hand the bookkeeping to the device (a13)."""
         ga = self.gen_arch
-        kw = {}
-        if ga.use_tskit:
-            # species.py:891-905 layout: rows = non-neutral loci; the device reads row r as bit nonneut_loci[r]
-            traits = list((ga.traits or {}).values())
-            kw = dict(tskit_layout=True,
-                      trait_mus=[t.mu or 0 for t in traits] if self.mutate else None,
-                      trait_alpha_distr=[(t.alpha_distr_mu, t.alpha_distr_sigma, t.max_alpha_mag) for t in traits],
-                      trait_loci_idxs=[t.loci_idxs for t in traits], delet_loci_idxs=ga.delet_loci_idxs)
+        kw = self._tskit_mutation_kw()
         nonneut = set(int(v) for v in ga.nonneut_loci)
         nn_sorted = np.array(sorted(nonneut), dtype=np.int64)
         if not self.mutate:
@@ -1200,6 +1199,18 @@ class Species:
         self._dev.set_mutation(ga.mu_neut or 0, ga.mu_delet or 0, ga._mutables, nn_sorted, ga.delet_loci,
                                ga.delet_loci_s, ga.delet_alpha_distr_shape, ga.delet_alpha_distr_scale,
                                log_capacity=max(ga.L, 16), **kw)
+
+    def _tskit_mutation_kw(self):
+        """set_mutation's use_tskit arguments: species.py:891-905 layout (rows = non-neutral loci, read through
+        the reference's index arrays as written)."""
+        ga = self.gen_arch
+        if not ga.use_tskit:
+            return {}
+        traits = list((ga.traits or {}).values())
+        return dict(tskit_layout=True,
+                    trait_mus=[t.mu or 0 for t in traits] if self.mutate else None,
+                    trait_alpha_distr=[(t.alpha_distr_mu, t.alpha_distr_sigma, t.max_alpha_mag) for t in traits],
+                    trait_loci_idxs=[t.loci_idxs for t in traits], delet_loci_idxs=ga.delet_loci_idxs)
 
     def _sync_mutations(self):
         """Pull the device's mutation log and bookkeeping into gen_arch (what mutation.py:199-205

@@ -61,7 +61,12 @@ struct gnx_ctx {
   std::vector<unsigned char> graph_key;
   int device = 0;
   int num_sms = 148;
-  int Wq = 0, Wwords = 0;
+  int Wq = 0, Wwords = 0;            // 128-bit units / 32-bit words per homologue of a genotype row
+  int WqL = 0;                      // 128-bit units of L bits (by-locus rows, recombination paths as simulated)
+  // column layout (gnx_create_cols): a row holds col_cap columns, column j = non-neutral locus col_locus[j]
+  bool cols = false;
+  int col_cap = 0;
+  int32_t* d_cols = nullptr;        // [1 + 2L]: n_cols, col_locus[L], col_of_locus[L] (-1: no column)
   int ncell = 0;
   int64_t n_hint = 0;               // last population size seen by the host (grid sizing only)
   Pop pop{};
@@ -213,7 +218,8 @@ static void mating_grid(const gnx_config_t& c, double* cs, int* ncx, int* ncy) {
 static int create_impl(const gnx_config_t* cfg, gnx_ctx* ctx);
 extern "C" int gnx_destroy(gnx_ctx* ctx);
 
-extern "C" int gnx_create(const gnx_config_t* cfg, gnx_ctx** out) {
+static int create_ctx(const gnx_config_t* cfg, int32_t col_cap, int32_t n_cols, const int32_t* host_col_locus,
+                      gnx_ctx** out) {
   ARG(cfg && out, "null cfg/out");
   ARG(cfg->abi_version == GNX_ABI_VERSION, "abi_version mismatch");
   ARG(cfg->dim_x > 0 && cfg->dim_y > 0 && cfg->n_layers > 0 && cfg->n_layers <= GNX_MAX_LAYERS, "landscape dims");
@@ -223,9 +229,37 @@ extern "C" int gnx_create(const gnx_config_t* cfg, gnx_ctx** out) {
   int ndev = 0;
   CK(cudaGetDeviceCount(&ndev));
   if (ndev == 0) { g_last_error = "no CUDA device"; return GNX_ERR_CUDA; }
+  if (col_cap > 0) {
+    ARG(cfg->L > 0 && n_cols >= 0 && n_cols <= col_cap && (n_cols == 0 || host_col_locus), "columns");
+    std::vector<uint8_t> seen(cfg->L, 0);
+    for (int j = 0; j < n_cols; ++j) {
+      ARG(host_col_locus[j] >= 0 && host_col_locus[j] < cfg->L, "column locus out of range");
+      ARG(!seen[host_col_locus[j]], "a locus holds two columns");
+      seen[host_col_locus[j]] = 1;
+    }
+  }
   gnx_ctx* ctx = new gnx_ctx();
   ctx->cfg = *cfg;
-  const int r = create_impl(cfg, ctx);
+  ctx->cols = col_cap > 0;
+  ctx->col_cap = 128 * ((std::max(col_cap, 0) + 127) / 128);
+  int r = create_impl(cfg, ctx);
+  if (r == GNX_OK && ctx->cols) {
+    const int L = cfg->L;
+    std::vector<int32_t> h((size_t)1 + 2 * L, 0);
+    h[0] = n_cols;
+    for (int l = 0; l < L; ++l) h[1 + L + l] = -1;
+    for (int j = 0; j < n_cols; ++j) {
+      h[1 + j] = host_col_locus[j];
+      h[1 + L + host_col_locus[j]] = j;
+    }
+    r = dmalloc(ctx, &ctx->d_cols, h.size());
+    if (r == GNX_OK &&
+        (cudaMemcpyAsync(ctx->d_cols, h.data(), h.size() * 4, cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess ||
+         cudaStreamSynchronize(ctx->stream) != cudaSuccess)) {
+      g_last_error = "copying the column map";
+      r = GNX_ERR_CUDA;
+    }
+  }
   if (r != GNX_OK) {                       // streams, events and every buffer allocated so far
     const std::string keep = g_last_error;
     gnx_destroy(ctx);
@@ -234,6 +268,14 @@ extern "C" int gnx_create(const gnx_config_t* cfg, gnx_ctx** out) {
   }
   *out = ctx;
   return GNX_OK;
+}
+
+extern "C" int gnx_create(const gnx_config_t* cfg, gnx_ctx** out) { return create_ctx(cfg, 0, 0, nullptr, out); }
+
+extern "C" int gnx_create_cols(const gnx_config_t* cfg, int32_t col_capacity, int32_t n_cols,
+                               const int32_t* host_col_locus, gnx_ctx** out) {
+  ARG(col_capacity > 0, "col_capacity");
+  return create_ctx(cfg, col_capacity, n_cols, host_col_locus, out);
 }
 
 // Quantile table of |theta|, theta ~ von Mises(0, kappa): the half-distribution's inverse CDF at
@@ -276,7 +318,8 @@ static int create_impl(const gnx_config_t* cfg, gnx_ctx* ctx) {
   CK(cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming));
   if (const char* ng = getenv("GNX_NO_GRAPH")) ctx->use_graph = !(ng[0] && ng[0] != '0');
   const int64_t cap = cfg->capacity;
-  ctx->Wq = std::max(1, (cfg->L + 127) / 128);
+  ctx->WqL = std::max(1, (cfg->L + 127) / 128);
+  ctx->Wq = ctx->cols ? ctx->col_cap / 128 : ctx->WqL;
   ctx->Wwords = 4 * ctx->Wq;
   Pop& P = ctx->pop;
   P.cap = (int)cap;
@@ -436,6 +479,33 @@ static void free_bucket(std::vector<void*>& b) {
   b.clear();
 }
 
+// column layout: the current columns (col_locus[0 .. n_cols)) and the column of every locus (-1: none).
+// Synchronises.
+static int read_cols(gnx_ctx* ctx, std::vector<int32_t>* col_locus, std::vector<int32_t>* col_of_locus = nullptr) {
+  const int L = ctx->cfg.L;
+  std::vector<int32_t> h((size_t)1 + 2 * L);
+  CK(cudaMemcpyAsync(h.data(), ctx->d_cols, h.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  col_locus->assign(h.begin() + 1, h.begin() + 1 + h[0]);
+  if (col_of_locus) col_of_locus->assign(h.begin() + 1 + L, h.end());
+  return GNX_OK;
+}
+
+// the recombination paths as simulated (host_paths, [n_paths][4 WqL]) at the bits of the genotype rows: the
+// same array by locus, bit j = the path at locus col_locus[j] in the column layout
+static std::vector<uint32_t> paths_at_rows(const gnx_ctx* ctx, const std::vector<int32_t>& col_locus) {
+  if (!ctx->cols) return ctx->host_paths;
+  const size_t WL = (size_t)4 * ctx->WqL, W = (size_t)4 * ctx->Wq;
+  const int n = ctx->cfg.n_recomb_paths;
+  std::vector<uint32_t> out((size_t)n * W, 0u);
+  for (int p = 0; p < n; ++p)
+    for (size_t j = 0; j < col_locus.size(); ++j) {
+      const int l = col_locus[j];
+      out[p * W + (j >> 5)] |= ((ctx->host_paths[p * WL + (l >> 5)] >> (l & 31)) & 1u) << (j & 31);
+    }
+  return out;
+}
+
 extern "C" int gnx_destroy(gnx_ctx* ctx) {
   if (!ctx) return GNX_OK;
   cudaSetDevice(ctx->device);
@@ -591,26 +661,39 @@ extern "C" int gnx_set_traits(gnx_ctx* ctx, int32_t n_traits, const gnx_trait_t*
   const int NW = 4 * Wq;      // CSR over 32-bit words
   std::vector<int32_t> chunk_ptr((size_t)std::max(1, n_traits) * (NW + 1), 0);
   const size_t plane = (size_t)ctx->cfg.dim_x * ctx->cfg.dim_y;
+  std::vector<int32_t> col_locus, col_of;                      // column layout: the bit of a locus is its column
+  if (ctx->cols) {
+    int r = read_cols(ctx, &col_locus, &col_of);
+    if (r != GNX_OK) return r;
+  }
   for (int t = 0; t < n_traits; ++t) {
     const gnx_trait_t& tr = traits[t];
     ARG(tr.n_loci >= 0 && (tr.n_loci == 0 || (tr.host_loci && tr.host_alpha)), "trait loci");
     ARG(tr.layer >= 0 && tr.layer < ctx->cfg.n_layers, "trait layer");
     std::vector<int> order(tr.n_loci);
     for (int k = 0; k < tr.n_loci; ++k) order[k] = k;
+    for (int k = 0; k < tr.n_loci; ++k) {
+      ARG(tr.host_loci[k] >= 0 && tr.host_loci[k] < ctx->cfg.L, "trait locus out of range");
+      ARG(!ctx->cols || col_of[tr.host_loci[k]] >= 0, "trait locus without a column");
+    }
+    // Trait.loci order (by locus) for the host copies, the bit read for the tables
+    auto bit_of = [&](int k) { return ctx->cols ? col_of[tr.host_loci[k]] : tr.host_loci[k]; };
     std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return tr.host_loci[a] < tr.host_loci[b]; });
+    for (int kk = 0; kk < tr.n_loci; ++kk) {
+      ctx->host_trait_loci[t].push_back(tr.host_loci[order[kk]]);
+      ctx->host_trait_alpha[t].push_back(tr.host_alpha[order[kk]]);
+    }
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return bit_of(a) < bit_of(b); });
     int q = 0;
     chunk_ptr[(size_t)t * (NW + 1)] = (int32_t)te_locus.size();
     for (int kk = 0; kk < tr.n_loci; ++kk) {
       const int k = order[kk];
-      const int locus = tr.host_loci[k];
-      ARG(locus >= 0 && locus < ctx->cfg.L, "trait locus out of range");
-      while (q < locus / 32) chunk_ptr[(size_t)t * (NW + 1) + (++q)] = (int32_t)te_locus.size();
-      ctx->host_trait_loci[t].push_back(locus);
-      ctx->host_trait_alpha[t].push_back(tr.host_alpha[k]);
-      te_locus.push_back(locus);
+      const int locus = tr.host_loci[k], bit = bit_of(k);
+      while (q < bit / 32) chunk_ptr[(size_t)t * (NW + 1) + (++q)] = (int32_t)te_locus.size();
+      te_locus.push_back(bit);
       te_alpha.push_back(tr.host_alpha[k]);
       te_dom.push_back(host_dom ? 1.0 + (double)host_dom[locus] : 1.0);
-      te_pack.push_back(TraitEntry{(locus >> 5) * 8, (int32_t)(1u << (locus & 31)), 0.5 * tr.host_alpha[k]});
+      te_pack.push_back(TraitEntry{(bit >> 5) * 8, (int32_t)(1u << (bit & 31)), 0.5 * tr.host_alpha[k]});
     }
     while (q < NW) chunk_ptr[(size_t)t * (NW + 1) + (++q)] = (int32_t)te_locus.size();
     T.n_loci[t] = tr.n_loci;
@@ -650,7 +733,7 @@ extern "C" int gnx_set_recomb_paths(gnx_ctx* ctx, const uint32_t* host_packed_pa
   USE_DEVICE(ctx);
   ARG(ctx->cfg.n_recomb_paths > 0, "n_recomb_paths");
   uint4* d = nullptr;
-  const size_t n = (size_t)ctx->cfg.n_recomb_paths * ctx->Wq;
+  const size_t n = (size_t)ctx->cfg.n_recomb_paths * ctx->WqL;     // as simulated: by locus
   CK(cudaStreamSynchronize(ctx->stream));
   if (ctx->mut.enabled && ctx->mut.tskit_layout) {     // the mutation bookkeeping patches the old path array
     if (ctx->mut.own_tables) ctx->traits = ctx->traits_as_set;
@@ -659,13 +742,19 @@ extern "C" int gnx_set_recomb_paths(gnx_ctx* ctx, const uint32_t* host_packed_pa
     ctx->mut_delet = false;
   }
   if (ctx->d_paths) { cudaFree(ctx->d_paths); ctx->d_paths = nullptr; }
-  CK(cudaMalloc((void**)&d, std::max<size_t>(n, 1) * sizeof(uint4)));
+  ctx->host_paths.assign(host_packed_paths, host_packed_paths + n * 4);
+  std::vector<int32_t> col_locus;
+  if (ctx->cols) {
+    int r = read_cols(ctx, &col_locus);
+    if (r != GNX_OK) return r;
+  }
+  const std::vector<uint32_t> rows = paths_at_rows(ctx, col_locus);   // what k_gametes reads
+  CK(cudaMalloc((void**)&d, std::max<size_t>(rows.size() / 4, 1) * sizeof(uint4)));
   ctx->d_paths = d;
-  CK(cudaMemcpyAsync(d, host_packed_paths, n * sizeof(uint4), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(d, rows.data(), rows.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   ctx->prm.paths = d;
   ctx->have_paths = true;
-  ctx->host_paths.assign(host_packed_paths, host_packed_paths + n * 4);
   return GNX_OK;
 }
 
@@ -1402,12 +1491,20 @@ extern "C" int gnx_set_mutation(gnx_ctx* ctx, const gnx_mutation_t* m) {
     for (int t = 0; m->host_trait_mu && t < ctx->cfg.n_traits; ++t)
       ARG(!(m->host_trait_mu[t] > 0), "trait mutation is not supported under strip decomposition");
   }
+  // the column layout carries the use_tskit = True semantics: its genotype bits are non-neutral loci only
+  ARG(!ctx->cols || (m && m->tskit_layout), "a context with the column layout needs tskit_layout = 1");
   CK(cudaStreamSynchronize(ctx->stream));
+  std::vector<int32_t> col_locus, col_of;
+  if (ctx->cols) {
+    int r = read_cols(ctx, &col_locus, &col_of);
+    if (r != GNX_OK) return r;
+  }
   if (ctx->mut.enabled && ctx->mut.own_tables) {
     ctx->traits = ctx->traits_as_set;                  // back to the tables gnx_set_traits built
-    if (ctx->mut.tskit_layout && ctx->d_paths && !ctx->host_paths.empty())   // undo the path patches
-      CK(cudaMemcpyAsync(ctx->d_paths, ctx->host_paths.data(), ctx->host_paths.size() * 4, cudaMemcpyHostToDevice,
-                         ctx->stream));
+    if (ctx->mut.tskit_layout && ctx->d_paths && !ctx->host_paths.empty()) {   // undo the path patches
+      const std::vector<uint32_t> rows = paths_at_rows(ctx, col_locus);
+      CK(cudaMemcpyAsync(ctx->d_paths, rows.data(), rows.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+    }
     CK(cudaStreamSynchronize(ctx->stream));
   }
   free_bucket(ctx->mut_allocs);
@@ -1430,6 +1527,10 @@ extern "C" int gnx_set_mutation(gnx_ctx* ctx, const gnx_mutation_t* m) {
   ARG(m->n_nonneut >= 0 && m->n_nonneut <= ctx->cfg.L && (m->n_nonneut == 0 || m->host_nonneut_loci), "nonneut_loci");
   ARG(m->n_delet >= 0 && m->n_delet <= ctx->cfg.L && (m->n_delet == 0 || (m->host_delet_loci && m->host_delet_s)),
       "delet_loci");
+  ARG(!ctx->cols || (int)col_locus.size() == m->n_nonneut, "the columns must be the non-neutral loci");
+  for (int k = 0; ctx->cols && k < m->n_nonneut; ++k)
+    ARG(m->host_nonneut_loci[k] >= 0 && m->host_nonneut_loci[k] < ctx->cfg.L && col_of[m->host_nonneut_loci[k]] >= 0,
+        "a non-neutral locus without a column");
   const bool own = tskit_layout || trait_mu_sum > 0;
   if (own) {
     if (nT > 0 && !ctx->have_traits) { g_last_error = "gnx_set_traits must precede gnx_set_mutation"; return GNX_ERR_STATE; }
@@ -1464,6 +1565,13 @@ extern "C" int gnx_set_mutation(gnx_ctx* ctx, const gnx_mutation_t* m) {
   M.T = nT;
   M.NW = 4 * ctx->Wq;
   M.Wq = ctx->Wq;
+  M.WqL = ctx->WqL;
+  if (ctx->cols) {
+    M.col_n = ctx->d_cols;
+    M.col_locus = ctx->d_cols + 1;
+    M.col_of_locus = ctx->d_cols + 1 + L;
+    M.col_cap = ctx->col_cap;
+  }
   M.log_cap = std::max(m->log_capacity, 1);
   DM(ctx, &M.mutables, (size_t)std::max(L, m->n_mutables), &ctx->mut_allocs);
   DM(ctx, &M.nonneut, (size_t)L + 1, &ctx->mut_allocs);
@@ -1552,18 +1660,18 @@ extern "C" int gnx_set_mutation(gnx_ctx* ctx, const gnx_mutation_t* m) {
       M.paths_orig = orig;
       M.paths = (uint4*)ctx->d_paths;
       M.n_paths = ctx->cfg.n_recomb_paths;
-      patched = ctx->host_paths;
+      patched = paths_at_rows(ctx, col_locus);
       if (m->host_subsetters) {
         const size_t W32 = (size_t)4 * ctx->Wq;
         for (int pth = 0; pth < M.n_paths; ++pth)
           for (int j = 0; j < m->n_nonneut; ++j) {
-            const int l = m->host_nonneut_loci[j];
+            const int l = m->host_nonneut_loci[j], bit = ctx->cols ? col_of[l] : l;
             const uint32_t b = m->host_subsetters[(size_t)pth * m->n_nonneut + j] & 1u;
-            uint32_t& w = patched[(size_t)pth * W32 + (l >> 5)];
-            w = (w & ~(1u << (l & 31))) | (b << (l & 31));
+            uint32_t& w = patched[(size_t)pth * W32 + (bit >> 5)];
+            w = (w & ~(1u << (bit & 31))) | (b << (bit & 31));
           }
       }
-      CK(cudaMemcpyAsync(ctx->d_paths, patched.data(), nw * 4, cudaMemcpyHostToDevice, s));
+      CK(cudaMemcpyAsync(ctx->d_paths, patched.data(), patched.size() * 4, cudaMemcpyHostToDevice, s));
       CK(cudaStreamSynchronize(s));
     }
   }
@@ -1636,6 +1744,93 @@ extern "C" int gnx_read_mutation_tables(gnx_ctx* ctx, int32_t trait, int32_t* n_
     CK(cudaMemcpyAsync(host_delet_loci_idxs, M.tskit_layout ? M.delet_idxs : M.delet_loci, (size_t)counts[2] * 4,
                        cudaMemcpyDeviceToHost, s));
   CK(cudaStreamSynchronize(s));
+  return GNX_OK;
+}
+
+// ---- column layout ---------------------------------------------------------------------------
+extern "C" int gnx_read_cols(gnx_ctx* ctx, int32_t* host_col_locus, int32_t* n_cols, int32_t* col_capacity) {
+  ARG(ctx, "null ctx");
+  if (!ctx->cols) { g_last_error = "the context does not hold the column layout"; return GNX_ERR_STATE; }
+  USE_DEVICE(ctx);
+  Counters h;
+  int r = read_counters(ctx, &h);
+  if (r != GNX_OK) return r;
+  std::vector<int32_t> col_locus;
+  if ((r = read_cols(ctx, &col_locus)) != GNX_OK) return r;
+  if (n_cols) *n_cols = (int32_t)col_locus.size();
+  if (col_capacity) *col_capacity = ctx->col_cap;
+  if (host_col_locus && !col_locus.empty()) memcpy(host_col_locus, col_locus.data(), col_locus.size() * 4);
+  return check_device_err(h);
+}
+
+// a fresh [n_rows][wn] copy of the rows of *p ([n_rows][wo]), new units zero; *p is freed (and replaced in bucket)
+static int widen_rows(gnx_ctx* ctx, std::vector<void*>* bucket, uint4** p, size_t n_rows, int wo, int wn) {
+  uint4* q = nullptr;
+  CK(cudaMalloc((void**)&q, std::max<size_t>(n_rows * wn, 1) * sizeof(uint4)));
+  PROF(ctx, "k_widen_rows");
+  k_widen_rows<<<grid_for(ctx, 8), 256, 0, ctx->stream>>>(*p, q, (long long)n_rows, wo, wn);
+  LAUNCHED(ctx);
+  CK(cudaStreamSynchronize(ctx->stream));
+  if (bucket) std::replace(bucket->begin(), bucket->end(), (void*)*p, (void*)q);
+  CK(cudaFree(*p));
+  *p = q;
+  return GNX_OK;
+}
+
+static int widen_csr(gnx_ctx* ctx, std::vector<void*>& bucket, int32_t** p, int nwo, int nwn) {
+  const int nt = std::max(1, ctx->cfg.n_traits);
+  int32_t* q = nullptr;
+  CK(cudaMalloc((void**)&q, (size_t)nt * (nwn + 1) * sizeof(int32_t)));
+  k_widen_csr<<<grid_for(ctx, 1), 256, 0, ctx->stream>>>(*p, q, nt, nwo, nwn);
+  LAUNCHED(ctx);
+  CK(cudaStreamSynchronize(ctx->stream));
+  std::replace(bucket.begin(), bucket.end(), (void*)*p, (void*)q);
+  CK(cudaFree(*p));
+  *p = q;
+  return GNX_OK;
+}
+
+extern "C" int gnx_widen_cols(gnx_ctx* ctx, int32_t col_capacity) {
+  ARG(ctx, "null ctx");
+  if (!ctx->cols) { g_last_error = "the context does not hold the column layout"; return GNX_ERR_STATE; }
+  ARG(col_capacity > ctx->col_cap, "col_capacity must exceed the current one");
+  USE_DEVICE(ctx);
+  CK(cudaStreamSynchronize(ctx->stream));
+  const int wo = ctx->Wq, wn = (col_capacity + 127) / 128;
+  int r;
+  Pop& P = ctx->pop;
+  // genotype rows of every slot; the staging buffer of upload / download only needs the new size
+  if ((r = widen_rows(ctx, &ctx->allocs, &P.G, (size_t)P.cap * 2, wo, wn)) != GNX_OK) return r;
+  if ((r = widen_rows(ctx, &ctx->allocs, &ctx->d_stage_genomes, (size_t)P.cap * 2, wo, wn)) != GNX_OK) return r;
+  if (ctx->d_paths) {
+    uint4* d = (uint4*)ctx->d_paths;
+    if ((r = widen_rows(ctx, nullptr, &d, (size_t)ctx->cfg.n_recomb_paths, wo, wn)) != GNX_OK) return r;
+    ctx->d_paths = d;
+    ctx->prm.paths = d;
+  }
+  // the trait CSR over words: the tables of gnx_set_traits and those the mutation bookkeeping owns
+  const bool mut_tables = ctx->mut.enabled && ctx->mut.own_tables;
+  if (ctx->have_traits && ctx->traits_as_set.chunk_ptr) {
+    int32_t* cp = const_cast<int32_t*>(ctx->traits_as_set.chunk_ptr);
+    if ((r = widen_csr(ctx, ctx->trait_allocs, &cp, 4 * wo, 4 * wn)) != GNX_OK) return r;
+    ctx->traits_as_set.chunk_ptr = cp;
+    if (!mut_tables) ctx->traits.chunk_ptr = cp;
+  }
+  Mut& M = ctx->mut;
+  if (mut_tables) {
+    if ((r = widen_csr(ctx, ctx->mut_allocs, &M.chunk_ptr, 4 * wo, 4 * wn)) != GNX_OK) return r;
+    ctx->traits.chunk_ptr = M.chunk_ptr;
+  }
+  ctx->Wq = wn;
+  ctx->Wwords = 4 * wn;
+  ctx->col_cap = 128 * wn;
+  P.Wq = wn;
+  if (M.enabled) {
+    M.Wq = wn;
+    M.NW = 4 * wn;
+    M.paths = (uint4*)ctx->d_paths;
+    if (M.col_of_locus) M.col_cap = ctx->col_cap;
+  }
   return GNX_OK;
 }
 
@@ -1971,6 +2166,7 @@ extern "C" int gnx_strip_enable(gnx_ctx* ctx, const gnx_strip_config_t* sc) {
   ARG(sc->world >= 1 && sc->world <= GNX_STRIP_MAX_WORLD && sc->rank >= 0 && sc->rank < sc->world, "rank / world");
   ARG(ctx->cfg.mating_radius > 0, "strip decomposition needs a mating radius (panmixia has no locality)");
   ARG(!ctx->tsk.enabled, "strip decomposition does not carry tskit rows");
+  ARG(!ctx->cols, "strip decomposition does not carry the column genotype layout");
   ARG(!ctx->mut.enabled || !ctx->mut.own_tables,
       "strip decomposition does not carry the tskit genotype layout or trait mutation");
   ARG(!ctx->prm.ordered, "injected draws are not supported under strip decomposition");
@@ -2547,7 +2743,15 @@ extern "C" int gnx_stats_genotypes_region(gnx_ctx* ctx, double x_min, double x_m
   int r = read_counters(ctx, &hc);
   cudaFree(d);
   if (r != GNX_OK) return r;
-  for (int l = 0; l < ctx->cfg.L; ++l) { host_c1[l] = h[l]; host_het[l] = h[nbits + l]; }
+  if (ctx->cols) {                                    // column j counts locus col_locus[j]; no column: zero
+    std::vector<int32_t> col_locus;
+    if ((r = read_cols(ctx, &col_locus)) != GNX_OK) return r;
+    memset(host_c1, 0, (size_t)ctx->cfg.L * 8);
+    memset(host_het, 0, (size_t)ctx->cfg.L * 8);
+    for (size_t j = 0; j < col_locus.size(); ++j) { host_c1[col_locus[j]] = h[j]; host_het[col_locus[j]] = h[nbits + j]; }
+  } else {
+    for (int l = 0; l < ctx->cfg.L; ++l) { host_c1[l] = h[l]; host_het[l] = h[nbits + l]; }
+  }
   memcpy(fit_sum, &h[2 * nbits], 8);
   *n = (int64_t)h[2 * nbits + 1];
   return check_device_err(hc);
@@ -2563,7 +2767,10 @@ extern "C" int gnx_stats_ld(gnx_ctx* ctx, uint64_t* host_n11, int64_t* n) {
   if (ctx->burn || ctx->cfg.L == 0) { g_last_error = "no genomes on the device"; return GNX_ERR_STATE; }
   int r = materialise(ctx);
   if (r != GNX_OK) return r;
-  const int Wu = (ctx->cfg.L + 31) / 32, Lp = 32 * Wu;
+  std::vector<int32_t> col_locus;
+  if (ctx->cols && (r = read_cols(ctx, &col_locus)) != GNX_OK) return r;
+  // the column layout counts over its columns and scatters the pairs to their loci below
+  const int Wu = ctx->cols ? std::max<int>(1, ((int)col_locus.size() + 31) / 32) : (ctx->cfg.L + 31) / 32, Lp = 32 * Wu;
   const int ntile = Wu * (Wu + 1) / 2;
   // enough (tile, haplotype range) items to fill the machine a few times over
   const int nsplit = std::max(1, std::min(4096, (ctx->num_sms * 64 + ntile - 1) / ntile));
@@ -2573,12 +2780,27 @@ extern "C" int gnx_stats_ld(gnx_ctx* ctx, uint64_t* host_n11, int64_t* n) {
   PROF(ctx, "k_stats_ld");
   k_stats_ld<<<grid_for(ctx, 8), 256, 0, ctx->stream>>>(ctx->pop, ctx->d_c, d, Wu, Lp, nsplit);
   LAUNCHED(ctx);
-  cudaError_t e = cudaMemcpyAsync(host_n11, d, (size_t)Lp * Lp * 8, cudaMemcpyDeviceToHost, ctx->stream);
+  std::vector<unsigned long long> hcols(ctx->cols ? (size_t)Lp * Lp : 0);
+  cudaError_t e = cudaMemcpyAsync(ctx->cols ? hcols.data() : (unsigned long long*)host_n11, d, (size_t)Lp * Lp * 8,
+                                  cudaMemcpyDeviceToHost, ctx->stream);
   Counters hc;
   r = read_counters(ctx, &hc);
   cudaFree(d);
   if (e != cudaSuccess) { g_last_error = cudaGetErrorString(e); return GNX_ERR_CUDA; }
   if (r != GNX_OK) return r;
+  if (ctx->cols) {
+    // the by-locus answer: entry (i, j) of loci i, j with j / 32 >= i / 32, from the column pair (a, b) -- the
+    // device filled the column word-triangle b / 32 >= a / 32 of the symmetric counts
+    const size_t LpL = (size_t)32 * ((ctx->cfg.L + 31) / 32);
+    memset(host_n11, 0, LpL * LpL * 8);
+    const int nc = (int)col_locus.size();
+    for (int a = 0; a < nc; ++a)
+      for (int b = 0; b < nc; ++b) {
+        const int i = col_locus[a], j = col_locus[b];
+        if (j / 32 < i / 32) continue;
+        host_n11[(size_t)i * LpL + j] = b / 32 >= a / 32 ? hcols[(size_t)a * Lp + b] : hcols[(size_t)b * Lp + a];
+      }
+  }
   *n = hc.n;
   return check_device_err(hc);
 }
@@ -2709,7 +2931,7 @@ extern "C" int gnx_tskit_enable(gnx_ctx* ctx, int64_t edge_capacity, int64_t bir
   Tsk& T = ctx->tsk;
   memset(&T, 0, sizeof T);
   // breakpoints of every cached path: loci where the path switches homologue (genome.py:194-199)
-  const int L = ctx->cfg.L, W = ctx->Wwords, np = ctx->cfg.n_recomb_paths;
+  const int L = ctx->cfg.L, W = 4 * ctx->WqL, np = ctx->cfg.n_recomb_paths;   // paths as simulated: by locus
   std::vector<int32_t> ptr(np + 1, 0), pos;
   for (int k = 0; k < np; ++k) {
     const uint32_t* row = &ctx->host_paths[(size_t)k * W];
@@ -2924,7 +3146,7 @@ extern "C" int gnx_genome_init_end(gnx_ctx* ctx) {
   cudaStream_t s = ctx->stream;
   PROF(ctx, "k_gi_write");
   k_gi_write<<<grid_for(ctx, 8), 256, 0, s>>>(ctx->pop, ctx->d_c, ctx->d_gi_state, ctx->d_gi_lkey, ctx->d_gi_write,
-                                              ctx->cfg.L);
+                                              ctx->cfg.L, ctx->d_cols);
   LAUNCHED(ctx);
   if (ctx->cfg.n_traits > 0 && ctx->have_traits) {
     int r = gnx_phenotype(ctx);

@@ -311,8 +311,13 @@ struct Mut {
   int32_t* chunk_ptr;
   int32_t NW;                      // 32-bit words per homologue
   uint4* paths;                    // cached recombination paths the gamete kernel reads (patched, tskit layout)
-  const uint4* paths_orig;         // as simulated: bit l = (#breakpoints <= l) % 2
-  int32_t n_paths, Wq;
+  const uint4* paths_orig;         // as simulated: bit l = (#breakpoints <= l) % 2, [n_paths][WqL]
+  int32_t n_paths, Wq, WqL;        // 128-bit units per row of `paths` / of `paths_orig`
+  // column layout (gnx_create_cols): genotype bit j holds non-neutral locus col_locus[j]; NULL otherwise
+  int32_t* col_n;                  // [1] columns in use
+  int32_t* col_locus;              // [L]
+  int32_t* col_of_locus;           // [L], -1: no column
+  int32_t col_cap;                 // columns a row holds (128 * Wq)
   gnx_mutation_row_t* log;
   int32_t log_cap;
   int32_t L;

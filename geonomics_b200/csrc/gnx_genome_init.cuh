@@ -192,11 +192,12 @@ __global__ void __launch_bounds__(256) k_gi_select(GiLocus* st, const int32_t* _
   }
 }
 
-// one thread per (entry, 32-locus word): both homologue words of the row.  Loci outside `write`
-// (neutral loci of the tskit layout) and the padding beyond L stay zero.
+// one thread per (entry, 32-bit word): both homologue words of the row.  Loci outside `write`
+// (neutral loci of the tskit layout) and the padding beyond L stay zero.  cols (column layout,
+// {n_cols, col_locus[]}): bit j of the row is locus col_locus[j], the unused columns stay zero.
 __global__ void __launch_bounds__(256) k_gi_write(Pop pop, const Counters* c, const GiLocus* __restrict__ st,
                                                   const uint32_t* __restrict__ lkey, const uint8_t* __restrict__ write,
-                                                  int L) {
+                                                  int L, const int32_t* __restrict__ cols) {
   const int n = c->n, cur = c->cur, Ww = 4 * pop.Wq;
   const long long total = (long long)n * Ww;
   uint32_t* G = reinterpret_cast<uint32_t*>(pop.G);
@@ -205,7 +206,11 @@ __global__ void __launch_bounds__(256) k_gi_write(Pop pop, const Counters* c, co
     const long long id = pop.idx[cur][i];
     uint32_t h0 = 0u, h1 = 0u;
     for (int j = 0; j < 32; ++j) {
-      const int l = 32 * w + j;
+      int l = 32 * w + j;
+      if (cols) {
+        if (l >= cols[0]) break;
+        l = cols[1 + l];
+      }
       if (l >= L) break;
       if (!write[l]) continue;
       const GiLocus s = st[l];

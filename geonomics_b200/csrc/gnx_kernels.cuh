@@ -1558,7 +1558,8 @@ __global__ void __launch_bounds__(256) k_phenotype_all(Pop pop, Traits tr, const
 //   trait, delet_loci_idxs never) and the trait tables are rebuilt to read bit
 //   nonneut[idxs[k]].  The whole CTA then patches bit `locus` of every cached path to the
 //   homologue the path is on in FRONT of the locus (genome.py:133-160: bisect_left of the
-//   breakpoints), which is bit locus - 1 of the path as simulated.
+//   breakpoints), which is bit locus - 1 of the path as simulated.  Column layout: the locus takes
+//   the next free column, and that column stands for bit `locus` in all of the above.
 // ========================================================================================
 __device__ inline int lower_bound_i32(const int32_t* a, int n, int v) {
   int lo = 0, hi = n;
@@ -1585,6 +1586,7 @@ __device__ inline void mut_rebuild_tables(const Mut& mu, Counters* c) {
         int r = ti[k];
         if (r < 0 || r >= nn) { c->err |= GNX_ERRBIT_MUTIDX; r = r < 0 ? 0 : nn - 1; }   // IndexError in the reference
         eff = mu.nonneut[r];
+        if (mu.col_of_locus) eff = mu.col_of_locus[eff];
       }
       const double al = ta[k];
       const double dm = mu.dom1p ? mu.dom1p[tl[k]] : 1.0;      // selection.py:37: dom[trait.loci]
@@ -1619,6 +1621,7 @@ __device__ inline void mut_rebuild_tables(const Mut& mu, Counters* c) {
       int r = mu.delet_idxs[k];
       if (r < 0 || r >= nn) { c->err |= GNX_ERRBIT_MUTIDX; r = r < 0 ? 0 : nn - 1; }
       eff = mu.nonneut[r];
+      if (mu.col_of_locus) eff = mu.col_of_locus[eff];
     }
     mu.delet_eff[k] = eff;
   }
@@ -1628,6 +1631,25 @@ __global__ void k_mut_rebuild(Mut mu, Counters* c) {
   if (threadIdx.x == 0 && blockIdx.x == 0) mut_rebuild_tables(mu, c);
 }
 
+// Widening of the column layout (gnx_widen_cols): every row of wo 128-bit units becomes a row of
+// wn > wo units, the new columns zero (genotype rows of every slot, compact recombination paths).
+__global__ void __launch_bounds__(256) k_widen_rows(const uint4* __restrict__ src, uint4* __restrict__ dst,
+                                                    long long n_rows, int wo, int wn) {
+  const long long total = n_rows * wn;
+  for (long long k = GTID; k < total; k += GSTRIDE) {
+    const long long r = k / wn;
+    const int q = (int)(k - r * wn);
+    dst[k] = q < wo ? src[r * wo + q] : make_uint4(0u, 0u, 0u, 0u);
+  }
+}
+// ... and the trait CSR over 32-bit words: no entry reads a new word, so the new word ranges are empty
+__global__ void k_widen_csr(const int32_t* __restrict__ src, int32_t* __restrict__ dst, int n_tables, int nwo, int nwn) {
+  for (int k = GTID; k < n_tables * (nwn + 1); k += GSTRIDE) {
+    const int t = k / (nwn + 1), q = k - t * (nwn + 1);
+    dst[k] = src[t * (nwo + 1) + min(q, nwo)];
+  }
+}
+
 // STRIP: one strip of a decomposed landscape (by-locus layout only: no tskit layout, trait mutation or
 // tskit rows).  Every rank replays the species-wide sequence -- the births of all ranks, keyed by the
 // species-wide max_ind_idx (k_strip_id_base left both in Counters) -- and so keeps identical tables and
@@ -1635,6 +1657,7 @@ __global__ void k_mut_rebuild(Mut mu, Counters* c) {
 template <bool STRIP>
 __global__ void __launch_bounds__(256) k_mutate(Pop pop, Params prm, Traits tr, DevDraws dr, Mut mu, Counters* c, int tsk_on) {
   __shared__ int new_loci[GNX_MUT_MAX_NEW];
+  __shared__ int new_bits[GNX_MUT_MAX_NEW];    // the genotype bit of each: the locus, or its column
   __shared__ int n_new;
   if (blockIdx.x != 0) return;
   if (threadIdx.x == 0) {
@@ -1652,6 +1675,8 @@ __global__ void __launch_bounds__(256) k_mutate(Pop pop, Params prm, Traits tr, 
       while (type < mu.n_types - 1 && ut >= mu.cdf[type]) ++type;
       if (mu.counts[0] == 0) { c->err |= GNX_ERRBIT_MUTABLES; break; }    // list.pop() on an empty list
       if (type >= 1 && mu.tskit_layout && n_new >= GNX_MUT_MAX_NEW) { c->err |= GNX_ERRBIT_CAPACITY; break; }
+      // column layout: a non-neutral mutation needs a free column; the host widens the rows between steps
+      if (type >= 1 && mu.col_of_locus && *mu.col_n >= mu.col_cap) { c->err |= GNX_ERRBIT_CAPACITY; break; }
       const double s_raw = type == 1 ? (dr.mut_s ? dr.mut_s[m] : sample_gamma(g, mu.s_shape, mu.s_scale)) : 0.0;
       const double sel = fmin(s_raw, 1.0);                                  // genome.py:692
       const int locus = mu.mutables[--mu.counts[0]];                        // mutation.py:73 / :95
@@ -1668,6 +1693,12 @@ __global__ void __launch_bounds__(256) k_mutate(Pop pop, Params prm, Traits tr, 
         for (int k = nn; k > idx; --k) mu.nonneut[k] = mu.nonneut[k - 1];
         mu.nonneut[idx] = locus;
         mu.counts[1] = nn + 1;
+        if (mu.col_of_locus) {                                              // the next free column
+          const int cn = *mu.col_n;
+          mu.col_locus[cn] = locus;
+          mu.col_of_locus[locus] = cn;
+          *mu.col_n = cn + 1;
+        }
         if (type == 1) {
           int nd = mu.counts[2];
           const int di = lower_bound_i32(mu.delet_loci, nd, locus);
@@ -1711,7 +1742,7 @@ __global__ void __launch_bounds__(256) k_mutate(Pop pop, Params prm, Traits tr, 
           for (int k = 0; k < mu.counts[2]; ++k) mu.delet_eff[k] = mu.delet_loci[k];
         // mutation.py:117: spp[individ].g[idx, homol] = 1
         row = lower_bound_i32(mu.nonneut, mu.counts[1], locus);
-        const int bit = mu.tskit_layout ? locus : row;
+        const int bit = !mu.tskit_layout ? row : mu.col_of_locus ? mu.col_of_locus[locus] : locus;
         if (!STRIP || (unsigned)(o - c->births_lo) < (unsigned)c->B) {      // this rank holds offspring o
           uint32_t* hw = reinterpret_cast<uint32_t*>(pop.G + ((size_t)pop.gslot[cur][i] * 2 + homol) * Wq);
           hw[bit >> 5] |= 1u << (bit & 31);
@@ -1736,7 +1767,10 @@ __global__ void __launch_bounds__(256) k_mutate(Pop pop, Params prm, Traits tr, 
             pop.z[cur][(size_t)tt * pop.cap + i] = nl > 1 ? 0.5 + acc : acc;
           }
         }
-        if (mu.tskit_layout) new_loci[n_new++] = locus;
+        if (mu.tskit_layout) {
+          new_loci[n_new] = locus;
+          new_bits[n_new++] = bit;
+        }
       }
       const int nl = mu.counts[3];
       if (nl < mu.log_cap) {
@@ -1762,12 +1796,12 @@ __global__ void __launch_bounds__(256) k_mutate(Pop pop, Params prm, Traits tr, 
   // genome.py:133-160 _update_subsetters: the inserted homologue is the one the path is on in front of the locus
   if (mu.tskit_layout && n_new > 0) {
     for (int pth = threadIdx.x; pth < mu.n_paths; pth += blockDim.x) {
-      const uint32_t* src = reinterpret_cast<const uint32_t*>(mu.paths_orig + (size_t)pth * mu.Wq);
+      const uint32_t* src = reinterpret_cast<const uint32_t*>(mu.paths_orig + (size_t)pth * mu.WqL);
       uint32_t* dst = reinterpret_cast<uint32_t*>(mu.paths + (size_t)pth * mu.Wq);
       for (int k = 0; k < n_new; ++k) {
-        const int l = new_loci[k];
+        const int l = new_loci[k], j = new_bits[k];
         const uint32_t b = l > 0 ? (src[(l - 1) >> 5] >> ((l - 1) & 31)) & 1u : 0u;
-        dst[l >> 5] = (dst[l >> 5] & ~(1u << (l & 31))) | (b << (l & 31));
+        dst[j >> 5] = (dst[j >> 5] & ~(1u << (j & 31))) | (b << (j & 31));
       }
     }
   }

@@ -82,7 +82,11 @@ class DeviceSpecies:
                disp_distr (name, p1, p2), direction_mu, direction_kappa, choose_nearest,
                inverse_dist, density_grid_window_width, move_surf / disp_surf (dicts or None)
     gen_arch : dict with L, paths (uint8[n_paths, L]), traits (list of dicts loci/alpha/phi/
-               gamma/lyr_num/univ_adv), dom (int8[L])   or None (no genomes)
+               gamma/lyr_num/univ_adv), dom (int8[L])   or None (no genomes);
+               cols (the starting non-neutral loci, ascending) selects the column layout of a use_tskit
+               species (gnx_create_cols): genotype rows hold one column per non-neutral locus, and
+               upload(g=...) / download()['g'] take and give the reference's rows [n, n_nonneut, 2] in
+               ascending locus order; col_capacity (optional): the starting columns per row
     """
 
     def __init__(self, land_dim, rasters, prm, gen_arch=None, capacity=None, seed=0,
@@ -99,7 +103,15 @@ class DeviceSpecies:
         traits = (gen_arch or {}).get('traits') or []
         self.n_traits = len(traits)
         self.Lg = int(gen_arch['L']) if gen_arch is not None else 0
-        self.W = gp.words_per_hap(self.Lg)
+        cols = None if gen_arch is None else gen_arch.get('cols')
+        self.cols = cols is not None
+        if self.cols:
+            cols = np.ascontiguousarray(cols, dtype=np.int32)
+            self.W = gp.words_per_hap(int(gen_arch.get('col_capacity') or gp.col_capacity(len(cols))))
+            self.col_capacity = 32 * self.W
+        else:
+            self.W = gp.words_per_hap(self.Lg)
+        self._col_budget = None
         if capacity is None:
             ksum = float(np.sum(rasters[int(prm.get('K_layer', 0))]) * float(prm.get('K_factor', 1.0)))
             capacity = int(max(4096, 3.0 * ksum))
@@ -145,7 +157,11 @@ class DeviceSpecies:
         self._cfg = cfg
 
         self._ctx = C.c_void_p()
-        _lib.check(L.gnx_create(C.byref(cfg), C.byref(self._ctx)), 'gnx_create')
+        if self.cols:
+            _lib.check(L.gnx_create_cols(C.byref(cfg), self.col_capacity, len(cols), _ptr(cols, _lib.c_int32_p),
+                                         C.byref(self._ctx)), 'gnx_create_cols')
+        else:
+            _lib.check(L.gnx_create(C.byref(cfg), C.byref(self._ctx)), 'gnx_create')
         _lib.check(L.gnx_set_rasters(self._ctx, _ptr(rasters, _lib.c_double_p)), 'gnx_set_rasters')
         self._rasters_host = rasters
 
@@ -394,6 +410,27 @@ class DeviceSpecies:
             m.host_subsetters = sb.ctypes.data_as(C.POINTER(C.c_uint8))
         _lib.check(self._L.gnx_set_mutation(self._ctx, C.byref(m)), 'gnx_set_mutation')
         self._mut_tskit = bool(tskit_layout)
+        if self.cols:
+            nonneutral = float(mu_delet) > 0 or (trait_mus is not None and any(float(v) > 0 for v in trait_mus))
+            self._col_budget = gp.ColumnBudget(len(self.read_cols()), self.col_capacity,
+                                               gp.MUT_MAX_NEW if nonneutral else 0, 128 * ((self.Lg + 127) // 128))
+
+    # ---- column layout -----------------------------------------------------------------------
+    def read_cols(self):
+        """int32[n_cols]: the locus of every column, in column order (gnx_read_cols; synchronises)."""
+        out = np.zeros(max(1, self.Lg), np.int32)
+        n, cap = C.c_int32(), C.c_int32()
+        _lib.check(self._L.gnx_read_cols(self._ctx, _ptr(out, _lib.c_int32_p), C.byref(n), C.byref(cap)),
+                   'gnx_read_cols')
+        return out[:n.value].copy()
+
+    def widen_cols(self, col_capacity):
+        """Re-pack the rows to col_capacity columns (between steps; the next step captures its graph again)."""
+        _lib.check(self._L.gnx_widen_cols(self._ctx, int(col_capacity)), 'gnx_widen_cols')
+        self.W = gp.words_per_hap(col_capacity)
+        self.col_capacity = 32 * self.W
+        if self._col_budget is not None:
+            self._col_budget.capacity = self.col_capacity
 
     @staticmethod
     def _mut_type_name(t):
@@ -466,7 +503,7 @@ class DeviceSpecies:
         if idx is not None:
             bufs['idx'] = np.ascontiguousarray(idx, dtype=np.int64)
         if genomes_packed is None and g is not None:
-            genomes_packed = gp.pack_genomes(g)
+            genomes_packed = gp.rows_to_cols(g, self.read_cols(), self.W) if self.cols else gp.pack_genomes(g)
         if genomes_packed is not None:
             gpk = np.ascontiguousarray(genomes_packed, dtype=np.uint32)
             assert gpk.shape == (n, 2, self.W), (gpk.shape, (n, 2, self.W))
@@ -498,7 +535,11 @@ class DeviceSpecies:
         _lib.check(self._L.gnx_download_population(self._ctx, C.byref(p)), 'gnx_download_population')
         out = {k: v for k, v in bufs.items() if k != 'n'}
         out['max_ind_idx'] = int(p.max_ind_idx)
-        if 'genomes' in out and unpack:
+        if 'genomes' in out and self.cols:
+            out['col_locus'] = self.read_cols()
+            if unpack:
+                out['g'] = gp.cols_to_rows(out['genomes'], out['col_locus'])
+        elif 'genomes' in out and unpack:
             out['g'] = gp.unpack_genomes(out['genomes'], self.Lg)
         return out
 
@@ -580,7 +621,16 @@ class DeviceSpecies:
 
     # ---- stepping ------------------------------------------------------------------------
     def step(self, n_steps=1, sync=False):
-        _lib.check(self._L.gnx_step(self._ctx, int(n_steps)), 'gnx_step')
+        n_steps = int(n_steps)
+        while self._col_budget is not None and n_steps > 0:
+            # column layout: widen before a step could run out of free columns
+            k, cap = self._col_budget.take(n_steps, lambda: len(self.read_cols()))
+            if cap > self.col_capacity:
+                self.widen_cols(cap)
+            _lib.check(self._L.gnx_step(self._ctx, k), 'gnx_step')
+            n_steps -= k
+        if n_steps > 0:
+            _lib.check(self._L.gnx_step(self._ctx, n_steps), 'gnx_step')
         if sync:
             self.sync()
 

@@ -376,7 +376,9 @@ int gnx_tskit_renumber(gnx_ctx* ctx);
  *        behind the insertion point of the mutated trait itself and delet_loci_idxs never, so
  *        after mutations they may address other rows than the trait's / deleterious loci; the
  *        phenotype (selection.py:30) and the deleterious fitness (selection.py:86-88) read row
- *        idxs[k], i.e. bit nonneut_loci[idxs[k]].  Each log row carries the tskit node of the
+ *        idxs[k], i.e. bit nonneut_loci[idxs[k]].  A context of gnx_create_cols keeps the same
+ *        semantics on one COLUMN per non-neutral locus: bit col_of_locus[l] stands for bit l above, a
+ *        non-neutral mutation takes the next free column, and the path patch goes to that column.  Each log row carries the tskit node of the
  *        mutated homologue (mutations-table row of mutation.py:44-58: site = locus, node,
  *        derived_state '1', time = -t) when tskit recording is enabled.
  *      gnx_set_traits must precede gnx_set_mutation; re-setting the traits disables mutation. */
@@ -425,6 +427,26 @@ int gnx_read_mutations(gnx_ctx* ctx, gnx_mutation_row_t* rows, int32_t max_rows,
  * Without tskit_layout the idxs are the rows of the loci themselves. */
 int gnx_read_mutation_tables(gnx_ctx* ctx, int32_t trait, int32_t* n_loci, int32_t* host_loci, double* host_alpha,
                              int32_t* host_loci_idxs, int32_t* host_delet_loci_idxs);
+
+/* ---- column genotype layout of a use_tskit species --------------------------------------------
+ * The by-locus layout keeps one bit per locus even under tskit_layout, where only the non-neutral loci
+ * carry information.  A context created by gnx_create_cols keeps col_capacity COLUMNS per homologue
+ * instead (rounded up to a multiple of 128; a homologue is 16 * col_capacity / 128 bytes): column j holds
+ * non-neutral locus col_locus[j].  host_col_locus names the starting columns (usually the ascending
+ * non-neutral loci); every non-neutral mutation takes the next free column; columns are never freed and no
+ * bit ever moves.  Everything observable is as under the by-locus tskit layout (gnx_set_mutation must give
+ * tskit_layout = 1 and host_nonneut_loci = the column loci; gnx_set_traits takes loci, all of them columns;
+ * gnx_set_recomb_paths takes the paths as simulated, by locus), except that gnx_population_t.genomes,
+ * GNX_F_GENOMES and gnx_genome_init_end use column rows [n][2][4 * col_capacity / 128].  gnx_stats_genotypes
+ * (_region) and gnx_stats_ld count over the columns and return the by-locus arrays, zero at loci without a
+ * column.  A non-neutral mutation that finds no free column inside a step is GNX_ERR_CAPACITY: the caller
+ * widens between steps (gnx_widen_cols re-packs the genotype rows, the paths and the trait tables to the
+ * wider rows; the next gnx_step captures its graph again).  Not supported under strip decomposition. */
+int gnx_create_cols(const gnx_config_t* cfg, int32_t col_capacity, int32_t n_cols, const int32_t* host_col_locus,
+                    gnx_ctx** out);
+/* the current columns: host_col_locus [L] (column order) or NULL; synchronises */
+int gnx_read_cols(gnx_ctx* ctx, int32_t* host_col_locus, int32_t* n_cols, int32_t* col_capacity);
+int gnx_widen_cols(gnx_ctx* ctx, int32_t col_capacity);
 
 /* ---- device assignment of the starting genomes (species.py:956-1094, genome.py:1108-1157) -----------
  * An alternative to uploading host-built genotypes after the burn-in.  Locus l gets exactly
