@@ -170,6 +170,13 @@ class TskitRows(C.Structure):
     ]
 
 
+class StepStatus(C.Structure):
+    _fields_ = [('steps_run', C.c_int32), ('stopped', C.c_int32),
+                ('need_entries', C.c_int64), ('need_slots', C.c_int64), ('need_births', C.c_int64),
+                ('need_edges', C.c_int64), ('capacity', C.c_int64), ('born_capacity', C.c_int64),
+                ('edge_capacity', C.c_int64)]
+
+
 class GenomeInit(C.Structure):
     _fields_ = [
         ('seed', C.c_uint64),
@@ -231,6 +238,10 @@ SIGNATURES = {
     'gnx_set_life_history': (C.c_int, [_ctx, C.POINTER(Config)]),
     'gnx_step': (C.c_int, [_ctx, C.c_int32]),
     'gnx_sync': (C.c_int, [_ctx]),
+    'gnx_set_growth_guard': (C.c_int, [_ctx, C.c_int32]),
+    'gnx_step_status': (C.c_int, [_ctx, C.POINTER(StepStatus)]),
+    'gnx_reserve': (C.c_int, [_ctx, C.c_int64]),
+    'gnx_tskit_reserve': (C.c_int, [_ctx, C.c_int64, C.c_int64]),
     'gnx_walk_host': (C.c_int, [_ctx, C.POINTER(Population), C.c_int32]),
     'gnx_walk_host_begin': (C.c_int, [_ctx, C.POINTER(Population), C.c_int32]),
     'gnx_walk_host_end': (C.c_int, [_ctx, C.POINTER(Population)]),

@@ -26,7 +26,7 @@ from collections import OrderedDict
 import numpy as np
 
 from . import genome_pack as gp
-from .device import DeviceSpecies
+from .device import DeviceSpecies, growth_capacity
 
 
 # ---------------------------------------------------------------------------------------------
@@ -710,8 +710,10 @@ class Species:
         else:
             if capacity is None:
                 capacity = int(max(4096, 3.0 * float(np.sum(self.K)), 2 * self.start_N))
+            # the population may outgrow the starting capacity (a K raised by a landscape or demographic
+            # change, a high lambda): the buffers grow between steps
             self._dev = DeviceSpecies(land.dim, rasters, self._device_params(), ga, capacity=capacity,
-                                      seed=self._seed, res_ratio=self._land_res_ratio)
+                                      seed=self._seed, res_ratio=self._land_res_ratio, grow=True)
         land._listeners.append(self)
         self._dev.set_burn(not self.burned)
         self._dev.upload(p['x'], p['y'], p['age'], p['sex'], p['idx'], max_ind_idx=self.max_ind_idx,
@@ -864,7 +866,17 @@ class Species:
                 self._step(k)
                 done += k
             return
-        self._dev.step(n)
+        stop = self._dev.step(n)
+        while stop is not None:
+            # a step would overflow the tskit row buffers: drain them, grow them only if one step still
+            # needs more, and go on (every step runs: walk's `ran < n` keeps meaning extinction)
+            births, edges = self._drain_tskit()
+            need_b, need_e = stop['need_births'] - births, stop['need_edges'] - edges
+            ecap, bcap = stop['edge_capacity'], stop['born_capacity']
+            if need_b > bcap or need_e > ecap:
+                self._dev.tskit_reserve(growth_capacity(need_e, ecap) if need_e > ecap else ecap,
+                                        growth_capacity(need_b, bcap) if need_b > bcap else bcap)
+            stop = self._dev.step(stop['steps_left'])
         recs = self._dev.step_records()
         if tsk:
             self._drain_tskit()
@@ -1139,8 +1151,10 @@ class Species:
     def _drain_tskit(self):
         """Device row buffers -> self._tc (species.py:692-736 rows, in the reference's order)."""
         if self._tc is None or self._dev is None:
-            return
-        self._tc.append_births(self._dev.tskit_drain())
+            return 0, 0
+        rows = self._dev.tskit_drain()
+        self._tc.append_births(rows)
+        return len(rows['idx']), len(rows['left'])
 
     def _sort_and_simplify_table_collection(self):
         """species.py:1107-1219: sort + simplify on the current nodes, then nodes 2k, 2k + 1 in species order and

@@ -108,6 +108,14 @@ struct gnx_ctx {
   uint32_t* d_cs_tab = nullptr;
   int64_t records_pending = 0;          // step records written since the last gnx_read_step_records
   int64_t graph_launches = 0, graph_captures = 0;
+  // growth guard (gnx_set_growth_guard): the device status block k_step_guard writes, and the last
+  // gnx_step batch as the host saw it (steps enqueued, steps run and a stop found by a host check)
+  bool grow_guard = false;
+  gnx_step_status_t* d_grow = nullptr;
+  int32_t tsk_max_bp = 0;               // largest breakpoint count of a cached path (gnx_tskit_enable)
+  int64_t grow_enqueued = 0, grow_host_run = 0;
+  bool grow_host_stop = false, grow_graph = false;   // grow_graph: the batch launched a guarded graph
+  gnx_step_status_t grow_host_need{};
   void* d_paths = nullptr;
   void* d_surf_tab[2] = {nullptr, nullptr};
   // strip domain decomposition (gnx_strip.cuh)
@@ -1067,6 +1075,13 @@ static int run_scan(gnx_ctx* ctx, F f, const char* name);
 // Deaths a fused step left flagged are applied now (explicit stable compaction), so that every
 // host-facing view sees exactly the live population.
 static int materialise(gnx_ctx* ctx) {
+  if (ctx->grow_guard && !ctx->capturing) {
+    // the guard may have skipped the steps that would have left deaths pending: ask the device
+    Counters h;
+    int r = read_counters(ctx, &h);
+    if (r != GNX_OK) return r;
+    ctx->pending = h.pending != 0;
+  }
   if (!ctx->pending) return GNX_OK;
   MortalityScan ms{ctx->pop, ctx->work, ctx->d_c, ctx->burn};
   int r = run_scan(ctx, ms, "scan_mortality");
@@ -2074,8 +2089,55 @@ static void step_key(const gnx_ctx* ctx, std::vector<unsigned char>* key) {
   put(&ctx->dens, sizeof ctx->dens);
   put(&ctx->tsk, sizeof ctx->tsk);
   put(&ctx->mut, sizeof ctx->mut);
-  const int flags[3] = {ctx->burn, ctx->have_density ? 1 : 0, ctx->mut_delet ? 1 : 0};
+  const int flags[5] = {ctx->burn, ctx->have_density ? 1 : 0, ctx->mut_delet ? 1 : 0, ctx->grow_guard ? 1 : 0,
+                        ctx->tsk_max_bp};
   put(flags, sizeof flags);
+}
+
+static GrowthBound growth_bound(const gnx_ctx* ctx) {
+  GrowthBound g;
+  g.lambda = ctx->cfg.n_births_lambda;
+  g.fixed = ctx->cfg.n_births_fixed ? 1 : 0;
+  g.genomes = ctx->burn ? 0 : 1;
+  g.tsk = (ctx->tsk.enabled && !ctx->burn) ? 1 : 0;
+  g.edges_per_birth = 2 * (ctx->tsk_max_bp + 1);
+  g.cap = ctx->pop.cap;
+  g.born_cap = ctx->tsk.born_cap;
+  g.edge_cap = ctx->tsk.edge_cap;
+  return g;
+}
+
+// The guarded step: k_step_guard -> IF node whose body holds the captured step as a child graph.
+// Nothing is captured into the conditional body; `step` is cloned into it (the caller destroys it).
+static int guard_graph(gnx_ctx* ctx, cudaGraph_t step, cudaGraph_t* out) {
+  cudaGraph_t g = nullptr;
+  CK(cudaGraphCreate(&g, 0));
+  cudaGraphConditionalHandle h;
+  GrowthBound gb = growth_bound(ctx);
+  const Counters* c = ctx->d_c;
+  void* args[4] = {&c, &gb, &ctx->d_grow, &h};
+  cudaKernelNodeParams kp = {};
+  kp.func = (void*)k_step_guard;
+  kp.gridDim = dim3(1);
+  kp.blockDim = dim3(1);
+  kp.kernelParams = args;
+  cudaGraphNodeParams cp = {};
+  cp.type = cudaGraphNodeTypeConditional;
+  cp.conditional.type = cudaGraphCondTypeIf;
+  cp.conditional.size = 1;
+  cudaGraphNode_t guard, cond, child;
+  cudaError_t e = cudaGraphConditionalHandleCreate(&h, g, 0, 0);
+  if (e == cudaSuccess) e = cudaGraphAddKernelNode(&guard, g, nullptr, 0, &kp);
+  cp.conditional.handle = h;
+  if (e == cudaSuccess) e = cudaGraphAddNode(&cond, g, &guard, 1, &cp);
+  if (e == cudaSuccess) e = cudaGraphAddChildGraphNode(&child, cp.conditional.phGraph_out[0], nullptr, 0, step);
+  if (e != cudaSuccess) {
+    cudaGraphDestroy(g);
+    g_last_error = std::string("building the guarded step graph: ") + cudaGetErrorString(e);
+    return GNX_ERR_CUDA;
+  }
+  *out = g;
+  return GNX_OK;
 }
 
 static void drop_graph(gnx_ctx* ctx) {
@@ -2096,6 +2158,14 @@ static int capture_step(gnx_ctx* ctx) {
   ctx->launches = launches0;                 // nothing ran yet
   if (r != GNX_OK) { if (graph) cudaGraphDestroy(graph); return r; }
   if (e != cudaSuccess) { g_last_error = cudaGetErrorString(e); return GNX_ERR_CUDA; }
+  if (ctx->grow_guard) {
+    cudaGraph_t guarded = nullptr;
+    r = guard_graph(ctx, graph, &guarded);
+    cudaGraphDestroy(graph);
+    if (r != GNX_OK) return r;
+    graph = guarded;
+    ctx->graph_kernels += 1;
+  }
   e = cudaGraphInstantiate(&ctx->graph_exec, graph, 0);
   cudaGraphDestroy(graph);
   if (e != cudaSuccess) { ctx->graph_exec = nullptr; g_last_error = cudaGetErrorString(e); return GNX_ERR_CUDA; }
@@ -2120,6 +2190,11 @@ extern "C" int gnx_step(gnx_ctx* ctx, int32_t n_steps) {
     return GNX_ERR_STATE;
   }
   const bool lazy = ctx->cfg.mating_radius > 0;
+  if (ctx->grow_guard) {                     // a new batch for gnx_step_status
+    ctx->grow_enqueued = ctx->grow_host_run = 0;
+    ctx->grow_host_stop = ctx->grow_graph = false;
+    CK(cudaMemsetAsync(ctx->d_grow, 0, sizeof(gnx_step_status_t), ctx->stream));
+  }
   std::vector<unsigned char> key;
   for (int k = 0; k < n_steps; ++k) {
     if (ctx->prm.ordered) {
@@ -2138,17 +2213,215 @@ extern "C" int gnx_step(gnx_ctx* ctx, int32_t n_steps) {
         }
       }
       CK(cudaGraphLaunch(ctx->graph_exec, ctx->stream));
+      ctx->grow_graph = ctx->grow_guard;
       ctx->launches += ctx->graph_kernels;
       ctx->graph_launches += 1;
     } else {
+      if (ctx->grow_guard) {                 // the same check as k_step_guard, on the host
+        Counters h;
+        int r = read_counters(ctx, &h);
+        if (r != GNX_OK) return r;
+        if (!growth_check(growth_bound(ctx), h.n, h.n_slots, h.n_free, h.n_born, h.n_edges, &ctx->grow_host_need)) {
+          ctx->grow_host_stop = true;
+          break;                             // every later step would stop as well
+        }
+        ctx->grow_host_run += 1;
+      }
       int r = one_step(ctx);
       if (r != GNX_OK) return r;
     }
+    ctx->grow_enqueued += 1;
     ctx->records_pending += 1;
     ctx->steps_done += 1;
     ctx->pending = lazy;
     ctx->order_valid = false;
   }
+  return GNX_OK;
+}
+
+extern "C" int gnx_set_growth_guard(gnx_ctx* ctx, int32_t on) {
+  ARG(ctx, "null ctx");
+  if (ctx->d_strip) { g_last_error = "the growth guard is not supported under strip decomposition"; return GNX_ERR_STATE; }
+  USE_DEVICE(ctx);
+  if (on && !ctx->d_grow) DM(ctx, &ctx->d_grow, 1);
+  ctx->grow_guard = on != 0;
+  ctx->grow_enqueued = ctx->grow_host_run = 0;
+  ctx->grow_host_stop = ctx->grow_graph = false;
+  return GNX_OK;
+}
+
+extern "C" int gnx_step_status(gnx_ctx* ctx, gnx_step_status_t* out) {
+  ARG(ctx && out, "null");
+  if (!ctx->grow_guard) { g_last_error = "the growth guard is off"; return GNX_ERR_STATE; }
+  USE_DEVICE(ctx);
+  gnx_step_status_t st;
+  CK(cudaMemcpyAsync(&st, ctx->d_grow, sizeof st, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  st.steps_run += (int32_t)ctx->grow_host_run;
+  if (ctx->grow_host_stop || !ctx->grow_graph) {       // the last check of the batch ran on the host
+    st.stopped = ctx->grow_host_stop ? 1 : 0;
+    st.need_entries = ctx->grow_host_need.need_entries;
+    st.need_slots = ctx->grow_host_need.need_slots;
+    st.need_births = ctx->grow_host_need.need_births;
+    st.need_edges = ctx->grow_host_need.need_edges;
+  }
+  // launches the guard skipped wrote no record and did not advance the step counter
+  const int64_t skipped = ctx->grow_enqueued - st.steps_run;
+  ctx->records_pending -= skipped;
+  ctx->steps_done -= skipped;
+  ctx->grow_enqueued = st.steps_run;
+  st.capacity = ctx->pop.cap;
+  st.born_capacity = ctx->tsk.enabled ? ctx->tsk.born_cap : 0;
+  st.edge_capacity = ctx->tsk.enabled ? ctx->tsk.edge_cap : 0;
+  *out = st;
+  Counters h;
+  int r = read_counters(ctx, &h);
+  if (r != GNX_OK) return r;
+  return check_device_err(h);
+}
+
+// ---- re-allocation of the buffers sized from a capacity ----------------------------------------
+// One buffer to grow: rows x (old -> new) bytes, row r at r * old / r * new (a [rows][cap] array);
+// rows = 1 for everything laid out by entry.
+struct Regrow {
+  void** p;
+  size_t old_bytes, new_bytes;
+  size_t rows;
+  std::vector<void*>* bucket;
+  void* q;
+};
+
+// Allocates every new buffer before it frees an old one: a failed allocation leaves the context on its
+// old buffers.  The old contents are copied (state and scratch alike) and the rest is zeroed.
+static int regrow(gnx_ctx* ctx, std::vector<Regrow>& v) {
+  for (auto& g : v) {
+    g.q = nullptr;
+    if (cudaMalloc(&g.q, std::max<size_t>(g.new_bytes, 1)) != cudaSuccess) {
+      cudaGetLastError();
+      for (auto& f : v) if (f.q) cudaFree(f.q);
+      g_last_error = "out of device memory growing the buffers (the context keeps its old ones)";
+      return GNX_ERR_CUDA;
+    }
+  }
+  cudaStream_t s = ctx->stream;
+  for (auto& g : v) {
+    CK(cudaMemsetAsync(g.q, 0, std::max<size_t>(g.new_bytes, 1), s));
+    const size_t po = g.old_bytes / g.rows, pn = g.new_bytes / g.rows;
+    for (size_t r = 0; r < g.rows; ++r)
+      CK(cudaMemcpyAsync((char*)g.q + r * pn, (const char*)*g.p + r * po, po, cudaMemcpyDeviceToDevice, s));
+  }
+  CK(cudaStreamSynchronize(s));
+  for (auto& g : v) {
+    std::replace(g.bucket->begin(), g.bucket->end(), *g.p, g.q);
+    CK(cudaFree(*g.p));
+    *g.p = g.q;
+  }
+  return GNX_OK;
+}
+
+template <class T>
+static void regrow_add(std::vector<Regrow>& v, T** p, size_t n_old, size_t n_new, std::vector<void*>* bucket,
+                       size_t rows = 1) {
+  v.push_back(Regrow{reinterpret_cast<void**>(p), std::max<size_t>(n_old, 1) * rows * sizeof(T),
+                     std::max<size_t>(n_new, 1) * rows * sizeof(T), rows, bucket, nullptr});
+}
+
+extern "C" int gnx_reserve(gnx_ctx* ctx, int64_t capacity) {
+  ARG(ctx, "null ctx");
+  if (ctx->d_strip) { g_last_error = "gnx_reserve: a strip keeps its capacity"; return GNX_ERR_STATE; }
+  ARG(capacity < (1ll << 31) - 4096, "capacity");
+  if (capacity <= ctx->pop.cap) return GNX_OK;
+  USE_DEVICE(ctx);
+  CK(cudaStreamSynchronize(ctx->stream));
+  Pop& P = ctx->pop;
+  Work& W = ctx->work;
+  const size_t co = (size_t)P.cap, cn = (size_t)capacity;
+  const size_t T1 = std::max(1, ctx->cfg.n_traits), row = (size_t)2 * ctx->Wq;
+  auto hist = [](size_t c) { return (size_t)256 * (c / RS_TILE + 2); };
+  auto tiles = [&](size_t c) { return std::max(std::max(c, (size_t)ctx->ncell), hist(c)) / SCAN_TILE + 2; };
+  auto heavy = [](size_t c) { return c / 4 + 1024; };
+  std::vector<Regrow> v;
+  std::vector<void*>* A = &ctx->allocs;
+  for (int h = 0; h < 2; ++h) {
+    regrow_add(v, &P.xy[h], co, cn, A);
+    regrow_add(v, &P.age[h], co, cn, A);
+    regrow_add(v, &P.sex[h], co, cn, A);
+    regrow_add(v, &P.idx[h], co, cn, A);
+    regrow_add(v, &P.gslot[h], co, cn, A);
+    regrow_add(v, &P.z[h], co, cn, A, T1);              // [T][cap]
+    regrow_add(v, &P.fit[h], co, cn, A);
+    regrow_add(v, &P.ord[h], co, cn, A);
+    regrow_add(v, &W.sort_keys[h], co, cn, A);
+    regrow_add(v, &W.sort_vals[h], co, cn, A);
+    if (ctx->tsk.enabled)
+      for (int b = 0; b < 2; ++b) regrow_add(v, &P.node[h][b], co, cn, &ctx->tsk_allocs);
+  }
+  regrow_add(v, &P.G, co * row, cn * row, A);
+  regrow_add(v, &P.free_slots, co, cn, A);
+  regrow_add(v, &ctx->d_stage_genomes, co * row, cn * row, A);
+  regrow_add(v, &ctx->d_stage_z, co * T1, cn * T1, A);
+  regrow_add(v, &W.mkey, co, cn, A);
+  regrow_add(v, &W.bucket, co, cn, A);
+  regrow_add(v, &W.skey, co, cn, A);
+  regrow_add(v, &W.inv, co, cn, A);
+  regrow_add(v, &W.perm, co, cn, A);
+  regrow_add(v, &W.sort_hist, hist(co), hist(cn), A);
+  double* scratch = static_cast<double*>(W.scratch);
+  regrow_add(v, &scratch, 2 * co * T1, 2 * cn * T1, A);
+  regrow_add(v, &W.mate, co, cn, A);
+  regrow_add(v, &W.heavy, heavy(co), heavy(cn), A);
+  regrow_add(v, &W.fm_list, co, cn, A);
+  regrow_add(v, &W.n_nbrs, co, cn, A);
+  regrow_add(v, &W.pairs, 2 * co, 2 * cn, A);
+  regrow_add(v, &W.pair_slots, 2 * co, 2 * cn, A);
+  regrow_add(v, &W.nb, co, cn, A);
+  regrow_add(v, &W.off_start, co, cn, A);
+  regrow_add(v, &W.off_pair, co, cn, A);
+  regrow_add(v, &W.mid, co, cn, A);
+  regrow_add(v, &W.alive, co, cn, A);
+  regrow_add(v, &W.death_p, co, cn, A);
+  regrow_add(v, &W.disp_tries, co, cn, A);
+  regrow_add(v, &W.tile_sums, tiles(co), tiles(cn), A);
+  regrow_add(v, &W.e_out, co * ctx->cfg.n_layers, cn * ctx->cfg.n_layers, A);
+  int r = regrow(ctx, v);
+  if (r != GNX_OK) return r;
+  W.scratch = scratch;
+  W.heavy_cap = (int32_t)heavy(cn);
+  P.cap = (int32_t)capacity;
+  ctx->cfg.capacity = capacity;
+  ctx->prm.c.capacity = capacity;
+  return GNX_OK;                       // the pointers changed: the next gnx_step captures its graph again
+}
+
+extern "C" int gnx_tskit_reserve(gnx_ctx* ctx, int64_t edge_capacity, int64_t birth_capacity) {
+  ARG(ctx, "null ctx");
+  if (!ctx->tsk.enabled) { g_last_error = "tskit recording not enabled"; return GNX_ERR_STATE; }
+  ARG(edge_capacity < (1ll << 31) && birth_capacity < (1ll << 31), "capacities");
+  USE_DEVICE(ctx);
+  CK(cudaStreamSynchronize(ctx->stream));
+  Tsk& T = ctx->tsk;
+  const size_t T1 = std::max(1, ctx->cfg.n_traits);
+  const size_t eo = (size_t)T.edge_cap, en = (size_t)std::max<int64_t>(edge_capacity, T.edge_cap);
+  const size_t bo = (size_t)T.born_cap, bn = (size_t)std::max<int64_t>(birth_capacity, T.born_cap);
+  std::vector<Regrow> v;
+  std::vector<void*>* B = &ctx->tsk_allocs;
+  if (en > eo) {
+    regrow_add(v, &T.e_left, eo, en, B);
+    regrow_add(v, &T.e_right, eo, en, B);
+    regrow_add(v, &T.e_parent, eo, en, B);
+    regrow_add(v, &T.e_child, eo, en, B);
+  }
+  if (bn > bo) {
+    regrow_add(v, &T.b_idx, bo, bn, B);
+    regrow_add(v, &T.b_x, bo, bn, B);
+    regrow_add(v, &T.b_y, bo, bn, B);
+    regrow_add(v, &T.b_z, bo, bn, B, T1);               // [T][born_cap]
+    regrow_add(v, &T.b_time, bo, bn, B);
+  }
+  int r = regrow(ctx, v);
+  if (r != GNX_OK) return r;
+  T.edge_cap = (int32_t)en;
+  T.born_cap = (int32_t)bn;
   return GNX_OK;
 }
 
@@ -2166,6 +2439,7 @@ extern "C" int gnx_strip_enable(gnx_ctx* ctx, const gnx_strip_config_t* sc) {
   ARG(sc->world >= 1 && sc->world <= GNX_STRIP_MAX_WORLD && sc->rank >= 0 && sc->rank < sc->world, "rank / world");
   ARG(ctx->cfg.mating_radius > 0, "strip decomposition needs a mating radius (panmixia has no locality)");
   ARG(!ctx->tsk.enabled, "strip decomposition does not carry tskit rows");
+  ARG(!ctx->grow_guard, "a strip keeps its capacity: turn the growth guard off first");
   ARG(!ctx->cols, "strip decomposition does not carry the column genotype layout");
   ARG(!ctx->mut.enabled || !ctx->mut.own_tables,
       "strip decomposition does not carry the tskit genotype layout or trait mutation");
@@ -2946,6 +3220,8 @@ extern "C" int gnx_tskit_enable(gnx_ctx* ctx, int64_t edge_capacity, int64_t bir
   int r;
   if ((r = upload_vec(ctx, ptr, &T.bp_ptr, ctx->tsk_allocs)) != GNX_OK) return r;
   if ((r = upload_vec(ctx, pos, &T.bp_pos, ctx->tsk_allocs)) != GNX_OK) return r;
+  ctx->tsk_max_bp = 0;
+  for (int k = 0; k < np; ++k) ctx->tsk_max_bp = std::max(ctx->tsk_max_bp, ptr[k + 1] - ptr[k]);
   T.L = (double)L;
   T.edge_cap = (int32_t)edge_capacity;
   T.born_cap = (int32_t)birth_capacity;

@@ -1508,6 +1508,51 @@ struct TskitScan {
   }
 };
 
+// ---- growth guard (gnx_set_growth_guard) --------------------------------------------------
+// What one step may need, judged from the counters at step start.  Every focal makes at most one
+// pair (mating.py:62-63), so P <= n: fixed births give at most lambda * n newborns; Poisson births
+// sum to Poisson(lambda * P), bounded by ceil(lambda n + 10 sqrt(lambda n)) + 32 (tail below 1e-15,
+// DESIGN.md section 8).  n counts the dead the previous step only flagged, so it is an upper bound.
+struct GrowthBound {
+  double lambda;
+  int32_t fixed;            // n_births_fixed: lambda is the integer litter size
+  int32_t genomes;          // genome slots are taken (not in burn-in, which returns none)
+  int32_t tsk;              // tskit rows are written
+  int32_t edges_per_birth;  // 2 * (largest breakpoint count of a cached path + 1)
+  int64_t cap, born_cap, edge_cap;
+};
+
+__host__ __device__ inline int64_t growth_max_births(double lambda, int fixed, int64_t n) {
+  if (fixed) return (int64_t)(int32_t)lambda * n;
+  const double m = lambda * (double)n;
+  return (int64_t)ceil(m + 10.0 * sqrt(m)) + 32;
+}
+
+// fills the capacities the step needs; 1: they all fit, the step may run
+__host__ __device__ inline int growth_check(const GrowthBound& g, int64_t n, int64_t n_slots, int64_t n_free,
+                                            int64_t n_born, int64_t n_edges, gnx_step_status_t* need) {
+  const int64_t B = growth_max_births(g.lambda, g.fixed, n);
+  need->need_entries = n + B;
+  need->need_slots = g.genomes ? n_slots + (B > n_free ? B - n_free : 0) : 0;   // newborns take free slots first
+  need->need_births = g.tsk ? n_born + B : 0;
+  need->need_edges = g.tsk ? n_edges + B * g.edges_per_birth : 0;
+  return need->need_entries <= g.cap && need->need_slots <= g.cap && need->need_births <= g.born_cap &&
+         need->need_edges <= g.edge_cap;
+}
+
+// first node of a guarded step graph: runs the step body (IF conditional) only when it cannot overflow
+__global__ void k_step_guard(const Counters* c, GrowthBound g, gnx_step_status_t* st, cudaGraphConditionalHandle h) {
+  gnx_step_status_t need;
+  const int ok = growth_check(g, c->n, c->n_slots, c->n_free, c->n_born, c->n_edges, &need);
+  st->steps_run += ok;
+  st->stopped = !ok;
+  st->need_entries = need.need_entries;
+  st->need_slots = need.need_slots;
+  st->need_births = need.need_births;
+  st->need_edges = need.need_edges;
+  cudaGraphSetConditional(h, ok);
+}
+
 __global__ void k_after_births(Counters* c, int tsk_enabled) {
   const int B = c->B;
   if (tsk_enabled) {

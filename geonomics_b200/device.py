@@ -69,6 +69,22 @@ def cell_stats_from_sums(sum_diff, sum_sq_diff, ncell):
     return mean, float(np.sqrt(max(sum_sq_diff / float(ncell) - mean * mean, 0.0)))
 
 
+def max_births(lam, fixed, n):
+    """Most births one step of n individuals can have (k_step_guard): every focal makes at most one pair,
+    so fixed births give at most lam * n; Poisson births ceil(lam n + 10 sqrt(lam n)) + 32, whose tail
+    probability is below 1e-15."""
+    if fixed:
+        return int(lam) * int(n)
+    m = float(lam) * float(n)
+    return int(np.ceil(m + 10.0 * np.sqrt(m))) + 32
+
+
+def growth_capacity(need, capacity):
+    """The size to grow a buffer of `capacity` to when a step needs `need`: at least double, so that a
+    population growing steadily re-allocates a logarithmic number of times."""
+    return max(int(need), 2 * int(capacity))
+
+
 class DeviceSpecies:
     """One Species resident on the GPU.
 
@@ -87,10 +103,13 @@ class DeviceSpecies:
                species (gnx_create_cols): genotype rows hold one column per non-neutral locus, and
                upload(g=...) / download()['g'] take and give the reference's rows [n, n_nonneut, 2] in
                ascending locus order; col_capacity (optional): the starting columns per row
+    grow     : let the population outgrow `capacity`: every step first checks that it cannot overflow a
+               buffer, and step() grows the buffers in front of a step that could (gnx_set_growth_guard);
+               the run is bit-identical to one started at the larger capacity
     """
 
     def __init__(self, land_dim, rasters, prm, gen_arch=None, capacity=None, seed=0,
-                 disp_tries_injected=6, res_ratio=(1.0, 1.0)):
+                 disp_tries_injected=6, res_ratio=(1.0, 1.0), grow=False):
         L = _lib.lib()
         self._L = L
         self.land_dim = (int(land_dim[0]), int(land_dim[1]))
@@ -179,6 +198,9 @@ class DeviceSpecies:
             _lib.check(L.gnx_set_surface_tables(self._ctx, _ptr(mv, _lib.c_uint16_p), _ptr(dv, _lib.c_uint16_p)),
                        'gnx_set_surface_tables')
         self._keep = []
+        self.grow = bool(grow)
+        if self.grow:
+            _lib.check(L.gnx_set_growth_guard(self._ctx, 1), 'gnx_set_growth_guard')
 
     # ---- setup -----------------------------------------------------------------------
     def set_recomb_paths(self, paths):
@@ -621,18 +643,53 @@ class DeviceSpecies:
 
     # ---- stepping ------------------------------------------------------------------------
     def step(self, n_steps=1, sync=False):
+        """Enqueue n_steps steps.  With grow, the population capacity is grown (reserve) in front of any
+        step that could outgrow it, and the call returns None once every step ran, or the step_status()
+        dict, with 'steps_left', of a stop on the tskit row buffers (the caller drains them, grows them
+        with tskit_reserve if one step still needs more, and steps on)."""
         n_steps = int(n_steps)
-        while self._col_budget is not None and n_steps > 0:
-            # column layout: widen before a step could run out of free columns
-            k, cap = self._col_budget.take(n_steps, lambda: len(self.read_cols()))
-            if cap > self.col_capacity:
-                self.widen_cols(cap)
+        while n_steps > 0:
+            k = n_steps
+            if self._col_budget is not None:
+                # column layout: widen before a step could run out of free columns
+                k, cap = self._col_budget.take(n_steps, lambda: len(self.read_cols()))
+                if cap > self.col_capacity:
+                    self.widen_cols(cap)
             _lib.check(self._L.gnx_step(self._ctx, k), 'gnx_step')
-            n_steps -= k
-        if n_steps > 0:
-            _lib.check(self._L.gnx_step(self._ctx, n_steps), 'gnx_step')
+            if not self.grow:
+                n_steps -= k
+                continue
+            st = self.step_status()
+            n_steps -= st['steps_run']
+            if not st['stopped']:
+                continue
+            need = max(st['need_entries'], st['need_slots'])
+            if need > self.capacity:
+                self.reserve(growth_capacity(need, self.capacity))
+            else:
+                st['steps_left'] = n_steps
+                return st
         if sync:
             self.sync()
+        return None
+
+    def step_status(self):
+        """The last gnx_step batch (grow only; synchronises): steps_run, stopped, and the capacities the
+        next step needs (need_entries, need_slots, need_births, need_edges) beside the current ones."""
+        s = _lib.StepStatus()
+        _lib.check(self._L.gnx_step_status(self._ctx, C.byref(s)), 'gnx_step_status')
+        return {name: int(getattr(s, name)) for name, _ in s._fields_}
+
+    def reserve(self, capacity):
+        """Grow the population capacity to `capacity` individuals (never shrinks; between steps)."""
+        _lib.check(self._L.gnx_reserve(self._ctx, int(capacity)), 'gnx_reserve')
+        self.capacity = max(self.capacity, int(capacity))
+        self._cfg.capacity = self.capacity
+
+    def tskit_reserve(self, edge_capacity, birth_capacity):
+        """Grow the tskit row buffers, keeping the rows buffered since the last drain."""
+        _lib.check(self._L.gnx_tskit_reserve(self._ctx, int(edge_capacity), int(birth_capacity)),
+                   'gnx_tskit_reserve')
 
     def sync(self):
         _lib.check(self._L.gnx_sync(self._ctx), 'gnx_sync')

@@ -247,6 +247,32 @@ int gnx_set_life_history(gnx_ctx* ctx, const gnx_config_t* cfg);
  * density chain); the graph is re-captured when a setter changed any kernel argument.
  * GNX_NO_GRAPH=1 in the environment keeps plain stream launches. */
 int gnx_step(gnx_ctx* ctx, int32_t n_steps);
+/* ---- growth between steps ----------------------------------------------------------------
+ * gnx_set_growth_guard(ctx, 1): every step first checks, from the device counters, whether it could
+ * overflow the population capacity (entries, genome slots) or the tskit row buffers; a step that
+ * could does not start (nothing moves, no draws, Counters.t stays) and neither does any later step
+ * of the same gnx_step batch.  The caller reads gnx_step_status, grows the buffers (gnx_reserve,
+ * gnx_tskit_reserve) and steps again: Philox draws are keyed by (seed, id, site, t), so the run is
+ * bit-identical to one that had the larger buffers from the start.  Graph-launched steps check on
+ * the device (a guard kernel in front of an IF conditional node holding the step), the first step
+ * of a context and GNX_NO_GRAPH steps on the host.  Off by default; GNX_ERR_STATE on a strip. */
+typedef struct {
+  int32_t steps_run;          /* steps of the last gnx_step batch that ran */
+  int32_t stopped;            /* 1: the batch stopped in front of a step that could overflow */
+  int64_t need_entries;       /* population capacity the next step needs (n + most births) */
+  int64_t need_slots;         /* genome slots it needs (within the population capacity) */
+  int64_t need_births;        /* tskit birth rows it needs (0 without recording) */
+  int64_t need_edges;         /* tskit edge rows it needs (0 without recording) */
+  int64_t capacity, born_capacity, edge_capacity;   /* the current sizes */
+} gnx_step_status_t;
+int gnx_set_growth_guard(gnx_ctx* ctx, int32_t on);
+/* Synchronises; reconciles the host's step bookkeeping with the steps the device skipped. */
+int gnx_step_status(gnx_ctx* ctx, gnx_step_status_t* out);
+/* Grow the population capacity (never shrinks): every buffer sized from it is re-allocated and its
+ * contents copied.  On an allocation failure GNX_ERR_CUDA, and the context keeps its old buffers. */
+int gnx_reserve(gnx_ctx* ctx, int64_t capacity);
+/* Grow the tskit row buffers; the rows buffered since the last drain are kept. */
+int gnx_tskit_reserve(gnx_ctx* ctx, int64_t edge_capacity, int64_t birth_capacity);
 /* ---- strip domain decomposition of one landscape over several GPUs (SURVEY.md section 8e-2) ---
  * What shards (reference file:line): the mate search species.py:2157-2215 / spatial.py:191-245
  * (halo of the individuals within one mating-grid row of a strip edge, with their genome rows),
