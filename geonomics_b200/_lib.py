@@ -256,6 +256,8 @@ SIGNATURES = {
                                      c_int32_p, c_int32_p, c_double_p, c_int32_p]),
     'gnx_read_mutation_tables': (C.c_int, [_ctx, C.c_int32, c_int32_p, c_int32_p, c_double_p, c_int32_p, c_int32_p]),
     'gnx_create_cols': (C.c_int, [C.POINTER(Config), C.c_int32, C.c_int32, c_int32_p, C.POINTER(_ctx)]),
+    'gnx_set_clock': (C.c_int, [_ctx, C.c_int64, C.c_int64]),
+    'gnx_read_paths': (C.c_int, [_ctx, c_uint32_p, C.c_int64]),
     'gnx_read_cols': (C.c_int, [_ctx, c_int32_p, c_int32_p, c_int32_p]),
     'gnx_widen_cols': (C.c_int, [_ctx, C.c_int32]),
     'gnx_genome_init_begin': (C.c_int, [_ctx, C.POINTER(GenomeInit), C.POINTER(C.c_void_p), c_int64_p]),

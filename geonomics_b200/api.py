@@ -709,21 +709,26 @@ class Species:
                 self._dev = NcclStrips(land.dim, rasters, self._device_params(), ga, capacity, group=self._strips, **kw)
         else:
             if capacity is None:
-                capacity = int(max(4096, 3.0 * float(np.sum(self.K)), 2 * self.start_N))
+                capacity = int(max(4096, 3.0 * float(np.sum(self.K)), 2 * max(self.start_N, len(p['x']))))
             # the population may outgrow the starting capacity (a K raised by a landscape or demographic
             # change, a high lambda): the buffers grow between steps
             self._dev = DeviceSpecies(land.dim, rasters, self._device_params(), ga, capacity=capacity,
                                       seed=self._seed, res_ratio=self._land_res_ratio, grow=True)
         land._listeners.append(self)
         self._dev.set_burn(not self.burned)
-        self._dev.upload(p['x'], p['y'], p['age'], p['sex'], p['idx'], max_ind_idx=self.max_ind_idx,
-                         genomes_packed=p.get('genomes'))
+        self._upload(p)
         self._init_pop = None
         self._invalidate()
         self._burnin_spat_tester = None
+        self._burnin_base = None
         if not self.burned:                                   # species.py:469-470
             from .burnin import SpatialTester
             self._burnin_spat_tester = SpatialTester(self._dev)
+            self._burnin_base = (p['x'], p['y'])              # the device compares the next update with these counts
+
+    def _upload(self, p):
+        self._dev.upload(p['x'], p['y'], p['age'], p['sex'], p['idx'], max_ind_idx=self.max_ind_idx,
+                         genomes_packed=p.get('genomes'), z=p.get('z'), fit=p.get('fit'))
 
     def _do_spatial_burnin_test(self, num_timesteps_back):
         """species.py:572-578."""
@@ -731,6 +736,7 @@ class Species:
             from .burnin import SpatialTester
             self._burnin_spat_tester = SpatialTester(self._dev)
         self._burnin_spat_tester.update(self._dev)
+        self._burnin_base = None
         return self._burnin_spat_tester.run_test(num_timesteps_back)
 
     def _detach(self):
@@ -783,6 +789,73 @@ class Species:
                                    np.sort(np.asarray(ga.nonneut_loci, dtype=np.int64)), ga.delet_loci, ga.delet_loci_s,
                                    ga.delet_alpha_distr_shape, ga.delet_alpha_distr_scale,
                                    log_capacity=max(ga.L, 16), **self._tskit_mutation_kw())
+
+    # ---- checkpoints (Model.save / load_model) ----------------------------------------------------
+    _DEVICE_ATTRS = ('_dev', '_cache', '_inds', '_land', '_strips', '_init_pop')
+
+    def _checkpoint(self):
+        """Everything a resumed species needs, at a step boundary, without a device handle: the host attributes
+        (life-history overrides, K, changer, burn-in tester, gen_arch with its mutation bookkeeping, surface tables
+        as built, tskit tables), the population as downloaded (packed genomes, z, fitness) and the device's clock,
+        capacity, column map, path patches and tskit node ids."""
+        self._drain_tskit()
+        self._sync_mutations()
+        ck = dict(attrs={k: v for k, v in self.__dict__.items() if k not in self._DEVICE_ATTRS},
+                  state=self._dev.download(genomes=bool(self.burned and self.gen_arch is not None), unpack=False),
+                  clock=self._dev.clock(), capacity=int(self._dev.capacity))
+        if getattr(self._dev, 'cols', False):
+            ck['cols'] = (self._dev.read_cols(), self._dev.col_capacity)
+            ck['subsetters'] = self._dev.subsetters()
+        if self.burned and self.__dict__.get('_tc') is not None:
+            c = self._dev.counters()
+            ck['tskit'] = dict(nodes=self._node_ids(), next_node=c['n_nodes'], next_row=c['n_ind_rows'],
+                               capacity=self._dev.tskit_capacity)
+        return ck
+
+    @classmethod
+    def _from_checkpoint(cls, ck, land, strips):
+        """The host side of a checkpointed species on `land`, not yet on the device (_resume)."""
+        spp = cls.__new__(cls)
+        spp.__dict__.update(ck['attrs'])
+        spp._land, spp._strips = land, strips
+        spp._dev = spp._cache = spp._inds = None
+        st = ck['state']
+        spp._init_pop = {k: st[k] for k in ('x', 'y', 'age', 'sex', 'idx', 'z', 'fit', 'genomes') if k in st}
+        return spp
+
+    def _resume(self, ck, capacity=None):
+        """Re-attach from a checkpoint: upload the population, restore the burn-in counts, K, the mutation
+        bookkeeping and the tskit node ids, and set the device clock last, so that every later draw is the one
+        the saved run would have made."""
+        p = self._init_pop
+        tester, base = ck['attrs'].get('_burnin_spat_tester'), ck['attrs'].get('_burnin_base')
+        self._attach(capacity=capacity, cols=ck.get('cols'))  # life history, rasters, surface tables, burn flag
+        if base is not None and not self.burned:
+            # the tester's last counts are those of an earlier population (the one it was attached with)
+            self._dev.upload(base[0], base[1])
+            self._dev.burnin_cell_stats()
+            self._upload(p)
+        self._burnin_spat_tester, self._burnin_base = tester, base
+        if self.__dict__.get('_K_overridden'):
+            self._dev.set_K(self.K)
+        ga = self.gen_arch
+        if self.burned and ga is not None and (self.mutate or ga.use_tskit):
+            nn = np.sort(np.asarray(ga.nonneut_loci, dtype=np.int64))
+            kw = self._tskit_mutation_kw()
+            if ck.get('subsetters') is not None:
+                kw['subsetters'] = ck['subsetters']
+            if self.mutate:
+                self._dev.set_mutation(ga.mu_neut or 0, ga.mu_delet or 0, ga._mutables, nn, ga.delet_loci,
+                                       ga.delet_loci_s, ga.delet_alpha_distr_shape, ga.delet_alpha_distr_scale,
+                                       log_capacity=max(ga.L, 16), **kw)
+            else:
+                self._dev.set_mutation(0, 0, [], nn, ga.delet_loci, ga.delet_loci_s, log_capacity=16, **kw)
+        tk = ck.get('tskit')
+        if tk is not None:
+            self._dev.tskit_enable(*tk['capacity'])
+            self._dev.tskit_set_nodes(tk['nodes'][:, 0], tk['nodes'][:, 1], tk['next_node'], tk['next_row'])
+        self._dev.set_clock(*ck['clock'])
+        self._invalidate()
 
     def _on_raster_change(self, lyr_num, rast):
         if self._dev is not None:
@@ -1291,12 +1364,14 @@ def _make_species(land, name, idx, spp_params, seed=0, strips=None):
     mv = spp_params.get('movement', {})
     if spp._move and 'move_surf' in mv:
         ms = dict(mv['move_surf'])
-        lyr = [k for k, v in land.items() if v.name == ms.pop('layer')]
+        name = ms.pop('layer')
+        lyr = [k for k, v in land.items() if v.name == name]
         assert len(lyr) == 1
         spp._move_surf = _ConductanceSurface(land[lyr[0]], **ms)
     if 'disp_surf' in mv:
         ds = dict(mv['disp_surf'])
-        lyr = [k for k, v in land.items() if v.name == ds.pop('layer')]
+        name = ds.pop('layer')
+        lyr = [k for k, v in land.items() if v.name == name]
         assert len(lyr) == 1
         spp._disp_surf = _ConductanceSurface(land[lyr[0]], **ds)
     if 'change' in spp_params:                               # species.py:3373-3395
@@ -1654,6 +1729,32 @@ class Model:
             return parallel.gather_trajectories({it: v for it, v in self.iterations.items() if it in mine}, dist)
         return self.iterations
 
+    # ---- checkpoints ----------------------------------------------------------------------------
+    _DEVICE_ATTRS = ('land', 'comm', 'strips')
+
+    def save(self, path):
+        """Write the model, at the step boundary it stands at, to one file that load_model resumes from bit for
+        bit, on one GPU or on any number of strips: the model's own state (params, clocks, remaining iterations
+        and the originals they start from), numpy's and random's global streams, the landscape with its changer,
+        and every species (Species._checkpoint).  Under a process group every rank calls save; rank 0 writes
+        and the other ranks wait for it."""
+        import random
+        from . import _lib, checkpoint
+        species = {n: spp._checkpoint() for n, spp in self.comm.items()}
+        payload = dict(model={k: v for k, v in self.__dict__.items() if k not in self._DEVICE_ATTRS},
+                       land=self._bare_land(), comm=dict(t=self.comm.t, burned=self.comm.burned), species=species,
+                       strips=_strip_world(self.strips), rng=(np.random.get_state(), random.getstate()))
+        group = None if self.strips is None or isinstance(self.strips, (int, np.integer)) else self.strips
+        if group is None:
+            checkpoint.write(path, payload, _lib.lib().gnx_abi_version())
+            return
+        import torch.distributed as dist
+        try:
+            if dist.get_rank(group) == 0:
+                checkpoint.write(path, payload, _lib.lib().gnx_abi_version())
+        finally:
+            dist.barrier(group=group)
+
     # ---- getters (model.py:2787-3176) ---------------------------------------------------
     def _spp(self, spp):
         return self.comm[spp] if isinstance(spp, int) else [s for s in self.comm.values() if s.name == spp][0]
@@ -1694,6 +1795,38 @@ class Model:
         """model.py:3399-3446: idx, z, e, age, sex, x, y of everyone or of n individuals drawn at random (CSV)."""
         from . import writers
         return writers.write_geodata(filepath, self._spp(spp), n=n)
+
+
+def load_model(path, strips=None):
+    """A Model resumed from the file Model.save wrote: walking or running it on gives what the saved model
+    would have given.  strips has its meaning in make_model and need not match the decomposition the file was
+    written from.  Under a process group every rank reads the file.  A file of another checkpoint format or
+    C-ABI version is refused (checkpoint.CheckpointError)."""
+    import random
+    from . import _lib, checkpoint
+    world = _strip_world(strips)
+    ck = checkpoint.read(path, _lib.GNX_ABI_VERSION)
+    m = Model.__new__(Model)
+    m.__dict__.update(ck['model'])
+    m.strips = strips
+    m.land = ck['land']
+    m.land._listeners = []
+    spps = {n: Species._from_checkpoint(sc, m.land, strips) for n, sc in ck['species'].items()}
+    if world is not None:
+        for spp in spps.values():
+            _check_strip_species(spp, world)
+    # a capacity is per strip under a decomposition: it carries over only between single contexts
+    same = world is None and ck['strips'] is None
+    for n, spp in spps.items():
+        spp._resume(ck['species'][n], capacity=ck['species'][n]['capacity'] if same else None)
+    if not same:
+        for snap in (m.orig_comm or {}).values():
+            snap['capacity'] = None
+    m.comm = Community(m.land, spps)
+    m.comm.t, m.comm.burned = ck['comm']['t'], ck['comm']['burned']
+    np.random.set_state(ck['rng'][0])
+    random.setstate(ck['rng'][1])
+    return m
 
 
 def make_model(parameters=None, verbose=False, name=None, genome_init='host', strips=None):

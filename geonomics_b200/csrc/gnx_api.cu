@@ -2250,6 +2250,34 @@ extern "C" int gnx_set_growth_guard(gnx_ctx* ctx, int32_t on) {
   return GNX_OK;
 }
 
+extern "C" int gnx_set_clock(gnx_ctx* ctx, int64_t t, int64_t tsk_t0) {
+  ARG(ctx && t >= 0, "t must be >= 0");
+  USE_DEVICE(ctx);
+  Counters h;
+  int r = read_counters(ctx, &h);
+  if (r != GNX_OK) return r;
+  if (ctx->grow_guard) ctx->pending = h.pending != 0;     // the guard may have skipped the step that left deaths
+  if (ctx->pending || ctx->gi_stage != 0) {
+    g_last_error = "gnx_set_clock: a step or a genome assignment is pending (download or upload the population first)";
+    return GNX_ERR_STATE;
+  }
+  PROF(ctx, "k_set_clock");
+  k_set_clock<<<1, 1, 0, ctx->stream>>>(ctx->d_c, t, tsk_t0);
+  LAUNCHED(ctx);
+  CK(cudaStreamSynchronize(ctx->stream));
+  return check_device_err(h);
+}
+
+extern "C" int gnx_read_paths(gnx_ctx* ctx, uint32_t* host_paths, int64_t n_words) {
+  ARG(ctx && host_paths, "null");
+  if (!ctx->have_paths) { g_last_error = "recombination paths not set"; return GNX_ERR_STATE; }
+  ARG(n_words == (int64_t)ctx->cfg.n_recomb_paths * 4 * ctx->Wq, "n_words must be n_recomb_paths * 4 * Wq");
+  USE_DEVICE(ctx);
+  CK(cudaMemcpyAsync(host_paths, ctx->d_paths, (size_t)n_words * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return GNX_OK;
+}
+
 extern "C" int gnx_step_status(gnx_ctx* ctx, gnx_step_status_t* out) {
   ARG(ctx && out, "null");
   if (!ctx->grow_guard) { g_last_error = "the growth guard is off"; return GNX_ERR_STATE; }

@@ -1540,6 +1540,12 @@ __host__ __device__ inline int growth_check(const GrowthBound& g, int64_t n, int
          need->need_edges <= g.edge_cap;
 }
 
+// gnx_set_clock: the step counter and the tskit time origin of a run resumed from a checkpoint
+__global__ void k_set_clock(Counters* c, int64_t t, int64_t tsk_t0) {
+  c->t = t;
+  c->tsk_t0 = tsk_t0;
+}
+
 // first node of a guarded step graph: runs the step body (IF conditional) only when it cannot overflow
 __global__ void k_step_guard(const Counters* c, GrowthBound g, gnx_step_status_t* st, cudaGraphConditionalHandle h) {
   gnx_step_status_t need;

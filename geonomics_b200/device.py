@@ -198,6 +198,7 @@ class DeviceSpecies:
             _lib.check(L.gnx_set_surface_tables(self._ctx, _ptr(mv, _lib.c_uint16_p), _ptr(dv, _lib.c_uint16_p)),
                        'gnx_set_surface_tables')
         self._keep = []
+        self.tskit_capacity = (0, 0)               # (edge, birth) rows of the tskit buffers, once enabled
         self.grow = bool(grow)
         if self.grow:
             _lib.check(L.gnx_set_growth_guard(self._ctx, 1), 'gnx_set_growth_guard')
@@ -513,9 +514,9 @@ class DeviceSpecies:
         return p
 
     def upload(self, x, y, age=None, sex=None, idx=None, g=None, z=None, max_ind_idx=None,
-               genomes_packed=None):
+               genomes_packed=None, fit=None):
         """Upload a population in species order.  g: int8[N, L, 2] (reference layout) or
-        genomes_packed: u32[N, 2, W]."""
+        genomes_packed: u32[N, 2, W]; z and fit as downloaded (z otherwise follows from the genomes)."""
         n = len(x)
         bufs = dict(n=n, x=np.ascontiguousarray(x, dtype=np.float64), y=np.ascontiguousarray(y, dtype=np.float64))
         if age is not None:
@@ -532,6 +533,8 @@ class DeviceSpecies:
             bufs['genomes'] = gpk
         if z is not None and self.n_traits:
             bufs['z'] = np.ascontiguousarray(z, dtype=np.float64).reshape(n, self.n_traits)
+        if fit is not None:
+            bufs['fit'] = np.ascontiguousarray(fit, dtype=np.float64)
         if max_ind_idx is None:
             max_ind_idx = int(np.max(idx)) if idx is not None and n else n - 1
         bufs['max_ind_idx'] = max_ind_idx
@@ -690,6 +693,34 @@ class DeviceSpecies:
         """Grow the tskit row buffers, keeping the rows buffered since the last drain."""
         _lib.check(self._L.gnx_tskit_reserve(self._ctx, int(edge_capacity), int(birth_capacity)),
                    'gnx_tskit_reserve')
+        self.tskit_capacity = (max(self.tskit_capacity[0], int(edge_capacity)),
+                               max(self.tskit_capacity[1], int(birth_capacity)))
+
+    # ---- checkpoints ---------------------------------------------------------------------------
+    def clock(self):
+        """(t, tsk_t0): the step counter that keys every draw and the tskit time origin (synchronises)."""
+        c = self.counters()
+        return c['t'], c['tsk_t0']
+
+    def set_clock(self, t, tsk_t0=0):
+        """Continue the draws of a saved run (gnx_set_clock): after the upload, set_mutation and the tskit
+        calls, between steps."""
+        _lib.check(self._L.gnx_set_clock(self._ctx, int(t), int(tsk_t0)), 'gnx_set_clock')
+
+    def read_paths(self):
+        """uint32[n_paths, 4 * Wq]: the recombination paths the gamete kernel reads, at the genotype bits
+        (gnx_read_paths); under the tskit layout they carry the patches of the columns mutations added."""
+        out = np.zeros((self._cfg.n_recomb_paths, self.W), np.uint32)
+        _lib.check(self._L.gnx_read_paths(self._ctx, _ptr(out, _lib.c_uint32_p), out.size), 'gnx_read_paths')
+        return out
+
+    def subsetters(self):
+        """uint8[n_paths, n_cols]: the homologue every path reads at each non-neutral locus in ascending locus
+        order -- the `subsetters` argument of set_mutation that rebuilds the paths read_paths returns."""
+        col_locus = self.read_cols()
+        bits = np.argsort(col_locus, kind='stable')                 # the column of each ascending locus
+        rows = self.read_paths()
+        return ((rows[:, bits >> 5] >> (bits & 31).astype(np.uint32)) & 1).astype(np.uint8)
 
     def sync(self):
         _lib.check(self._L.gnx_sync(self._ctx), 'gnx_sync')
@@ -708,6 +739,7 @@ class DeviceSpecies:
     # ---- tskit record buffering (species.py:692-736) ---------------------------------------
     def tskit_enable(self, edge_capacity, birth_capacity):
         _lib.check(self._L.gnx_tskit_enable(self._ctx, int(edge_capacity), int(birth_capacity)), 'gnx_tskit_enable')
+        self.tskit_capacity = (int(edge_capacity), int(birth_capacity))
 
     def tskit_set_nodes(self, node0, node1, next_node_id, next_individual_row):
         a = np.ascontiguousarray(node0, dtype=np.int32)
@@ -808,6 +840,8 @@ class DeviceSpecies:
         out['err'] = int(c[12])
         out['n_rec'] = int(c[13])
         out['gs_iters'] = (int(c[14]), int(c[15]))
+        out['n_nodes'], out['n_ind_rows'] = int(c[20]), int(c[21])      # next tskit node id / individuals row
+        out['tsk_t0'] = int(c[24:26].view(np.int64)[0])
         # lengths of the fix list (exact-order cells) and the deferred list (d waits for max(N)) of the last
         # density evaluation
         out['density_lists'] = (int(c[46]), int(c[47]))

@@ -281,6 +281,14 @@ class _Strips:
         for r in self.ranks:
             r.dev.set_mutation(*args, **kw)
 
+    def set_clock(self, t, tsk_t0=0):
+        """DeviceSpecies.set_clock on every strip: the ranks step in lockstep and share one clock."""
+        for r in self.ranks:
+            r.dev.set_clock(t, tsk_t0)
+
+    def clock(self):
+        return self.ranks[0].dev.clock()
+
     def read_mutations(self, max_rows=4096):
         """Drain the mutation logs; each rank's must equal the undecomposed run's, so the ranks of this
         process must agree.  Returns (rows, state) as DeviceSpecies.read_mutations does."""
@@ -316,12 +324,13 @@ class _Strips:
             r.dev.genome_init_end()
 
     # ---- population in / out
-    def upload(self, x, y, age=None, sex=None, idx=None, g=None, max_ind_idx=None, genomes_packed=None):
+    def upload(self, x, y, age=None, sex=None, idx=None, g=None, max_ind_idx=None, genomes_packed=None, z=None,
+               fit=None):
         """Upload each rank's share of a population every process holds on the host."""
         idx = np.arange(len(x), dtype=np.int64) if idx is None else np.asarray(idx)
         if max_ind_idx is None and len(idx):
             max_ind_idx = int(idx.max())
-        cols = dict(x=x, y=y, age=age, sex=sex, idx=idx, g=g, genomes_packed=genomes_packed)
+        cols = dict(x=x, y=y, age=age, sex=sex, idx=idx, g=g, genomes_packed=genomes_packed, z=z, fit=fit)
         own = owner_of(y, self.bounds, self.cs, self.ncy)
         for r in self.ranks:
             m = own == r.rank

@@ -273,6 +273,21 @@ int gnx_step_status(gnx_ctx* ctx, gnx_step_status_t* out);
 int gnx_reserve(gnx_ctx* ctx, int64_t capacity);
 /* Grow the tskit row buffers; the rows buffered since the last drain are kept. */
 int gnx_tskit_reserve(gnx_ctx* ctx, int64_t edge_capacity, int64_t birth_capacity);
+/* ---- resuming a checkpoint ----------------------------------------------------------------------
+ * gnx_set_clock writes the time-step counter Counters.t (the Philox counter word of every draw) and the
+ * tskit time origin Counters.tsk_t0 (node time = -(t - tsk_t0)) on the context's stream, so that a population
+ * uploaded from a checkpoint continues the draws of the run it was saved from.  Call it last, after the
+ * upload, gnx_set_mutation and the tskit calls (gnx_tskit_enable sets tsk_t0 to the current t).  The step
+ * kernels read both values from Counters, never as graph arguments, so a captured step graph stays valid.
+ * GNX_ERR_STATE while a step is pending (its deaths are only flagged: download or upload first) or a device
+ * genome assignment is under way; on a strip every rank is given the same values. */
+int gnx_set_clock(gnx_ctx* ctx, int64_t t, int64_t tsk_t0);
+/* The cached recombination paths as the gamete kernel reads them: n_words = n_recomb_paths * 4 * (128-bit
+ * units of a genotype row) words, bit j of path p = the homologue path p reads at genotype bit j.  Under the
+ * tskit layout these are the reference's subsetters: k_mutate patches the bit of a column a mutation adds with
+ * the path in front of its locus (genome.py:133-160), which the paths as simulated do not give back, so a
+ * checkpoint carries them into gnx_set_mutation's host_subsetters.  Synchronises. */
+int gnx_read_paths(gnx_ctx* ctx, uint32_t* host_paths, int64_t n_words);
 /* ---- strip domain decomposition of one landscape over several GPUs (SURVEY.md section 8e-2) ---
  * What shards (reference file:line): the mate search species.py:2157-2215 / spatial.py:191-245
  * (halo of the individuals within one mating-grid row of a strip edge, with their genome rows),
