@@ -177,6 +177,22 @@ class StepStatus(C.Structure):
                 ('edge_capacity', C.c_int64)]
 
 
+class Tables(C.Structure):
+    _fields_ = [
+        ('sequence_length', C.c_double),
+        ('n_nodes', C.c_int64),
+        ('node_flags', c_int32_p), ('node_time', c_double_p), ('node_population', c_int32_p),
+        ('node_individual', c_int32_p),
+        ('n_edges', C.c_int64),
+        ('edge_left', c_double_p), ('edge_right', c_double_p), ('edge_parent', c_int32_p), ('edge_child', c_int32_p),
+        ('n_individuals', C.c_int64), ('n_location', C.c_int32),
+        ('individual_flags', c_int32_p), ('individual_location', c_double_p), ('individual_idx', c_int64_p),
+        ('n_sites', C.c_int64), ('site_position', c_double_p),
+        ('n_mutations', C.c_int64),
+        ('mutation_site', c_int32_p), ('mutation_node', c_int32_p), ('mutation_time', c_double_p),
+    ]
+
+
 class GenomeInit(C.Structure):
     _fields_ = [
         ('seed', C.c_uint64),
@@ -258,6 +274,8 @@ SIGNATURES = {
     'gnx_create_cols': (C.c_int, [C.POINTER(Config), C.c_int32, C.c_int32, c_int32_p, C.POINTER(_ctx)]),
     'gnx_set_clock': (C.c_int, [_ctx, C.c_int64, C.c_int64]),
     'gnx_read_paths': (C.c_int, [_ctx, c_uint32_p, C.c_int64]),
+    'gnx_simplify': (C.c_int, [_ctx, C.POINTER(Tables), c_int32_p, C.c_int64, c_int64_p]),
+    'gnx_simplify_result': (C.c_int, [_ctx, C.POINTER(Tables)]),
     'gnx_read_cols': (C.c_int, [_ctx, c_int32_p, c_int32_p, c_int32_p]),
     'gnx_widen_cols': (C.c_int, [_ctx, C.c_int32]),
     'gnx_genome_init_begin': (C.c_int, [_ctx, C.POINTER(GenomeInit), C.POINTER(C.c_void_p), c_int64_p]),

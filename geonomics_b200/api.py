@@ -1234,7 +1234,7 @@ class Species:
         the individuals rows in species order (gnx_tskit_renumber).  sort()/simplify() are tskit's own."""
         self._drain_tskit()
         n = len(self)
-        self._tc.sort_and_simplify(self._node_ids().reshape(-1))
+        self._tc.sort_and_simplify(self._node_ids().reshape(-1), self._dev)
         # the samples are nodes 0 .. 2N - 1 in the order given (species.py:1148-1152); nodes where their ancestry
         # coalesces follow, with the individuals they belong to, so the NEXT rows continue from the table sizes
         self._dev.tskit_set_nodes(2 * np.arange(n, dtype=np.int32), 2 * np.arange(n, dtype=np.int32) + 1,

@@ -5,7 +5,7 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 SOURCES = ['gnx_api.cu']
-DEPS = ['gnx_api.cu', 'gnx_kernels.cuh', 'gnx_scan.cuh', 'gnx_common.cuh', 'gnx_strip.cuh', 'gnx_genome_init.cuh', '../../include/gnx_b200.h']
+DEPS = ['gnx_api.cu', 'gnx_kernels.cuh', 'gnx_scan.cuh', 'gnx_common.cuh', 'gnx_strip.cuh', 'gnx_genome_init.cuh', 'gnx_simplify.cuh', '../../include/gnx_b200.h']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
               '-Xcompiler', '-fPIC', '-shared']
 

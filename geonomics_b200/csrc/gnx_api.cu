@@ -10,6 +10,7 @@
 #include <algorithm>
 #include "gnx_kernels.cuh"
 #include "gnx_genome_init.cuh"
+#include "gnx_simplify.cuh"
 
 static thread_local std::string g_last_error;
 
@@ -139,6 +140,9 @@ struct gnx_ctx {
   int32_t* d_gi_active = nullptr;       // [2]: loci still active, loci with more carriers than keys
   int64_t gi_t = 0;                     // Counters.t when the genomes were written (the rows describe that population)
   std::vector<void*> gi_allocs;
+  // the last gnx_simplify result (device columns and their sizes) until gnx_simplify_result copies it out
+  gnx_tables_t simp{};
+  std::vector<void*> simp_allocs;
 };
 
 template <class T>
@@ -527,6 +531,7 @@ extern "C" int gnx_destroy(gnx_ctx* ctx) {
   free_bucket(ctx->mut_allocs);
   free_bucket(ctx->strip_allocs);
   free_bucket(ctx->gi_allocs);
+  free_bucket(ctx->simp_allocs);
   for (void* m : ctx->strip_ipc_opened) cudaIpcCloseMemHandle(m);
   ctx->strip_ipc_opened.clear();
   if (ctx->strip_block) cudaFree(ctx->strip_block);
@@ -1111,14 +1116,14 @@ static int build_order(gnx_ctx* ctx, const Counters& h, bool exclude_dead) {
   int in = 0;
   for (int shift = 0; shift < bits; shift += 8) {
     PROF(ctx, "k_radix_hist");
-    k_radix_hist<<<std::min(ntiles, grid_for(ctx, 8)), RS_BLOCK, 0, s>>>(W.sort_keys[in], n, shift, W.sort_hist, ntiles);
+    k_radix_hist<<<std::min(ntiles, grid_for(ctx, 8)), RS_BLOCK, 0, s>>>(W.sort_keys[in], n, nullptr, shift, W.sort_hist);
     LAUNCHED(ctx);
-    RadixScan rs{W.sort_hist, 256 * ntiles};
+    RadixScan rs{W.sort_hist, n, nullptr};
     int r = run_scan(ctx, rs, "scan_radix");
     if (r != GNX_OK) return r;
     PROF(ctx, "k_radix_scatter");
     k_radix_scatter<<<std::min(ntiles, grid_for(ctx, 8)), RS_BLOCK, 0, s>>>(W.sort_keys[in], W.sort_vals[in], W.sort_keys[in ^ 1],
-                                                                      W.sort_vals[in ^ 1], n, shift, W.sort_hist, ntiles);
+                                                                      W.sort_vals[in ^ 1], n, nullptr, shift, W.sort_hist);
     LAUNCHED(ctx);
     in ^= 1;
   }
@@ -1246,20 +1251,25 @@ extern "C" int gnx_download_population(gnx_ctx* ctx, gnx_population_t* pop) {
 
 // ---- stages -----------------------------------------------------------------------------
 
+// tile_sums / ticket: the ctx's own (sized from the capacity) unless a caller scanning something
+// larger brings its own
 template <class F>
-static int run_scan(gnx_ctx* ctx, F f, const char* name) {
+static int run_scan(gnx_ctx* ctx, F f, const char* name, u64* tile_sums, unsigned int* ticket) {
   cudaStream_t s = ctx->stream;
   char nm[64];
   snprintf(nm, sizeof nm, "%s.reduce", name);
   PROF(ctx, nm);
-  scan_reduce_kernel<F><<<grid_for(ctx, SCAN_GRID), SCAN_BLOCK, 0, s>>>(f, ctx->d_c, ctx->work.tile_sums,
-                                                                       ctx->work.scan_ticket);
+  scan_reduce_kernel<F><<<grid_for(ctx, SCAN_GRID), SCAN_BLOCK, 0, s>>>(f, ctx->d_c, tile_sums, ticket);
   LAUNCHED(ctx);
   snprintf(nm, sizeof nm, "%s.apply", name);
   PROF(ctx, nm);
-  scan_apply_kernel<F><<<grid_for(ctx, SCAN_GRID), SCAN_BLOCK, 0, s>>>(f, ctx->d_c, ctx->work.tile_sums);
+  scan_apply_kernel<F><<<grid_for(ctx, SCAN_GRID), SCAN_BLOCK, 0, s>>>(f, ctx->d_c, tile_sums);
   LAUNCHED(ctx);
   return GNX_OK;
+}
+template <class F>
+static int run_scan(gnx_ctx* ctx, F f, const char* name) {
+  return run_scan(ctx, f, name, ctx->work.tile_sums, ctx->work.scan_ticket);
 }
 
 // injected draws are indexed by species-order ordinal: make pop.ord / work.inv current.
@@ -2275,6 +2285,423 @@ extern "C" int gnx_read_paths(gnx_ctx* ctx, uint32_t* host_paths, int64_t n_word
   USE_DEVICE(ctx);
   CK(cudaMemcpyAsync(host_paths, ctx->d_paths, (size_t)n_words * 4, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
+  return GNX_OK;
+}
+
+// ---- sort + simplify of the tskit tables (gnx_simplify.cuh) ------------------------------------------
+#define TRY(call)                        \
+  do {                                   \
+    int r_ = (call);                     \
+    if (r_ != GNX_OK) return r_;         \
+  } while (0)
+
+static int bits_for(long long x) {          // bits of the largest value x (at least 1)
+  int b = 1;
+  while (b < 62 && (x >> b) != 0) ++b;
+  return b;
+}
+
+template <class T>
+static int simp_upload(gnx_ctx* ctx, std::vector<void*>& bucket, const T* host, int64_t n, T** dev) {
+  DM(ctx, dev, (size_t)n, &bucket);
+  if (n > 0) CK(cudaMemcpyAsync(*dev, host, (size_t)n * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
+  return GNX_OK;
+}
+
+// scratch of one radix sort / scan family: ping-pong pairs, histogram and scan tile sums for n_cap items
+struct SimpSort {
+  unsigned long long* key[2];
+  int32_t* val[2];
+  uint32_t* hist;
+  u64* tile_sums;
+  unsigned int* ticket;
+  int n_cap;
+};
+
+static int simp_sort_alloc(gnx_ctx* ctx, std::vector<void*>& bucket, int64_t n_cap, int64_t scan_cap, SimpSort* z) {
+  n_cap = std::max<int64_t>(n_cap, 1);
+  const int64_t ntiles = (n_cap + RS_TILE - 1) / RS_TILE;
+  scan_cap = std::max<int64_t>(std::max<int64_t>(scan_cap, n_cap), 256 * ntiles);
+  for (int k = 0; k < 2; ++k) {
+    DM(ctx, &z->key[k], (size_t)n_cap, &bucket);
+    DM(ctx, &z->val[k], (size_t)n_cap, &bucket);
+  }
+  DM(ctx, &z->hist, (size_t)256 * ntiles, &bucket);
+  DM(ctx, &z->tile_sums, (size_t)(scan_cap / SCAN_TILE + 2), &bucket);
+  DM(ctx, &z->ticket, 1, &bucket);
+  z->n_cap = (int)n_cap;
+  return GNX_OK;
+}
+
+// LSD radix sort of z->key[0] / z->val[0] on the low `bits` key bits; n items, or *n_dev when given.
+// *in = the buffer holding the result.
+static int simp_sort(gnx_ctx* ctx, SimpSort& z, int n, const int* n_dev, int bits, int* in) {
+  const int grid = std::max(1, std::min((z.n_cap + RS_TILE - 1) / RS_TILE, grid_for(ctx, 8)));
+  *in = 0;
+  for (int shift = 0; shift < bits; shift += 8) {
+    PROF(ctx, "k_radix_hist");
+    k_radix_hist<<<grid, RS_BLOCK, 0, ctx->stream>>>(z.key[*in], n, n_dev, shift, z.hist);
+    LAUNCHED(ctx);
+    TRY(run_scan(ctx, RadixScan{z.hist, n, n_dev}, "scan_radix", z.tile_sums, z.ticket));
+    PROF(ctx, "k_radix_scatter");
+    k_radix_scatter<<<grid, RS_BLOCK, 0, ctx->stream>>>(z.key[*in], z.val[*in], z.key[*in ^ 1], z.val[*in ^ 1], n,
+                                                        n_dev, shift, z.hist);
+    LAUNCHED(ctx);
+    *in ^= 1;
+  }
+  return GNX_OK;
+}
+
+template <class F>
+static int simp_scan(gnx_ctx* ctx, const SimpSort& z, F f, const char* name) {
+  return run_scan(ctx, f, name, z.tile_sums, z.ticket);
+}
+
+static int read_ints(gnx_ctx* ctx, const int32_t* dev, int32_t* host, size_t n) {
+  CK(cudaMemcpyAsync(host, dev, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return GNX_OK;
+}
+
+static int simplify_impl(gnx_ctx* ctx, const gnx_tables_t* T, const int32_t* samples, int64_t n_samples,
+                         std::vector<void*>& B, std::vector<void*>& A, int64_t* out_sizes) {
+  const int64_t lim = 1ll << 29;
+  ARG(T->n_nodes >= 0 && T->n_nodes < lim && T->n_edges >= 0 && T->n_edges < lim && T->n_individuals >= 0 &&
+      T->n_individuals < lim && T->n_sites >= 0 && T->n_sites < lim && T->n_mutations >= 0 && T->n_mutations < lim,
+      "table sizes");
+  ARG(n_samples >= 0 && n_samples <= T->n_nodes && (n_samples == 0 || samples), "samples");
+  ARG(T->n_location >= 0 && T->sequence_length >= 0, "n_location / sequence_length");
+  ARG((T->n_nodes == 0 || (T->node_time && T->node_population && T->node_individual)) &&
+      (T->n_edges == 0 || (T->edge_left && T->edge_right && T->edge_parent && T->edge_child)) &&
+      (T->n_individuals == 0 || (T->individual_flags && T->individual_idx &&
+                                 (T->n_location == 0 || T->individual_location))) &&
+      (T->n_sites == 0 || T->site_position) &&
+      (T->n_mutations == 0 || (T->mutation_site && T->mutation_node && T->mutation_time)), "null column");
+  cudaStream_t st = ctx->stream;
+  const int n_in = (int)T->n_nodes, E = (int)T->n_edges, ns = (int)n_samples;
+  const int GD = grid_for(ctx, 4);
+  auto gr = [&](int64_t n) { return (int)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, grid_for(ctx, 8))); };
+
+  Simp S{};
+  S.n_in = n_in;
+  S.n_edges = E;
+  S.n_ind = (int)T->n_individuals;
+  S.n_sites = (int)T->n_sites;
+  S.n_mut = (int)T->n_mutations;
+  S.n_samples = ns;
+  S.L = T->sequence_length;
+  int32_t *d_pop, *d_iflags;
+  double *d_mtime, *d_iloc;
+  int64_t* d_iidx;
+  TRY(simp_upload(ctx, B, T->node_time, n_in, (double**)&S.time));
+  TRY(simp_upload(ctx, B, T->node_population, n_in, &d_pop));
+  TRY(simp_upload(ctx, B, T->node_individual, n_in, (int32_t**)&S.ind));
+  TRY(simp_upload(ctx, B, T->edge_left, E, (double**)&S.el));
+  TRY(simp_upload(ctx, B, T->edge_right, E, (double**)&S.er));
+  TRY(simp_upload(ctx, B, T->edge_parent, E, (int32_t**)&S.ep));
+  TRY(simp_upload(ctx, B, T->edge_child, E, (int32_t**)&S.ec));
+  TRY(simp_upload(ctx, B, T->site_position, T->n_sites, (double**)&S.site_pos));
+  TRY(simp_upload(ctx, B, T->mutation_site, T->n_mutations, (int32_t**)&S.m_site));
+  TRY(simp_upload(ctx, B, T->mutation_node, T->n_mutations, (int32_t**)&S.m_node));
+  TRY(simp_upload(ctx, B, T->mutation_time, T->n_mutations, &d_mtime));
+  TRY(simp_upload(ctx, B, T->individual_flags, T->n_individuals, &d_iflags));
+  TRY(simp_upload(ctx, B, T->individual_location, T->n_individuals * T->n_location, &d_iloc));
+  TRY(simp_upload(ctx, B, T->individual_idx, T->n_individuals, &d_iidx));
+  TRY(simp_upload(ctx, B, samples, ns, (int32_t**)&S.samples));
+  DM(ctx, &S.smap, (size_t)n_in, &B);
+  CK(cudaMemsetAsync(S.smap, 0xff, (size_t)n_in * 4, st));
+  int32_t* hsz;                        // sizes the host reads back
+  DM(ctx, &S.err, 1, &B);
+  DM(ctx, &hsz, 4, &B);
+
+  // ---- refuse what the algorithm cannot take
+  PROF(ctx, "k_simp_check_edges");
+  k_simp_check_edges<<<gr(E), 256, 0, st>>>(S);
+  LAUNCHED(ctx);
+  PROF(ctx, "k_simp_check_rest");
+  k_simp_check_rest<<<gr(std::max<int64_t>({(int64_t)n_in, T->n_mutations, n_samples})), 256, 0, st>>>(S);
+  LAUNCHED(ctx);
+  int32_t err = 0;
+  TRY(read_ints(ctx, S.err, &err, 1));
+  ARG(!(err & SE_ID), "an edge names a node that does not exist");
+  ARG(!(err & SE_TIME), "an edge whose parent is not older than its child");
+  ARG(!(err & SE_INTERVAL), "an edge outside 0 <= left < right <= sequence_length");
+  ARG(!(err & SE_IND), "a node names an individual that does not exist");
+  ARG(!(err & SE_SITE), "a mutation names a site that does not exist");
+  ARG(!(err & SE_SAMPLE), "a sample is out of range or repeated");
+
+  // ---- distinct positions; edges sorted as TableCollection.sort(); levels and groups
+  const int n_pos = 2 * E + 2;
+  SimpSort z;
+  TRY(simp_sort_alloc(ctx, B, std::max(n_pos, n_in), std::max<int64_t>(T->n_individuals, T->n_mutations), &z));
+  int in = 0;
+  PROF(ctx, "k_simp_pos_keys");
+  k_simp_pos_keys<<<gr(E), 256, 0, st>>>(S, z.key[0]);
+  LAUNCHED(ctx);
+  TRY(simp_sort(ctx, z, n_pos, nullptr, 64, &in));
+  DM(ctx, &S.uniq, (size_t)n_pos, &B);
+  TRY(simp_scan(ctx, z, UniqScan{z.key[in], S.uniq, hsz, n_pos}, "scan_simp_uniq"));
+  int32_t n_uniq = 0;
+  TRY(read_ints(ctx, hsz, &n_uniq, 1));
+  S.pb = bits_for(n_uniq - 1);
+  const int nb_node = bits_for(std::max(n_in - 1, 0));
+
+  int32_t* prank;
+  DM(ctx, &prank, (size_t)n_in, &B);
+  PROF(ctx, "k_simp_time_keys");
+  k_simp_time_keys<<<gr(n_in), 256, 0, st>>>(S.time, nullptr, n_in, z.key[0], z.val[0]);
+  LAUNCHED(ctx);
+  TRY(simp_sort(ctx, z, n_in, nullptr, 64, &in));
+  PROF(ctx, "k_simp_rank");
+  k_simp_rank<<<gr(n_in), 256, 0, st>>>(z.val[in], n_in, prank);
+  LAUNCHED(ctx);
+  uint32_t *lr, *rr;
+  DM(ctx, &lr, (size_t)E, &B);
+  DM(ctx, &rr, (size_t)E, &B);
+  PROF(ctx, "k_simp_edge_keys");
+  k_simp_edge_keys<<<gr(E), 256, 0, st>>>(S, n_uniq, lr, rr, z.key[0], z.val[0]);
+  LAUNCHED(ctx);
+  TRY(simp_sort(ctx, z, E, nullptr, nb_node + S.pb, &in));
+  if (in) {                                          // the second pass starts from buffer 0
+    CK(cudaMemcpyAsync(z.val[0], z.val[1], (size_t)E * 4, cudaMemcpyDeviceToDevice, st));
+  }
+  PROF(ctx, "k_simp_edge_keys2");
+  k_simp_edge_keys2<<<gr(E), 256, 0, st>>>(S, prank, z.val[0], z.key[0]);
+  LAUNCHED(ctx);
+  TRY(simp_sort(ctx, z, E, nullptr, nb_node, &in));
+  DM(ctx, &S.sl, (size_t)E, &B);
+  DM(ctx, &S.sr, (size_t)E, &B);
+  DM(ctx, &S.sp, (size_t)E, &B);
+  DM(ctx, &S.sc, (size_t)E, &B);
+  DM(ctx, &S.grp_of, (size_t)E, &B);
+  DM(ctx, &S.grp_parent, (size_t)E, &B);
+  DM(ctx, &S.lvl_start, (size_t)E + 1, &B);
+  DM(ctx, &S.lvl_g0, (size_t)E + 1, &B);
+  PROF(ctx, "k_simp_edge_gather");
+  k_simp_edge_gather<<<gr(E), 256, 0, st>>>(S, z.val[in], lr, rr);
+  LAUNCHED(ctx);
+  TRY(simp_scan(ctx, z, LevelScan{S, hsz}, "scan_simp_levels"));
+  int32_t lg[2] = {0, 0};
+  TRY(read_ints(ctx, hsz, lg, 2));
+  const int n_levels = lg[0];
+  std::vector<int32_t> lvl_start(n_levels + 1), lvl_g0(n_levels + 1);
+  TRY(read_ints(ctx, S.lvl_start, lvl_start.data(), n_levels + 1));
+  TRY(read_ints(ctx, S.lvl_g0, lvl_g0.data(), n_levels + 1));
+  int max_ne = 1, max_ng = 1;
+  for (int k = 0; k < n_levels; ++k) {
+    max_ne = std::max(max_ne, lvl_start[k + 1] - lvl_start[k]);
+    max_ng = std::max(max_ng, lvl_g0[k + 1] - lvl_g0[k]);
+  }
+
+  // ---- the levels, youngest first; pools that overflow are grown and the levels run again
+  int64_t cap_p = std::max<int64_t>(4096, 2 * (int64_t)max_ne);
+  int64_t cap_a = (int64_t)ns + 2 * (int64_t)E + 4096, cap_r = 2 * (int64_t)E + 4096;
+  int32_t sv[SV_N];
+  SimpSort ze{};
+  for (;;) {
+    ARG(cap_p < lim && cap_a < 2 * lim && cap_r < 2 * lim, "the simplification needs more than 2^29 pieces");
+    S.cap_p = (int)cap_p;
+    S.cap_a = (int)cap_a;
+    S.cap_r = (int)cap_r;
+    const size_t P2 = 2 * (size_t)cap_p;
+    DM(ctx, &S.sv, SV_N, &A);
+    DM(ctx, &S.a_off, (size_t)n_in, &A);
+    DM(ctx, &S.a_end, (size_t)n_in, &A);
+    DM(ctx, &S.a_lo, (size_t)cap_a, &A);
+    DM(ctx, &S.a_hi, (size_t)cap_a, &A);
+    DM(ctx, &S.a_node, (size_t)cap_a, &A);
+    DM(ctx, &S.pcnt, (size_t)max_ne, &A);
+    DM(ctx, &S.pj, (size_t)max_ne, &A);
+    DM(ctx, &S.pc_node, (size_t)cap_p, &A);
+    DM(ctx, &S.rcnt, (size_t)cap_p, &A);
+    DM(ctx, &S.inv, P2, &A);
+    DM(ctx, &S.cover, 2 * P2, &A);
+    DM(ctx, &S.bex, P2, &A);
+    DM(ctx, &S.b_pos, P2, &A);
+    DM(ctx, &S.b_end, P2, &A);
+    DM(ctx, &S.b_cls, P2, &A);
+    DM(ctx, &S.b_node, P2, &A);
+    DM(ctx, &S.b_g, P2, &A);
+    DM(ctx, &S.flag, (size_t)max_ng, &A);
+    DM(ctx, &S.vout, (size_t)max_ng, &A);
+    DM(ctx, &S.out_src, (size_t)ns + n_in, &A);
+    DM(ctx, &S.r_lo, (size_t)cap_r, &A);
+    DM(ctx, &S.r_hi, (size_t)cap_r, &A);
+    DM(ctx, &S.r_par, (size_t)cap_r, &A);
+    DM(ctx, &S.r_child, (size_t)cap_r, &A);
+    TRY(simp_sort_alloc(ctx, A, (int64_t)P2, max_ne, &ze));
+    for (int k = 0; k < 2; ++k) {
+      S.ev_key[k] = ze.key[k];
+      S.ev_val[k] = ze.val[k];
+    }
+    // rank of L among the positions: the last one
+    PROF(ctx, "k_simp_init_samples");
+    k_simp_init_samples<<<gr(ns), 256, 0, st>>>(S, (uint32_t)(n_uniq - 1));
+    LAUNCHED(ctx);
+    for (int k = 0; k < n_levels; ++k) {
+      const int e0 = lvl_start[k], ne = lvl_start[k + 1] - e0, g0 = lvl_g0[k], ng = lvl_g0[k + 1] - g0;
+      PROF(ctx, "k_simp_count");
+      k_simp_count<<<gr(ne), 256, 0, st>>>(S, e0, ne);
+      LAUNCHED(ctx);
+      TRY(simp_scan(ctx, ze, PieceScan{S, ne}, "scan_simp_pieces"));
+      PROF(ctx, "k_simp_pieces");
+      k_simp_pieces<<<GD, 256, 0, st>>>(S, e0, ne, g0);
+      LAUNCHED(ctx);
+      int ein = 0;
+      TRY(simp_sort(ctx, ze, 0, S.sv + SV_NEV, bits_for(std::max(ng - 1, 0)) + S.pb, &ein));
+      PROF(ctx, "k_simp_event_inv");
+      k_simp_event_inv<<<GD, 256, 0, st>>>(S, ze.val[ein]);
+      LAUNCHED(ctx);
+      TRY(simp_scan(ctx, ze, CoverScan{S, ze.val[ein]}, "scan_simp_cover"));
+      TRY(simp_scan(ctx, ze, BoundScan{S, ze.key[ein]}, "scan_simp_bounds"));
+      CK(cudaMemsetAsync(S.flag, 0, (size_t)ng * 4, st));
+      PROF(ctx, "k_simp_flag");
+      k_simp_flag<<<GD, 256, 0, st>>>(S);
+      LAUNCHED(ctx);
+      TRY(simp_scan(ctx, ze, ParentScan{S, g0, ng}, "scan_simp_parents"));
+      TRY(simp_scan(ctx, ze, SegScan{S, g0}, "scan_simp_segments"));
+      PROF(ctx, "k_simp_runs");
+      k_simp_runs<<<GD, 256, 0, st>>>(S, g0, false);
+      LAUNCHED(ctx);
+      TRY(simp_scan(ctx, ze, RunScan{S}, "scan_simp_runs"));
+      PROF(ctx, "k_simp_runs");
+      k_simp_runs<<<GD, 256, 0, st>>>(S, g0, true);
+      LAUNCHED(ctx);
+      PROF(ctx, "k_simp_level_end");
+      k_simp_level_end<<<1, 32, 0, st>>>(S);
+      LAUNCHED(ctx);
+    }
+    TRY(read_ints(ctx, S.sv, sv, SV_N));
+    if (!sv[SV_OVF]) break;
+    cap_p = std::max<int64_t>(2 * cap_p, sv[SV_NEED_P]);
+    cap_a = std::max<int64_t>(2 * cap_a, sv[SV_NEED_A]);
+    cap_r = std::max<int64_t>(2 * cap_r, sv[SV_NEED_R]);
+    CK(cudaStreamSynchronize(st));
+    free_bucket(A);
+  }
+  const int n_out = sv[SV_OUT], R = sv[SV_RTOP];
+
+  // ---- the result: nodes, individuals, mutations, edges in final order
+  std::vector<void*>& Rb = ctx->simp_allocs;
+  gnx_tables_t& O = ctx->simp;
+  O = gnx_tables_t{};
+  O.sequence_length = T->sequence_length;
+  O.n_location = T->n_location;
+  DM(ctx, &O.node_flags, (size_t)n_out, &Rb);
+  DM(ctx, &O.node_time, (size_t)n_out, &Rb);
+  DM(ctx, &O.node_population, (size_t)n_out, &Rb);
+  DM(ctx, &O.node_individual, (size_t)n_out, &Rb);
+  DM(ctx, &O.individual_flags, (size_t)T->n_individuals, &Rb);
+  DM(ctx, &O.individual_location, (size_t)(T->n_individuals * T->n_location), &Rb);
+  DM(ctx, &O.individual_idx, (size_t)T->n_individuals, &Rb);
+  DM(ctx, &O.mutation_site, (size_t)T->n_mutations, &Rb);
+  DM(ctx, &O.mutation_node, (size_t)T->n_mutations, &Rb);
+  DM(ctx, &O.mutation_time, (size_t)T->n_mutations, &Rb);
+  DM(ctx, &O.edge_left, (size_t)R, &Rb);
+  DM(ctx, &O.edge_right, (size_t)R, &Rb);
+  DM(ctx, &O.edge_parent, (size_t)R, &Rb);
+  DM(ctx, &O.edge_child, (size_t)R, &Rb);
+  int32_t* remap;
+  DM(ctx, &remap, (size_t)T->n_individuals, &B);
+  PROF(ctx, "k_simp_mark_ind");
+  k_simp_mark_ind<<<gr(n_out), 256, 0, st>>>(S, n_out, remap);
+  LAUNCHED(ctx);
+  TRY(simp_scan(ctx, z, IndScan{S.n_ind, (int)T->n_location, remap, d_iflags, d_iloc, d_iidx, O.individual_flags,
+                                O.individual_location, O.individual_idx, hsz}, "scan_simp_individuals"));
+  PROF(ctx, "k_simp_nodes_out");
+  k_simp_nodes_out<<<gr(n_out), 256, 0, st>>>(S, n_out, d_pop, remap, O.node_flags, O.node_time, O.node_population,
+                                              O.node_individual);
+  LAUNCHED(ctx);
+  TRY(simp_scan(ctx, z, MutScan{S, d_mtime, O.mutation_site, O.mutation_node, O.mutation_time, hsz + 1},
+                "scan_simp_mutations"));
+  SimpSort zr;
+  TRY(simp_sort_alloc(ctx, B, std::max(n_out, R), 0, &zr));
+  int32_t* orank;
+  DM(ctx, &orank, (size_t)n_out, &B);
+  PROF(ctx, "k_simp_time_keys");
+  k_simp_time_keys<<<gr(n_out), 256, 0, st>>>(S.time, S.out_src, n_out, zr.key[0], zr.val[0]);
+  LAUNCHED(ctx);
+  TRY(simp_sort(ctx, zr, n_out, nullptr, 64, &in));
+  PROF(ctx, "k_simp_rank");
+  k_simp_rank<<<gr(n_out), 256, 0, st>>>(zr.val[in], n_out, orank);
+  LAUNCHED(ctx);
+  const int nb_out = bits_for(std::max(n_out - 1, 0));
+  PROF(ctx, "k_simp_run_keys");
+  k_simp_run_keys<<<gr(R), 256, 0, st>>>(S, R, zr.key[0], zr.val[0]);
+  LAUNCHED(ctx);
+  TRY(simp_sort(ctx, zr, R, nullptr, nb_out + S.pb, &in));
+  if (in) CK(cudaMemcpyAsync(zr.val[0], zr.val[1], (size_t)R * 4, cudaMemcpyDeviceToDevice, st));
+  PROF(ctx, "k_simp_run_keys2");
+  k_simp_run_keys2<<<gr(R), 256, 0, st>>>(S, R, orank, zr.val[0], zr.key[0]);
+  LAUNCHED(ctx);
+  TRY(simp_sort(ctx, zr, R, nullptr, nb_out, &in));
+  TRY(simp_scan(ctx, zr, SquashScan{S, R, zr.val[in], O.edge_left, O.edge_right, O.edge_parent, O.edge_child,
+                                    hsz + 2}, "scan_simp_squash"));
+  int32_t outn[3];
+  TRY(read_ints(ctx, hsz, outn, 3));
+  O.n_nodes = n_out;
+  O.n_individuals = outn[0];
+  O.n_mutations = outn[1];
+  O.n_edges = outn[2];
+  O.n_sites = T->n_sites;
+  out_sizes[0] = O.n_nodes;
+  out_sizes[1] = O.n_edges;
+  out_sizes[2] = O.n_individuals;
+  out_sizes[3] = O.n_mutations;
+  return GNX_OK;
+}
+
+extern "C" int gnx_simplify(gnx_ctx* ctx, const gnx_tables_t* tables, const int32_t* samples, int64_t n_samples,
+                            int64_t* out_sizes) {
+  ARG(ctx && tables && out_sizes, "null");
+  USE_DEVICE(ctx);
+  CK(cudaStreamSynchronize(ctx->stream));
+  free_bucket(ctx->simp_allocs);
+  ctx->simp = gnx_tables_t{};
+  std::vector<void*> scratch, pools;            // pools: the level pass's, grown and replaced on overflow
+  int r = simplify_impl(ctx, tables, samples, n_samples, scratch, pools, out_sizes);
+  cudaStreamSynchronize(ctx->stream);
+  free_bucket(scratch);
+  free_bucket(pools);
+  if (r != GNX_OK) {
+    free_bucket(ctx->simp_allocs);
+    ctx->simp = gnx_tables_t{};
+  }
+  return r;
+}
+
+extern "C" int gnx_simplify_result(gnx_ctx* ctx, gnx_tables_t* out) {
+  ARG(ctx && out, "null");
+  const gnx_tables_t& O = ctx->simp;
+  if (ctx->simp_allocs.empty()) { g_last_error = "no gnx_simplify result to copy"; return GNX_ERR_STATE; }
+  ARG(out->n_nodes == O.n_nodes && out->n_edges == O.n_edges && out->n_individuals == O.n_individuals &&
+      out->n_mutations == O.n_mutations && out->n_location == O.n_location, "sizes differ from gnx_simplify's");
+  USE_DEVICE(ctx);
+  cudaStream_t st = ctx->stream;
+  auto get = [&](void* h, const void* d, size_t bytes) -> int {
+    if (bytes == 0) return GNX_OK;
+    ARG(h, "null column");
+    CK(cudaMemcpyAsync(h, d, bytes, cudaMemcpyDeviceToHost, st));
+    return GNX_OK;
+  };
+  const size_t nn = (size_t)O.n_nodes, ne = (size_t)O.n_edges, ni = (size_t)O.n_individuals, nm = (size_t)O.n_mutations;
+  TRY(get(out->node_flags, O.node_flags, nn * 4));
+  TRY(get(out->node_time, O.node_time, nn * 8));
+  TRY(get(out->node_population, O.node_population, nn * 4));
+  TRY(get(out->node_individual, O.node_individual, nn * 4));
+  TRY(get(out->edge_left, O.edge_left, ne * 8));
+  TRY(get(out->edge_right, O.edge_right, ne * 8));
+  TRY(get(out->edge_parent, O.edge_parent, ne * 4));
+  TRY(get(out->edge_child, O.edge_child, ne * 4));
+  TRY(get(out->individual_flags, O.individual_flags, ni * 4));
+  TRY(get(out->individual_location, O.individual_location, ni * (size_t)O.n_location * 8));
+  TRY(get(out->individual_idx, O.individual_idx, ni * 8));
+  TRY(get(out->mutation_site, O.mutation_site, nm * 4));
+  TRY(get(out->mutation_node, O.mutation_node, nm * 4));
+  TRY(get(out->mutation_time, O.mutation_time, nm * 8));
+  CK(cudaStreamSynchronize(st));
+  free_bucket(ctx->simp_allocs);
+  ctx->simp = gnx_tables_t{};
   return GNX_OK;
 }
 

@@ -2648,7 +2648,8 @@ __global__ void k_end_step(Counters* c, Work w, int burn, int record) {
 // Species order on demand.  The reference's Species is an OrderedDict in ascending id; the
 // host-facing views (download, field reads, injected draws, tskit renumbering) need each
 // entry's rank by id: an LSD radix sort of (id, entry) pairs, 8 bits per pass, only as many
-// passes as the largest id has bits.
+// passes as the largest id has bits.  A pass takes its size from n, or from device memory when
+// n_dev is given (the table simplification, gnx_simplify.cuh, sorts arrays the host never sizes).
 // ========================================================================================
 #define RS_BLOCK 256
 #define RS_ITEMS 8
@@ -2663,9 +2664,13 @@ __global__ void __launch_bounds__(256) k_order_keys(Pop pop, Work w, const Count
   }
 }
 
-__global__ void __launch_bounds__(RS_BLOCK) k_radix_hist(const unsigned long long* __restrict__ keys, int n, int shift,
-                                                          uint32_t* hist, int ntiles) {
+__device__ __forceinline__ int radix_tiles(int n) { return max(1, (n + RS_TILE - 1) / RS_TILE); }
+
+__global__ void __launch_bounds__(RS_BLOCK) k_radix_hist(const unsigned long long* __restrict__ keys, int n,
+                                                          const int* n_dev, int shift, uint32_t* hist) {
   __shared__ uint32_t h[256];
+  if (n_dev) n = *n_dev;
+  const int ntiles = radix_tiles(n);
   for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     h[threadIdx.x] = 0u;
     __syncthreads();
@@ -2682,8 +2687,9 @@ __global__ void __launch_bounds__(RS_BLOCK) k_radix_hist(const unsigned long lon
 
 struct RadixScan {
   uint32_t* hist;
-  int len;
-  __device__ int size(const Counters*) const { return len; }
+  int n;
+  const int* n_dev;
+  __device__ int size(const Counters*) const { return 256 * radix_tiles(n_dev ? *n_dev : n); }
   __device__ u64 value(int i) const { return hist[i]; }
   __device__ void apply(int i, u64, u64 ex) const { hist[i] = (uint32_t)ex; }
   __device__ void total(Counters*, u64) const {}
@@ -2691,9 +2697,11 @@ struct RadixScan {
 
 __global__ void __launch_bounds__(RS_BLOCK) k_radix_scatter(const unsigned long long* __restrict__ kin,
                                                              const int32_t* __restrict__ vin, unsigned long long* kout,
-                                                             int32_t* vout, int n, int shift, const uint32_t* hist,
-                                                             int ntiles) {
+                                                             int32_t* vout, int n, const int* n_dev, int shift,
+                                                             const uint32_t* hist) {
   __shared__ uint32_t base[256];
+  if (n_dev) n = *n_dev;
+  const int ntiles = radix_tiles(n);
   __shared__ uint32_t wcnt[RS_BLOCK / 32][256];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {

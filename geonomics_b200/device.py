@@ -714,6 +714,65 @@ class DeviceSpecies:
         _lib.check(self._L.gnx_read_paths(self._ctx, _ptr(out, _lib.c_uint32_p), out.size), 'gnx_read_paths')
         return out
 
+    def simplify_tables(self, tc, sample_nodes):
+        """TableCollection.sort() + simplify(sample_nodes, filter_individuals=True, filter_sites=False) of a
+        tables.TableColumns on this context's device (gnx_simplify), in place; row for row what
+        tables.simplify_columns gives.  The columns are copied up, simplified and copied back."""
+        cols = {}
+
+        def col(name, a, dtype, typ):
+            cols[name] = np.ascontiguousarray(a, dtype=dtype)
+            return _ptr(cols[name], typ)
+
+        f8, i4, i8 = (np.float64, _lib.c_double_p), (np.int32, _lib.c_int32_p), (np.int64, _lib.c_int64_p)
+        t = _lib.Tables()
+        t.sequence_length = float(tc.sequence_length)
+        t.n_nodes, t.n_edges = tc.nodes.num_rows, tc.edges.num_rows
+        t.n_individuals, t.n_location = tc.individuals.num_rows, tc.n_loc
+        t.n_sites, t.n_mutations = tc.sites.num_rows, tc.mutations.num_rows
+        t.node_time = col('nt', tc.nodes.time, *f8)
+        t.node_population = col('np', tc.nodes.population, *i4)
+        t.node_individual = col('ni', tc.nodes.individual, *i4)
+        t.edge_left, t.edge_right = col('el', tc.edges.left, *f8), col('er', tc.edges.right, *f8)
+        t.edge_parent, t.edge_child = col('ep', tc.edges.parent, *i4), col('ec', tc.edges.child, *i4)
+        t.individual_flags = col('if', tc.individuals.flags, *i4)
+        t.individual_location = col('il', tc.individuals.location, *f8)
+        t.individual_idx = col('ii', tc.individuals.idx, *i8)
+        t.site_position = col('sp', tc.sites.position, *f8)
+        t.mutation_site, t.mutation_node = col('ms', tc.mutations.site, *i4), col('mn', tc.mutations.node, *i4)
+        t.mutation_time = col('mt', tc.mutations.time, *f8)
+        samples = np.ascontiguousarray(sample_nodes, dtype=np.int32)
+        sizes = np.zeros(4, np.int64)
+        _lib.check(self._L.gnx_simplify(self._ctx, C.byref(t), _ptr(samples, _lib.c_int32_p), len(samples),
+                                        _ptr(sizes, _lib.c_int64_p)), 'gnx_simplify')
+        nn, ne, ni, nm = (int(v) for v in sizes)
+        nodes = dict(flags=np.zeros(nn, np.int32), time=np.zeros(nn), population=np.zeros(nn, np.int32),
+                     individual=np.zeros(nn, np.int32))
+        edges = dict(left=np.zeros(ne), right=np.zeros(ne), parent=np.zeros(ne, np.int32), child=np.zeros(ne, np.int32))
+        inds = dict(flags=np.zeros(ni, np.int32), location=np.zeros((ni, tc.n_loc)), idx=np.zeros(ni, np.int64))
+        muts = dict(site=np.zeros(nm, np.int32), node=np.zeros(nm, np.int32), time=np.zeros(nm))
+        o = _lib.Tables()
+        o.sequence_length, o.n_location = t.sequence_length, tc.n_loc
+        o.n_nodes, o.n_edges, o.n_individuals, o.n_sites, o.n_mutations = nn, ne, ni, t.n_sites, nm
+        o.node_flags, o.node_time = _ptr(nodes['flags'], _lib.c_int32_p), _ptr(nodes['time'], _lib.c_double_p)
+        o.node_population = _ptr(nodes['population'], _lib.c_int32_p)
+        o.node_individual = _ptr(nodes['individual'], _lib.c_int32_p)
+        o.edge_left, o.edge_right = _ptr(edges['left'], _lib.c_double_p), _ptr(edges['right'], _lib.c_double_p)
+        o.edge_parent, o.edge_child = _ptr(edges['parent'], _lib.c_int32_p), _ptr(edges['child'], _lib.c_int32_p)
+        o.individual_flags = _ptr(inds['flags'], _lib.c_int32_p)
+        o.individual_location = _ptr(inds['location'], _lib.c_double_p)
+        o.individual_idx = _ptr(inds['idx'], _lib.c_int64_p)
+        o.mutation_site, o.mutation_node = _ptr(muts['site'], _lib.c_int32_p), _ptr(muts['node'], _lib.c_int32_p)
+        o.mutation_time = _ptr(muts['time'], _lib.c_double_p)
+        _lib.check(self._L.gnx_simplify_result(self._ctx, C.byref(o)), 'gnx_simplify_result')
+        for tab in (tc.nodes, tc.edges, tc.individuals, tc.mutations):
+            tab.truncate(0)
+        tc.individuals.append_columns(**inds)
+        tc.nodes.append_columns(**nodes)
+        tc.edges.append_columns(**edges)
+        tc.mutations.append_columns(**muts)
+        return tc
+
     def subsetters(self):
         """uint8[n_paths, n_cols]: the homologue every path reads at each non-neutral locus in ascending locus
         order -- the `subsetters` argument of set_mutation that rebuilds the paths read_paths returns."""

@@ -5,7 +5,7 @@ the rows of every birth into device buffers (include/gnx_b200.h, "tskit record b
 module keeps them on the host as numpy COLUMNS -- the layout `TableCollection.*.append_columns` /
 `set_columns` take -- and turns them into a real `tskit.TableCollection` when tskit is importable
 (`to_tskit`).  tskit and msprime are absent from the build image: nothing here imports them at module
-level, and `sort_and_simplify` says so instead of falling back to anything.
+level; without tskit `sort_and_simplify` runs the restated algorithm on the species' device.
 """
 import numpy as np
 
@@ -134,11 +134,12 @@ class TableColumns:
                                  derived_state_offset=np.arange(nm + 1, dtype=np.uint64))
         return tc
 
-    def sort_and_simplify(self, sample_nodes):
+    def sort_and_simplify(self, sample_nodes, dev=None):
         """species.py:1107-1152: TableCollection.sort(); simplify(current nodes, filter_individuals=True,
         filter_sites=False).  With tskit installed its own C implementation runs on a real TableCollection
-        (`to_tskit`) and the result is read back.  Without it (this image) the published algorithm is run here
-        (`simplify_columns`): parity with tskit unpinned, invariants checked by the tests."""
+        (`to_tskit`) and the result is read back.  Without it, the published algorithm as `simplify_columns`
+        restates it (parity with tskit unpinned, invariants checked by the tests): on the device of `dev`, a
+        DeviceSpecies (gnx_simplify, row for row what `simplify_columns` gives), or here when there is none."""
         try:
             import tskit          # noqa: F401
             have = getattr(tskit, '__file__', None) is not None
@@ -150,6 +151,8 @@ class TableColumns:
             tc.simplify(np.asarray(sample_nodes, dtype=np.int32), filter_individuals=True, filter_sites=False)
             self._load(tc)
             return tc
+        if dev is not None:
+            return dev.simplify_tables(self, sample_nodes)
         simplify_columns(self, sample_nodes)
         return self
 

@@ -288,6 +288,43 @@ int gnx_set_clock(gnx_ctx* ctx, int64_t t, int64_t tsk_t0);
  * the path in front of its locus (genome.py:133-160), which the paths as simulated do not give back, so a
  * checkpoint carries them into gnx_set_mutation's host_subsetters.  Synchronises. */
 int gnx_read_paths(gnx_ctx* ctx, uint32_t* host_paths, int64_t n_words);
+/* ---- sort + simplify of the tskit tables (gnx_simplify.cuh) ---------------------------------------
+ * The columns of geonomics_b200.tables.TableColumns: nodes (time, population, individual; flags are
+ * written, not read), edges, individuals (n_location doubles per row), site positions and mutations.
+ * gnx_simplify reads them, does TableCollection.sort() + simplify(samples, filter_individuals=True,
+ * filter_sites=False) as tables.simplify_columns restates it, row for row, and returns the output sizes
+ * out_sizes[4] = nodes, edges, individuals, mutations (the sites are unchanged).  The result stays on the
+ * device until gnx_simplify_result copies it into host columns of exactly those sizes (the n_* fields of
+ * `out` say so) and frees it.  Both run on the ctx's stream and synchronise; scratch lives for the call.
+ * GNX_ERR_ARG for an edge whose parent is not older than its child, an edge outside 0 <= left < right <=
+ * sequence_length, a node id, sample, site or individual out of range, or a repeated sample. */
+typedef struct {
+  double sequence_length;
+  int64_t n_nodes;
+  int32_t* node_flags;
+  double* node_time;
+  int32_t* node_population;
+  int32_t* node_individual;
+  int64_t n_edges;
+  double* edge_left;
+  double* edge_right;
+  int32_t* edge_parent;
+  int32_t* edge_child;
+  int64_t n_individuals;
+  int32_t n_location;
+  int32_t* individual_flags;
+  double* individual_location;   /* [n_individuals][n_location] */
+  int64_t* individual_idx;
+  int64_t n_sites;
+  double* site_position;
+  int64_t n_mutations;
+  int32_t* mutation_site;
+  int32_t* mutation_node;
+  double* mutation_time;
+} gnx_tables_t;
+int gnx_simplify(gnx_ctx* ctx, const gnx_tables_t* tables, const int32_t* samples, int64_t n_samples,
+                 int64_t* out_sizes);
+int gnx_simplify_result(gnx_ctx* ctx, gnx_tables_t* out);
 /* ---- strip domain decomposition of one landscape over several GPUs (SURVEY.md section 8e-2) ---
  * What shards (reference file:line): the mate search species.py:2157-2215 / spatial.py:191-245
  * (halo of the individuals within one mating-grid row of a strip edge, with their genome rows),
